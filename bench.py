@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- enhanced audio-seconds per second through the fused STFT -> mask -> iSTFT + loss path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline workload (BASELINE.json configs[1]): VoiceBank-DEMAND-shaped synthetic batch, 16 kHz, 64 x 4 s
@@ -26,7 +26,12 @@ The same JSON line carries a `configs` object with the other BASELINE.json confi
 
 Timed regions: the ranks are aligned by a collective ON THE STREAM right before the first event, the metric sums of the
 pass accumulate on the device (se_finalize_metrics_acc) and are all-reduced once before the second event; nothing between
-the events reads back to the host.
+the events reads back to the host.  Every timed loop runs exactly --steps steps.
+
+--dump-outputs DIR (rank 0): after the timed pass, the arrays its last step returned (EnhancementEngine.eval_step's
+loss_per_utt, sisdr, gain, wav_predicted, mask) and the pass's device sums [sum loss, sum SI-SDR, utterances] are written
+as DIR/<name>.npy, float32 (pass_sums: float64), about 33 MB in all.  The inputs are seeded, so two builds run with the
+same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -222,6 +227,19 @@ class Ctx:
         return t.item()
 
 
+DUMP_KEYS = ("loss_per_utt", "sisdr", "gain", "wav_predicted", "mask")
+
+
+def dump_outputs(path, step_out, acc):
+    """--dump-outputs: one step's eval_step arrays as float32 and the pass's float64 sums, as <path>/<name>.npy."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: step_out[k].float() for k in DUMP_KEYS}
+    arrays["pass_sums"] = acc.double()
+    for name, t in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), t.detach().cpu().numpy())
+
+
 def make_engine(se, ctx, n_fft, precision=1):
     g = GEOMETRY[n_fft]
     pre = se.OnlinePreprocessor(sample_rate=SR, win_ms=g["win_ms"], hop_ms=g["hop_ms"], n_freq=g["n_freq"], n_mels=40, n_mfcc=13).to(ctx.dev)
@@ -337,7 +355,7 @@ def bench_longform(ctx, se, args):
     lengths = torch.full((B,), T, dtype=torch.int64, device=ctx.dev)
     acc = torch.zeros(3, device=ctx.dev, dtype=torch.float64)
     g = engine.capture_bound(lengths, wavs, metric_acc=acc)
-    steps = max(2, min(args.steps, 5))
+    steps = args.steps
     for _ in range(2):
         g["graph"].replay()
     acc.zero_()
@@ -381,7 +399,7 @@ def bench_training(ctx, se, args):
     lengths, wavs = lengths.to(ctx.dev), wavs.to(ctx.dev)
     fused = engine.fused_training_supported(crit, B, wavs.shape[2])
     st = engine.capture_train(lengths, wavs, crit, opt, 1.0)
-    steps = max(5, args.steps)
+    steps = args.steps
     for _ in range(3):
         st["graph"].replay()
 
@@ -444,7 +462,7 @@ def bench_scoring(ctx, se, args):
         return grads, sampler_ops.matching(grads[12:], grads[:12])
     for _ in range(3):
         grads, scores = one()
-    steps = max(5, min(args.steps, 20))
+    steps = args.steps
 
     def run():
         for _ in range(steps):
@@ -486,7 +504,7 @@ def bench_scoring(ctx, se, args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200, help="timed steps of every timed loop")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--ring", type=int, default=8, help="distinct batches the device-resident run rotates over")
@@ -497,7 +515,10 @@ def main():
     ap.add_argument("--head-precision", type=int, default=1, help="0 = fp32 SIMT head, 1 = TF32 tcgen05 head")
     ap.add_argument("--long-utts", type=int, default=1024, help="utterances (60 s each) of the long-form configuration, in total")
     ap.add_argument("--skip-configs", action="store_true", help="headline only (no `configs` object)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the arrays the last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -537,9 +558,10 @@ def main():
     # ---------------------------------------------------------------- device-resident timed run
     acc = torch.zeros(3, device=dev, dtype=torch.float64)     # [sum loss, sum SI-SDR, utterances] of the pass, kept on the device
     if args.eager:
-        steps = [lambda l=l, w=w: engine.eval_step(l, w, metric_acc=acc) for l, w in ring]
+        outputs = [{} for _ in ring]                   # what each ring slot's latest step returned
+        steps = [lambda l=l, w=w, o=o: o.update(engine.eval_step(l, w, metric_acc=acc)) for (l, w), o in zip(ring, outputs)]
     else:
-        graphs = [engine.capture_bound(l, w, metric_acc=acc) for l, w in ring]
+        graphs = outputs = [engine.capture_bound(l, w, metric_acc=acc) for l, w in ring]
         steps = [g["graph"].replay for g in graphs]
     # Consecutive steps work on independent batches: with --streams S > 1, step i is enqueued on stream i % S, so the
     # ramp-up and tail of one step's kernels overlap the neighbouring step's kernels (every ring slot owns its buffers).
@@ -571,6 +593,8 @@ def main():
     ms_total = ctx.timed(timed_pass)
     value = world * audio_s_per_step * args.steps / (ms_total * 1e-3)
     pass_loss, pass_sisdr, pass_n = float(acc[0] / acc[2]), float(acc[1] / acc[2]), float(acc[2])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs[(args.steps - 1) % len(outputs)], acc)
 
     # ---------------------------------------------------------------- per-kernel timing, roofline of the dominant kernel
     kernel_ms, alg_bytes = time_eval_kernels(ctx, se, engine, pre, head, ring, N_FFT, HOP, reps=10)
