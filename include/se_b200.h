@@ -166,15 +166,36 @@ int se_l1_logspec_bwd(const float* log_predicted, const float* linear_tar, const
  * S = linear_tar, X = linear_inp, G = offset; voiced[u,f] = 10 log10(sum_k S + eps) > 10 log10(max_{u,f} sum_k S + eps)
  * - db_interval (the maximum runs over the whole padded batch, as in the reference).  Workspaces (caller-owned):
  * ws_energy (n_utt * n_frames) floats, ws_max 1 float, ws_sums2 (n_utt, 2) doubles; loss: 1 float.
- * bwd: grad_offset = grad_loss[0] * d loss / d offset (0 on padded frames), from the forward's workspaces.
- * Under data parallelism the batch maximum needs an all-reduce(max) of ws_max between the two forward kernels; the
- * single-process form here is what the reference computes. */
+ * bwd: grad_offset = grad_loss[0] * d loss / d offset (0 on padded frames), from the forward's workspaces (ws_max holds the
+ * batch maximum as a plain float).
+ * This form takes the maximum over the batch it is given.  Under data parallelism the maximum must be the GLOBAL batch's: use
+ * the split form below (se_wsd_energy -> all-reduce(max) of its 1-float buffer -> se_wsd_mask_step), which se_wsd_bwd can
+ * also differentiate (its ws_energy / ws_max are se_wsd_energy's outputs). */
 int se_wsd_fwd(const float* linear_inp, const float* offset, const float* linear_tar, const int64_t* stft_len, int64_t n_utt,
                int64_t n_frames, int64_t K, float alpha, float db_interval, float eps, float* ws_energy, float* ws_max,
                double* ws_sums2, float* loss, void* stream);
 int se_wsd_bwd(const float* linear_inp, const float* offset, const float* linear_tar, const int64_t* stft_len, int64_t n_utt,
                int64_t n_frames, int64_t K, float alpha, float db_interval, float eps, const float* ws_energy,
                const float* ws_max, const float* grad_loss, float* grad_offset, void* stream);
+
+/* ---- the same objective split at the batch maximum (data-parallel form), on row-padded tensors --------------------------------
+ * se_wsd_energy: energy[u * n_frames + f] = sum_{k<K} linear_tar[u, f, k] over EVERY frame of the padded batch (rows ld_tar floats
+ *   apart, columns >= K never read; summation order of se_wsd_fwd) and max_energy[0] = their maximum, written as a plain float32 --
+ *   so that torch.distributed.all_reduce(op=MAX) of that 1-element buffer gives the maximum of the global batch.  Sums of
+ *   any sign are ordered as floats; NaN energies take no part (if every energy is NaN, max_energy is NaN).
+ * se_wsd_mask_step: the objective's part of one training step (the counterpart of se_sisdr_mask_step), reading the maximum from
+ *   max_energy AFTER any all-reduce: sums2 (n_utt, 2) doubles = {sum ((S - G S) voiced)^2, sum (G max(X - S, 0))^2} over the
+ *   valid frames, loss_per_utt[u] = alpha sums2[u, 0] + (1 - alpha) sums2[u, 1] (may be NULL), loss_mean (1 float) = their batch
+ *   mean, and grad_offset = d loss_mean / d offset (ld_g floats between rows; 0 on padded frames and pad columns), skipped when
+ *   NULL (se_linear_head_bwd_wsd rebuilds it inside the weight-gradient kernel).  Rows of offset / linear_inp / linear_tar are
+ *   ld_* floats apart (float4 loads when every ld is a multiple of 4 and the pointers are 16-byte aligned).  lengths / len_hop as
+ *   in se_sisdr_mask_step; sums_zeroed != 0: sums2 is already zero. */
+int se_wsd_energy(const float* linear_tar, int64_t ld_tar, int64_t n_utt, int64_t n_frames, int64_t K, float* energy, float* max_energy,
+                  void* stream);
+int se_wsd_mask_step(const float* offset, int64_t ld_off, const float* linear_inp, int64_t ld_inp, const float* linear_tar, int64_t ld_tar,
+                     const int64_t* lengths, int64_t len_hop, int64_t n_utt, int64_t n_frames, int64_t K, float alpha, float db_interval,
+                     float eps, const float* energy, const float* max_energy, double* sums2, int sums_zeroed, float* loss_per_utt,
+                     float* loss_mean, float* grad_offset, int64_t ld_g, void* stream);
 
 /* ---- K4c: batched waveform SI-SDR (evaluation.py:5-10 over runner.py:587-602) -----
  * sisdr[u] = sisdr_eval(src[u, :len[u]], tar[u, :len[u]]).  ws_sums3: caller workspace of
@@ -240,6 +261,20 @@ int se_linear_head_bwd_sisdr(const float* x, int64_t ldx, const double* stat_sum
                              const int64_t* lengths, int64_t len_hop, const double* sums3, float loss_eps, int64_t n_utt, int64_t n_frames,
                              int64_t D_in, int64_t D_out, int act, float* ws_partials, int64_t ws_floats, float* grad_W, float* grad_b,
                              void* stream);
+
+/* se_linear_head_bwd_wsd: se_linear_head_bwd_fused with the backward of objective.WSD folded in: d loss / d offset =
+ * (1 / n_utt) (alpha 2 (S - G S)(-S) voiced + (1 - alpha) 2 G max(X - S, 0)^2) is rebuilt per element from offset (G), linear_inp (X)
+ * and linear_tar (S), with one voiced flag per frame from energy and the threshold from max_energy (se_wsd_energy, after any
+ * all-reduce), so grad_offset is never written or read.  Padded frames carry no gradient.  lengths / len_hop as in se_wsd_mask_step.
+ * Same operands and alignment rules as se_linear_head_bwd_sisdr (_supported; otherwise SE_ERR_UNSUPPORTED: use se_wsd_mask_step's
+ * grad_offset + se_linear_head_bwd_fused). */
+int se_linear_head_bwd_wsd_supported(int64_t n_utt, int64_t n_frames, int64_t D_in, int64_t D_out, int64_t ldx, int64_t ld_off,
+                                     int64_t ld_inp, int64_t ld_tar);
+int se_linear_head_bwd_wsd(const float* x, int64_t ldx, const double* stat_sums, int64_t ld_stats, float cmvn_eps, const float* offset,
+                           int64_t ld_off, const float* linear_inp, int64_t ld_inp, const float* linear_tar, int64_t ld_tar,
+                           const int64_t* lengths, int64_t len_hop, const float* energy, const float* max_energy, float alpha,
+                           float db_interval, float loss_eps, int64_t n_utt, int64_t n_frames, int64_t D_in, int64_t D_out, int act,
+                           float* ws_partials, int64_t ws_floats, float* grad_W, float* grad_b, void* stream);
 
 /* ---- spectral SI-SDR objective on predicted = offset * linear_inp (objective.py:86-100 after model.py:33) ----------------
  * Same sums / loss as se_sisdr_spec_fwd without materialising `predicted`; rows of the three tensors are ld_* floats apart

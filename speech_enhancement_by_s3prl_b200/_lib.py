@@ -65,6 +65,12 @@ _SIGNATURES = {
     "se_mix_batch": [c_f, i64, c_f, c_f, i64, c_f, c_f, i64, i64, c_float, c_float, c_f, c_f, c_f],
     "se_wsd_fwd": [c_f, c_f, c_f, c_f, i64, i64, i64, c_float, c_float, c_float, c_f, c_f, c_f, c_f, c_f],
     "se_wsd_bwd": [c_f, c_f, c_f, c_f, i64, i64, i64, c_float, c_float, c_float, c_f, c_f, c_f, c_f, c_f],
+    "se_wsd_energy": [c_f, i64, i64, i64, i64, c_f, c_f, c_f],
+    "se_wsd_mask_step": [c_f, i64, c_f, i64, c_f, i64, c_f, i64, i64, i64, i64, c_float, c_float, c_float, c_f, c_f, c_f, c_int, c_f, c_f,
+                         c_f, i64, c_f],
+    "se_linear_head_bwd_wsd_supported": [i64, i64, i64, i64, i64, i64, i64, i64],
+    "se_linear_head_bwd_wsd": [c_f, i64, c_f, i64, c_float, c_f, i64, c_f, i64, c_f, i64, c_f, i64, c_f, c_f, c_float, c_float, c_float, i64,
+                               i64, i64, i64, c_int, c_f, i64, c_f, c_f, c_f],
     "se_sisdr_wave": [c_f, i64, c_f, i64, c_f, i64, i64, c_float, c_f, c_f, c_f],
     "se_masked_normalize_db": [c_f, i64, c_f, i64, i64, c_f, c_f, i64, c_float, c_f, c_f, i64, c_f],
     "se_length_masks": [c_f, i64, i64, c_f, c_f],

@@ -9,7 +9,8 @@
 //
 // TWO kernels share the plan, the epilogue and the reduction:
 //   linear_head_bwd_tma_kernel<LOSS>  (further down; 16-byte aligned, row-padded operands -- the engine's tensors): TMA lands the
-//       operands as they lie in HBM, MN-major tcgen05 operands, in-place rewrite; LOSS also folds the SISDR objective's backward in
+//       operands as they lie in HBM, MN-major tcgen05 operands, in-place rewrite; LOSS = kLossSisdr / kLossWsd also folds the
+//       backward of that objective in
 //   linear_head_bwd_tc_kernel         (below; any strides -- the autograd custom op on un-padded tensors): transposing producers
 //
 // linear_head_bwd_tc_kernel:
@@ -123,9 +124,12 @@ struct BwdArgs {
     int n_main, n_tail;
     float* partials;               // (splits, m_rows, 272)
     int m_rows;                    // m_tiles * 128 + simt_rows
-    // LOSS kernel: grad_offset is not read; d loss / d offset of objective.SISDR on predicted = offset * linear_inp is rebuilt per element
+    // LOSS kernels: grad_offset is not read; d loss / d offset of objective.SISDR on predicted = offset * linear_inp (or of objective.WSD)
+    // is rebuilt per element
     const float* inp; const float* tar; long long ld_inp, ld_tar;
     const double* sums3; const long long* lengths; int len_hop; float loss_eps; float grad_uniform; const float* grad_out;
+    // kLossWsd: objective.WSD instead -- frame energies (n_utt * n_frames) and the batch maximum (1 float) of se_wsd_energy
+    float alpha, db_interval; const float* energy; const float* max_energy;
     int m_tiles, simt_rows;        // tensor-core tiles; leftover rows [128 m_tiles, 128 m_tiles + simt_rows) done by SIMT CTAs
 };
 
@@ -443,9 +447,9 @@ constexpr int kTOffShift = kTOffScale + kMaxUtt * kTStatLd * 4;
 constexpr int kTOffBar = kTOffShift + kMaxUtt * kTStatLd * 4;
 constexpr int kTNumBars = 3 * kTStages + 1;                     // full, norm, empty per stage + accum
 constexpr int kTOffTmem = kTOffBar + kTNumBars * 8;
-constexpr int kTOffCoef = kTOffTmem + 16;                       // LOSS: [kMaxUtt] (c_t, c_s) + [kMaxUtt] valid frames
-constexpr int kTSmemBytes = kTOffCoef + kMaxUtt * 12;
-// LOSS variant (the SISDR objective's backward folded in): stages of inp | offset | tar | x = 12 + 9 boxes, two of them
+constexpr int kTOffCoef = kTOffTmem + 16;                       // LOSS: [kMaxUtt] (c_t, c_s) + [kMaxUtt] valid frames + WSD threshold
+constexpr int kTSmemBytes = kTOffCoef + kMaxUtt * 12 + 16;
+// LOSS variants (an objective's backward folded in): stages of inp | offset | tar | x = 12 + 9 boxes, two of them
 constexpr int kLStages = 2, kLOffT = 8 * kTBox, kLOffX = 12 * kTBox, kLStageBytes = (12 + kTMaxXBoxes) * kTBox;
 static_assert(kLStages * kLStageBytes <= kTStages * kTStageBytes && BM * kStageLd * 4 <= kLStages * kLStageBytes, "LOSS ring inside the plain ring");
 constexpr int kTWorkWarps = 16, kTWorkThreads = kTWorkWarps * 32, kTThreads = kTWorkThreads + 64;   // + MMA warp + TMA warp
@@ -498,14 +502,27 @@ __device__ __forceinline__ float sisdr_grad(float o, float x, float t, float2 c)
     const float g = (c.x * ti + c.y * (pi * rs)) * (0.5f * rs) * x;
     return pi > 0.0f ? g : 0.0f;
 }
+// grad_offset of one element of objective.WSD: G = offset, X = linear_inp, S = linear_tar, scale = 1 / B -- the expression of
+// wsd_mask_bwd_kernel (ops_kernels.cu) term for term, so that both routes round the same fp32 values to TF32
+__device__ __forceinline__ float wsd_grad(float G, float X, float S, bool voiced, float alpha, float scale) {
+    const float n = fmaxf(X - S, 0.0f);
+    return scale * ((voiced ? alpha * 2.0f * (S - G * S) * (-S) : 0.0f) + (1.0f - alpha) * 2.0f * G * n * n);
+}
+constexpr int kLossNone = 0, kLossSisdr = 1, kLossWsd = 2;
+// c: SISDR's per-utterance coefficients, or (1 if the row's frame is voiced else 0, unused) for WSD
+template <int LOSS>
+__device__ __forceinline__ float loss_grad(float o, float x, float t, float2 c, const BwdArgs& a) {
+    return LOSS == kLossWsd ? wsd_grad(o, x, t, c.x != 0.0f, a.alpha, a.grad_uniform) : sisdr_grad(o, x, t, c);
+}
 
-template <bool LOSS>
+template <int LOSS>
 __global__ void __launch_bounds__(kTThreads, 1) linear_head_bwd_tma_kernel(const __grid_constant__ CUtensorMap tmG,
                                                                             const __grid_constant__ CUtensorMap tmO,
                                                                             const __grid_constant__ CUtensorMap tmX,
                                                                             const __grid_constant__ CUtensorMap tmT, const BwdArgs a) {
     constexpr int STAGES = LOSS ? kLStages : kTStages, STAGE_BYTES = LOSS ? kLStageBytes : kTStageBytes;
     constexpr int OFF_X = LOSS ? kLOffX : kTOffX;
+    static_assert(LOSS == kLossNone || LOSS == kLossSisdr || LOSS == kLossWsd, "loss kind");
     extern __shared__ __align__(1024) unsigned char smem[];
     const uint32_t sbase = smem_u32(smem);
     float* s_scale = reinterpret_cast<float*>(smem + kTOffScale);
@@ -515,6 +532,7 @@ __global__ void __launch_bounds__(kTThreads, 1) linear_head_bwd_tma_kernel(const
                    bar_accum = bar_empty + 8 * kTStages;
     float2* s_coef = reinterpret_cast<float2*>(smem + kTOffCoef);
     int* s_valid = reinterpret_cast<int*>(smem + kTOffCoef + kMaxUtt * 8);
+    float* s_thres = reinterpret_cast<float*>(smem + kTOffCoef + kMaxUtt * 12);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int split = blockIdx.x, n0 = blockIdx.y * BM;
     long long ra = (long long)split * a.rows_per_split;
@@ -569,13 +587,16 @@ __global__ void __launch_bounds__(kTThreads, 1) linear_head_bwd_tma_kernel(const
         float2 c = make_float2(0.f, 0.f);
         int valid = 0;
         if (u * a.n_frames < a.R) {
-            c = sisdr_coef(a.sums3 + 3 * u, (double)a.loss_eps, a.grad_out ? (double)a.grad_out[u] : (double)a.grad_uniform);
+            if (LOSS == kLossSisdr)
+                c = sisdr_coef(a.sums3 + 3 * u, (double)a.loss_eps, a.grad_out ? (double)a.grad_out[u] : (double)a.grad_uniform);
             long long v = a.n_frames;
             if (a.lengths) v = a.len_hop > 0 ? a.lengths[u] / a.len_hop + 1 : a.lengths[u];
             valid = (int)(v < a.n_frames ? v : a.n_frames);
         }
         s_coef[threadIdx.x] = c;
         s_valid[threadIdx.x] = valid;
+        if (LOSS == kLossWsd && threadIdx.x == 0)                      // voicing threshold of the (all-reduced) batch maximum, once per CTA
+            *s_thres = 10.0f * log10f(__ldg(a.max_energy) + a.loss_eps) - a.db_interval;
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
@@ -627,6 +648,7 @@ __global__ void __launch_bounds__(kTThreads, 1) linear_head_bwd_tma_kernel(const
         const int row = tl >> 3, pc = tl & 7, lc = pc ^ ((row & 3) << 1);  // this thread's row of every box, physical / logical 16-byte chunk
         const bool do_left = a.simt_rows > 0 && blockIdx.y == 0;           // leftover output row n_left (at most one here)
         const int n_left = a.m_tiles * BM;
+        const float thres = LOSS == kLossWsd ? *s_thres : 0.0f;
         constexpr int kXPer = (kTMaxXBoxes + 1) / 2;                       // x boxes per thread: j = th, th + 2, ...
         float4 acc_l[kXPer];
 #pragma unroll
@@ -643,12 +665,17 @@ __global__ void __launch_bounds__(kTThreads, 1) linear_head_bwd_tma_kernel(const
             if (LOSS) {                                                    // padded frames of the utterance carry no loss
                 const int fr = (int)(r0 + row - (u_first + ui) * a.n_frames);
                 if (fr >= s_valid[ui]) live = 0.0f;
-                coef = s_coef[ui];
+                if (LOSS == kLossSisdr) {
+                    coef = s_coef[ui];
+                } else {                                                   // WSD: one voiced flag per row (frame)
+                    const bool voiced = r0 + row < a.R && 10.0f * log10f(__ldg(a.energy + r0 + row) + a.loss_eps) > thres;
+                    coef = make_float2(voiced ? 1.0f : 0.0f, 0.0f);
+                }
             }
             float dzl = 0.0f;
             if (do_left && live != 0.0f) {                                 // in flight while the stage lands
                 const float ol = __ldg(a.offset + (r0 + row) * a.ld_off + n_left);
-                const float gl = LOSS ? sisdr_grad(ol, __ldg(a.inp + (r0 + row) * a.ld_inp + n_left), __ldg(a.tar + (r0 + row) * a.ld_tar + n_left), coef)
+                const float gl = LOSS ? loss_grad<LOSS>(ol, __ldg(a.inp + (r0 + row) * a.ld_inp + n_left), __ldg(a.tar + (r0 + row) * a.ld_tar + n_left), coef, a)
                                       : __ldg(a.grad_offset + (r0 + row) * a.ld_off + n_left);
                 dzl = dact(gl, ol, a.act);
             }
@@ -664,8 +691,8 @@ __global__ void __launch_bounds__(kTThreads, 1) linear_head_bwd_tma_kernel(const
                 const float4 o = O[ci];
                 if (LOSS) {                                                // G holds linear_inp: rebuild d loss / d offset first
                     const float4 tt = Tt[ci];
-                    g = make_float4(sisdr_grad(o.x, g.x, tt.x, coef), sisdr_grad(o.y, g.y, tt.y, coef), sisdr_grad(o.z, g.z, tt.z, coef),
-                                    sisdr_grad(o.w, g.w, tt.w, coef));
+                    g = make_float4(loss_grad<LOSS>(o.x, g.x, tt.x, coef, a), loss_grad<LOSS>(o.y, g.y, tt.y, coef, a),
+                                    loss_grad<LOSS>(o.z, g.z, tt.z, coef, a), loss_grad<LOSS>(o.w, g.w, tt.w, coef, a));
                 }
                 G[ci] = make_float4(to_tf32(live * dact(g.x, o.x, a.act)), to_tf32(live * dact(g.y, o.y, a.act)),
                                     to_tf32(live * dact(g.z, o.z, a.act)), to_tf32(live * dact(g.w, o.w, a.act)));
@@ -859,9 +886,11 @@ int64_t se_linear_head_bwd_tc_workspace(int64_t n_utt, int64_t n_frames, int64_t
     return (int64_t)g.splits * g.m_rows * kMaxBRows;
 }
 
-struct LossArgs {          // the SISDR objective's backward folded into the weight gradient (TMA kernel only)
+struct LossArgs {          // an objective's backward folded into the weight gradient (TMA kernel only)
     const float* inp; int64_t ld_inp; const float* tar; int64_t ld_tar; const double* sums3; const int64_t* lengths; int64_t len_hop;
     float eps, grad_uniform; const float* grad_out;
+    int kind = kLossSisdr;                                     // kLossWsd: energy / max_energy / alpha / db_interval instead of sums3
+    float alpha = 0.0f, db_interval = 0.0f; const float* energy = nullptr; const float* max_energy = nullptr;
 };
 static int head_bwd_impl(const float* x, int64_t ldx, const float* mean, const float* std, const double* stat_sums, int64_t ld_stats,
                          float cmvn_eps, const float* offset, const float* grad_offset, int64_t ld_off, int64_t n_utt,
@@ -918,6 +947,25 @@ int se_linear_head_bwd_sisdr(const float* x, int64_t ldx, const double* stat_sum
     SE_REQUIRE(ld_inp >= D_out && ld_tar >= D_out && len_hop >= 0 && len_hop < (1LL << 30), "bad stride / hop");
     SE_REQUIRE(!stat_sums || n_frames >= 2, "CMVN statistics need at least two frames");
     LossArgs l{linear_inp, ld_inp, linear_tar, ld_tar, sums3, lengths, len_hop, loss_eps, 1.0f / (float)n_utt, nullptr};
+    return head_bwd_impl(x, ldx, nullptr, nullptr, stat_sums, ld_stats, cmvn_eps, offset, nullptr, ld_off, n_utt, n_frames, D_in, D_out, act,
+                         ws_partials, ws_floats, grad_W, grad_b, stream, nullptr, &l);
+}
+
+int se_linear_head_bwd_wsd_supported(int64_t n_utt, int64_t n_frames, int64_t D_in, int64_t D_out, int64_t ldx, int64_t ld_off,
+                                     int64_t ld_inp, int64_t ld_tar) {
+    return se_linear_head_bwd_sisdr_supported(n_utt, n_frames, D_in, D_out, ldx, ld_off, ld_inp, ld_tar);   // same kernel, same operands
+}
+
+int se_linear_head_bwd_wsd(const float* x, int64_t ldx, const double* stat_sums, int64_t ld_stats, float cmvn_eps, const float* offset,
+                           int64_t ld_off, const float* linear_inp, int64_t ld_inp, const float* linear_tar, int64_t ld_tar,
+                           const int64_t* lengths, int64_t len_hop, const float* energy, const float* max_energy, float alpha,
+                           float db_interval, float loss_eps, int64_t n_utt, int64_t n_frames, int64_t D_in, int64_t D_out, int act,
+                           float* ws_partials, int64_t ws_floats, float* grad_W, float* grad_b, void* stream) {
+    SE_REQUIRE(linear_inp && linear_tar && energy && max_energy && grad_W, "null pointer");
+    SE_REQUIRE(ld_inp >= D_out && ld_tar >= D_out && len_hop >= 0 && len_hop < (1LL << 30), "bad stride / hop");
+    SE_REQUIRE(!stat_sums || n_frames >= 2, "CMVN statistics need at least two frames");
+    LossArgs l{linear_inp, ld_inp, linear_tar, ld_tar, nullptr, lengths, len_hop, loss_eps, 1.0f / (float)n_utt, nullptr,
+               kLossWsd, alpha, db_interval, energy, max_energy};
     return head_bwd_impl(x, ldx, nullptr, nullptr, stat_sums, ld_stats, cmvn_eps, offset, nullptr, ld_off, n_utt, n_frames, D_in, D_out, act,
                          ws_partials, ws_floats, grad_W, grad_b, stream, nullptr, &l);
 }
@@ -987,17 +1035,22 @@ static int head_bwd_impl(const float* x, int64_t ldx, const float* mean, const f
         a.inp = loss->inp; a.ld_inp = loss->ld_inp; a.tar = loss->tar; a.ld_tar = loss->ld_tar; a.sums3 = loss->sums3;
         a.lengths = (const long long*)loss->lengths; a.len_hop = (int)loss->len_hop; a.loss_eps = loss->eps;
         a.grad_uniform = loss->grad_uniform; a.grad_out = loss->grad_out;
+        a.alpha = loss->alpha; a.db_interval = loss->db_interval; a.energy = loss->energy; a.max_energy = loss->max_energy;
     }
     static unsigned long long opted_t = 0;
     if (tma_ok && secommon::first_use_on_device(opted_t)) {
-        SE_CUDA_CHECK(cudaFuncSetAttribute(linear_head_bwd_tma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTSmemBytes));
-        SE_CUDA_CHECK(cudaFuncSetAttribute(linear_head_bwd_tma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTSmemBytes));
+        SE_CUDA_CHECK(cudaFuncSetAttribute(linear_head_bwd_tma_kernel<kLossNone>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTSmemBytes));
+        SE_CUDA_CHECK(cudaFuncSetAttribute(linear_head_bwd_tma_kernel<kLossSisdr>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTSmemBytes));
+        SE_CUDA_CHECK(cudaFuncSetAttribute(linear_head_bwd_tma_kernel<kLossWsd>, cudaFuncAttributeMaxDynamicSharedMemorySize, kTSmemBytes));
     }
-    if (loss) {
-        linear_head_bwd_tma_kernel<true><<<dim3((unsigned)g.splits, (unsigned)g.m_tiles), kTThreads, kTSmemBytes, st>>>(tmG, tmO, tmX, tmT, a);
+    if (loss && loss->kind == kLossWsd) {
+        linear_head_bwd_tma_kernel<kLossWsd><<<dim3((unsigned)g.splits, (unsigned)g.m_tiles), kTThreads, kTSmemBytes, st>>>(tmG, tmO, tmX, tmT, a);
+        rc = secommon::check_launch("linear_head_bwd_tma_kernel<wsd>");
+    } else if (loss) {
+        linear_head_bwd_tma_kernel<kLossSisdr><<<dim3((unsigned)g.splits, (unsigned)g.m_tiles), kTThreads, kTSmemBytes, st>>>(tmG, tmO, tmX, tmT, a);
         rc = secommon::check_launch("linear_head_bwd_tma_kernel<loss>");
     } else if (tma_ok) {
-        linear_head_bwd_tma_kernel<false><<<dim3((unsigned)g.splits, (unsigned)g.m_tiles), kTThreads, kTSmemBytes, st>>>(tmG, tmO, tmX, tmX, a);
+        linear_head_bwd_tma_kernel<kLossNone><<<dim3((unsigned)g.splits, (unsigned)g.m_tiles), kTThreads, kTSmemBytes, st>>>(tmG, tmO, tmX, tmX, a);
         rc = secommon::check_launch("linear_head_bwd_tma_kernel");
     } else {
         linear_head_bwd_tc_kernel<<<dim3((unsigned)g.splits, (unsigned)g.m_tiles), kThreads, kSmemBytes, st>>>(a);

@@ -437,15 +437,17 @@ __global__ void l1_logspec_bwd_kernel(const float* __restrict__ logp, const floa
 
 // ------------------------------------------------------------------ weighted speech distortion objective (objective.py:120-153)
 // energy[u,f] = sum_k S[u,f,k] for EVERY frame (the reference takes energy.max() over the whole padded batch), and the
-// batch maximum.  One warp per frame; energies are >= 0 in practice (power spectra), so the maximum is an atomicMax on
-// the float's bit pattern, with negative sums clamped out of the comparison the way max() of mixed signs would need.
-__global__ void wsd_energy_kernel(const float* __restrict__ tar, long long n_rows, int K, float* __restrict__ energy,
+// batch maximum.  One warp per frame (rows ld floats apart).  The maximum stays a plain float in memory, so that an
+// all-reduce(max) of the buffer across data-parallel ranks gives the global one: the caller fills it with 0xff bytes (a
+// NaN that every value replaces), non-negative sums go through a signed atomicMax of the bit pattern (their order as
+// ints), negative ones through an unsigned atomicMin (reversed order), and a non-negative value beats a negative one in both.
+__global__ void wsd_energy_kernel(const float* __restrict__ tar, long long ld, long long n_rows, int K, float* __restrict__ energy,
                                   float* __restrict__ max_energy) {
     const int lane = threadIdx.x & 31;
     const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
     float best = -INFINITY;
     for (long long r = warp; r < n_rows; r += nwarps) {
-        const float* t = tar + r * K;
+        const float* t = tar + r * ld;
         float s = 0.0f;
         for (int k = lane; k < K; k += 32) s += t[k];
         s = secommon::warp_sum(s);
@@ -453,14 +455,16 @@ __global__ void wsd_energy_kernel(const float* __restrict__ tar, long long n_row
         best = fmaxf(best, s);
     }
     if (lane == 0 && best > -INFINITY) {
-        // order-preserving integer image of a float: flip all bits of negatives, the sign bit of non-negatives
-        const unsigned bits = __float_as_uint(best);
-        atomicMax(reinterpret_cast<unsigned*>(max_energy), (bits & 0x80000000u) ? ~bits : (bits | 0x80000000u));
+        if (best >= 0.0f) atomicMax(reinterpret_cast<int*>(max_energy), __float_as_int(best));
+        else atomicMin(reinterpret_cast<unsigned*>(max_energy), __float_as_uint(best));
     }
 }
-__device__ __forceinline__ float wsd_decode_max(const float* max_energy) {
-    const unsigned key = *reinterpret_cast<const unsigned*>(max_energy);
-    return __uint_as_float((key & 0x80000000u) ? (key & 0x7fffffffu) : ~key);
+__device__ __forceinline__ float wsd_decode_max(const float* max_energy) { return *max_energy; }
+int launch_wsd_energy(const float* tar, long long ld, long long rows, int K, float* energy, float* max_energy, cudaStream_t st) {
+    SE_CUDA_CHECK(cudaMemsetAsync(max_energy, 0xff, sizeof(float), st));
+    const long long want = (rows + 7) / 8;
+    wsd_energy_kernel<<<(unsigned)(want < 148 * 8 ? want : 148 * 8), 256, 0, st>>>(tar, ld, rows, K, energy, max_energy);
+    return secommon::check_launch("wsd_energy_kernel");
 }
 // per-utterance sums over valid frames: sums2[u] = { sum ((S - G S) voiced)^2, sum (G N)^2 }, N = max(X - S, 0)
 __global__ void wsd_sums_kernel(const float* __restrict__ inp, const float* __restrict__ off, const float* __restrict__ tar,
@@ -513,6 +517,105 @@ __global__ void wsd_bwd_kernel(const float* __restrict__ inp, const float* __res
             g = scale * ((voiced ? alpha * 2.0f * (S - G * S) * (-S) : 0.0f) + (1.0f - alpha) * 2.0f * G * n * n);
         }
         grad_off[i] = g;
+    }
+}
+
+// ---- the same objective on row-strided tensors (the training step's padded spectra), lengths as in the SISDR mask kernels and
+// the batch maximum read from a device buffer that may have been all-reduced across ranks in between (se_wsd_energy)
+struct WsdMaskArgs : SisdrMaskArgs {           // sums3 holds the (n_utt, 2) sums here
+    float alpha, db_interval;
+    const float* energy; const float* max_energy;
+};
+__device__ __forceinline__ float wsd_thres(const WsdMaskArgs& a) { return 10.0f * log10f(wsd_decode_max(a.max_energy) + a.eps) - a.db_interval; }
+
+template <int V>
+__global__ void __launch_bounds__(256) wsd_mask_sums_kernel(const WsdMaskArgs a) {
+    const int u = blockIdx.x / a.chunks, chunk = blockIdx.x - u * a.chunks;
+    const int valid = mask_valid_frames(a, u);
+    const int KV = (a.K + V - 1) / V;
+    const int per = (valid + a.chunks - 1) / a.chunks;
+    const int f_lo = chunk * per, f_hi = min(valid, f_lo + per);
+    const long long row0 = (long long)u * a.n_frames;
+    const float thres = wsd_thres(a);
+    float acc[2] = {0.f, 0.f};
+    const int items = max(f_hi - f_lo, 0) * KV;
+#pragma unroll 4
+    for (int i = threadIdx.x; i < items; i += blockDim.x) {
+        const int fr = i / KV, c = (i - fr * KV) * V;
+        const long long r = row0 + f_lo + fr;
+        float x[V], t[V], o[V];
+        ldv<V>(a.inp + r * a.ld_inp + c, x);
+        ldv<V>(a.tar + r * a.ld_tar + c, t);
+        ldv<V>(a.offset + r * a.ld_off + c, o);
+        const bool voiced = 10.0f * log10f(a.energy[r] + a.eps) > thres;
+#pragma unroll
+        for (int e = 0; e < V; ++e)
+            if (c + e < a.K) {
+                const float d = voiced ? t[e] - o[e] * t[e] : 0.0f;
+                const float n = o[e] * fmaxf(x[e] - t[e], 0.0f);
+                acc[0] += d * d;
+                acc[1] += n * n;
+            }
+    }
+    block_accumulate_to<2, float>(acc, a.sums3 + (long long)u * 2);
+}
+
+// one block: loss_per_utt[u] = alpha sd_u + (1 - alpha) rn_u and the batch mean (the arithmetic of wsd_finish_kernel)
+__global__ void __launch_bounds__(256) wsd_finish_mean_kernel(const double* __restrict__ sums2, int n_utt, float alpha,
+                                                              float* __restrict__ loss, float* __restrict__ loss_mean) {
+    __shared__ double part[2][8];
+    double sp = 0.0, no = 0.0;
+    for (int u = threadIdx.x; u < n_utt; u += blockDim.x) {
+        const double s = sums2[2 * u], n = sums2[2 * u + 1];
+        if (loss) loss[u] = (float)((double)alpha * s + (1.0 - (double)alpha) * n);
+        sp += s;
+        no += n;
+    }
+    sp = secommon::warp_sum(sp);
+    no = secommon::warp_sum(no);
+    if ((threadIdx.x & 31) == 0) { part[0][threadIdx.x >> 5] = sp; part[1][threadIdx.x >> 5] = no; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        sp = no = 0.0;
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) { sp += part[0][w]; no += part[1][w]; }
+        *loss_mean = (float)(((double)alpha * sp + (1.0 - (double)alpha) * no) / n_utt);
+    }
+}
+
+// d loss_mean / d offset (upstream gradient grad_uniform = 1 / B), whole rows of grad_offset: 0 on padded frames and pad columns
+template <int V>
+__global__ void __launch_bounds__(256) wsd_mask_bwd_kernel(const WsdMaskArgs a) {
+    const int u = blockIdx.x / a.chunks, chunk = blockIdx.x - u * a.chunks;
+    const int valid = mask_valid_frames(a, u);
+    const int KV = (int)(a.ld_g / V) < (a.K + V - 1) / V ? (a.K + V - 1) / V : (int)(a.ld_g / V);
+    const int per = (a.n_frames + a.chunks - 1) / a.chunks;
+    const int f_lo = chunk * per, f_hi = min(a.n_frames, f_lo + per);
+    const float thres = wsd_thres(a);
+    const float scale = a.grad_uniform;
+    const long long row0 = (long long)u * a.n_frames;
+    const int items = max(f_hi - f_lo, 0) * KV;
+#pragma unroll 4
+    for (int i = threadIdx.x; i < items; i += blockDim.x) {
+        const int fr = i / KV, c = (i - fr * KV) * V;
+        const int f = f_lo + fr;
+        const long long r = row0 + f;
+        float g[V];
+#pragma unroll
+        for (int e = 0; e < V; ++e) g[e] = 0.0f;
+        if (f < valid && c < a.K) {
+            float x[V], t[V], o[V];
+            ldv<V>(a.inp + r * a.ld_inp + c, x);
+            ldv<V>(a.tar + r * a.ld_tar + c, t);
+            ldv<V>(a.offset + r * a.ld_off + c, o);
+            const bool voiced = 10.0f * log10f(a.energy[r] + a.eps) > thres;
+#pragma unroll
+            for (int e = 0; e < V; ++e)
+                if (c + e < a.K) {
+                    const float S = t[e], G = o[e], n = fmaxf(x[e] - S, 0.0f);
+                    g[e] = scale * ((voiced ? a.alpha * 2.0f * (S - G * S) * (-S) : 0.0f) + (1.0f - a.alpha) * 2.0f * G * n * n);
+                }
+        }
+        if (c + V <= a.ld_g) stv<V>(a.grad_offset + r * a.ld_g + c, g);
     }
 }
 
@@ -1114,12 +1217,8 @@ int se_wsd_fwd(const float* linear_inp, const float* offset, const float* linear
     SE_REQUIRE(linear_inp && offset && linear_tar && ws_energy && ws_max && ws_sums2 && loss && n_utt > 0 && n_frames > 0 && K > 0,
                "bad argument");
     cudaStream_t st = (cudaStream_t)stream;
-    SE_CUDA_CHECK(cudaMemsetAsync(ws_max, 0, sizeof(float), st));                 // key 0 = below every float
     SE_CUDA_CHECK(cudaMemsetAsync(ws_sums2, 0, sizeof(double) * 2 * n_utt, st));
-    const long long rows = n_utt * n_frames;
-    const long long want = (rows + 7) / 8;
-    wsd_energy_kernel<<<(unsigned)(want < 148 * 8 ? want : 148 * 8), 256, 0, st>>>(linear_tar, rows, (int)K, ws_energy, ws_max);
-    int rc = secommon::check_launch("wsd_energy_kernel");
+    int rc = launch_wsd_energy(linear_tar, K, n_utt * n_frames, (int)K, ws_energy, ws_max, st);
     if (rc != SE_OK) return rc;
     const int chunks = pick_chunks(n_utt, n_frames * K, 8192);
     wsd_sums_kernel<<<(unsigned)(n_utt * chunks), kThreads, 0, st>>>(linear_inp, offset, linear_tar, (const long long*)stft_len,
@@ -1140,6 +1239,43 @@ int se_wsd_bwd(const float* linear_inp, const float* offset, const float* linear
         linear_inp, offset, linear_tar, (const long long*)stft_len, (int)n_utt, (int)n_frames, (int)K, alpha, db_interval, eps,
         ws_energy, ws_max, grad_loss, grad_offset, total);
     return secommon::check_launch("wsd_bwd_kernel");
+}
+
+int se_wsd_energy(const float* linear_tar, int64_t ld_tar, int64_t n_utt, int64_t n_frames, int64_t K, float* energy, float* max_energy,
+                  void* stream) {
+    SE_REQUIRE(linear_tar && energy && max_energy && n_utt > 0 && n_frames > 0 && K > 0, "bad argument");
+    SE_REQUIRE(ld_tar >= K, "row stride smaller than K");
+    return launch_wsd_energy(linear_tar, ld_tar, n_utt * n_frames, (int)K, energy, max_energy, (cudaStream_t)stream);
+}
+
+int se_wsd_mask_step(const float* offset, int64_t ld_off, const float* linear_inp, int64_t ld_inp, const float* linear_tar, int64_t ld_tar,
+                     const int64_t* lengths, int64_t len_hop, int64_t n_utt, int64_t n_frames, int64_t K, float alpha, float db_interval,
+                     float eps, const float* energy, const float* max_energy, double* sums2, int sums_zeroed, float* loss_per_utt,
+                     float* loss_mean, float* grad_offset, int64_t ld_g, void* stream) {
+    SE_REQUIRE(offset && linear_inp && linear_tar && energy && max_energy && sums2 && loss_mean && n_utt > 0 && n_frames > 0 && K > 0,
+               "bad argument");
+    SE_REQUIRE(ld_off >= K && ld_inp >= K && ld_tar >= K && (!grad_offset || ld_g >= K), "row stride smaller than K");
+    SE_REQUIRE(len_hop >= 0 && len_hop < (1LL << 30), "len_hop=%lld out of range", (long long)len_hop);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!sums_zeroed) SE_CUDA_CHECK(cudaMemsetAsync(sums2, 0, sizeof(double) * 2 * n_utt, st));
+    WsdMaskArgs a{};
+    a.offset = offset; a.inp = linear_inp; a.tar = linear_tar; a.ld_off = ld_off; a.ld_inp = ld_inp; a.ld_tar = ld_tar;
+    a.stft_len = (const long long*)lengths; a.len_hop = (int)len_hop; a.n_utt = (int)n_utt; a.n_frames = (int)n_frames; a.K = (int)K;
+    a.chunks = pick_chunks(n_utt, n_frames * K, 2048); a.sums3 = sums2; a.eps = eps;
+    a.grad_uniform = 1.0f / (float)n_utt; a.grad_offset = grad_offset; a.ld_g = ld_g;
+    a.alpha = alpha; a.db_interval = db_interval; a.energy = energy; a.max_energy = max_energy;
+    const long long need = (K + 3) / 4 * 4;
+    const bool v4 = vec4_ok(offset, ld_off) && vec4_ok(linear_inp, ld_inp) && vec4_ok(linear_tar, ld_tar) && ld_inp >= need && ld_tar >= need &&
+                    ld_off >= need && (!grad_offset || (vec4_ok(grad_offset, ld_g) && ld_g >= need));
+    if (v4) wsd_mask_sums_kernel<4><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
+    else wsd_mask_sums_kernel<1><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
+    int rc = secommon::check_launch("wsd_mask_sums_kernel");
+    if (rc != SE_OK) return rc;
+    wsd_finish_mean_kernel<<<1, 256, 0, st>>>(sums2, (int)n_utt, alpha, loss_per_utt, loss_mean);
+    if ((rc = secommon::check_launch("wsd_finish_mean_kernel")) != SE_OK || !grad_offset) return rc;
+    if (v4) wsd_mask_bwd_kernel<4><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
+    else wsd_mask_bwd_kernel<1><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
+    return secommon::check_launch("wsd_mask_bwd_kernel");
 }
 
 int se_l1_logspec_fwd(const float* log_predicted, const float* linear_tar, const int64_t* stft_len, int64_t n_utt,

@@ -75,6 +75,15 @@ def reduce_sums(vec):
     return vec
 
 
+def global_max(t):
+    """All-reduce (max) a small tensor in place; returns it.  objective.WSD thresholds voicing against the loudest frame of
+    the WHOLE batch (objective.py:132-133), so every rank needs the maximum over all shards.  No-op at world size 1; under NCCL
+    it may run inside CUDA-graph capture."""
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    return t
+
+
 def global_means(per_utt_loss, per_utt_metric):
     """Batch means exactly as the single-process reference defines them (objective.py:100,
     runner.py:602): sum the per-utterance terms locally, all-reduce [sum_loss, sum_metric, count],

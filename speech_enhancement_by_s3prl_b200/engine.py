@@ -42,6 +42,7 @@ class EnhancementEngine:
         self.ch_inp = int(getattr(preprocessor, "channel_inp", 0))
         self.ch_tar = int(getattr(preprocessor, "channel_tar", 1))
         self._graphs = {}
+        self._side_streams = {}
         self.fused_training = os.environ.get("SE_B200_FUSED_TRAIN", "1") != "0"  # train_step without autograd (see fused_training_supported)
         self.launches_per_step = 5          # library kernels per eval_step (set by eval_step: 4 on the fused path)
 
@@ -214,11 +215,11 @@ class EnhancementEngine:
         return (int(cfg.get("delta", 0)) + 1) * self.pre._n_mels
 
     def fused_training_supported(self, objective, B, T):
-        """True if train_step can take the fused route: LinearResidual with the SISDR objective and the tensor-core head, on the
-        (log-)power spectrum or on a mel feature config (pseudo_noise.yaml:10-15), shapes inside the TMA head's / the split-K
-        backward's range."""
+        """True if train_step can take the fused route: LinearResidual with the SISDR or the WSD objective and the tensor-core
+        head, on the (log-)power spectrum or on a mel feature config (pseudo_noise.yaml:10-15), shapes inside the TMA head's / the
+        split-K backward's range."""
         from . import model, objective as obj
-        if not self.fused_training or self.precision != 1 or type(objective) is not obj.SISDR:
+        if not self.fused_training or self.precision != 1 or type(objective) not in (obj.SISDR, obj.WSD):
             return False
         if type(self.head) is not model.LinearResidual:
             return False
@@ -235,7 +236,11 @@ class EnhancementEngine:
         """runner.py:431-460 in seven kernels, no autograd graph: K1 (noisy: power + log-power + CMVN sums), K1 (clean:
         power), TMA head, SISDR sums + finish on offset * linear_inp, its backward straight to grad_offset, split-K
         tensor-core weight gradient + reduction.  With a mel ``feat_cfg`` the head input comes from the fused K1b kernel
-        (mel -> log -> deltas) and one sums pass instead.  Leaves the gradients in ``.grad`` and returns the loss."""
+        (mel -> log -> deltas) and one sums pass instead.  objective.WSD: the frame energies of linear_tar and their maximum
+        first (all-reduced across data-parallel ranks on a side stream while the head runs), then the WSD sums + finish and
+        its backward in the weight-gradient kernel.  Leaves the gradients in ``.grad`` and returns the loss."""
+        from . import objective as obj
+        wsd = type(objective) is obj.WSD
         B, C, T = wavs.shape
         dev = wavs.device
         head = self.head
@@ -270,14 +275,35 @@ class EnhancementEngine:
                 linear_tar = ops.stft_padded(wavs, self.ch_tar, self.n_fft, self.hop, window, logpower=False)
             wpad = self._padded_weight()            # current: refreshed in place after every update (_clip_and_step)
             stats = stat_sums if head.cmvn else None
+            if wsd:
+                # the voicing threshold needs the loudest frame of the GLOBAL batch: its 4-byte all-reduce runs on a side stream
+                # under the head's forward (nothing to fork at world size 1)
+                energy, emax = ops.wsd_energy(linear_tar, K)
+                main = torch.cuda.current_stream(dev)
+                side = self._side_stream(dev) if dp.world()[1] > 1 else None
+                if side is not None:
+                    side.wait_stream(main)
+                    with torch.cuda.stream(side):
+                        dp.global_max(emax)
             offset = ops.linear_head_tma(feats, D, wpad, head.linear.bias, head.activation, stats, head.eps)
             # frames = lengths // hop + 1, the batch-mean loss and d loss / d offset inside three launches
             lens = _c64(lengths)
-            fold = ops.linear_head_bwd_sisdr_supported(B, feats.shape[1], D, K, feats.shape[2], offset.shape[2], linear_inp.shape[2],
-                                                       linear_tar.shape[2])
-            loss, _, grad_offset, _ = ops.sisdr_mask_step(offset, linear_inp, linear_tar, lens, self.hop, K, objective.eps,
-                                                           sums3=sums3, sums_zeroed=True, want_grad=not fold)
-            if fold:            # the objective's backward runs inside the weight-gradient kernel: no grad_offset tensor
+            fold = (ops.linear_head_bwd_wsd_supported if wsd else ops.linear_head_bwd_sisdr_supported)(
+                B, feats.shape[1], D, K, feats.shape[2], offset.shape[2], linear_inp.shape[2], linear_tar.shape[2])
+            if wsd:
+                if side is not None:
+                    main.wait_stream(side)
+                sums2 = sums3.view(-1)[:2 * B].view(B, 2)          # the zeroed workspace's sums part, as (B, 2)
+                loss, _, grad_offset, _ = ops.wsd_mask_step(offset, linear_inp, linear_tar, lens, self.hop, K, energy, emax,
+                                                            objective.alpha, objective.db_interval, objective.eps, sums2=sums2,
+                                                            sums_zeroed=True, want_grad=not fold)
+            else:
+                loss, _, grad_offset, _ = ops.sisdr_mask_step(offset, linear_inp, linear_tar, lens, self.hop, K, objective.eps,
+                                                               sums3=sums3, sums_zeroed=True, want_grad=not fold)
+            if fold and wsd:    # the objective's backward runs inside the weight-gradient kernel: no grad_offset tensor
+                gw, gb = ops.linear_head_bwd_wsd(feats, D, stats, head.eps, offset, linear_inp, linear_tar, lens, self.hop, energy, emax, K,
+                                                 head.activation, objective.alpha, objective.db_interval, objective.eps)
+            elif fold:
                 gw, gb = ops.linear_head_bwd_sisdr(feats, D, stats, head.eps, offset, linear_inp, linear_tar, lens, self.hop, sums3, K,
                                                    head.activation, objective.eps)
             else:
@@ -288,6 +314,13 @@ class EnhancementEngine:
                 else:
                     p.grad.add_(g)
         return loss
+
+    def _side_stream(self, device):
+        """One side stream per device for the WSD maximum's all-reduce (kept: a captured step records it as a fork / join)."""
+        key = str(device)
+        if key not in self._side_streams:
+            self._side_streams[key] = torch.cuda.Stream(device=device)
+        return self._side_streams[key]
 
     def _clip_and_step(self, optimizer, grad_clip):
         """runner.py:463-470; two launches with se_b200.ClipAdam (NaN / inf norms skipped on the device), torch's kernels

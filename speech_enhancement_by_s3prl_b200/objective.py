@@ -46,7 +46,9 @@ class L1(nn.Module):
 class WSD(nn.Module):
     """objective.py:120-153 -- weighted speech distortion: alpha * speech distortion on voiced frames + (1 - alpha) *
     residual noise, both summed per utterance over valid frames and averaged over the batch.  Fused forward and
-    backward (w.r.t. ``offset``); ``linear_inp`` / ``linear_tar`` are data and get no gradient, as in the reference's use."""
+    backward (w.r.t. ``offset``); ``linear_inp`` / ``linear_tar`` are data and get no gradient, as in the reference's use.
+    The voicing threshold comes from the loudest frame of the whole batch, all-reduced across data-parallel ranks
+    (``dp.global_max``): while a process group of world size > 1 is initialized, every rank must call it for every batch."""
 
     def __init__(self, alpha=0.5, db_interval=30, eps=1e-10, **kwargs):
         super().__init__()

@@ -11,7 +11,7 @@ import math
 
 import torch
 
-from . import _lib
+from . import _lib, dp
 
 ACT = {"Identity": 0, "ReLU": 1, "Sigmoid": 2}
 NSUMS = 6
@@ -234,6 +234,70 @@ def linear_head_bwd_sisdr(x, D_in, stat_sums, cmvn_eps, offset, linear_inp, line
                                           gw.data_ptr(), gb.data_ptr(), _stream())
         _lib.check(rc, "se_linear_head_bwd_sisdr")
     return gw, gb
+
+
+def linear_head_bwd_wsd_supported(B, F, D_in, D_out, ldx, ld_off, ld_inp, ld_tar):
+    return bool(_lib.load().se_linear_head_bwd_wsd_supported(B, F, int(D_in), int(D_out), ldx, ld_off, ld_inp, ld_tar))
+
+
+def linear_head_bwd_wsd(x, D_in, stat_sums, cmvn_eps, offset, linear_inp, linear_tar, lengths, hop, energy, emax, D_out, activation,
+                        alpha=0.5, db_interval=30.0, loss_eps=1e-10):
+    """``linear_head_bwd_sisdr`` for the batch-mean objective.WSD loss: d loss / d offset is rebuilt inside the weight-gradient
+    kernel from offset / linear_inp / linear_tar (B, F, LD*) row-padded, the frame energies (B, F) and the batch maximum (1,) of
+    ``wsd_energy`` (all-reduced first under data parallelism).  Returns (grad_W (D_out, D_in), grad_b (D_out,))."""
+    B, F, LDx = x.shape
+    lib = _lib.load()
+    with torch.cuda.device(x.device):
+        ws_floats = lib.se_linear_head_bwd_tc_workspace(B, F, int(D_in), int(D_out))
+        if ws_floats <= 0:
+            raise RuntimeError(f"se_linear_head_bwd_wsd: shape (B={B}, F={F}, D_in={D_in}, D_out={D_out}) is not supported")
+        ws = torch.empty(ws_floats, device=x.device)
+        gw = torch.empty(D_out, D_in, device=x.device)
+        gb = torch.empty(D_out, device=x.device)
+        rc = lib.se_linear_head_bwd_wsd(x.data_ptr(), LDx, _p(stat_sums), 0 if stat_sums is None else stat_sums.shape[1], float(cmvn_eps),
+                                        offset.data_ptr(), offset.shape[2], linear_inp.data_ptr(), linear_inp.shape[2],
+                                        linear_tar.data_ptr(), linear_tar.shape[2], lengths.data_ptr(), int(hop), energy.data_ptr(),
+                                        emax.data_ptr(), float(alpha), float(db_interval), float(loss_eps), B, F, int(D_in), int(D_out),
+                                        ACT[activation], ws.data_ptr(), ws_floats, gw.data_ptr(), gb.data_ptr(), _stream())
+        _lib.check(rc, "se_linear_head_bwd_wsd")
+    return gw, gb
+
+
+def wsd_energy(linear_tar, K):
+    """objective.WSD's frame energies and their maximum: linear_tar (B, F, LD) row-padded (columns >= K are not read) ->
+    (energy (B, F), emax (1,) float32 -- the rank-local batch maximum, ready for ``dp.global_max``)."""
+    linear_tar = _chk(linear_tar, "linear_tar")
+    assert linear_tar.dim() == 3 and linear_tar.stride(2) == 1 and linear_tar.stride(1) == linear_tar.shape[2]
+    B, F, LD = linear_tar.shape
+    dev = linear_tar.device
+    with torch.cuda.device(dev):
+        energy = torch.empty(B, F, device=dev)
+        emax = torch.empty(1, device=dev)
+        rc = _lib.load().se_wsd_energy(linear_tar.data_ptr(), LD, B, F, int(K), energy.data_ptr(), emax.data_ptr(), _stream())
+        _lib.check(rc, "se_wsd_energy")
+    return energy, emax
+
+
+def wsd_mask_step(offset, linear_inp, linear_tar, lengths, hop, K, energy, emax, alpha=0.5, db_interval=30.0, eps=1e-10, sums2=None,
+                  sums_zeroed=False, want_grad=True):
+    """The WSD objective's part of a training step on (B, F, LD) row-padded tensors (the counterpart of ``sisdr_mask_step``),
+    thresholding against the maximum in ``emax`` (after ``dp.global_max`` under data parallelism).  ``lengths``: SAMPLE lengths
+    with ``hop`` (frames = lengths // hop + 1) or frame counts with hop = 0.
+    Returns (loss (0-dim), loss_per_utt (B,), grad_offset (B, F, LDo) or None (want_grad=False), sums2 (B, 2) float64)."""
+    B, F, LDi = linear_inp.shape
+    dev = linear_inp.device
+    lengths = _c(lengths, "lengths", torch.int64)
+    with torch.cuda.device(dev):
+        if sums2 is None:
+            sums2, sums_zeroed = torch.zeros(B, 2, device=dev, dtype=torch.float64), True
+        out = torch.empty(B + 1, device=dev)
+        grad = torch.empty_like(offset) if want_grad else None
+        rc = _lib.load().se_wsd_mask_step(offset.data_ptr(), offset.shape[2], linear_inp.data_ptr(), LDi, linear_tar.data_ptr(),
+                                          linear_tar.shape[2], lengths.data_ptr(), int(hop), B, F, int(K), float(alpha), float(db_interval),
+                                          float(eps), energy.data_ptr(), emax.data_ptr(), sums2.data_ptr(), 1 if sums_zeroed else 0,
+                                          out.data_ptr(), out[B:].data_ptr(), _p(grad), 0 if grad is None else grad.shape[2], _stream())
+        _lib.check(rc, "se_wsd_mask_step")
+    return out[B], out[:B], grad, sums2
 
 
 def sisdr_mask_step(offset, linear_inp, linear_tar, lengths, hop, K, eps=1e-10, sums3=None, sums_zeroed=False, want_grad=True):
@@ -702,29 +766,26 @@ def l1_logspec_sums(log_predicted, linear_tar, stft_len, eps=1e-10):
 
 
 # --------------------------------------------------------------------------- mask head
-@torch.library.custom_op("se_b200::wsd", mutates_args=())
-def _wsd(linear_inp: torch.Tensor, offset: torch.Tensor, linear_tar: torch.Tensor, stft_len: torch.Tensor, alpha: float,
-         db_interval: float, eps: float) -> tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
-    """objective.WSD forward -> (loss (1,), frame energies (B, F), batch-maximum key (1,)) -- the last two feed the backward."""
+@torch.library.custom_op("se_b200::wsd_sums", mutates_args=())
+def _wsd_sums(linear_inp: torch.Tensor, offset: torch.Tensor, linear_tar: torch.Tensor, stft_len: torch.Tensor, energy: torch.Tensor,
+              emax: torch.Tensor, alpha: float, db_interval: float, eps: float) -> torch.Tensor:
+    """objective.WSD forward from the frame energies and the batch maximum of ``wsd_energy`` -> loss (1,)."""
     linear_inp, offset, linear_tar = _c(linear_inp, "linear_inp"), _c(offset, "offset"), _c(linear_tar, "linear_tar")
     B, F, K = linear_tar.shape
     dev = linear_tar.device
     with torch.cuda.device(dev):
-        energy = torch.empty(B, F, device=dev)
-        emax = torch.empty(1, device=dev)
         sums2 = torch.empty(B, 2, device=dev, dtype=torch.float64)
         loss = torch.empty(1, device=dev)
-        rc = _lib.load().se_wsd_fwd(linear_inp.data_ptr(), offset.data_ptr(), linear_tar.data_ptr(), stft_len.data_ptr(), B, F, K,
-                                    alpha, db_interval, eps, energy.data_ptr(), emax.data_ptr(), sums2.data_ptr(),
-                                    loss.data_ptr(), _stream())
-        _lib.check(rc, "se_wsd_fwd")
-    return loss, energy, emax
+        rc = _lib.load().se_wsd_mask_step(offset.data_ptr(), K, linear_inp.data_ptr(), K, linear_tar.data_ptr(), K, stft_len.data_ptr(), 0,
+                                          B, F, K, alpha, db_interval, eps, energy.data_ptr(), emax.data_ptr(), sums2.data_ptr(), 0, None,
+                                          loss.data_ptr(), None, 0, _stream())
+        _lib.check(rc, "se_wsd_mask_step")
+    return loss
 
 
-@_wsd.register_fake
-def _(linear_inp, offset, linear_tar, stft_len, alpha, db_interval, eps):
-    B, F, K = linear_tar.shape
-    return linear_tar.new_empty(1), linear_tar.new_empty(B, F), linear_tar.new_empty(1)
+@_wsd_sums.register_fake
+def _(linear_inp, offset, linear_tar, stft_len, energy, emax, alpha, db_interval, eps):
+    return linear_tar.new_empty(1)
 
 
 @torch.library.custom_op("se_b200::wsd_bwd", mutates_args=())
@@ -748,26 +809,33 @@ def _(linear_inp, offset, linear_tar, stft_len, alpha, db_interval, eps, energy,
 
 
 def _wsd_setup(ctx, inputs, output):
-    linear_inp, offset, linear_tar, stft_len, alpha, db_interval, eps = inputs
-    _, energy, emax = output
+    linear_inp, offset, linear_tar, stft_len, energy, emax, alpha, db_interval, eps = inputs
     ctx.save_for_backward(linear_inp, offset, linear_tar, stft_len, energy, emax)
     ctx.cfg = (alpha, db_interval, eps)
 
 
-def _wsd_backward(ctx, grad_loss, grad_energy, grad_emax):
+def _wsd_backward(ctx, grad_loss):
     linear_inp, offset, linear_tar, stft_len, energy, emax = ctx.saved_tensors
     alpha, db_interval, eps = ctx.cfg
     grad = torch.ops.se_b200.wsd_bwd(linear_inp, offset, linear_tar, stft_len, alpha, db_interval, eps, energy, emax, grad_loss)
-    return None, grad, None, None, None, None, None          # the spectra are data: only the head's offset gets a gradient
+    return None, grad, None, None, None, None, None, None, None   # the spectra are data: only the head's offset gets a gradient
 
 
-_wsd.register_autograd(_wsd_backward, setup_context=_wsd_setup)
+_wsd_sums.register_autograd(_wsd_backward, setup_context=_wsd_setup)
 
 
 def wsd(linear_inp, offset, linear_tar, stft_len, alpha=0.5, db_interval=30.0, eps=1e-10):
-    """objective.py:120-153 as one fused forward (+ backward w.r.t. offset).  Returns the scalar loss."""
+    """objective.py:120-153 (+ backward w.r.t. offset).  Returns the scalar loss.  The frame energies and their maximum come first
+    and the maximum is all-reduced across data-parallel ranks (``dp.global_max``) before the sums: every rank then thresholds
+    voicing against the loudest frame of the GLOBAL batch, as the single-process reference does.
+    That all-reduce is a collective: while a process group of world size > 1 is initialized, EVERY rank must call this for
+    every batch (a call made on some ranks only -- e.g. evaluation on rank 0 alone -- waits for the others forever)."""
     stft_len = _c(stft_len, "stft_len", torch.int64)
-    return torch.ops.se_b200.wsd(linear_inp, offset, linear_tar, stft_len, float(alpha), float(db_interval), float(eps))[0][0]
+    linear_tar = _c(linear_tar, "linear_tar")
+    energy, emax = wsd_energy(linear_tar, linear_tar.shape[2])
+    dp.global_max(emax)
+    return torch.ops.se_b200.wsd_sums(linear_inp, offset, linear_tar, stft_len, energy, emax, float(alpha), float(db_interval),
+                                      float(eps))[0]
 
 
 @torch.library.custom_op("se_b200::linear_head", mutates_args=())
