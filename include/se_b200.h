@@ -126,14 +126,18 @@ int se_mask_istft_ex(const float* noisy, const float* clean, int64_t utt_stride,
  * reference's (target_db_or_nan = NaN; runner.py:570 + utils.py:38-40) or a fixed level
  * in dB (runner.py:266 default -25); wav *= gain in place over [0, width);
  * sisdr_wave[u] = evaluation.sisdr_eval(gain*y[:len], c[:len]);
- * loss_spec[u]  = per-utterance term of objective.SISDR (its batch mean is the loss).
- * Any of gain / sisdr_wave / loss_spec may be NULL; wav may be NULL (no scaling). */
+ * loss_spec[u]  = per-utterance term of objective.SISDR (its batch mean is the loss); meaningful only if the sums
+ *                came from se_mask_istft with want_spec (otherwise the spectral sums are 0 and the term is 100 dB).
+ * lengths[u] is clamped to [0, T] as se_mask_istft clamps it, so the means divide by the samples that were summed;
+ * lengths NULL = T.  Any of gain / sisdr_wave / loss_spec may be NULL; wav may be NULL (no scaling). */
 int se_finalize_metrics(const double* sums, const int64_t* lengths, int64_t n_utt, int64_t T,
                         float target_db_or_nan, float* wav, int64_t wav_stride, int64_t width,
                         float* gain, float* sisdr_wave, float* loss_spec, void* stream);
 /* Same, and metric_acc[0..2] (doubles, caller-owned, never zeroed here) += [sum_u loss_spec, sum_u sisdr_wave, n_utt]:
  * the running sums an evaluation pass averages at its end (runner.py:602; objective.py:100) stay on the device, so
- * a pass over many batches -- and the one all-reduce of a data-parallel pass -- needs no host read per batch. */
+ * a pass over many batches -- and the one all-reduce of a data-parallel pass -- needs no host read per batch.
+ * A term is added only if it is produced: metric_acc[0] only when loss_spec != NULL, metric_acc[1] only when
+ * sisdr_wave != NULL (pass loss_spec = NULL when the sums were made without want_spec); metric_acc[2] always counts. */
 int se_finalize_metrics_acc(const double* sums, const int64_t* lengths, int64_t n_utt, int64_t T,
                             float target_db_or_nan, float* wav, int64_t wav_stride, int64_t width,
                             float* gain, float* sisdr_wave, float* loss_spec, double* metric_acc, void* stream);
@@ -205,7 +209,8 @@ int se_sisdr_wave(const float* src, int64_t src_stride, const float* tar, int64_
 
 /* ---- a11: masked_normalize_decibel (utils.py:31-46) -------------------------------
  * out = audio * sqrt(10^(target/10) / (masked_mean(audio^2) + eps)); target per row is
- * target_db[u] if target_db != NULL, else the masked level of ref[u] (utils.py:38-40).
+ * target_db[u] if target_db != NULL, else the masked level of ref[u] (utils.py:38-40).  masked_mean divides by
+ * min(lengths[u], width) + 1e-8 whatever eps is (utils.py:26: the reference's masked_mean keeps its own default).
  * ws_sums3: caller workspace of n_utt x 3 doubles.  out may alias audio. */
 int se_masked_normalize_db(const float* audio, int64_t stride, const int64_t* lengths, int64_t n_utt, int64_t width,
                            const float* target_db, const float* ref, int64_t ref_stride, float eps,

@@ -56,7 +56,8 @@ __global__ void finalize_metrics_kernel(const double* __restrict__ sums, const l
         for (int q = 0; q < 8; ++q) if (i0 + q * bd < n4) v[q] = r4[i0 + q * bd];
     }
     const double* s = sums + (long long)u * SE_NSUMS;
-    const double len = lengths ? (double)lengths[u] : (double)T;
+    // clamped to [0, T] as se_mask_istft clamps it for the sums: the means divide by the samples that were summed
+    const double len = lengths ? (double)min((long long)T, max(0LL, lengths[u])) : (double)T;
     const double eps_mean = 1e-8;                                       // utils.py:26, utils.py:31
     const double mean_yy = s[SE_SUM_YY] / (len + eps_mean);
     const double level = level_or_neg < 0.0 ? s[SE_SUM_CC] / (len + eps_mean) : level_or_neg;
@@ -68,8 +69,8 @@ __global__ void finalize_metrics_kernel(const double* __restrict__ sums, const l
         if (sisdr_wave) sisdr_wave[u] = sd;
         if (loss_spec) loss_spec[u] = ls;
         if (metric_acc) {                                               // running sums of an evaluation pass (runner.py:602)
-            atomicAdd(metric_acc, (double)ls);
-            atomicAdd(metric_acc + 1, (double)sd);
+            if (loss_spec) atomicAdd(metric_acc, (double)ls);           // only the terms this call produces
+            if (sisdr_wave) atomicAdd(metric_acc + 1, (double)sd);
             atomicAdd(metric_acc + 2, 1.0);
         }
     }
@@ -698,16 +699,19 @@ __global__ void sisdr_wave_finish_kernel(const double* __restrict__ sums3, int n
     if (u < n_utt) out[u] = (float)sisdr_from_sums(sums3[3 * u], sums3[3 * u + 1], sums3[3 * u + 2], (double)eps);
 }
 
-// out = audio * sqrt(10^(target/10) / (mean(audio^2) + eps)); sums3[u] = (<a,r>, <r,r>, <a,a>) with r = ref
+// out = audio * sqrt(10^(target/10) / (mean(audio^2) + eps)); sums3[u] = (<a,r>, <r,r>, <a,a>) with r = ref.
+// The masked means divide by len + 1e-8 whatever eps is (utils.py:26 masked_mean's own default); eps enters only the
+// gain's denominator (utils.py:42).
 __global__ void normalize_db_kernel(const float* __restrict__ audio, long long stride, const long long* __restrict__ lengths,
                                     int width, const float* __restrict__ target_db, int have_ref, float eps,
                                     const double* __restrict__ sums3, float* __restrict__ out, long long out_stride, int chunks) {
     const int u = blockIdx.x / chunks, chunk = blockIdx.x - u * chunks;
-    const double len = lengths ? (double)min((long long)width, lengths[u]) : (double)width;
-    const double mean_aa = sums3[3 * u + 2] / (len + (double)eps);
+    const double len = lengths ? (double)min((long long)width, max(0LL, lengths[u])) : (double)width;
+    const double eps_mean = 1e-8;
+    const double mean_aa = sums3[3 * u + 2] / (len + eps_mean);
     double tdb;
     if (target_db) tdb = (double)target_db[u];
-    else tdb = have_ref ? 10.0 * log10(sums3[3 * u + 1] / (len + (double)eps)) : -25.0;
+    else tdb = have_ref ? 10.0 * log10(sums3[3 * u + 1] / (len + eps_mean)) : -25.0;
     const float g = (float)sqrt(pow(10.0, tdb / 10.0) / (mean_aa + (double)eps));
     const int per = (width + chunks - 1) / chunks;
     const int lo = chunk * per, hi = min(width, lo + per);

@@ -55,9 +55,11 @@ class EnhancementEngine:
 
     def eval_step(self, lengths, wavs, want_spec_loss=True, metric_acc=None, ws=None):
         """lengths (B,) int64, wavs (B, C, T) fp32, both on the GPU.
-        Returns dict(loss_per_utt (B,), sisdr (B,), wav_predicted (B, T), gain (B,)).
+        Returns dict(loss_per_utt (B,), sisdr (B,), wav_predicted (B, T), gain (B,)); loss_per_utt is None when
+        want_spec_loss is False (the spectral SI-SDR sums are not computed then).
         metric_acc: float64 (3,) device tensor += [sum loss, sum SI-SDR, utterances] (the running sums of an evaluation
-        pass, runner.py:587-602; ``dp.means_from_acc`` turns them into the global means with one all-reduce).
+        pass, runner.py:587-602; ``dp.means_from_acc`` turns them into the global means with one all-reduce).  Without
+        want_spec_loss the loss sum is left as it is; SI-SDR and the count are still added.
         ws: a ``step_workspace`` that this call may use and must leave zeroed (captured steps); None = a fresh one per call."""
         B, C, T = wavs.shape
         dev = wavs.device
@@ -115,7 +117,8 @@ class EnhancementEngine:
                                               head.eps, precision=self.precision)
                 wav, sums = ops.mask_istft(wavs, self.ch_inp, self.ch_tar, mask, lengths, self.n_fft, self.hop, window,
                                            pad_to=T, want_sums=True, want_spec=want_spec_loss, mask_padded=True)
-            gain, sisdr, loss = ops.finalize_metrics(sums, lengths, T, wav=wav, target_db=None, metric_acc=metric_acc)
+            gain, sisdr, loss = ops.finalize_metrics(sums, lengths, T, wav=wav, target_db=None, want_loss=want_spec_loss,
+                                                     metric_acc=metric_acc)
         return {"loss_per_utt": loss, "sisdr": sisdr, "wav_predicted": wav, "gain": gain, "mask": mask[..., :K]}
 
     def _padded_weight(self, force=False):

@@ -469,7 +469,8 @@ def mask_istft(wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, 
 def finalize_metrics(sums, lengths, T, wav=None, target_db=None, want_gain=True, want_sisdr=True, want_loss=True,
                      metric_acc=None):
     """Gain / waveform SI-SDR / spectral-SISDR terms from the sums of mask_istft; scales wav in place.
-    metric_acc: float64 (3,) running [sum loss, sum SI-SDR, utterances] of an evaluation pass, updated on the device."""
+    metric_acc: float64 (3,) running [sum loss, sum SI-SDR, utterances] of an evaluation pass, updated on the device
+    (the loss sum only with want_loss, the SI-SDR sum only with want_sisdr).  lengths are clamped to [0, T]."""
     B = sums.shape[0]
     dev = sums.device
     with torch.cuda.device(dev):
