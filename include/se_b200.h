@@ -207,6 +207,20 @@ int se_wsd_mask_step(const float* offset, int64_t ld_off, const float* linear_in
 int se_sisdr_wave(const float* src, int64_t src_stride, const float* tar, int64_t tar_stride, const int64_t* lengths,
                   int64_t n_utt, int64_t T, float eps, double* ws_sums3, float* sisdr, void* stream);
 
+/* ---- STOI / ESTOI (pystoi 0.3.x: stoi(clean, processed, fs), extended=False / True) -----------------------
+ * stoi[u], estoi[u] of ref[u, :len[u]] (the clean reference, pystoi's x) and est[u, :len[u]] (the processed
+ * signal); lengths NULL = T, otherwise clamped to [0, T].  Resampled to 10 kHz unless fs == 10000; fewer than
+ * 30 STFT frames after silent-frame removal (also no frame at all) gives 1e-5.  Supported rates: 10000 / fs
+ * reduced to p / q with p, q <= 48 (8, 16, 32, 48 kHz; 10 kHz without resampling); others SE_ERR_UNSUPPORTED.
+ * se_stoi_workspace: bytes of `ws` (<= 0: unsupported fs or shape).  stoi, estoi, n_kept (frames kept by the
+ * silent-frame removal) are each optional, but stoi or estoi must be given.  acc (optional, 3 doubles, never
+ * zeroed here) += [sum stoi, sum estoi, n_utt], each sum only when that output is given.  No host
+ * synchronisation, no allocation: capturable.  Per-utterance results are bitwise reproducible. */
+int64_t se_stoi_workspace(int64_t n_utt, int64_t T, int fs);
+int se_stoi(const float* est, int64_t est_stride, const float* ref, int64_t ref_stride, const int64_t* lengths,
+            int64_t n_utt, int64_t T, int fs, void* ws, int64_t ws_bytes,
+            float* stoi, float* estoi, int32_t* n_kept, double* acc, void* stream);
+
 /* ---- a11: masked_normalize_decibel (utils.py:31-46) -------------------------------
  * out = audio * sqrt(10^(target/10) / (masked_mean(audio^2) + eps)); target per row is
  * target_db[u] if target_db != NULL, else the masked level of ref[u] (utils.py:38-40).  masked_mean divides by

@@ -72,6 +72,8 @@ _SIGNATURES = {
     "se_linear_head_bwd_wsd": [c_f, i64, c_f, i64, c_float, c_f, i64, c_f, i64, c_f, i64, c_f, i64, c_f, c_f, c_float, c_float, c_float, i64,
                                i64, i64, i64, c_int, c_f, i64, c_f, c_f, c_f],
     "se_sisdr_wave": [c_f, i64, c_f, i64, c_f, i64, i64, c_float, c_f, c_f, c_f],
+    "se_stoi_workspace": [i64, i64, c_int],
+    "se_stoi": [c_f, i64, c_f, i64, c_f, i64, i64, c_int, c_f, i64, c_f, c_f, c_f, c_f, c_f],
     "se_masked_normalize_db": [c_f, i64, c_f, i64, i64, c_f, c_f, i64, c_float, c_f, c_f, i64, c_f],
     "se_length_masks": [c_f, i64, i64, c_f, c_f],
     "se_cmvn_stats": [c_f, i64, i64, i64, c_f, c_f, c_f],

@@ -53,14 +53,16 @@ class EnhancementEngine:
         LD = ops.round4(self.n_fft // 2 + 1)
         return torch.zeros(B * (2 * LD + ops.NSUMS), device=device, dtype=torch.float64)
 
-    def eval_step(self, lengths, wavs, want_spec_loss=True, metric_acc=None, ws=None):
+    def eval_step(self, lengths, wavs, want_spec_loss=True, metric_acc=None, ws=None, want_stoi=False, stoi_acc=None):
         """lengths (B,) int64, wavs (B, C, T) fp32, both on the GPU.
         Returns dict(loss_per_utt (B,), sisdr (B,), wav_predicted (B, T), gain (B,)); loss_per_utt is None when
         want_spec_loss is False (the spectral SI-SDR sums are not computed then).
         metric_acc: float64 (3,) device tensor += [sum loss, sum SI-SDR, utterances] (the running sums of an evaluation
         pass, runner.py:587-602; ``dp.means_from_acc`` turns them into the global means with one all-reduce).  Without
         want_spec_loss the loss sum is left as it is; SI-SDR and the count are still added.
-        ws: a ``step_workspace`` that this call may use and must leave zeroed (captured steps); None = a fresh one per call."""
+        ws: a ``step_workspace`` that this call may use and must leave zeroed (captured steps); None = a fresh one per call.
+        want_stoi: also return "stoi" and "estoi" (B,) of wav_predicted against the target channel, at the preprocessor's
+        sample rate (``ops.stoi``); stoi_acc: float64 (3,) device tensor += [sum STOI, sum ESTOI, utterances]."""
         B, C, T = wavs.shape
         dev = wavs.device
         window = self.pre._frame_window
@@ -119,7 +121,11 @@ class EnhancementEngine:
                                            pad_to=T, want_sums=True, want_spec=want_spec_loss, mask_padded=True)
             gain, sisdr, loss = ops.finalize_metrics(sums, lengths, T, wav=wav, target_db=None, want_loss=want_spec_loss,
                                                      metric_acc=metric_acc)
-        return {"loss_per_utt": loss, "sisdr": sisdr, "wav_predicted": wav, "gain": gain, "mask": mask[..., :K]}
+            out = {"loss_per_utt": loss, "sisdr": sisdr, "wav_predicted": wav, "gain": gain, "mask": mask[..., :K]}
+            if want_stoi:
+                # after K3' (both metrics are invariant to the gain of the estimate); the clean channel is read in place
+                out["stoi"], out["estoi"] = ops.stoi(wav, wavs[:, self.ch_tar], lengths, fs=self.pre._sample_rate, acc=stoi_acc)
+        return out
 
     def _padded_weight(self, force=False):
         """16-byte-row (and, for the tensor cores, TF32-rounded) copy of the head weight.
@@ -145,10 +151,10 @@ class EnhancementEngine:
         return buf
 
     # ------------------------------------------------------------------ CUDA-graph replay of the step
-    def capture_bound(self, lengths, wavs, metric_acc=None):
+    def capture_bound(self, lengths, wavs, metric_acc=None, want_stoi=False, stoi_acc=None):
         """Capture eval_step into a CUDA graph that reads the GIVEN device tensors in place
         (no staging copy).  Returns dict(graph=, lengths=, wavs=, loss_per_utt=, sisdr=, wav_predicted=, ...).
-        metric_acc: see eval_step (every replay adds the batch's sums to it)."""
+        metric_acc, want_stoi, stoi_acc: see eval_step (every replay adds the batch's sums to the accumulators)."""
         device = wavs.device
         ops.prepare(self.n_fft)
         if self.pre._frame_window.device != device:
@@ -158,12 +164,12 @@ class EnhancementEngine:
         ws = self.step_workspace(wavs.shape[0], device)          # zeroed once here; every replay leaves it zeroed
         with torch.cuda.stream(side):
             for _ in range(2):                                   # warm up allocator + lazy init outside capture
-                self.eval_step(lengths, wavs, ws=ws)             # (no metric_acc: warm-up batches are not part of a pass)
+                self.eval_step(lengths, wavs, ws=ws, want_stoi=want_stoi)   # (no accumulators: warm-up batches are not part of a pass)
         torch.cuda.current_stream(device).wait_stream(side)
         torch.cuda.synchronize(device)
         graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(graph):
-            out = self.eval_step(lengths, wavs, metric_acc=metric_acc, ws=ws)
+            out = self.eval_step(lengths, wavs, metric_acc=metric_acc, ws=ws, want_stoi=want_stoi, stoi_acc=stoi_acc)
         static = {"lengths": lengths, "wavs": wavs, "graph": graph, "ws": ws}
         static.update(out)
         return static

@@ -526,6 +526,34 @@ def sisdr_wave(src, tar, lengths=None, eps=1e-10):
     return out
 
 
+def stoi(est, ref, lengths=None, fs=16000, want_stoi=True, want_estoi=True, acc=None, n_kept=None):
+    """Batched STOI / ESTOI (pystoi 0.3.x): est = processed, ref = clean reference, both (B, T) views with unit sample stride
+    (row strides may differ, e.g. a channel of a (B, C, T) batch).  Returns (stoi, estoi), each (B,) fp32 or None.
+    acc: float64 (3,) device tensor += [sum stoi, sum estoi, B] (each sum only when that metric is requested).
+    n_kept: optional (B,) int32 output, the frames kept by the silent-frame removal."""
+    est, ref = _chk(est, "est"), _chk(ref, "ref")
+    assert est.dim() == 2 and est.shape == ref.shape and est.stride(1) == 1 and ref.stride(1) == 1
+    if not (want_stoi or want_estoi):
+        raise ValueError("ops.stoi: request stoi, estoi or both")
+    B, T = est.shape
+    lengths = _c(lengths, "lengths", torch.int64)
+    acc = _chk(acc, "acc", torch.float64)
+    n_kept = _chk(n_kept, "n_kept", torch.int32)
+    lib = _lib.load()
+    ws_bytes = lib.se_stoi_workspace(B, T, int(fs))
+    if ws_bytes <= 0:
+        raise RuntimeError(f"se_b200.stoi: unsupported sample rate {fs} or shape {tuple(est.shape)} "
+                           "(10000 / fs reduced to p / q needs p, q <= 48)")
+    with torch.cuda.device(est.device):
+        ws = torch.empty(ws_bytes, device=est.device, dtype=torch.uint8)
+        s = torch.empty(B, device=est.device) if want_stoi else None
+        e = torch.empty(B, device=est.device) if want_estoi else None
+        rc = lib.se_stoi(est.data_ptr(), est.stride(0), ref.data_ptr(), ref.stride(0), _p(lengths), B, T, int(fs), ws.data_ptr(),
+                         ws_bytes, _p(s), _p(e), _p(n_kept), _p(acc), _stream())
+        _lib.check(rc, "se_stoi")
+    return s, e
+
+
 def masked_normalize_db(audio, lengths, target_db=None, ref=None, eps=1e-8):
     """utils.masked_normalize_decibel on lengths instead of (B, T) int64 masks."""
     audio = _chk(audio, "audio")
