@@ -385,12 +385,12 @@ int se_linear_head_fused(const float* x, int64_t ldx, const double* stat_sums, i
 
 /* se_stft_features2: se_stft_features with BOTH spectral tensors of the channel -- power ("linear", what the objectives and
  * `predicted = linears * offset` consume) and log-power (the head's feature) -- from one transform; either may be NULL.
- * stat_sums holds the sums of logpower if it is given, else of power.  One launch for n_fft 512 / hop 256. */
+ * stat_sums holds the sums of logpower if it is given, else of power.  One launch for n_fft 512 / hop 256, 1024 / 256 and 400 / 160. */
 int se_stft_features2(const float* wav, int64_t n_utt, int64_t utt_stride, int64_t T, int n_fft, int hop, const float* window,
                       float log_eps, float* power, float* logpower, int64_t spec_stride, double* stat_sums, int64_t ld_stats,
                       int flags, void* stream);
 /* se_stft_features_pair: se_stft_features2 of the input channel AND the power spectrum of a second channel (the clean target,
- * runner.py:433: linear_tar) in ONE launch of the register-resident kernels (n_fft 1024 / hop 256 and 400 / hop 160;
+ * runner.py:433: linear_tar) in ONE launch of the register-resident kernels (n_fft 512 / hop 256, 1024 / 256 and 400 / 160;
  * se_stft_features_pair_supported, else SE_ERR_UNSUPPORTED: call se_stft_features2 twice).  wav points at the input channel of
  * utterance 0, the second channel lies chan_step floats further in every utterance.  power2: (2, n_utt, n_frames, spec_stride) --
  * [0] the input channel's power, [1] the second channel's; logpower / stat_sums: the input channel only. */

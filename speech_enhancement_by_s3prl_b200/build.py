@@ -49,7 +49,7 @@ def is_stale():
 
 
 def build_library(force=False, verbose=False, extra_flags=(), out_path=None):
-    """extra_flags / out_path: experiment builds (e.g. -DSE_K3_MIN_BLOCKS=4 into another file, loaded via SE_B200_LIB)."""
+    """extra_flags / out_path: experiment builds (e.g. -DSE_GEO512_K3_MINB=1 into another file, loaded via SE_B200_LIB)."""
     if out_path is None and not force and not is_stale():
         return LIB_PATH
     build_dir = os.path.join(PKG_DIR, "build")

@@ -1,5 +1,5 @@
-// Device helpers shared by the register-resident fast paths (fast512.cu: n_fft 512 / hop 256; fastgeo.cu: n_fft 1024 / hop
-// 256 and n_fft 400 / hop 160): approximate transcendental wrappers, cp.async staging primitives, the real-input split /
+// Device helpers of the register-resident fast paths (fastgeo.cu: n_fft 512 / hop 256, n_fft 1024 / hop 256 and n_fft 400 /
+// hop 160): approximate transcendental wrappers, cp.async staging primitives, the real-input split /
 // inverse merge of one pair of bins, the mask application and the programmatic-dependent-launch fences.
 #pragma once
 #include "fft_core.cuh"
@@ -22,7 +22,7 @@ __device__ __forceinline__ float fast_log(float x) {
 }
 
 // ---- asynchronous staging (cp.async): the global loads of frame i+1 are in flight while frame i is
-// transformed, so no half-warp ever waits on a DRAM round trip between its transforms.
+// transformed, so no lane group ever waits on a DRAM round trip between its transforms.
 __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {
     const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gmem_src) : "memory");

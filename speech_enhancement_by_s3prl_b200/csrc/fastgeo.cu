@@ -1,5 +1,6 @@
-// libse_b200.so -- register-resident fast paths for the geometries beside n_fft 512 / hop 256 (fast512.cu):
+// libse_b200.so -- register-resident fast paths, one kernel template over three geometries:
 //
+//   Geo512    n_fft 512  / hop 256   (BASELINE configs[1], the headline)      one frame per group of 16 lanes, 2 groups per warp
 //   Geo1024   n_fft 1024 / hop 256   (BASELINE configs[3], long-form)        one frame per WARP
 //   Geo400    n_fft 400  / hop 160   (the reference's default 25 ms / 10 ms, pretrain_sample.yaml:46-48; configs[2], [4])
 //                                                                             one frame per group of 10 lanes, 3 groups per warp
@@ -8,17 +9,19 @@
 //   mask_istft_run_kernel   K3: frame -> rFFT -> x sqrt(mask) -> irFFT -> window -> overlap-add in registers along a run of
 //                               consecutive frames -> / envelope -> wav, plus the per-utterance metric sums
 //
-// Same structure as fast512.cu (a lane group owns a RUN of consecutive frames, FFT values live in registers, only the
-// transposes of the FFT go through shared memory, no block-level barrier in the frame loops), generalised in two ways:
+// A lane group owns a RUN of consecutive frames, FFT values live in registers, only the transposes of the FFT go through
+// shared memory, and there is no block-level barrier in the frame loops.  All groups of a warp run in lock-step, so every
+// shuffle and __syncwarp uses the full warp mask.  The geometries differ in two places:
 //
-//   * FFT cores.  Geo1024: the 512-point complex transform of a frame is two 256-point half-warp transforms
+//   * FFT cores.  Geo512: the 256-point complex transform of a frame is one 16-lane transform (fft256_warp.cuh).
+//     Geo1024: the 512-point complex transform of a frame is two 256-point 16-lane transforms
 //     (fft256_warp.cuh) plus ONE radix-2 exchange between the halves (16 shuffles): decimation in time on the way
 //     forward (strided "time" layout in, blocked "spectral" layout out), decimation in frequency on the way back
 //     (blocked in, strided out), so neither direction needs a second transpose.  Geo400: 200 = 20 x 10 -- a
 //     prime-factor (Good-Thomas, twiddle-free) 20-point DFT in registers, one transpose through shared memory, the
 //     twiddles, then two prime-factor 10-point DFTs; lane j holds element j + 10 s before and after.
 //     tools/lane_model.py is the lane-level numpy model these index maps were checked with.
-//   * Overlap-add with N / hop > 2 (1024/256: 4 frames cover a sample; 400/160: 2 or 3).  Frame f EMITS the window of
+//   * Overlap-add (512/256: 2 frames cover a sample; 1024/256: 4; 400/160: 2 or 3).  Frame f EMITS the window of
 //     hop samples [f hop - N/2, f hop - N/2 + hop) that no later frame touches; the rest of its windowed inverse
 //     transform stays in the register carry.  A run that owns emit windows e0..e1 walks frames e0 - halo .. e1
 //     (halo = ceil(N / hop) - 1 frames recomputed at the start of every run) and, past the last frame of the
@@ -41,6 +44,7 @@ namespace {
 
 constexpr unsigned kFull = 0xffffffffu;
 
+struct Geo512  { enum { N = 512,  M = 256, H = 256, G = 16, V = 16, GPW = 2, IDLE = 0, NB = 2, HB = 1, VB = 8, NP = 8,  XBUF = 2048 }; };
 struct Geo1024 { enum { N = 1024, M = 512, H = 256, G = 32, V = 16, GPW = 1, IDLE = 0, NB = 4, HB = 1, VB = 4, NP = 8, XBUF = 4224 }; };
 struct Geo400  { enum { N = 400,  M = 200, H = 160, G = 10, V = 20, GPW = 3, IDLE = 1, NB = 5, HB = 2, VB = 4, NP = 10, XBUF = 1792 }; };
 
@@ -92,6 +96,29 @@ __device__ __forceinline__ void pfa10(float2 (&x)[10]) {
 // bin M/2 sits in slot V/2 of the group's leader lane, whose pair 0 is (DC, Nyquist).
 template <class Geo> struct Core;
 
+template <> struct Core<Geo512> {
+    float2 tw[15], twn[8];
+    float2* xbuf;
+    int j, tidx, ln;
+    bool leader, active;
+    __device__ __forceinline__ void init(int lane, unsigned char* region, const Tables& tab) {
+        j = lane & 15; tidx = j; ln = lane;                                             // group lane >> 4, its own region
+        leader = j == 0; active = true;
+        xbuf = reinterpret_cast<float2*>(region);
+        fft256w::load_lane_constants(j, tab.twM, tab.twN, tw, twn);
+    }
+    static __device__ __forceinline__ int group_of(int lane) { return lane >> 4; }
+    static __device__ __forceinline__ int lane_in_group(int lane) { return lane & 15; }
+    __device__ __forceinline__ int pair_bin(int q) const { return j + 16 * q; }
+    __device__ __forceinline__ void fft(float2 (&v)[16]) { fft256w::fft256<-1>(v, xbuf, j, tw); }
+    __device__ __forceinline__ void post_forward(float2 (&)[16]) {}
+    __device__ __forceinline__ void pre_inverse(float2 (&)[16]) {}
+    __device__ __forceinline__ void fetch_mirror(const float2 (&v)[16], float2 (&zm)[8], int lane) const { fft256w::fetch_mirror(v, lane, zm); }
+    __device__ __forceinline__ void scatter_mirror(const float2 (&ca)[8], const float2 (&cb)[8], float2 cmid, float2 (&v)[16]) const {
+        fft256w::scatter_mirror(ca, cb, cmid, ln, v);
+    }
+};
+
 template <> struct Core<Geo1024> {
     float2 tw[15], tc[8], twn[8];
     float2* xbuf;
@@ -116,7 +143,7 @@ template <> struct Core<Geo1024> {
     static __device__ __forceinline__ int group_of(int) { return 0; }
     static __device__ __forceinline__ int lane_in_group(int lane) { return lane; }
     __device__ __forceinline__ int pair_bin(int q) const { return j + 16 * (q + 8 * h); }
-    __device__ __forceinline__ void fft(float2 (&v)[16]) { fft256w::fft256<-1>(v, xbuf, j, tw, kFull); }
+    __device__ __forceinline__ void fft(float2 (&v)[16]) { fft256w::fft256<-1>(v, xbuf, j, tw); }
     // decimation in time: Z[k] = E[k] + W^k O[k], Z[k + 256] = E[k] - W^k O[k]; half h keeps k = j + 16 (q + 8 h)
     __device__ __forceinline__ void post_forward(float2 (&v)[16]) {
 #pragma unroll
@@ -224,7 +251,8 @@ template <class Geo> struct Sz {
     static constexpr int TAB_BYTES = (2 * M * 8 + 127) / 128 * 128; // s_win2 | s_bw2
 };
 // position of bin k in the staged mask row.  Geo1024: the two halves of a warp read bins 128 apart in the same instruction, so
-// every 128 bins are skewed by 16 floats (16 banks); Geo400: plain.
+// every 128 bins are skewed by 16 floats (16 banks); Geo400: plain; Geo512: plain, each group reads 16 consecutive bins of its
+// own row, and the two rows of a warp sit 16 banks apart (K3Sz::GSTRIDE).
 template <class Geo> __device__ __forceinline__ int mpos(int k) { return Geo::G == 32 ? k + ((k >> 7) << 4) : k; }
 
 // stage one block of Bs floats starting at original coordinate t0 (reflect outside [0, T)); jg = lane in group
@@ -288,6 +316,19 @@ __device__ __forceinline__ float edge_scale(const float* __restrict__ w, int t, 
     return ei / ee;
 }
 
+// se_set_trace: one TraceScope record per CTA (kernel id 1 = K1, 3 = K3), from the TRACE instantiations that the launchers
+// pick when a trace buffer is set, so that the kernels without it are unchanged.  Thread 0 parks the start time in the last 8
+// bytes of the dynamic shared memory: a register would stay live across the frame loops.
+__device__ __forceinline__ void trace_begin(unsigned char* smem_end) {
+    if (threadIdx.x == 0) reinterpret_cast<unsigned long long*>(smem_end)[-1] = secommon::TraceScope::now();
+}
+__device__ __forceinline__ void trace_end(unsigned long long* buf, int kernel_id, const unsigned char* smem_end) {
+    __syncthreads();
+    secommon::TraceScope trace(buf, kernel_id);
+    trace.t0 = reinterpret_cast<const unsigned long long*>(smem_end)[-1];
+    trace.finish();
+}
+
 struct GeoRunPlan { int per_utt; int runs_per_utt; long long total_runs; };      // per_utt frames (K1) / emit windows (K3)
 // run ri of `rpu` over `n` items: n / rpu each, the first n % rpu runs one more
 __device__ __forceinline__ void run_range(int ri, int n, int rpu, int& first, int& len) {
@@ -298,6 +339,9 @@ __device__ __forceinline__ void run_range(int ri, int n, int rpu, int& first, in
 
 // ------------------------------------------------------------------ K1
 template <class Geo> struct K1Cfg;
+// Geo512: small CTAs (2 warps, four per SM at up to 255 registers per thread): with two steps in flight the other step's
+// kernels get SMs back in finer grains (8-warp CTAs: +1.4 us per step at 64 x 4 s, round 2)
+template <> struct K1Cfg<Geo512>  { static constexpr int WARPS = 2, MIN_BLOCKS = 4; };
 template <> struct K1Cfg<Geo1024> { static constexpr int WARPS = 4, MIN_BLOCKS = 2; };
 template <> struct K1Cfg<Geo400>  { static constexpr int WARPS = 4, MIN_BLOCKS = 2; };
 template <class Geo> struct K1Sz {
@@ -306,7 +350,7 @@ template <class Geo> struct K1Sz {
     static constexpr int GSTRIDE = (GROUP_BYTES + 127) / 128 * 128 + (Geo::G == 10 ? 80 : 0);   // ... + 80 -> conflict-free column reads)
     static constexpr int WARP_BYTES = (Geo::GPW + Geo::IDLE) * GSTRIDE;
     static constexpr int GROUPS = K1Cfg<Geo>::WARPS * Geo::GPW;
-    static constexpr size_t SMEM = Sz<Geo>::TAB_BYTES + (size_t)K1Cfg<Geo>::WARPS * WARP_BYTES + GROUPS * 4 + 16;
+    static constexpr size_t SMEM = Sz<Geo>::TAB_BYTES + (size_t)K1Cfg<Geo>::WARPS * WARP_BYTES + GROUPS * 4 + 16;   // + trace start
 };
 
 // x[r] = raw samples (2m, 2m+1), m = tidx + G r, of the frame starting at original coordinate t0
@@ -329,9 +373,10 @@ __device__ __forceinline__ void load_frame(float2 (&x)[Geo::V], const float* __r
     }
 }
 
-template <class Geo, bool PHASE, bool STATS>
+template <class Geo, bool PHASE, bool STATS, bool TRACE>
 __global__ void __launch_bounds__(K1Cfg<Geo>::WARPS * 32, K1Cfg<Geo>::MIN_BLOCKS) stft_run_kernel(StftArgs a, GeoRunPlan plan) {
     extern __shared__ __align__(128) unsigned char smem[];
+    if (TRACE) trace_begin(smem + K1Sz<Geo>::SMEM);
     using S = Sz<Geo>;
     constexpr int M = S::M, H = S::H, G = S::G, V = S::V, NP = S::NP, N = S::N;
     constexpr int WARPS = K1Cfg<Geo>::WARPS, THREADS = WARPS * 32, GROUPS = K1Sz<Geo>::GROUPS;
@@ -456,12 +501,19 @@ __global__ void __launch_bounds__(K1Cfg<Geo>::WARPS * 32, K1Cfg<Geo>::MIN_BLOCKS
             }
         }
     }
+    if (TRACE) trace_end(a.trace, 1, smem + K1Sz<Geo>::SMEM);
 }
 
 // ------------------------------------------------------------------ K3
 template <class Geo> struct K3Cfg;
 // warps per CTA / CTAs per SM the register cap is set for (8 resident warps per SM either way; the occupancy sweeps of round 2
 // -- 12 warps at a 168-register cap lose 30 % to spills -- are in DESIGN.md 4.2)
+#ifndef SE_GEO512_K3_WARPS
+#define SE_GEO512_K3_WARPS 4
+#endif
+#ifndef SE_GEO512_K3_MINB
+#define SE_GEO512_K3_MINB 2
+#endif
 #ifndef SE_GEO1024_K3_WARPS
 #define SE_GEO1024_K3_WARPS 4
 #endif
@@ -474,22 +526,25 @@ template <class Geo> struct K3Cfg;
 #ifndef SE_GEO400_K3_MINB
 #define SE_GEO400_K3_MINB 1
 #endif
+template <> struct K3Cfg<Geo512>  { static constexpr int WARPS = SE_GEO512_K3_WARPS, MIN_BLOCKS = SE_GEO512_K3_MINB; };
 template <> struct K3Cfg<Geo1024> { static constexpr int WARPS = SE_GEO1024_K3_WARPS, MIN_BLOCKS = SE_GEO1024_K3_MINB; };
 template <> struct K3Cfg<Geo400>  { static constexpr int WARPS = SE_GEO400_K3_WARPS, MIN_BLOCKS = SE_GEO400_K3_MINB; };
 template <class Geo> struct K3Sz {
     using S = Sz<Geo>;
     static constexpr int RING_BYTES = S::RB * S::Bs * 4;
     static constexpr int GROUP_BYTES = Geo::XBUF + 2 * RING_BYTES + S::MROW * 4;
-    static constexpr int GSTRIDE = (GROUP_BYTES + 127) / 128 * 128 + (Geo::G == 10 ? 80 : 0);
+    // Geo400: + 80 -> conflict-free column reads; Geo512: + 64 -> the two groups' mask rows 16 banks apart
+    static constexpr int GSTRIDE = (GROUP_BYTES + 127) / 128 * 128 + (Geo::G == 10 ? 80 : Geo::G == 16 ? 64 : 0);
     static constexpr int IDLE_BYTES = Geo::IDLE ? (Geo::XBUF + 127) / 128 * 128 : 0;      // idle lanes only need transpose scratch
     static constexpr int WARP_BYTES = Geo::GPW * GSTRIDE + IDLE_BYTES;
     static constexpr int GROUPS = K3Cfg<Geo>::WARPS * Geo::GPW;
-    static constexpr size_t SMEM = S::TAB_BYTES + (size_t)K3Cfg<Geo>::WARPS * WARP_BYTES + 16;
+    static constexpr size_t SMEM = S::TAB_BYTES + (size_t)K3Cfg<Geo>::WARPS * WARP_BYTES + 16;                 // + trace start
 };
 
-template <class Geo, bool PM>
+template <class Geo, bool PM, bool TRACE>
 __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS) mask_istft_run_kernel(MaskIstftArgs a, GeoRunPlan plan) {
     extern __shared__ __align__(128) unsigned char smem[];
+    if (TRACE) trace_begin(smem + K3Sz<Geo>::SMEM);
     using S = Sz<Geo>;
     constexpr int N = S::N, M = S::M, H = S::H, G = S::G, V = S::V, NP = S::NP, Bs = S::Bs, RB = S::RB, HS = S::HS;
     constexpr int WARPS = K3Cfg<Geo>::WARPS, THREADS = WARPS * 32, GROUPS = K3Sz<Geo>::GROUPS;
@@ -761,21 +816,29 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
             }
         }
     }
+    if (TRACE) trace_end(a.trace, 3, smem + K3Sz<Geo>::SMEM);
 }
 
 template <class Geo> long long resident_groups(int warps, int min_blocks) {
     return (long long)secommon::device_sms() * min_blocks * warps * Geo::GPW;
 }
 
-template <class Geo> int prepare_geo() {
+template <class Geo, bool TRACE> int prepare_geo() {
 #define SE_OPT(K, BYTES) SE_CUDA_CHECK(cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(BYTES)))
-    SE_OPT((stft_run_kernel<Geo, false, false>), K1Sz<Geo>::SMEM);
-    SE_OPT((stft_run_kernel<Geo, true, false>), K1Sz<Geo>::SMEM);
-    SE_OPT((stft_run_kernel<Geo, false, true>), K1Sz<Geo>::SMEM);
-    SE_OPT((mask_istft_run_kernel<Geo, false>), K3Sz<Geo>::SMEM);
-    SE_OPT((mask_istft_run_kernel<Geo, true>), K3Sz<Geo>::SMEM);
+    SE_OPT((stft_run_kernel<Geo, false, false, TRACE>), K1Sz<Geo>::SMEM);
+    SE_OPT((stft_run_kernel<Geo, true, false, TRACE>), K1Sz<Geo>::SMEM);
+    SE_OPT((stft_run_kernel<Geo, false, true, TRACE>), K1Sz<Geo>::SMEM);
+    SE_OPT((mask_istft_run_kernel<Geo, false, TRACE>), K3Sz<Geo>::SMEM);
+    SE_OPT((mask_istft_run_kernel<Geo, true, TRACE>), K3Sz<Geo>::SMEM);
 #undef SE_OPT
-    return SE_OK;
+    return TRACE ? SE_OK : prepare_geo<Geo, true>();
+}
+
+template <class Geo, bool PHASE, bool STATS> void launch_stft_kernel(const StftArgs& a, const GeoRunPlan& plan, unsigned grid, cudaStream_t st) {
+    constexpr int THREADS = K1Cfg<Geo>::WARPS * 32;
+    constexpr size_t SMEM = K1Sz<Geo>::SMEM;
+    if (a.trace) stft_run_kernel<Geo, PHASE, STATS, true><<<grid, THREADS, SMEM, st>>>(a, plan);
+    else stft_run_kernel<Geo, PHASE, STATS, false><<<grid, THREADS, SMEM, st>>>(a, plan);
 }
 
 template <class Geo> int launch_stft_geo(const StftArgs& a, cudaStream_t st) {
@@ -798,10 +861,9 @@ template <class Geo> int launch_stft_geo(const StftArgs& a, cudaStream_t st) {
     plan.total_runs = (long long)a.n_utt * rpu;
     const long long grid = (plan.total_runs + GROUPS - 1) / GROUPS;
     if (grid > 0x7fffffffLL) return secommon::fail(SE_ERR_BAD_ARG, "grid too large");
-    const size_t smem = K1Sz<Geo>::SMEM;
-    if (a.stat_sums) stft_run_kernel<Geo, false, true><<<(unsigned)grid, WARPS * 32, smem, st>>>(a, plan);
-    else if (a.phase) stft_run_kernel<Geo, true, false><<<(unsigned)grid, WARPS * 32, smem, st>>>(a, plan);
-    else stft_run_kernel<Geo, false, false><<<(unsigned)grid, WARPS * 32, smem, st>>>(a, plan);
+    if (a.stat_sums) launch_stft_kernel<Geo, false, true>(a, plan, (unsigned)grid, st);
+    else if (a.phase) launch_stft_kernel<Geo, true, false>(a, plan, (unsigned)grid, st);
+    else launch_stft_kernel<Geo, false, false>(a, plan, (unsigned)grid, st);
     return secommon::check_launch("stft_run_kernel");
 }
 
@@ -813,11 +875,8 @@ template <class Geo> int launch_mask_istft_geo(const MaskIstftArgs& a, cudaStrea
     // `halo` frames); large batches: runs of about 64 windows.
     const int per_utt = a.n_frames - 1 + S::NV - S::E_MIN + 1;
     const long long slots = resident_groups<Geo>(WARPS, K3Cfg<Geo>::MIN_BLOCKS);
-    static int forced = -1;
-    if (forced < 0) { const char* e = getenv("SE_B200_RUN_LEN"); forced = e ? atoi(e) : 0; }
     long long rpu;
-    if (forced > 0) rpu = (per_utt + forced - 1) / forced;
-    else if ((long long)a.n_utt * per_utt <= slots * 32) {
+    if ((long long)a.n_utt * per_utt <= slots * 32) {
         rpu = slots / a.n_utt;
         const long long cap = per_utt / (4 * S::HALO);
         if (rpu > cap) rpu = cap;
@@ -840,8 +899,10 @@ template <class Geo> int launch_mask_istft_geo(const MaskIstftArgs& a, cudaStrea
     attr[0].val.programmaticStreamSerializationAllowed = (secommon::pdl_mask() & 2) ? 1 : 0;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    if (a.mask_is_power) SE_CUDA_CHECK(cudaLaunchKernelEx(&cfg, mask_istft_run_kernel<Geo, true>, a, plan));
-    else SE_CUDA_CHECK(cudaLaunchKernelEx(&cfg, mask_istft_run_kernel<Geo, false>, a, plan));
+    void (*kernel)(MaskIstftArgs, GeoRunPlan) =
+        a.mask_is_power ? (a.trace ? mask_istft_run_kernel<Geo, true, true> : mask_istft_run_kernel<Geo, true, false>)
+                        : (a.trace ? mask_istft_run_kernel<Geo, false, true> : mask_istft_run_kernel<Geo, false, false>);
+    SE_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kernel, a, plan));
     return secommon::check_launch("mask_istft_run_kernel");
 }
 
@@ -849,20 +910,25 @@ template <class Geo> int launch_mask_istft_geo(const MaskIstftArgs& a, cudaStrea
 
 namespace sefast {
 
-bool geo_supported(int n_fft, int hop) { return (n_fft == 1024 && hop == 256) || (n_fft == 400 && hop == 160); }
+bool geo_supported(int n_fft, int hop) {
+    return (n_fft == 512 && hop == 256) || (n_fft == 1024 && hop == 256) || (n_fft == 400 && hop == 160);
+}
 
 int prepare_geo_kernels(int n_fft) {
-    if (n_fft == 1024) return prepare_geo<Geo1024>();
-    if (n_fft == 400) return prepare_geo<Geo400>();
+    if (n_fft == 512) return prepare_geo<Geo512, false>();
+    if (n_fft == 1024) return prepare_geo<Geo1024, false>();
+    if (n_fft == 400) return prepare_geo<Geo400, false>();
     return SE_OK;
 }
 
 int launch_stft_run(const StftArgs& a, int n_fft, cudaStream_t st) {
+    if (n_fft == 512) return launch_stft_geo<Geo512>(a, st);
     if (n_fft == 1024) return launch_stft_geo<Geo1024>(a, st);
     return launch_stft_geo<Geo400>(a, st);
 }
 
 int launch_mask_istft_run(const MaskIstftArgs& a, int n_fft, cudaStream_t st) {
+    if (n_fft == 512) return launch_mask_istft_geo<Geo512>(a, st);
     if (n_fft == 1024) return launch_mask_istft_geo<Geo1024>(a, st);
     return launch_mask_istft_geo<Geo400>(a, st);
 }

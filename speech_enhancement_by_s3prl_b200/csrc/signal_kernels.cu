@@ -13,10 +13,7 @@ using namespace sekern;
 using secommon::fail;
 
 namespace sefast {
-int prepare512();
-int launch_stft512(const StftArgs& a, cudaStream_t st);
-int launch_mask_istft512(const MaskIstftArgs& a, cudaStream_t st);
-// fastgeo.cu: n_fft 1024 / hop 256 and n_fft 400 / hop 160
+// fastgeo.cu: n_fft 512 / hop 256, n_fft 1024 / hop 256 and n_fft 400 / hop 160
 bool geo_supported(int n_fft, int hop);
 int prepare_geo_kernels(int n_fft);
 int launch_stft_run(const StftArgs& a, int n_fft, cudaStream_t st);
@@ -87,7 +84,7 @@ int get_tables(int n_fft, DeviceTables* out) {
         switch (n_fft) {
             case 256: rc = opt_in_smem<256>(); break;
             case 400: rc = opt_in_smem<400>(); if (rc == SE_OK) rc = sefast::prepare_geo_kernels(400); break;
-            case 512: rc = opt_in_smem<512>(); if (rc == SE_OK) rc = sefast::prepare512(); break;
+            case 512: rc = opt_in_smem<512>(); if (rc == SE_OK) rc = sefast::prepare_geo_kernels(512); break;
             case 1024: rc = opt_in_smem<1024>(); if (rc == SE_OK) rc = sefast::prepare_geo_kernels(1024); break;
             case 2048: rc = opt_in_smem<2048>(); break;
         }
@@ -199,7 +196,6 @@ int se_stft_strided(const float* wav, int64_t n_utt, int64_t utt_stride, int64_t
     a.tab.window = window; a.tab.twM = t.twM; a.tab.twN = t.twN;
     a.power = power; a.phase = phase; a.logp = logpower; a.log_eps = log_eps; a.spec_stride = spec_stride;
     cudaStream_t st = (cudaStream_t)stream;
-    if (n_fft == 512 && !g_force_generic) return sefast::launch_stft512(a, st);
     if (sefast::geo_supported(n_fft, hop) && !g_force_generic) return sefast::launch_stft_run(a, n_fft, st);
     SE_DISPATCH_NFFT(n_fft, launch_stft, a, st)
 }
@@ -224,8 +220,7 @@ static int stft_features_impl(const float* wav, int64_t n_utt, int64_t utt_strid
     if (rc != SE_OK) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     if (!(flags & SE_FLAG_SUMS_ZEROED)) SE_CUDA_CHECK(cudaMemsetAsync(stat_sums, 0, sizeof(double) * 2 * ld_stats * n_utt, st));
-    const bool geo = sefast::geo_supported(n_fft, hop);
-    if (((n_fft == 512 && hop == 256) || geo) && !g_force_generic) {
+    if (sefast::geo_supported(n_fft, hop) && !g_force_generic) {
         DeviceTables t;
         if ((rc = get_tables(n_fft, &t)) != SE_OK) return rc;
         StftArgs a{};
@@ -236,7 +231,7 @@ static int stft_features_impl(const float* wav, int64_t n_utt, int64_t utt_strid
         a.stat_sums = stat_sums; a.ld_stats = ld_stats;
         a.trace = secommon::trace_ptr();
         if (flags & SE_FLAG_WS_SELF_CLEAN) { a.zero_ptr = stat_sums + 2 * ld_stats * n_utt; a.zero_count = (long long)SE_NSUMS * n_utt; }
-        return geo ? sefast::launch_stft_run(a, n_fft, st) : sefast::launch_stft512(a, st);
+        return sefast::launch_stft_run(a, n_fft, st);
     }
     if (flags & SE_FLAG_WS_SELF_CLEAN)                      // no fast path for this geometry: the same contract by a memset
         SE_CUDA_CHECK(cudaMemsetAsync(stat_sums + 2 * ld_stats * n_utt, 0, sizeof(double) * SE_NSUMS * n_utt, st));
@@ -256,8 +251,7 @@ int se_stft_features2(const float* wav, int64_t n_utt, int64_t utt_stride, int64
     if (rc != SE_OK) return rc;
     cudaStream_t st = (cudaStream_t)stream;
     if (!(flags & SE_FLAG_SUMS_ZEROED)) SE_CUDA_CHECK(cudaMemsetAsync(stat_sums, 0, sizeof(double) * 2 * ld_stats * n_utt, st));
-    const bool geo = sefast::geo_supported(n_fft, hop);
-    if (((n_fft == 512 && hop == 256) || geo) && !g_force_generic) {
+    if (sefast::geo_supported(n_fft, hop) && !g_force_generic) {
         DeviceTables t;
         if ((rc = get_tables(n_fft, &t)) != SE_OK) return rc;
         StftArgs a{};
@@ -267,7 +261,7 @@ int se_stft_features2(const float* wav, int64_t n_utt, int64_t utt_stride, int64
         a.power = power; a.logp = logpower; a.log_eps = log_eps; a.spec_stride = spec_stride;
         a.stat_sums = stat_sums; a.ld_stats = ld_stats;
         a.trace = secommon::trace_ptr();
-        return geo ? sefast::launch_stft_run(a, n_fft, st) : sefast::launch_stft512(a, st);
+        return sefast::launch_stft_run(a, n_fft, st);
     }
     rc = se_stft_strided(wav, n_utt, utt_stride, T, n_fft, hop, window, log_eps, power, nullptr, logpower, spec_stride, stream);
     if (rc != SE_OK) return rc;
@@ -355,7 +349,6 @@ int se_mask_istft_ex(const float* noisy, const float* clean, int64_t utt_stride,
     const long long stat_doubles = 2LL * ((n_fft / 2 + 1 + 3) / 4 * 4) * n_utt;         // (n_utt, round4(K), 2) right before `sums`
     const bool self_clean = (flags & SE_FLAG_WS_SELF_CLEAN) && sums;
     if (self_clean) { a.zero_ptr = sums - stat_doubles; a.zero_count = stat_doubles; }
-    if (n_fft == 512 && hop == 256 && a.n_frames >= 2 && !g_force_generic) return sefast::launch_mask_istft512(a, st);
     if (sefast::geo_supported(n_fft, hop) && a.n_frames >= 6 && !g_force_generic) return sefast::launch_mask_istft_run(a, n_fft, st);
     if (self_clean) SE_CUDA_CHECK(cudaMemsetAsync(sums - stat_doubles, 0, sizeof(double) * stat_doubles, st));   // generic path: by a memset
     SE_DISPATCH_NFFT(n_fft, launch_mask_istft, a, st)

@@ -127,4 +127,4 @@ def test_launch_planning_is_host_logic():
     assert lib.se_head_grad_embeddings_sisdr_supported(44, 1001, 201, 201, 204, 204, 204, 204) == 1
     # one K1 launch for both channels exists for the register-resident geometries of fastgeo.cu only
     assert lib.se_stft_features_pair_supported(400, 160) == 1 and lib.se_stft_features_pair_supported(1024, 256) == 1
-    assert lib.se_stft_features_pair_supported(512, 256) == 0 and lib.se_stft_features_pair_supported(400, 200) == 0
+    assert lib.se_stft_features_pair_supported(512, 256) == 1 and lib.se_stft_features_pair_supported(400, 200) == 0

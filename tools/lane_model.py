@@ -1,5 +1,5 @@
 """Lane-level numpy model of the register-resident FFT cores and of the run / overlap-add logic of
-csrc/fastgeo.cu (the n_fft 1024 / hop 256 and n_fft 400 / hop 160 fast paths).
+csrc/fastgeo.cu (the n_fft 512 / hop 256, n_fft 1024 / hop 256 and n_fft 400 / hop 160 fast paths).
 
 Every array is indexed [lane][slot] exactly like the registers of a warp; shuffles are fancy indexing.
 The CUDA code is a transcription of these functions, so index maps (mirror fetch, scatter, radix-2
@@ -8,6 +8,83 @@ exchange, prime-factor DFT-20 / DFT-10, emit windows, edge envelopes) are checke
     python tools/lane_model.py
 """
 import numpy as np
+
+
+# ----------------------------------------------------------------------------- G16V16: 256-point complex FFT on 16 lanes
+def fft256_groups(v):
+    """fft256 of each 16-lane group of a warp: lane (g = L >> 4, j = L & 15) slot r holds z_g[j + 16 r] on entry and
+    Z_g[j + 16 q] in slot q on exit."""
+    out = np.zeros_like(v)
+    for g in range(2):
+        seq = v[16 * g:16 * g + 16].T.reshape(256)              # seq[j + 16 r] = v[16 g + j, r]
+        out[16 * g:16 * g + 16] = np.fft.fft(seq).reshape(16, 16).T
+    return out
+
+
+def fetch_mirror256(v):
+    """zm[lane][q] = Z_g[256 - k], k = j + 16 q, q < 8: one shuffle per value inside the lane's group."""
+    L = np.arange(32)
+    j = L & 15
+    src = (L & 16) | ((16 - j) & 15)
+    zm = np.zeros((32, 8), complex)
+    for q in range(8):
+        offer = np.where(j == 0, v[:, (16 - q) & 15], v[:, 15 - q])
+        zm[:, q] = offer[src]
+    return zm
+
+
+def scatter_mirror256(ca, cb, cmid):
+    """ca[lane][q] = C_g[k], cb[lane][q] = C_g[256 - k]; cmid[lane] = C_g[128] (read on lane j = 0).  -> v[lane][s] = C_g[j + 16 s]."""
+    L = np.arange(32)
+    j = L & 15
+    src = (L & 16) | ((16 - j) & 15)
+    rcv = cb[src]
+    v = np.zeros((32, 16), complex)
+    v[:, :8] = ca
+    for q in range(7):
+        v[:, 15 - q] = np.where(j == 0, rcv[:, q + 1], rcv[:, q])
+    v[:, 8] = np.where(j == 0, cmid, rcv[:, 7])
+    return v
+
+
+def check_512():
+    """Two 512-sample real frames, one per 16-lane group of a warp (Core<Geo512>)."""
+    rng = np.random.default_rng(2)
+    L = np.arange(32)
+    j, g = L & 15, L >> 4
+    x = rng.standard_normal((2, 512))
+    z = x[:, 0::2] + 1j * x[:, 1::2]
+    Z, X = np.fft.fft(z), np.fft.rfft(x)
+    v = np.zeros((32, 16), complex)
+    for r in range(16):
+        v[:, r] = z[g, j + 16 * r]
+    v = fft256_groups(v)
+    for q in range(16):
+        assert np.allclose(v[:, q], Z[g, j + 16 * q])
+    zm = fetch_mirror256(v)
+    ca = np.zeros((32, 8), complex)
+    cb = np.zeros((32, 8), complex)
+    for q in range(8):
+        k = j + 16 * q
+        assert np.allclose(zm[:, q], Z[g, (256 - k) % 256])
+        w = np.exp(-2j * np.pi * k / 512)
+        e = 0.5 * (v[:, q] + np.conj(zm[:, q]))
+        o = -0.5j * (v[:, q] - np.conj(zm[:, q]))
+        xa, xb = e + o * w, np.conj(e - o * w)
+        assert np.allclose(xa, X[g, k]) and np.allclose(xb, X[g, 256 - k])
+        e2 = 0.5 * (xa + np.conj(xb))                         # inverse merge: Zinv[k], Zinv[256 - k] from X[k], X[256 - k]
+        o2 = 0.5 * (xa - np.conj(xb)) * np.conj(w)
+        ca[:, q] = np.conj(e2 + 1j * o2)
+        cb[:, q] = e2 - 1j * o2
+    lead = j == 0                                             # bin 128 pairs with itself: leader slot 8, X[128] = conj(Z[128])
+    assert np.allclose(v[lead, 8], Z[g[lead], 128]) and np.allclose(np.conj(Z[:, 128]), X[:, 128])
+    c = scatter_mirror256(ca, cb, np.conj(v[:, 8]))
+    for s in range(16):
+        assert np.allclose(c[:, s], np.conj(Z[g, j + 16 * s])), s
+    y = fft256_groups(c)                                      # the forward transform used as the inverse
+    for p in range(16):
+        assert np.allclose(np.conj(y[:, p]) / 256, z[g, j + 16 * p])
+    print("512 core (16-lane groups: forward, mirror fetch, scatter, inverse): ok")
 
 
 # ----------------------------------------------------------------------------- G32V16: 512-point complex FFT on a warp
@@ -292,6 +369,7 @@ def check_ola():
 
 
 if __name__ == "__main__":
+    check_512()
     check_1024()
     check_400()
     check_ola()

@@ -1,4 +1,4 @@
-// The 256-point half-warp FFT of the fast paths in isolation (no global memory in the loop): time per transform against the
+// The 256-point 16-lane FFT of the fast paths in isolation (no global memory in the loop): time per transform against the
 // number of resident warps.  nvcc -arch=sm_100a -O3 -std=c++17 -I../../speech_enhancement_by_s3prl_b200/csrc -I../../include -o fft_loop fft_loop.cu
 #include <cstdio>
 #include <cuda_runtime.h>
@@ -8,8 +8,7 @@ constexpr int ITERS = 512;
 template <int MODE> __global__ void __launch_bounds__(128) k(const float2* twM, const float2* twN, float2* out, float seed) {
     extern __shared__ __align__(16) unsigned char smem[];
     const int lane = threadIdx.x & 31, j = lane & 15, hw = threadIdx.x >> 4;
-    float2* xbuf = reinterpret_cast<float2*>(smem) + hw * M;
-    const unsigned hmask = half_mask(lane);
+    float2* xbuf = reinterpret_cast<float2*>(smem) + hw * 256;
     float2 tw[15], twn[8];
     load_lane_constants(j, twM, twN, tw, twn);
     float2 v[16];
@@ -17,7 +16,7 @@ template <int MODE> __global__ void __launch_bounds__(128) k(const float2* twM, 
     for (int r = 0; r < 16; ++r) v[r] = make_float2(seed * (j + 16 * r), seed);
 #pragma unroll 1
     for (int it = 0; it < ITERS; ++it) {
-        if (MODE == 0) fft256<-1>(v, xbuf, j, tw, hmask);
+        if (MODE == 0) fft256<-1>(v, xbuf, j, tw);
         if (MODE == 1) { bfly16<-1>(v); bfly16<-1>(v); }                       // butterflies only (no transpose, no twiddles)
         if (MODE == 2) {                                                        // twiddles only
 #pragma unroll
@@ -27,10 +26,10 @@ template <int MODE> __global__ void __launch_bounds__(128) k(const float2* twM, 
             float4* row = reinterpret_cast<float4*>(xbuf) + j * 8;
 #pragma unroll
             for (int c = 0; c < 8; ++c) row[c ^ (j & 7)] = make_float4(v[2 * c].x, v[2 * c].y, v[2 * c + 1].x, v[2 * c + 1].y);
-            __syncwarp(hmask);
+            __syncwarp();
 #pragma unroll
             for (int r = 0; r < 16; ++r) v[r] = xbuf[r * 16 + ((((j >> 1) ^ (r & 7)) << 1) | (j & 1))];
-            __syncwarp(hmask);
+            __syncwarp();
         }
     }
     float2 s = make_float2(0.f, 0.f);
@@ -42,7 +41,7 @@ template <int MODE> void run(const char* name, const float2* twM, const float2* 
     int sms; cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, 0);
     int clk; cudaDeviceGetAttribute(&clk, cudaDevAttrClockRate, 0);
     float2* out; cudaMalloc(&out, 1024);
-    const size_t smem = 8 * M * 8 + (ctas_per_sm == 1 ? 120 : ctas_per_sm == 2 ? 90 : ctas_per_sm == 3 ? 52 : 30) * 1024;  // caps residency
+    const size_t smem = 8 * 256 * 8 + (ctas_per_sm == 1 ? 120 : ctas_per_sm == 2 ? 90 : ctas_per_sm == 3 ? 52 : 30) * 1024;  // caps residency
     cudaFuncSetAttribute(k<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
     k<MODE><<<sms * ctas_per_sm, 128, smem>>>(twM, twN, out, 1e-3f); cudaDeviceSynchronize();

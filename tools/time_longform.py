@@ -1,5 +1,5 @@
 """Long-form evaluation pass (BASELINE configs[3] at one GPU's share of 8: 128 utterances x 60 s, n_fft 1024 / hop 256):
-ms per pass and per-kernel times.  SE_B200_RUN_LEN forces the K3 run length (emit windows per run).
+ms per pass and per-kernel times.
 python tools/time_longform.py [B] [seconds] [n_freq win_ms hop_ms]"""
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -46,5 +46,5 @@ with torch.no_grad():
     k2 = timeit(lambda: ops.linear_head_tma(feats, K, wpad, head.linear.bias, head.activation, sums, head.eps))
     k3 = timeit(lambda: ops.mask_istft(wavs, 0, 1, mask, lengths, n_fft, hop, window, pad_to=T, mask_padded=True, out=wav, sums=s6))
     k4 = timeit(lambda: ops.finalize_metrics(s6, lengths, T, wav=wav))
-print(f"RUN_LEN={os.environ.get('SE_B200_RUN_LEN', 'auto')}  B {B} x {secs:g} s n_fft {n_fft}: {ms:.3f} ms/pass = {B * secs / ms * 1e3 / 1e6:.3f} M audio-s/s | "
+print(f"B {B} x {secs:g} s n_fft {n_fft}: {ms:.3f} ms/pass = {B * secs / ms * 1e3 / 1e6:.3f} M audio-s/s | "
       f"K1 {k1:.3f} K2 {k2:.3f} K3 {k3:.3f} K3' {k4:.3f} ms", flush=True)
