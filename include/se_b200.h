@@ -371,7 +371,9 @@ int se_adam_clip_step_mirror(float* const* params, float* const* grads, float* c
  *   stat_sums (NULL = no CMVN); tcgen05 TF32 (W is read as TF32: pass it pre-rounded for round-to-nearest).
  *   One CTA per <=128-row tile, TMA tensor-map loads, accumulators in tensor memory, bulk-store epilogue.
  *   Returns SE_ERR_UNSUPPORTED outside its shape range (se_linear_head_fused_supported(...) == 0):
- *   D_in <= 288, D_out <= 272, n_frames >= 8, ldx and ldw multiples of 4, 16-byte aligned x and W. */
+ *   D_in <= 544, D_out <= 544 (more than 272 output columns run as column slabs), n_frames >= 8, ldx and ldw multiples of 4,
+ *   16-byte aligned x and W, and for D_out <= 272 a 128-row staging tile of ld_out (ld_out == round4(D_out)) or round4(D_out) + 4
+ *   floats per row that fits the 200 KB ring. */
 int se_stft_features(const float* wav, int64_t n_utt, int64_t utt_stride, int64_t T, int n_fft, int hop, const float* window,
                      float log_eps, int take_log, float* feat, int64_t feat_stride, double* stat_sums, int64_t ld_stats,
                      int flags, void* stream);
@@ -400,8 +402,9 @@ int se_stft_features_pair(const float* wav, int64_t n_utt, int64_t utt_stride, i
                           int64_t ld_stats, int flags, void* stream);
 
 /* Tensor-core form of se_linear_head_bwd (tcgen05 TF32 split-K GEMM; grad_b from a ones column of the same GEMM).
- * ws_partials: caller workspace of se_linear_head_bwd_tc_workspace(...) floats (0 = shape unsupported: D_in <= 271, n_frames >= 32
- * and a split of the rows may touch at most 4 utterances); ldx / ld_off = floats between rows of x / of offset and grad_offset. */
+ * ws_partials: caller workspace of se_linear_head_bwd_tc_workspace(...) floats (0 = shape unsupported: D_in <= 271 and
+ * n_frames >= 32).  A split of the rows touches at most 8 utterances: large batches of short utterances get shorter splits, and
+ * then more of them than one wave of CTAs.  ldx / ld_off = floats between rows of x / of offset and grad_offset. */
 int64_t se_linear_head_bwd_tc_workspace(int64_t n_utt, int64_t n_frames, int64_t D_in, int64_t D_out);
 int se_linear_head_bwd_tc(const float* x, int64_t ldx, const float* mean, const float* std, int64_t ld_stats, float cmvn_eps,
                           const float* offset, const float* grad_offset, int64_t ld_off, int64_t n_utt, int64_t n_frames,

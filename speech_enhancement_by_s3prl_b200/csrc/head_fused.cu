@@ -311,7 +311,14 @@ linear_head_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
         for (int kb = 0; kb < a.kblocks; ++kb) {
             const int s = kb % kStages;
             float4 wx = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (has_extra && kb * BK + 4 * cx + 4 <= (int)a.ldw) wx = __ldg(reinterpret_cast<const float4*>(a.w_extra + kb * BK + 4 * cx));
+            const int kx = kb * BK + 4 * cx;
+            if (has_extra && kx + 4 <= (int)a.ldw) wx = __ldg(reinterpret_cast<const float4*>(a.w_extra + kx));
+            if (kx + 4 > a.Din) {                                         // the weight row's padding past D_in may hold NaN (NaN * 0 = NaN)
+                wx.x = kx < a.Din ? wx.x : 0.f;
+                wx.y = kx + 1 < a.Din ? wx.y : 0.f;
+                wx.z = kx + 2 < a.Din ? wx.z : 0.f;
+                wx.w = 0.f;
+            }
             mbar_wait(bar_full + 8 * s, (kb / kStages) & 1);
             if (t == 0 && kb == 0) trace.mark(13);
             float4* tile = reinterpret_cast<float4*>(smem + kOffRing + s * kStageBytes);

@@ -1162,7 +1162,8 @@ def test_tensor_core_head_backward_matches_torch(se, B, F, Din, Dout, act, cmvn)
                                                    (2, 33, 256, 256, "Sigmoid", True), (7, 95, 201, 128, "Sigmoid", True)])
 def test_tma_head_backward_on_padded_operands_matches_torch(se, B, F, Din, Dout, act, cmvn):
     """se_linear_head_bwd_fused on the engine's row-padded tensors (16-byte rows: the TMA / MN-major tcgen05 kernel; NaN in the
-    padding columns must not leak) against torch in float64 -- including batches that need more splits than one wave of CTAs."""
+    padding columns must not leak) against torch in float64.  Batches that need more splits than one wave of CTAs are in
+    tests/test_head_gemm_f64.py."""
     from speech_enhancement_by_s3prl_b200 import ops
     assert ops.linear_head_bwd_fused_supported(B, F, Din, Dout)
     g = torch.Generator().manual_seed(Din + F + B)
