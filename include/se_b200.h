@@ -201,6 +201,31 @@ int se_wsd_mask_step(const float* offset, int64_t ld_off, const float* linear_in
                      float eps, const float* energy, const float* max_energy, double* sums2, int sums_zeroed, float* loss_per_utt,
                      float* loss_mean, float* grad_offset, int64_t ld_g, void* stream);
 
+/* ---- the evaluation step with objective.WSD (objective.py:127-153; runner.py:575 `criterion(**locals())`) ---------------------
+ * se_mask_istft_wsd: se_mask_istft_ex (same waveform output and SE_SUM_YC / SE_SUM_CC / SE_SUM_YY sums; clean and sums
+ *   required) that computes, instead of the spectral SI-SDR sums, the WSD terms of mask G = `mask`, X = |STFT(noisy)|^2 and
+ *   S = |STFT(clean)|^2 without materialising any spectrum:
+ *     frame_terms (n_utt, n_frames) float2 = {E_f = sum_k S over EVERY frame of the padded batch,
+ *                                             D_f = sum_k (S - G S)^2 on frames f < lengths[u] // hop + 1, else 0};
+ *     sums[u * SE_NSUMS + SE_SUM_SPEC_ST] += sum over valid frames of (G max(X - S, 0))^2;
+ *     wsd_state[0] (a float32 that rests at 0.0f) = max(itself, largest E_f), so that torch.distributed.all_reduce(op=MAX) of that
+ *     1-element buffer gives the maximum of the global batch.  wsd_state is 2 x 32 bits, zeroed once by the caller;
+ *     se_wsd_eval_finish puts it back to zero.
+ *   flags: SE_FLAG_SUMS_ZEROED and SE_FLAG_WS_SELF_CLEAN as in se_mask_istft_ex.  Register-resident geometries only
+ *   (se_mask_istft_wsd_supported, and T / hop + 1 >= 6 frames); otherwise SE_ERR_UNSUPPORTED: use se_wsd_energy and
+ *   se_wsd_mask_step on the spectra.
+ * se_wsd_eval_finish: after any all-reduce of wsd_state[0]: voiced[u, f] = 10 log10(E_f + eps) > 10 log10(wsd_state[0] + eps)
+ *   - db_interval; loss_per_utt[u] = alpha sum_f voiced D_f (double, fixed order) + (1 - alpha) sums[u, SE_SUM_SPEC_ST]; the batch
+ *   mean of loss_per_utt is objective.WSD's value.  metric_acc (or NULL) [0] += sum_u loss_per_utt; pair it with
+ *   se_finalize_metrics_acc(loss_spec = NULL), which adds the SI-SDR sum and the count. */
+int se_mask_istft_wsd_supported(int n_fft, int hop);
+int se_mask_istft_wsd(const float* noisy, const float* clean, int64_t utt_stride, const float* mask, int64_t mask_stride,
+                      const int64_t* lengths, int64_t n_utt, int64_t T, int n_fft, int hop, const float* window,
+                      float* wav_out, int64_t out_stride, int64_t pad_to, double* sums, float* frame_terms, float* wsd_state,
+                      int flags, void* stream);
+int se_wsd_eval_finish(const float* frame_terms, const double* sums, int64_t n_utt, int64_t n_frames, float alpha, float db_interval,
+                       float eps, float* wsd_state, float* loss_per_utt, double* metric_acc, void* stream);
+
 /* ---- K4c: batched waveform SI-SDR (evaluation.py:5-10 over runner.py:587-602) -----
  * sisdr[u] = sisdr_eval(src[u, :len[u]], tar[u, :len[u]]).  ws_sums3: caller workspace of
  * n_utt x 3 doubles (overwritten: <s,t>, <t,t>, <s,s>). */

@@ -68,6 +68,9 @@ _SIGNATURES = {
     "se_wsd_energy": [c_f, i64, i64, i64, i64, c_f, c_f, c_f],
     "se_wsd_mask_step": [c_f, i64, c_f, i64, c_f, i64, c_f, i64, i64, i64, i64, c_float, c_float, c_float, c_f, c_f, c_f, c_int, c_f, c_f,
                          c_f, i64, c_f],
+    "se_mask_istft_wsd_supported": [c_int, c_int],
+    "se_mask_istft_wsd": [c_f, c_f, i64, c_f, i64, c_f, i64, i64, c_int, c_int, c_f, c_f, i64, i64, c_f, c_f, c_f, c_int, c_f],
+    "se_wsd_eval_finish": [c_f, c_f, i64, i64, c_float, c_float, c_float, c_f, c_f, c_f, c_f],
     "se_linear_head_bwd_wsd_supported": [i64, i64, i64, i64, i64, i64, i64, i64],
     "se_linear_head_bwd_wsd": [c_f, i64, c_f, i64, c_float, c_f, i64, c_f, i64, c_f, i64, c_f, i64, c_f, c_f, c_float, c_float, c_float, i64,
                                i64, i64, i64, c_int, c_f, i64, c_f, c_f, c_f],

@@ -70,12 +70,14 @@ template <bool PM> __device__ __forceinline__ float2 apply_gain(float2 x, float 
     const float p = x.x * x.x + x.y * x.y;
     return p > 0.0f ? cscale(x, fast_sqrt(g) * rsqrtf(p)) : make_float2(fast_sqrt(g), 0.0f);
 }
-template <bool PM>
+// RELU = false (the WSD variant of K3): ra / rb keep the signed mask * |X|^2
+template <bool PM, bool RELU = true>
 __device__ __forceinline__ void mask_merge(float2 xa, float2 xb, float ga, float gb, float2 w, bool own, float& ra, float& rb,
                                            float2& ca, float2& cb) {
     if (own) {
-        ra = fmaxf(PM ? ga : ga * (xa.x * xa.x + xa.y * xa.y), 0.0f);
-        rb = fmaxf(PM ? gb : gb * (xb.x * xb.x + xb.y * xb.y), 0.0f);
+        ra = PM ? ga : ga * (xa.x * xa.x + xa.y * xa.y);
+        rb = PM ? gb : gb * (xb.x * xb.x + xb.y * xb.y);
+        if (RELU) { ra = fmaxf(ra, 0.0f); rb = fmaxf(rb, 0.0f); }
     }
     merge_pair_conj(apply_gain<PM>(xa, ga), apply_gain<PM>(xb, gb), w, ca, cb);
 }

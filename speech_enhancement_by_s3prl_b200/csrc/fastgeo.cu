@@ -529,10 +529,11 @@ template <class Geo> struct K3Cfg;
 template <> struct K3Cfg<Geo512>  { static constexpr int WARPS = SE_GEO512_K3_WARPS, MIN_BLOCKS = SE_GEO512_K3_MINB; };
 template <> struct K3Cfg<Geo1024> { static constexpr int WARPS = SE_GEO1024_K3_WARPS, MIN_BLOCKS = SE_GEO1024_K3_MINB; };
 template <> struct K3Cfg<Geo400>  { static constexpr int WARPS = SE_GEO400_K3_WARPS, MIN_BLOCKS = SE_GEO400_K3_MINB; };
-template <class Geo> struct K3Sz {
+// MB: staged mask rows per group (2 in the WSD variant, which reads frame f's row again in pass 2 while f + 1's is in flight)
+template <class Geo, int MB = 1> struct K3Sz {
     using S = Sz<Geo>;
     static constexpr int RING_BYTES = S::RB * S::Bs * 4;
-    static constexpr int GROUP_BYTES = Geo::XBUF + 2 * RING_BYTES + S::MROW * 4;
+    static constexpr int GROUP_BYTES = Geo::XBUF + 2 * RING_BYTES + MB * S::MROW * 4;
     // Geo400: + 80 -> conflict-free column reads; Geo512: + 64 -> the two groups' mask rows 16 banks apart
     static constexpr int GSTRIDE = (GROUP_BYTES + 127) / 128 * 128 + (Geo::G == 10 ? 80 : Geo::G == 16 ? 64 : 0);
     static constexpr int IDLE_BYTES = Geo::IDLE ? (Geo::XBUF + 127) / 128 * 128 : 0;      // idle lanes only need transpose scratch
@@ -541,24 +542,46 @@ template <class Geo> struct K3Sz {
     static constexpr size_t SMEM = S::TAB_BYTES + (size_t)K3Cfg<Geo>::WARPS * WARP_BYTES + 16;                 // + trace start
 };
 
-template <class Geo, bool PM, bool TRACE>
+// sum of v over the lane group (every lane of the group gets it; all 32 lanes must call).  Geo400's groups of 10 lanes: pairs
+// (j, j + 5), then the five pair sums, which lanes j and j + 5 both hold.
+template <class Geo> __device__ __forceinline__ float2 group_sum(float2 v, int lane, int jg, bool active) {
+    if constexpr (Geo::G == 10) {
+        const int base = lane - jg;
+        auto at = [&](int d) { return active ? base + (jg + d) % 10 : lane; };
+        const float2 p = cadd(v, shfl2(v, at(5)));
+        float2 s = cadd(p, shfl2(p, at(1)));
+        s = cadd(s, shfl2(s, at(2)));
+        return cadd(s, shfl2(p, at(4)));
+    } else {
+#pragma unroll
+        for (int o = Geo::G / 2; o > 0; o >>= 1) v = cadd(v, shfl2_xor(v, o));
+        return v;
+    }
+}
+
+// WSD: the variant of K3 for objective.WSD (objective.py:127-153).  Pass 2 runs for every real frame the run owns (frames past an
+// utterance's valid length included: the reference does not mask the energies) and writes per frame {E_f = sum_k S,
+// D_f = sum_k (S - G S)^2 (0 past the valid length)} to a.wsd_terms; sum_k (G max(X - S, 0))^2 over valid frames goes to the
+// SE_SUM_SPEC_ST slot of the sums, and the run's largest E_f to *a.wsd_max (float bits, atomicMax: energies are >= 0).
+template <class Geo, bool PM, bool TRACE, bool WSD = false>
 __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS) mask_istft_run_kernel(MaskIstftArgs a, GeoRunPlan plan) {
+    using Z = K3Sz<Geo, WSD ? 2 : 1>;
     extern __shared__ __align__(128) unsigned char smem[];
-    if (TRACE) trace_begin(smem + K3Sz<Geo>::SMEM);
+    if (TRACE) trace_begin(smem + Z::SMEM);
     using S = Sz<Geo>;
     constexpr int N = S::N, M = S::M, H = S::H, G = S::G, V = S::V, NP = S::NP, Bs = S::Bs, RB = S::RB, HS = S::HS;
-    constexpr int WARPS = K3Cfg<Geo>::WARPS, THREADS = WARPS * 32, GROUPS = K3Sz<Geo>::GROUPS;
+    constexpr int WARPS = K3Cfg<Geo>::WARPS, THREADS = WARPS * 32, GROUPS = Z::GROUPS;
     float2* s_win2 = reinterpret_cast<float2*>(smem);
     float2* s_bw2 = s_win2 + M;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int grp = Core<Geo>::group_of(lane), jg = Core<Geo>::lane_in_group(lane);
-    unsigned char* region = smem + S::TAB_BYTES + (size_t)warp * K3Sz<Geo>::WARP_BYTES + (size_t)grp * K3Sz<Geo>::GSTRIDE;
+    unsigned char* region = smem + S::TAB_BYTES + (size_t)warp * Z::WARP_BYTES + (size_t)grp * Z::GSTRIDE;
     // idle lanes (Geo400: 30, 31) execute every load of the frame loop too: they read the last real group's staging
     // (same addresses as its lanes 0, 1: a broadcast) and own only scratch for the transposes
     const int dgrp = grp < Geo::GPW ? grp : Geo::GPW - 1;
-    float* nring = reinterpret_cast<float*>(smem + S::TAB_BYTES + (size_t)warp * K3Sz<Geo>::WARP_BYTES + (size_t)dgrp * K3Sz<Geo>::GSTRIDE + Geo::XBUF);
+    float* nring = reinterpret_cast<float*>(smem + S::TAB_BYTES + (size_t)warp * Z::WARP_BYTES + (size_t)dgrp * Z::GSTRIDE + Geo::XBUF);
     float* cring = nring + RB * Bs;
-    float* mb = cring + RB * Bs;
+    float* mb = cring + RB * Bs;                                                    // WSD: two rows, frame f_first + it in row (it & 1)
     const bool lane_active = grp < Geo::GPW;
     const long long unit = (long long)blockIdx.x * GROUPS + warp * Geo::GPW + grp;
     const bool active = lane_active && unit < plan.total_runs;
@@ -614,7 +637,8 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
     float2 carry[V - HS];
 #pragma unroll
     for (int i = 0; i < V - HS; ++i) carry[i] = make_float2(0.0f, 0.0f);
-    float2 yy2 = make_float2(0.0f, 0.0f), yc2 = yy2, cc2 = yy2, st2 = yy2, tt2 = yy2, ss2 = yy2;
+    float2 yy2 = make_float2(0.0f, 0.0f), yc2 = yy2, cc2 = yy2, st2 = yy2, tt2 = yy2, ss2 = yy2;   // WSD: st2 = residual noise
+    float wmax = 0.0f;                                                              // WSD: largest frame energy of the run
 
     griddep_wait();                                                                 // the mask (and the zeroed sums) come from upstream kernels
     if (a.zero_ptr)                                                                 // SE_FLAG_WS_SELF_CLEAN: the CMVN sums the head has consumed
@@ -635,7 +659,10 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
         const bool live = it < my_iters;
         const bool real = live && f <= F - 1;
         const bool emit = live && f >= e0;
-        const bool own = spec && real && f < valid_frames && (f >= e0 || ri == 0);
+        // WSD: own = every real frame of the run (energies), wval = the valid ones among them (loss terms)
+        const bool own = WSD ? need_clean && real && (f >= e0 || ri == 0) : spec && real && f < valid_frames && (f >= e0 || ri == 0);
+        const bool wval = WSD && own && f < valid_frames;
+        const int moff = WSD ? (it & 1) * S::MROW : 0;
         const bool next_real = it + 1 < my_iters && f + 1 <= F - 1;
         if (next_real) {                                                            // the hop of frame f + 1 -> the free ring slots
 #pragma unroll
@@ -677,15 +704,16 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
                     float2 xa, xb;
                     split_pair(v[q], zm[q], core.twn[q], xa, xb);
                     // (Geo1024: q >= 1 keeps k and M - k inside one 128-bin skew block per lane: constant offsets from mlo / mhi)
-                    const float ga = (Geo::G == 32 && q > 0) ? mlo[16 * q] : mb[mpos<Geo>(k)];
-                    const float gb = (Geo::G == 32 && q > 0) ? mhi[-16 * q] : mb[mpos<Geo>(M - k)];
-                    mask_merge<PM>(xa, xb, ga, gb, core.twn[q], own, ra[q], rb[q], ca[q], cbv[q]);
+                    const float ga = (Geo::G == 32 && q > 0) ? mlo[moff + 16 * q] : mb[moff + mpos<Geo>(k)];
+                    const float gb = (Geo::G == 32 && q > 0) ? mhi[moff - 16 * q] : mb[moff + mpos<Geo>(M - k)];
+                    mask_merge<PM, !WSD>(xa, xb, ga, gb, core.twn[q], WSD ? wval : own, ra[q], rb[q], ca[q], cbv[q]);
                 }
-                const float gmid = mb[mpos<Geo>(M / 2)];
+                const float gmid = mb[moff + mpos<Geo>(M / 2)];
                 const float2 xmid = make_float2(2.0f * v[V / 2].x, -2.0f * v[V / 2].y);   // bin M/2 pairs with itself: X = 2 conj(Z[M/2])
-                if (own) rmid = fmaxf(PM ? gmid : gmid * (xmid.x * xmid.x + xmid.y * xmid.y), 0.0f);
+                if (WSD) { if (wval) rmid = gmid * (xmid.x * xmid.x + xmid.y * xmid.y); }
+                else if (own) rmid = fmaxf(PM ? gmid : gmid * (xmid.x * xmid.x + xmid.y * xmid.y), 0.0f);
                 __syncwarp();
-                if (next_real) stage_mask_row<Geo>(mb, mrow0 + (long long)(f + 1) * a.mask_stride, mask_padded, jg);
+                if (next_real) stage_mask_row<Geo>(mb + (S::MROW - moff) * WSD, mrow0 + (long long)(f + 1) * a.mask_stride, mask_padded, jg);
                 cp_async_commit();                                                  // group M(f + 1)
                 mask_group_open = false;
                 float2 ymid;                                                        // 2 Y[M/2]: conj(Zinv[M/2]), same factor 2 as merge_pair_conj
@@ -748,6 +776,46 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
                             }
                         }
                     }
+                }
+            } else if (WSD) {
+                // S = clean power, G re-read from the frame's mask row, ra / rb = G X: d = G X - G S is G (X - S), so the
+                // residual-noise term (G max(X - S, 0))^2 is d^2 where G d > 0, for a mask of any sign
+                float2 zm[NP];
+                core.fetch_mirror(v, zm, lane);
+                float2 ed = make_float2(0.0f, 0.0f);                                // (E_f, D_f) parts of this lane
+                if (own) {
+#pragma unroll
+                    for (int q = 0; q < NP; ++q) {
+                        const int k = core.pair_bin(q);
+                        float2 xa, xb;
+                        split_pair(v[q], zm[q], core.twn[q], xa, xb);
+                        const float2 pt = make_float2(xa.x * xa.x + xa.y * xa.y, xb.x * xb.x + xb.y * xb.y);
+                        ed.x += pt.x + pt.y;
+                        if (wval) {
+                            const float ga = (Geo::G == 32 && q > 0) ? mlo[moff + 16 * q] : mb[moff + mpos<Geo>(k)];
+                            const float gb = (Geo::G == 32 && q > 0) ? mhi[moff - 16 * q] : mb[moff + mpos<Geo>(M - k)];
+                            const float sa = pt.x - ga * pt.x, sb = pt.y - gb * pt.y;
+                            ed.y += sa * sa + sb * sb;
+                            const float da = ra[q] - ga * pt.x, db = rb[q] - gb * pt.y;
+                            st2.x += ga * da > 0.0f ? da * da : 0.0f;
+                            st2.y += gb * db > 0.0f ? db * db : 0.0f;
+                        }
+                    }
+                    if (core.leader) {
+                        const float ptm = 4.0f * (v[V / 2].x * v[V / 2].x + v[V / 2].y * v[V / 2].y);
+                        ed.x += ptm;
+                        if (wval) {
+                            const float gmid = mb[moff + mpos<Geo>(M / 2)];
+                            const float sm = ptm - gmid * ptm, dm = rmid - gmid * ptm;
+                            ed.y += sm * sm;
+                            acc[sekern::SUM_SPEC_ST] += gmid * dm > 0.0f ? dm * dm : 0.0f;
+                        }
+                    }
+                }
+                ed = group_sum<Geo>(ed, lane, jg, core.active);
+                if (own && core.leader) {
+                    reinterpret_cast<float2*>(a.wsd_terms)[(long long)u * F + f] = ed;
+                    wmax = fmaxf(wmax, ed.x);
                 }
             } else {
                 float2 zm[NP];
@@ -816,7 +884,9 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
             }
         }
     }
-    if (TRACE) trace_end(a.trace, 3, smem + K3Sz<Geo>::SMEM);
+    // one atomic per run; the buffer rests at 0.0f, and non-negative floats order as their bit patterns
+    if (WSD && active && core.leader && wmax > 0.0f) atomicMax(reinterpret_cast<int*>(a.wsd_max), __float_as_int(wmax));
+    if (TRACE) trace_end(a.trace, 3, smem + Z::SMEM);
 }
 
 template <class Geo> long long resident_groups(int warps, int min_blocks) {
@@ -830,6 +900,7 @@ template <class Geo, bool TRACE> int prepare_geo() {
     SE_OPT((stft_run_kernel<Geo, false, true, TRACE>), K1Sz<Geo>::SMEM);
     SE_OPT((mask_istft_run_kernel<Geo, false, TRACE>), K3Sz<Geo>::SMEM);
     SE_OPT((mask_istft_run_kernel<Geo, true, TRACE>), K3Sz<Geo>::SMEM);
+    SE_OPT((mask_istft_run_kernel<Geo, false, TRACE, true>), (K3Sz<Geo, 2>::SMEM));
 #undef SE_OPT
     return TRACE ? SE_OK : prepare_geo<Geo, true>();
 }
@@ -892,7 +963,7 @@ template <class Geo> int launch_mask_istft_geo(const MaskIstftArgs& a, cudaStrea
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3((unsigned)grid);
     cfg.blockDim = dim3(WARPS * 32);
-    cfg.dynamicSmemBytes = K3Sz<Geo>::SMEM;
+    cfg.dynamicSmemBytes = a.wsd_terms ? K3Sz<Geo, 2>::SMEM : K3Sz<Geo>::SMEM;
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;       // prologue overlaps the upstream kernel's tail
@@ -900,8 +971,9 @@ template <class Geo> int launch_mask_istft_geo(const MaskIstftArgs& a, cudaStrea
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     void (*kernel)(MaskIstftArgs, GeoRunPlan) =
-        a.mask_is_power ? (a.trace ? mask_istft_run_kernel<Geo, true, true> : mask_istft_run_kernel<Geo, true, false>)
-                        : (a.trace ? mask_istft_run_kernel<Geo, false, true> : mask_istft_run_kernel<Geo, false, false>);
+        a.wsd_terms ? (a.trace ? mask_istft_run_kernel<Geo, false, true, true> : mask_istft_run_kernel<Geo, false, false, true>)
+        : a.mask_is_power ? (a.trace ? mask_istft_run_kernel<Geo, true, true> : mask_istft_run_kernel<Geo, true, false>)
+                          : (a.trace ? mask_istft_run_kernel<Geo, false, true> : mask_istft_run_kernel<Geo, false, false>);
     SE_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kernel, a, plan));
     return secommon::check_launch("mask_istft_run_kernel");
 }

@@ -583,6 +583,42 @@ __global__ void __launch_bounds__(256) wsd_finish_mean_kernel(const double* __re
     }
 }
 
+// the evaluation step's WSD terms (se_mask_istft_wsd) -> loss_per_utt; one CTA per utterance.  Every thread sums its own run of
+// consecutive frames, then a fixed reduction order: the result does not change from run to run.  The last CTA to finish puts the
+// maximum and the CTA counter back to 0 for the next step (a captured step then needs no fill node).
+__global__ void __launch_bounds__(256) wsd_eval_finish_kernel(const float2* __restrict__ terms, const double* __restrict__ sums,
+                                                              int n_frames, float alpha, float db_interval, float eps,
+                                                              float* wsd_state, float* __restrict__ loss, double* __restrict__ metric_acc) {
+    __shared__ double part[8];
+    const int u = blockIdx.x;
+    const float thres = 10.0f * log10f(__ldcg(wsd_state) + eps) - db_interval;     // after any all-reduce of wsd_state[0]
+    const float2* row = terms + (long long)u * n_frames;
+    const int per = (n_frames + blockDim.x - 1) / blockDim.x;
+    const int lo = threadIdx.x * per, hi = min(n_frames, lo + per);
+    double sd = 0.0;
+    for (int f = lo; f < hi; ++f) {
+        const float2 t = row[f];
+        if (10.0f * log10f(t.x + eps) > thres) sd += (double)t.y;
+    }
+    sd = secommon::warp_sum(sd);
+    if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = sd;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        sd = 0.0;
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) sd += part[w];
+        const double rn = sums[(long long)u * SE_NSUMS + SE_SUM_SPEC_ST];
+        const float l = (float)((double)alpha * sd + (1.0 - (double)alpha) * rn);
+        loss[u] = l;
+        if (metric_acc) atomicAdd(metric_acc, (double)l);
+        __threadfence();
+        unsigned* done = reinterpret_cast<unsigned*>(wsd_state + 1);
+        if (atomicAdd(done, 1u) == gridDim.x - 1) {                                  // every CTA has read the maximum
+            wsd_state[0] = 0.0f;
+            *done = 0u;
+        }
+    }
+}
+
 // d loss_mean / d offset (upstream gradient grad_uniform = 1 / B), whole rows of grad_offset: 0 on padded frames and pad columns
 template <int V>
 __global__ void __launch_bounds__(256) wsd_mask_bwd_kernel(const WsdMaskArgs a) {
@@ -1280,6 +1316,16 @@ int se_wsd_mask_step(const float* offset, int64_t ld_off, const float* linear_in
     if (v4) wsd_mask_bwd_kernel<4><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
     else wsd_mask_bwd_kernel<1><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
     return secommon::check_launch("wsd_mask_bwd_kernel");
+}
+
+int se_wsd_eval_finish(const float* frame_terms, const double* sums, int64_t n_utt, int64_t n_frames, float alpha, float db_interval,
+                       float eps, float* wsd_state, float* loss_per_utt, double* metric_acc, void* stream) {
+    SE_REQUIRE(frame_terms && sums && wsd_state && loss_per_utt && n_utt > 0 && n_frames > 0, "bad argument");
+    SE_REQUIRE(n_utt <= 0x7fffffffLL && n_frames <= 0x7fffffffLL, "too many utterances or frames");
+    wsd_eval_finish_kernel<<<(unsigned)n_utt, 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const float2*>(frame_terms), sums,
+                                                                              (int)n_frames, alpha, db_interval, eps, wsd_state,
+                                                                              loss_per_utt, metric_acc);
+    return secommon::check_launch("wsd_eval_finish_kernel");
 }
 
 int se_l1_logspec_fwd(const float* log_predicted, const float* linear_tar, const int64_t* stft_len, int64_t n_utt,

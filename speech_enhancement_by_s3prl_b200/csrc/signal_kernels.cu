@@ -354,6 +354,44 @@ int se_mask_istft_ex(const float* noisy, const float* clean, int64_t utt_stride,
     SE_DISPATCH_NFFT(n_fft, launch_mask_istft, a, st)
 }
 
+int se_mask_istft_wsd_supported(int n_fft, int hop) { return (sefast::geo_supported(n_fft, hop) && !g_force_generic) ? 1 : 0; }
+
+int se_mask_istft_wsd(const float* noisy, const float* clean, int64_t utt_stride, const float* mask, int64_t mask_stride,
+                      const int64_t* lengths, int64_t n_utt, int64_t T, int n_fft, int hop, const float* window,
+                      float* wav_out, int64_t out_stride, int64_t pad_to, double* sums, float* frame_terms, float* wsd_state,
+                      int flags, void* stream) {
+    SE_REQUIRE(noisy && clean && mask && window && wav_out && sums && frame_terms && wsd_state, "null pointer");
+    SE_REQUIRE(mask_stride >= n_fft / 2 + 1, "mask_stride=%lld smaller than K", (long long)mask_stride);
+    SE_REQUIRE((reinterpret_cast<uintptr_t>(frame_terms) & 7) == 0 && (reinterpret_cast<uintptr_t>(wsd_state) & 7) == 0,
+               "frame_terms / wsd_state must be 8-byte aligned");
+    SE_REQUIRE(!(flags & (SE_FLAG_WANT_SPEC | SE_FLAG_MASK_IS_POWER)), "se_mask_istft_wsd: flags may hold SE_FLAG_SUMS_ZEROED and "
+               "SE_FLAG_WS_SELF_CLEAN only");
+    int rc = check_geometry(n_utt, T, n_fft, hop);
+    if (rc != SE_OK) return rc;
+    if (!se_mask_istft_wsd_supported(n_fft, hop) || T / hop + 1 < 6)       // the frame count se_mask_istft_ex's fast path needs
+        return fail(SE_ERR_UNSUPPORTED, "se_mask_istft_wsd: n_fft=%d hop=%d T=%lld has no register-resident kernel (use se_wsd_energy "
+                    "and se_wsd_mask_step on the spectra)", n_fft, hop, (long long)T);
+    DeviceTables t;
+    if ((rc = get_tables(n_fft, &t)) != SE_OK) return rc;
+    MaskIstftArgs a{};
+    a.noisy = noisy; a.clean = clean; a.utt_stride = utt_stride; a.mask = mask;
+    a.lengths = reinterpret_cast<const long long*>(lengths);
+    a.n_utt = (int)n_utt; a.T = (int)T; a.hop = hop; a.n_frames = (int)(T / hop) + 1;
+    a.tab.window = window; a.tab.twM = t.twM; a.tab.twN = t.twN;
+    a.wav_out = wav_out; a.out_stride = out_stride; a.out_len = hop * (a.n_frames - 1); a.pad_to = (int)pad_to;
+    a.sums = sums; a.want_spec = 0; a.mask_stride = mask_stride;
+    a.wsd_terms = frame_terms; a.wsd_max = wsd_state;
+    a.trace = secommon::trace_ptr();
+    SE_REQUIRE(out_stride >= a.out_len && out_stride >= pad_to, "out_stride=%lld too small", (long long)out_stride);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!(flags & SE_FLAG_SUMS_ZEROED)) SE_CUDA_CHECK(cudaMemsetAsync(sums, 0, sizeof(double) * SE_NSUMS * n_utt, st));
+    if (flags & SE_FLAG_WS_SELF_CLEAN) {
+        a.zero_ptr = sums - 2LL * ((n_fft / 2 + 1 + 3) / 4 * 4) * n_utt;
+        a.zero_count = 2LL * ((n_fft / 2 + 1 + 3) / 4 * 4) * n_utt;
+    }
+    return sefast::launch_mask_istft_run(a, n_fft, st);
+}
+
 __global__ void __launch_bounds__(256) pcm16_to_float_kernel(const short4* __restrict__ src, float4* __restrict__ dst, long long n4,
                                                              const short* __restrict__ src1, float* __restrict__ dst1, long long n) {
     const long long stride = (long long)gridDim.x * blockDim.x;

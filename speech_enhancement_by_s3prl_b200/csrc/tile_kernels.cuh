@@ -85,6 +85,8 @@ struct MaskIstftArgs {
     double* zero_ptr;          // SE_FLAG_WS_SELF_CLEAN: doubles zeroed after the upstream kernel has completed (or null)
     long long zero_count;
     int mask_is_power;         // `mask` holds the TARGET power spectrum: output = iSTFT(sqrt(mask) e^{i phase(noisy)}) (runner.py:266-281)
+    float* wsd_terms;          // se_mask_istft_wsd (fastgeo.cu only): (n_utt, n_frames) float2 {E_f, D_f}, or null
+    float* wsd_max;            // idem: the batch's largest E_f (1 float, at rest 0.0f)
 };
 
 SE_HD int imin(int a, int b) { return a < b ? a : b; }

@@ -25,6 +25,24 @@ def _c64(lengths):
     return lengths if lengths.dtype == torch.int64 and lengths.is_contiguous() else lengths.to(torch.int64).contiguous()
 
 
+def _eval_wsd(criterion):
+    """The evaluation step's loss: False for None / objective.SISDR (spectral SI-SDR), True for objective.WSD."""
+    from . import objective as obj
+    if criterion is None or type(criterion) is obj.SISDR:
+        return False
+    if type(criterion) is obj.WSD:
+        return True
+    raise RuntimeError(f"EnhancementEngine: no evaluation route for the criterion {type(criterion).__name__} (supported: None, "
+                       "objective.SISDR, objective.WSD)")
+
+
+def _criterion_key(criterion):
+    """What a captured evaluation step bakes in of its criterion."""
+    if not _eval_wsd(criterion):
+        return None
+    return ("WSD", float(criterion.alpha), float(criterion.db_interval), float(criterion.eps))
+
+
 class EnhancementEngine:
     def __init__(self, preprocessor, head, log_features=True, precision=0, feat_cfg=None):
         """preprocessor: se_b200 OnlinePreprocessor (gives n_fft / hop / window, channel_inp/tar);
@@ -47,22 +65,33 @@ class EnhancementEngine:
         self.launches_per_step = 5          # library kernels per eval_step (set by eval_step: 4 on the fused path)
 
     # ------------------------------------------------------------------ device-resident step
-    def step_workspace(self, B, device):
-        """Persistent, zeroed workspace of one captured evaluation step: [CMVN sums (B, round4(K), 2) | K3 sums (B, 6)] doubles.
+    def step_workspace(self, B, device, criterion=None):
+        """Persistent, zeroed workspace of one captured evaluation step: [CMVN sums (B, round4(K), 2) | K3 sums (B, 6)] doubles,
+        + one double (the WSD maximum and the finish kernel's CTA counter) with an objective.WSD criterion.
         The step's kernels leave it zeroed for the next replay (SE_FLAG_WS_SELF_CLEAN), so the graph has no fill node."""
         LD = ops.round4(self.n_fft // 2 + 1)
-        return torch.zeros(B * (2 * LD + ops.NSUMS), device=device, dtype=torch.float64)
+        extra = 1 if _eval_wsd(criterion) else 0
+        return torch.zeros(B * (2 * LD + ops.NSUMS) + extra, device=device, dtype=torch.float64)
 
-    def eval_step(self, lengths, wavs, want_spec_loss=True, metric_acc=None, ws=None, want_stoi=False, stoi_acc=None):
+    def eval_step(self, lengths, wavs, want_spec_loss=True, metric_acc=None, ws=None, want_stoi=False, stoi_acc=None,
+                  criterion=None):
         """lengths (B,) int64, wavs (B, C, T) fp32, both on the GPU.
         Returns dict(loss_per_utt (B,), sisdr (B,), wav_predicted (B, T), gain (B,)); loss_per_utt is None when
-        want_spec_loss is False (the spectral SI-SDR sums are not computed then).
+        want_spec_loss is False (the loss terms are not computed then).
+        criterion: the objective the validation loss is reported in (runner.py:575): None or an objective.SISDR (the spectral
+        SI-SDR), or an objective.WSD (its alpha, db_interval and eps; the voicing threshold comes from the loudest frame of the
+        global batch, so under data parallelism every rank must run the step for every batch).  On the register-resident
+        geometries (n_fft / hop 512 / 256, 1024 / 256, 400 / 160) the WSD terms come out of K3 itself; on any other geometry
+        from both channels' power spectra through ops.wsd_energy / ops.wsd_mask_step -- a slower route that materialises them.
         metric_acc: float64 (3,) device tensor += [sum loss, sum SI-SDR, utterances] (the running sums of an evaluation
         pass, runner.py:587-602; ``dp.means_from_acc`` turns them into the global means with one all-reduce).  Without
         want_spec_loss the loss sum is left as it is; SI-SDR and the count are still added.
-        ws: a ``step_workspace`` that this call may use and must leave zeroed (captured steps); None = a fresh one per call.
+        ws: a ``step_workspace`` (of the same criterion) that this call may use and must leave zeroed (captured steps); None = a
+        fresh one per call.
         want_stoi: also return "stoi" and "estoi" (B,) of wav_predicted against the target channel, at the preprocessor's
         sample rate (``ops.stoi``); stoi_acc: float64 (3,) device tensor += [sum STOI, sum ESTOI, utterances]."""
+        wsd = _eval_wsd(criterion) and want_spec_loss
+        want_spec_loss = want_spec_loss and not wsd             # the spectral SI-SDR sums of K3
         B, C, T = wavs.shape
         dev = wavs.device
         window = self.pre._frame_window
@@ -92,8 +121,7 @@ class EnhancementEngine:
                                          order=int(cfg.get("delta", 0)), K=K)
                 stat_sums = ops.feature_sums(feats, D) if head.cmvn else None
                 mask = ops.linear_head_tma(feats, D, wpad, head.linear.bias, head.activation, stat_sums, head.eps)
-                wav, sums = ops.mask_istft(wavs, self.ch_inp, self.ch_tar, mask, lengths, self.n_fft, self.hop, window,
-                                           pad_to=T, want_sums=True, want_spec=want_spec_loss, mask_padded=True)
+                k3 = {}
             elif self.precision == 1 and ops.linear_head_tma_supported(B, F, K, Dout, LD, wpad.shape[1], ops.round4(Dout)):
                 # K1 (+ CMVN sums) -> K2 (TMA + tcgen05 head) -> K3 -> K3': one zeroed workspace, no other memset, so
                 # the four kernels are chained by programmatic dependent launches
@@ -102,30 +130,70 @@ class EnhancementEngine:
                 if ws is None:
                     ws = torch.zeros(B * (2 * LD + ops.NSUMS), device=dev, dtype=torch.float64)
                 stat_sums = ws[:B * 2 * LD].view(B, LD, 2)
-                sums = ws[B * 2 * LD:].view(B, ops.NSUMS)
+                sums = ws[B * 2 * LD:B * (2 * LD + ops.NSUMS)].view(B, ops.NSUMS)
                 feats, _ = ops.stft_features(wavs, self.ch_inp, self.n_fft, self.hop, window, logpower=self.log_features,
                                              log_eps=self.pre.eps, stat_sums=stat_sums, self_clean=self_clean)
                 mask = ops.linear_head_tma(feats, K, wpad, head.linear.bias, head.activation,
                                              stat_sums if head.cmvn else None, head.eps)
-                wav, sums = ops.mask_istft(wavs, self.ch_inp, self.ch_tar, mask, lengths, self.n_fft, self.hop, window,
-                                           pad_to=T, want_sums=True, want_spec=want_spec_loss, mask_padded=True, sums=sums,
-                                           sums_zeroed=True, self_clean=self_clean)
+                k3 = dict(sums=sums, sums_zeroed=True, self_clean=self_clean)
             else:
+                self.launches_per_step = 5      # K1, K2 (+ CMVN statistics), the sums' fill, K3, K3'
                 feats = ops.stft_padded(wavs, self.ch_inp, self.n_fft, self.hop, window, logpower=self.log_features, log_eps=self.pre.eps)
                 mean = std = None
                 if head.cmvn:
                     mean, std = ops.cmvn_stats_padded(feats, K)
                 mask = ops.linear_head_padded(feats, K, wpad, head.linear.bias, head.activation, mean, std,
                                               head.eps, precision=self.precision)
+                k3 = {}
+            if wsd and ops.mask_istft_wsd_supported(self.n_fft, self.hop) and F >= 6:
+                # K3 with the WSD terms -> all-reduce(max) of its 4-byte maximum on the side stream under K3' -> the finish kernel
+                self.launches_per_step += 1
+                if ws is not None and ws.numel() == B * (2 * LD + ops.NSUMS) + 1:
+                    state = ws[B * (2 * LD + ops.NSUMS):].view(torch.float32)    # the step leaves it zeroed
+                else:
+                    state = torch.zeros(2, device=dev, dtype=torch.float32)
+                wav, sums, terms = ops.mask_istft_wsd(wavs, self.ch_inp, self.ch_tar, mask, lengths, self.n_fft, self.hop, window,
+                                                      pad_to=T, wsd_state=state, **k3)
+                main = torch.cuda.current_stream(dev)
+                side = self._side_stream(dev) if dp.world()[1] > 1 else None
+                if side is not None:
+                    side.wait_stream(main)
+                    with torch.cuda.stream(side):
+                        dp.global_max(state[:1])
+                gain, sisdr, _ = ops.finalize_metrics(sums, lengths, T, wav=wav, target_db=None, want_loss=False,
+                                                      metric_acc=metric_acc)
+                if side is not None:
+                    main.wait_stream(side)
+                loss = ops.wsd_eval_finish(terms, sums, state, criterion.alpha, criterion.db_interval, criterion.eps, metric_acc)
+            else:
                 wav, sums = ops.mask_istft(wavs, self.ch_inp, self.ch_tar, mask, lengths, self.n_fft, self.hop, window,
-                                           pad_to=T, want_sums=True, want_spec=want_spec_loss, mask_padded=True)
-            gain, sisdr, loss = ops.finalize_metrics(sums, lengths, T, wav=wav, target_db=None, want_loss=want_spec_loss,
-                                                     metric_acc=metric_acc)
+                                           pad_to=T, want_sums=True, want_spec=want_spec_loss, mask_padded=True, **k3)
+                gain, sisdr, loss = ops.finalize_metrics(sums, lengths, T, wav=wav, target_db=None, want_loss=want_spec_loss,
+                                                         metric_acc=metric_acc)
+                if wsd:
+                    self.launches_per_step += 8     # 2 STFTs, energies (+ fill), sums (+ fill), finish, the accumulator's sum + add
+                    loss = self._wsd_terms_from_spectra(wavs, mask, lengths, criterion, metric_acc)
             out = {"loss_per_utt": loss, "sisdr": sisdr, "wav_predicted": wav, "gain": gain, "mask": mask[..., :K]}
             if want_stoi:
                 # after K3' (both metrics are invariant to the gain of the estimate); the clean channel is read in place
                 out["stoi"], out["estoi"] = ops.stoi(wav, wavs[:, self.ch_tar], lengths, fs=self.pre._sample_rate, acc=stoi_acc)
         return out
+
+    def _wsd_terms_from_spectra(self, wavs, mask, lengths, criterion, metric_acc):
+        """objective.WSD's per-utterance terms where K3 has no WSD variant (other geometries, or fewer than 6 frames): both
+        channels' power spectra are materialised (B, F, LD) and go through the training step's split kernels -- energies and
+        their maximum (all-reduced across ranks), then the sums.  The slow route: two more STFTs and three passes over spectra."""
+        K = self.n_fft // 2 + 1
+        window = self.pre._frame_window
+        linear_inp = ops.stft_padded(wavs, self.ch_inp, self.n_fft, self.hop, window, logpower=False)
+        linear_tar = ops.stft_padded(wavs, self.ch_tar, self.n_fft, self.hop, window, logpower=False)
+        energy, emax = ops.wsd_energy(linear_tar, K)
+        dp.global_max(emax)
+        _, loss, _, _ = ops.wsd_mask_step(mask, linear_inp, linear_tar, lengths, self.hop, K, energy, emax, criterion.alpha,
+                                          criterion.db_interval, criterion.eps, want_grad=False)
+        if metric_acc is not None:
+            metric_acc[:1] += loss.sum(dtype=torch.float64)
+        return loss
 
     def _padded_weight(self, force=False):
         """16-byte-row (and, for the tensor cores, TF32-rounded) copy of the head weight.
@@ -151,42 +219,44 @@ class EnhancementEngine:
         return buf
 
     # ------------------------------------------------------------------ CUDA-graph replay of the step
-    def capture_bound(self, lengths, wavs, metric_acc=None, want_stoi=False, stoi_acc=None):
+    def capture_bound(self, lengths, wavs, metric_acc=None, want_stoi=False, stoi_acc=None, criterion=None):
         """Capture eval_step into a CUDA graph that reads the GIVEN device tensors in place
         (no staging copy).  Returns dict(graph=, lengths=, wavs=, loss_per_utt=, sisdr=, wav_predicted=, ...).
-        metric_acc, want_stoi, stoi_acc: see eval_step (every replay adds the batch's sums to the accumulators)."""
+        metric_acc, want_stoi, stoi_acc, criterion: see eval_step (every replay adds the batch's sums to the accumulators;
+        the criterion's constants are baked into the graph)."""
         device = wavs.device
         ops.prepare(self.n_fft)
         if self.pre._frame_window.device != device:
             self.pre.to(device)
         side = torch.cuda.Stream(device=device)
         side.wait_stream(torch.cuda.current_stream(device))
-        ws = self.step_workspace(wavs.shape[0], device)          # zeroed once here; every replay leaves it zeroed
+        ws = self.step_workspace(wavs.shape[0], device, criterion)   # zeroed once here; every replay leaves it zeroed
         with torch.cuda.stream(side):
             for _ in range(2):                                   # warm up allocator + lazy init outside capture
-                self.eval_step(lengths, wavs, ws=ws, want_stoi=want_stoi)   # (no accumulators: warm-up batches are not part of a pass)
+                self.eval_step(lengths, wavs, ws=ws, want_stoi=want_stoi, criterion=criterion)   # (no accumulators: warm-up
+                                                                                                   # batches are not part of a pass)
         torch.cuda.current_stream(device).wait_stream(side)
         torch.cuda.synchronize(device)
         graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(graph):
-            out = self.eval_step(lengths, wavs, metric_acc=metric_acc, ws=ws, want_stoi=want_stoi, stoi_acc=stoi_acc)
+            out = self.eval_step(lengths, wavs, metric_acc=metric_acc, ws=ws, want_stoi=want_stoi, stoi_acc=stoi_acc, criterion=criterion)
         static = {"lengths": lengths, "wavs": wavs, "graph": graph, "ws": ws}
         static.update(out)
         return static
 
-    def capture(self, B, C, T, device):
-        """Graph with its own static input buffers for a fixed (B, C, T); cached."""
-        key = (B, C, T, str(device))
+    def capture(self, B, C, T, device, criterion=None):
+        """Graph with its own static input buffers for a fixed (B, C, T) and criterion; cached."""
+        key = (B, C, T, str(device), _criterion_key(criterion))
         if key not in self._graphs:
             lengths = torch.full((B,), T, dtype=torch.int64, device=device)
             wavs = torch.zeros(B, C, T, device=device).normal_(0, 0.05)
-            self._graphs[key] = self.capture_bound(lengths, wavs)
+            self._graphs[key] = self.capture_bound(lengths, wavs, criterion=criterion)
         return self._graphs[key]
 
-    def eval_step_graph(self, lengths, wavs):
+    def eval_step_graph(self, lengths, wavs, criterion=None):
         """Same result as eval_step through the cached graph (inputs are copied into its static buffers)."""
         B, C, T = wavs.shape
-        st = self.capture(B, C, T, wavs.device)
+        st = self.capture(B, C, T, wavs.device, criterion)
         self._padded_weight()                                       # in-place refresh if the parameters changed since capture
         st["lengths"].copy_(lengths, non_blocking=True)
         st["wavs"].copy_(wavs, non_blocking=True)
@@ -194,22 +264,24 @@ class EnhancementEngine:
         return st
 
     # ------------------------------------------------------------------ host-facing step (e2e)
-    def eval_step_host(self, lengths_cpu, wavs_cpu):
+    def eval_step_host(self, lengths_cpu, wavs_cpu, criterion=None):
         """The call a user makes with collate_fn's output (CPU tensors): H2D of the batch, the fused
         step, D2H of the per-utterance loss terms and SI-SDR.  Returns (mean_loss, mean_sisdr, wav_predicted on device)."""
-        pipe = self.host_pipeline(*wavs_cpu.shape, depth=1)
+        pipe = self.host_pipeline(*wavs_cpu.shape, depth=1, criterion=criterion)
         pipe.submit(lengths_cpu, wavs_cpu)
         loss, sisdr = pipe.drain()[0]
         return float(loss.mean()), float(sisdr.mean()), pipe.slots[0]["wav_predicted"]
 
-    def host_pipeline(self, B, C, T, depth=2, device=None, pcm16=False, want_wav=False, copy_wav=True):
+    def host_pipeline(self, B, C, T, depth=2, device=None, pcm16=False, want_wav=False, copy_wav=True, criterion=None):
         """Host-facing evaluation loop for (B, C, T) batches; see HostPipeline.  pcm16: the host batches are int16 PCM
         (half the PCIe bytes; widened on the device); want_wav: the enhanced waveforms come back to pinned host memory
-        (copy_wav=False: as views of the slot's pinned buffer, valid until that slot is submitted to again)."""
-        key = ("pipe", B, C, T, depth, bool(pcm16), bool(want_wav), bool(copy_wav))
+        (copy_wav=False: as views of the slot's pinned buffer, valid until that slot is submitted to again);
+        criterion: the loss the per-utterance terms are in (see eval_step)."""
+        key = ("pipe", B, C, T, depth, bool(pcm16), bool(want_wav), bool(copy_wav), _criterion_key(criterion))
         if key not in self._graphs:
             device = device or torch.device("cuda", torch.cuda.current_device())
-            self._graphs[key] = HostPipeline(self, B, C, T, depth, device, pcm16=pcm16, want_wav=want_wav, copy_wav=copy_wav)
+            self._graphs[key] = HostPipeline(self, B, C, T, depth, device, pcm16=pcm16, want_wav=want_wav, copy_wav=copy_wav,
+                                             criterion=criterion)
         return self._graphs[key]
 
     # ------------------------------------------------------------------ training step (head fwd + bwd)
@@ -448,7 +520,7 @@ class HostPipeline:
 
     N_CH = 2
 
-    def __init__(self, engine, B, C, T, depth, device, pcm16=False, want_wav=False, copy_wav=True):
+    def __init__(self, engine, B, C, T, depth, device, pcm16=False, want_wav=False, copy_wav=True, criterion=None):
         assert engine.ch_inp in (0, 1) and engine.ch_tar in (0, 1), "pipeline ships channels 0 and 1 only"
         self.engine, self.shape, self.device = engine, (B, C, T), device
         self.pcm16, self.want_wav, self.copy_wav = bool(pcm16), bool(want_wav), bool(copy_wav)
@@ -458,12 +530,12 @@ class HostPipeline:
         self.pending = []
         self.h2d_bytes = B * self.N_CH * T * (2 if pcm16 else 4) + B * 8
         self.d2h_bytes = 2 * B * 4 + (B * T * 4 if want_wav else 0)
-        self.launches_per_step = 5 + (1 if pcm16 else 0)
+        self.launches_per_step = 5 + (1 if pcm16 else 0) + (1 if _eval_wsd(criterion) else 0)   # (+ the WSD finish kernel)
         with torch.cuda.stream(self.compute_stream):
             for _ in range(depth):
                 lengths = torch.full((B,), T, dtype=torch.int64, device=device)
                 wavs = torch.zeros(B, self.N_CH, T, device=device).normal_(0, 0.05)
-                st = engine.capture_bound(lengths, wavs)
+                st = engine.capture_bound(lengths, wavs, criterion=criterion)
                 st["result_host"] = torch.empty(2, B).pin_memory()
                 if self.pcm16:
                     st["pcm"] = torch.empty(B, self.N_CH, T, device=device, dtype=torch.int16)

@@ -466,6 +466,54 @@ def mask_istft(wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, 
     return out, (sums if want_sums else None)
 
 
+def mask_istft_wsd_supported(n_fft, hop):
+    """True if ``mask_istft_wsd`` has a kernel for this geometry (it also needs T // hop + 1 >= 6 frames)."""
+    return bool(_lib.load().se_mask_istft_wsd_supported(int(n_fft), int(hop)))
+
+
+def mask_istft_wsd(wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, wsd_state, sums=None, sums_zeroed=False,
+                   self_clean=False):
+    """``mask_istft`` whose sums carry objective.WSD's terms instead of the spectral SI-SDR ones (se_mask_istft_wsd).
+
+    mask (B, F, LD) row-padded; wsd_state: float32 (2,) device buffer, zero at rest (``se_wsd_eval_finish`` resets it); its
+    element 0 receives the rank-local largest frame energy (all-reduce it with ``dp.global_max`` before the finish).
+    Returns (wav (B, width), sums (B, 6) float64, frame_terms (B, F, 2) float32 = {frame energy, speech-distortion sum})."""
+    wavs, mask, window = _chk(wavs, "wavs"), _chk(mask, "mask"), _c(window, "window")
+    wsd_state = _chk(wsd_state, "wsd_state")
+    assert wavs.dim() == 3 and wavs.is_contiguous() and wsd_state.numel() == 2 and wsd_state.is_contiguous()
+    B, C, T = wavs.shape
+    F, K = T // hop + 1, n_fft // 2 + 1
+    assert mask.dim() == 3 and mask.shape[:2] == (B, F) and mask.shape[2] >= K and mask.stride(2) == 1 and mask.stride(1) == mask.shape[2]
+    lengths = _c(lengths, "lengths", torch.int64)
+    width = max(hop * (F - 1), int(pad_to))
+    with torch.cuda.device(wavs.device):
+        out = torch.empty(B, width, device=wavs.device, dtype=torch.float32)
+        if sums is None:
+            sums = torch.empty(B, NSUMS, device=wavs.device, dtype=torch.float64)
+        terms = torch.empty(B, F, 2, device=wavs.device, dtype=torch.float32)
+        flags = (FLAG_SUMS_ZEROED if sums_zeroed else 0) | (FLAG_WS_SELF_CLEAN if self_clean else 0)
+        rc = _lib.load().se_mask_istft_wsd(wavs.data_ptr() + 4 * int(ch_inp) * T, wavs.data_ptr() + 4 * int(ch_tar) * T, C * T,
+                                           mask.data_ptr(), mask.shape[2], _p(lengths), B, T, n_fft, hop, window.data_ptr(),
+                                           out.data_ptr(), out.stride(0), int(pad_to), sums.data_ptr(), terms.data_ptr(),
+                                           wsd_state.data_ptr(), flags, _stream())
+        _lib.check(rc, "se_mask_istft_wsd")
+    return out, sums, terms
+
+
+def wsd_eval_finish(frame_terms, sums, wsd_state, alpha=0.5, db_interval=30.0, eps=1e-10, metric_acc=None):
+    """objective.WSD's per-utterance terms from ``mask_istft_wsd``'s outputs (after any all-reduce of wsd_state[0]) -> loss_per_utt
+    (B,); metric_acc (float64 (3,) or None) [0] += their sum.  Leaves wsd_state zeroed for the next step."""
+    B, F, _ = frame_terms.shape
+    if metric_acc is not None:
+        assert metric_acc.dtype == torch.float64 and metric_acc.numel() >= 3 and metric_acc.is_contiguous()
+    with torch.cuda.device(frame_terms.device):
+        loss = torch.empty(B, device=frame_terms.device)
+        rc = _lib.load().se_wsd_eval_finish(frame_terms.data_ptr(), sums.data_ptr(), B, F, float(alpha), float(db_interval), float(eps),
+                                            wsd_state.data_ptr(), loss.data_ptr(), _p(metric_acc), _stream())
+        _lib.check(rc, "se_wsd_eval_finish")
+    return loss
+
+
 def finalize_metrics(sums, lengths, T, wav=None, target_db=None, want_gain=True, want_sisdr=True, want_loss=True,
                      metric_acc=None):
     """Gain / waveform SI-SDR / spectral-SISDR terms from the sums of mask_istft; scales wav in place.
