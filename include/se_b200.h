@@ -147,7 +147,8 @@ int se_finalize_metrics_acc(const double* sums, const int64_t* lengths, int64_t 
  *      f < stft_len[u] of src = sqrt(relu(predicted)), tar = sqrt(relu(linear_tar));
  *      loss_per_utt[u] = -10 log10(|a t|^2 / (|a t - s|^2 + eps) + eps), a = st/(tt+eps).
  * bwd: grad_predicted[u] = grad_out[u] * d loss_u / d predicted[u] (grad_out: (n_utt,), 1/B each
- *      for loss.mean(); 0 where predicted <= 0 or the frame is masked), from the saved sums. */
+ *      for loss.mean(); 0 where predicted <= 0 or the frame is masked), from the saved sums.
+ * Both are se_sisdr_mask_fwd / _bwd (below) on dense tensors: offset NULL and every row stride = K. */
 int se_sisdr_spec_fwd(const float* predicted, const float* linear_tar, const int64_t* stft_len, int64_t n_utt,
                       int64_t n_frames, int64_t K, float eps, double* sums3, float* loss_per_utt, void* stream);
 int se_sisdr_spec_bwd(const float* predicted, const float* linear_tar, const int64_t* stft_len, int64_t n_utt,
@@ -172,6 +173,8 @@ int se_l1_logspec_bwd(const float* log_predicted, const float* linear_tar, const
  * ws_energy (n_utt * n_frames) floats, ws_max 1 float, ws_sums2 (n_utt, 2) doubles; loss: 1 float.
  * bwd: grad_offset = grad_loss[0] * d loss / d offset (0 on padded frames), from the forward's workspaces (ws_max holds the
  * batch maximum as a plain float).
+ * Both are the strided forms below on dense tensors (every row stride = K): fwd = se_wsd_energy, then the sums and batch mean of
+ * se_wsd_mask_step; bwd = se_wsd_mask_step's backward scaled by grad_loss[0].
  * This form takes the maximum over the batch it is given.  Under data parallelism the maximum must be the GLOBAL batch's: use
  * the split form below (se_wsd_energy -> all-reduce(max) of its 1-float buffer -> se_wsd_mask_step), which se_wsd_bwd can
  * also differentiate (its ws_energy / ws_max are se_wsd_energy's outputs). */

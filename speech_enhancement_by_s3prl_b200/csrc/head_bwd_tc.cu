@@ -25,6 +25,7 @@
 // fp32 dot products accumulated by the B-operand producers of the first tile's CTAs (they hold xhat in registers anyway)
 // instead of a third tensor-core tile that would transpose the whole B operand again for one useful row.
 #include <cuda.h>
+#include "objective_math.cuh"
 #include "se_common.cuh"
 
 using secommon::fail;
@@ -482,31 +483,13 @@ __device__ __forceinline__ uint32_t make_idesc_mn(int n) {        // as make_ide
     return make_idesc(n) | (1u << 15) | (1u << 16);
 }
 
-// d loss_u / d predicted coefficients of objective.SISDR (the arithmetic of sisdr_mask_bwd_kernel in ops_kernels.cu)
-__device__ __forceinline__ float2 sisdr_coef(const double* sums3, double eps, double go) {
-    const double st = sums3[0], tt = sums3[1], ss = sums3[2];
-    const double al = st / (tt + eps);
-    const double A = al * al * tt;
-    const double D = al * al * tt - 2.0 * al * st + ss + eps;
-    const double R = A / D;
-    const double kappa = -10.0 / (log(10.0) * (R + eps) * D * D);
-    const double ca = 2.0 * al * tt / (tt + eps);
-    const double cd = 2.0 * (al * tt - st) / (tt + eps) - 2.0 * al;
-    return make_float2((float)(go * kappa * (ca * D - A * cd)), (float)(go * kappa * (-2.0 * A)));
-}
-// grad_offset of one element: predicted = o * x, target power t (sisdr_mask_bwd_kernel)
+// grad_offset of one element: predicted = o * x, target power t, c = sisdr_coef (objective_math.cuh)
 __device__ __forceinline__ float sisdr_grad(float o, float x, float t, float2 c) {
     const float pi = o * x, tp = fmaxf(t, 0.0f);
     const float rs = rsqrtf(fmaxf(pi, 1e-37f));                              // one MUFU each instead of sqrt + divide
     const float ti = tp * rsqrtf(fmaxf(tp, 1e-37f));
     const float g = (c.x * ti + c.y * (pi * rs)) * (0.5f * rs) * x;
     return pi > 0.0f ? g : 0.0f;
-}
-// grad_offset of one element of objective.WSD: G = offset, X = linear_inp, S = linear_tar, scale = 1 / B -- the expression of
-// wsd_mask_bwd_kernel (ops_kernels.cu) term for term, so that both routes round the same fp32 values to TF32
-__device__ __forceinline__ float wsd_grad(float G, float X, float S, bool voiced, float alpha, float scale) {
-    const float n = fmaxf(X - S, 0.0f);
-    return scale * ((voiced ? alpha * 2.0f * (S - G * S) * (-S) : 0.0f) + (1.0f - alpha) * 2.0f * G * n * n);
 }
 constexpr int kLossNone = 0, kLossSisdr = 1, kLossWsd = 2;
 // c: SISDR's per-utterance coefficients, or (1 if the row's frame is voiced else 0, unused) for WSD
@@ -596,7 +579,7 @@ __global__ void __launch_bounds__(kTThreads, 1) linear_head_bwd_tma_kernel(const
         s_coef[threadIdx.x] = c;
         s_valid[threadIdx.x] = valid;
         if (LOSS == kLossWsd && threadIdx.x == 0)                      // voicing threshold of the (all-reduced) batch maximum, once per CTA
-            *s_thres = 10.0f * log10f(__ldg(a.max_energy) + a.loss_eps) - a.db_interval;
+            *s_thres = wsd_threshold(__ldg(a.max_energy), a.loss_eps, a.db_interval);
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
@@ -668,7 +651,7 @@ __global__ void __launch_bounds__(kTThreads, 1) linear_head_bwd_tma_kernel(const
                 if (LOSS == kLossSisdr) {
                     coef = s_coef[ui];
                 } else {                                                   // WSD: one voiced flag per row (frame)
-                    const bool voiced = r0 + row < a.R && 10.0f * log10f(__ldg(a.energy + r0 + row) + a.loss_eps) > thres;
+                    const bool voiced = r0 + row < a.R && wsd_voiced(__ldg(a.energy + r0 + row), a.loss_eps, thres);
                     coef = make_float2(voiced ? 1.0f : 0.0f, 0.0f);
                 }
             }

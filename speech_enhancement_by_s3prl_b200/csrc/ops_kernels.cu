@@ -4,6 +4,7 @@
 // head GEMM, whose tensor-core (tcgen05) variant lives in head_tc.cu.
 #include <algorithm>
 #include <cmath>
+#include "objective_math.cuh"
 #include "se_common.cuh"
 
 using secommon::fail;
@@ -20,16 +21,6 @@ namespace {
 constexpr int kThreads = 256;
 
 __device__ __forceinline__ float relu(float x) { return x > 0.0f ? x : 0.0f; }
-
-// SI-SDR in dB from the three sums st = <s,t>, tt = <t,t>, ss = <s,s>  (evaluation.py:5-10,
-// objective.py:94-97): a = st/(tt+eps); 10 log10(|a t|^2 / (|a t - s|^2 + eps) + eps)
-__device__ __forceinline__ double sisdr_from_sums(double st, double tt, double ss, double eps) {
-    const double a = st / (tt + eps);
-    const double num = a * a * tt;
-    double den = a * a * tt - 2.0 * a * st + ss;
-    if (den < 0.0) den = 0.0;                      // rounding when s is (numerically) a multiple of t
-    return 10.0 * log10(num / (den + eps) + eps);
-}
 
 // ------------------------------------------------------------------ finalize (gain + metrics)
 // level_or_neg: 10^(target_dB/10) computed on the host, or < 0 to match the clean reference's own level.
@@ -97,31 +88,7 @@ __global__ void finalize_metrics_kernel(const double* __restrict__ sums, const l
 }
 
 // ------------------------------------------------------------------ spectral SI-SDR objective
-__global__ void sisdr_spec_sums_kernel(const float* __restrict__ pred, const float* __restrict__ tar,
-                                       const long long* __restrict__ stft_len, int n_frames, int K,
-                                       double* __restrict__ sums3, int chunks) {
-    const int u = blockIdx.x / chunks, chunk = blockIdx.x - u * chunks;
-    const long long valid = (long long)min((long long)n_frames, stft_len ? stft_len[u] : (long long)n_frames) * K;
-    const long long per = (valid + chunks - 1) / chunks;
-    const long long lo = chunk * per, hi = min(valid, lo + per);
-    const float* p = pred + (long long)u * n_frames * K;
-    const float* t = tar + (long long)u * n_frames * K;
-    float acc[3] = {0.f, 0.f, 0.f};
-    for (long long i = lo + threadIdx.x; i < hi; i += blockDim.x) {
-        const float rp = relu(p[i]), rt = relu(t[i]);
-        acc[0] += sqrtf(rp) * sqrtf(rt);
-        acc[1] += rt;
-        acc[2] += rp;
-    }
-    block_accumulate_to<3, float>(acc, sums3 + (long long)u * 3);
-}
-
-__global__ void sisdr_spec_finish_kernel(const double* __restrict__ sums3, int n_utt, float eps, float* __restrict__ loss) {
-    const int u = blockIdx.x * blockDim.x + threadIdx.x;
-    if (u < n_utt) loss[u] = (float)(-sisdr_from_sums(sums3[3 * u], sums3[3 * u + 1], sums3[3 * u + 2], (double)eps));
-}
-
-// one block: per-utterance losses and their batch mean (objective.py:100) in one launch
+// one block: per-utterance losses and (loss_mean != null) their batch mean (objective.py:100) in one launch
 __global__ void __launch_bounds__(256) sisdr_finish_mean_kernel(const double* __restrict__ sums3, int n_utt, float eps,
                                                                 float* __restrict__ loss, float* __restrict__ loss_mean) {
     __shared__ double part[8];
@@ -134,52 +101,17 @@ __global__ void __launch_bounds__(256) sisdr_finish_mean_kernel(const double* __
     acc = secommon::warp_sum(acc);
     if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = acc;
     __syncthreads();
-    if (threadIdx.x == 0) {
+    if (threadIdx.x == 0 && loss_mean) {
         double t = 0.0;
         for (int w = 0; w < (int)(blockDim.x >> 5); ++w) t += part[w];
         *loss_mean = (float)(t / (double)n_utt);
     }
 }
 
-__global__ void sisdr_spec_bwd_kernel(const float* __restrict__ pred, const float* __restrict__ tar,
-                                      const long long* __restrict__ stft_len, int n_utt, int n_frames, int K, float eps_f,
-                                      const double* __restrict__ sums3, const float* __restrict__ grad_out,
-                                      float* __restrict__ grad_pred, int chunks) {
-    const int u = blockIdx.x / chunks, chunk = blockIdx.x - u * chunks;
-    const long long total = (long long)n_frames * K;
-    const long long valid = (long long)min((long long)n_frames, stft_len ? stft_len[u] : (long long)n_frames) * K;
-    const long long per = (total + chunks - 1) / chunks;
-    const long long lo = chunk * per, hi = min(total, lo + per);
-    const double eps = eps_f;
-    const double st = sums3[3 * u], tt = sums3[3 * u + 1], ss = sums3[3 * u + 2];
-    const double a = st / (tt + eps);
-    const double A = a * a * tt;
-    const double D = a * a * tt - 2.0 * a * st + ss + eps;
-    const double R = A / D;
-    // loss_u = -10 log10(R + eps);  d loss_u / d s_i = kappa * ((ca*D - A*cd) t_i - 2 A s_i)
-    const double kappa = -10.0 / (log(10.0) * (R + eps) * D * D);
-    const double ca = 2.0 * a * tt / (tt + eps);
-    const double cd = 2.0 * (a * tt - st) / (tt + eps) - 2.0 * a;
-    const double go = (double)grad_out[u];                                 // d L / d loss_u (1/B for loss.mean())
-    const float c_t = (float)(go * kappa * (ca * D - A * cd));
-    const float c_s = (float)(go * kappa * (-2.0 * A));
-    const float* p = pred + (long long)u * total;
-    const float* t = tar + (long long)u * total;
-    float* g = grad_pred + (long long)u * total;
-    for (long long i = lo + threadIdx.x; i < hi; i += blockDim.x) {
-        float out = 0.0f;
-        const float pi = p[i];
-        if (i < valid && pi > 0.0f) {
-            const float s = sqrtf(pi), ti = sqrtf(relu(t[i]));
-            out = (c_t * ti + c_s * s) * (0.5f / s);                    // ds/dp = 1/(2 sqrt(p)), 0 where p <= 0
-        }
-        g[i] = out;
-    }
-}
-
-// ---- the same objective on predicted = offset * linear_inp (model.py:33) without materialising `predicted`, on row-strided
-// tensors (rows ld floats apart; V = 4: 16-byte aligned rows read as float4, V = 1: any stride).  The backward writes
-// d loss / d offset = d loss / d predicted * linear_inp directly (0 on padded frames and on the pad columns of a row).
+// The sums and the backward run on predicted = offset * linear_inp (model.py:33) without materialising `predicted`, on row-strided
+// tensors (rows ld floats apart; V = 4: 16-byte aligned rows read as float4, V = 1: any stride); offset = null: predicted =
+// linear_inp (the dense entry points pass ld = K).  The backward writes d loss / d offset = d loss / d predicted * linear_inp
+// directly (0 on padded frames and on the pad columns of a row).
 template <int V> __device__ __forceinline__ void ldv(const float* p, float (&v)[V]) {
     if (V == 4) { const float4 q = *reinterpret_cast<const float4*>(p); v[0] = q.x; v[1 % V] = q.y; v[2 % V] = q.z; v[3 % V] = q.w; }
     else v[0] = *p;
@@ -243,18 +175,7 @@ __global__ void __launch_bounds__(256) sisdr_mask_bwd_kernel(const SisdrMaskArgs
     const int KV = (int)(a.ld_g / V) < (a.K + V - 1) / V ? (a.K + V - 1) / V : (int)(a.ld_g / V);   // whole rows of grad_offset
     const int per = (a.n_frames + a.chunks - 1) / a.chunks;
     const int f_lo = chunk * per, f_hi = min(a.n_frames, f_lo + per);
-    const double eps = a.eps;
-    const double st = a.sums3[3 * u], tt = a.sums3[3 * u + 1], ss = a.sums3[3 * u + 2];
-    const double al = st / (tt + eps);
-    const double A = al * al * tt;
-    const double D = al * al * tt - 2.0 * al * st + ss + eps;
-    const double R = A / D;
-    const double kappa = -10.0 / (log(10.0) * (R + eps) * D * D);        // see sisdr_spec_bwd_kernel
-    const double ca = 2.0 * al * tt / (tt + eps);
-    const double cd = 2.0 * (al * tt - st) / (tt + eps) - 2.0 * al;
-    const double go = a.grad_out ? (double)a.grad_out[u] : (double)a.grad_uniform;
-    const float c_t = (float)(go * kappa * (ca * D - A * cd));
-    const float c_s = (float)(go * kappa * (-2.0 * A));
+    const float2 coef = sisdr_coef(a.sums3 + 3 * u, (double)a.eps, a.grad_out ? (double)a.grad_out[u] : (double)a.grad_uniform);
     const long long row0 = (long long)u * a.n_frames;
     const int items = max(f_hi - f_lo, 0) * KV;
 #pragma unroll 4
@@ -275,7 +196,7 @@ __global__ void __launch_bounds__(256) sisdr_mask_bwd_kernel(const SisdrMaskArgs
                 const float pi = a.offset ? o[e] * x[e] : x[e];
                 if (c + e < a.K && pi > 0.0f) {
                     const float sq = sqrtf(pi), ti = sqrtf(relu(t[e]));
-                    g[e] = (c_t * ti + c_s * sq) * (0.5f / sq) * (a.offset ? x[e] : 1.0f);
+                    g[e] = (coef.x * ti + coef.y * sq) * (0.5f / sq) * (a.offset ? x[e] : 1.0f);
                 }
             }
         }
@@ -460,74 +381,20 @@ __global__ void wsd_energy_kernel(const float* __restrict__ tar, long long ld, l
         else atomicMin(reinterpret_cast<unsigned*>(max_energy), __float_as_uint(best));
     }
 }
-__device__ __forceinline__ float wsd_decode_max(const float* max_energy) { return *max_energy; }
 int launch_wsd_energy(const float* tar, long long ld, long long rows, int K, float* energy, float* max_energy, cudaStream_t st) {
     SE_CUDA_CHECK(cudaMemsetAsync(max_energy, 0xff, sizeof(float), st));
     const long long want = (rows + 7) / 8;
     wsd_energy_kernel<<<(unsigned)(want < 148 * 8 ? want : 148 * 8), 256, 0, st>>>(tar, ld, rows, K, energy, max_energy);
     return secommon::check_launch("wsd_energy_kernel");
 }
-// per-utterance sums over valid frames: sums2[u] = { sum ((S - G S) voiced)^2, sum (G N)^2 }, N = max(X - S, 0)
-__global__ void wsd_sums_kernel(const float* __restrict__ inp, const float* __restrict__ off, const float* __restrict__ tar,
-                                const long long* __restrict__ stft_len, int n_frames, int K, float db_interval, float eps,
-                                const float* __restrict__ energy, const float* __restrict__ max_energy,
-                                double* __restrict__ sums2, int chunks) {
-    const int u = blockIdx.x / chunks, chunk = blockIdx.x - u * chunks;
-    const long long valid = (long long)min((long long)n_frames, stft_len ? stft_len[u] : (long long)n_frames) * K;
-    const long long per = (valid + chunks - 1) / chunks;
-    const long long lo = chunk * per, hi = min(valid, lo + per);
-    const long long base = (long long)u * n_frames * K;
-    const float thres = 10.0f * log10f(wsd_decode_max(max_energy) + eps) - db_interval;
-    float acc[2] = {0.f, 0.f};
-    for (long long i = lo + threadIdx.x; i < hi; i += blockDim.x) {
-        const int f = (int)(i / K);
-        const float S = tar[base + i], G = off[base + i], X = inp[base + i];
-        const bool voiced = 10.0f * log10f(energy[(long long)u * n_frames + f] + eps) > thres;
-        const float d = voiced ? S - G * S : 0.0f;
-        const float n = G * fmaxf(X - S, 0.0f);
-        acc[0] += d * d;
-        acc[1] += n * n;
-    }
-    block_accumulate_to<2, float>(acc, sums2 + (long long)u * 2);
-}
-__global__ void wsd_finish_kernel(const double* __restrict__ sums2, int n_utt, float alpha, float* __restrict__ loss) {
-    double sp = 0.0, no = 0.0;
-    for (int u = threadIdx.x; u < n_utt; u += blockDim.x) { sp += sums2[2 * u]; no += sums2[2 * u + 1]; }
-    sp = secommon::warp_sum(sp);
-    no = secommon::warp_sum(no);
-    if (threadIdx.x == 0) loss[0] = (float)(((double)alpha * sp + (1.0 - (double)alpha) * no) / n_utt);
-}
-// d loss / d G = grad * (1/B) * ( alpha * 2 (S - G S)(-S) voiced + (1 - alpha) * 2 G N^2 ) on valid frames, else 0
-__global__ void wsd_bwd_kernel(const float* __restrict__ inp, const float* __restrict__ off, const float* __restrict__ tar,
-                               const long long* __restrict__ stft_len, int n_utt, int n_frames, int K, float alpha,
-                               float db_interval, float eps, const float* __restrict__ energy,
-                               const float* __restrict__ max_energy, const float* __restrict__ grad_out,
-                               float* __restrict__ grad_off, long long total) {
-    const float thres = 10.0f * log10f(wsd_decode_max(max_energy) + eps) - db_interval;
-    const float scale = grad_out[0] / (float)n_utt;
-    const long long per_utt = (long long)n_frames * K;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-        const long long u = i / per_utt, r = i - u * per_utt;
-        const int f = (int)(r / K);
-        const long long nvalid = min((long long)n_frames, stft_len ? stft_len[u] : (long long)n_frames);
-        float g = 0.0f;
-        if (f < nvalid) {
-            const float S = tar[i], G = off[i], X = inp[i];
-            const bool voiced = 10.0f * log10f(energy[u * n_frames + f] + eps) > thres;
-            const float n = fmaxf(X - S, 0.0f);
-            g = scale * ((voiced ? alpha * 2.0f * (S - G * S) * (-S) : 0.0f) + (1.0f - alpha) * 2.0f * G * n * n);
-        }
-        grad_off[i] = g;
-    }
-}
-
-// ---- the same objective on row-strided tensors (the training step's padded spectra), lengths as in the SISDR mask kernels and
-// the batch maximum read from a device buffer that may have been all-reduced across ranks in between (se_wsd_energy)
-struct WsdMaskArgs : SisdrMaskArgs {           // sums3 holds the (n_utt, 2) sums here
+// Per-utterance sums over valid frames, sums2[u] = { sum ((S - G S) voiced)^2, sum (G N)^2 } with N = max(X - S, 0), and the
+// backward, on row-strided tensors (the training step's padded spectra; the dense entry points pass ld = K), lengths as in the
+// SISDR mask kernels and the batch maximum read from a device buffer that may have been all-reduced across ranks in between
+// (se_wsd_energy)
+struct WsdMaskArgs : SisdrMaskArgs {           // sums3 holds the (n_utt, 2) sums here; grad_out: d L / d loss_mean (one float)
     float alpha, db_interval;
     const float* energy; const float* max_energy;
 };
-__device__ __forceinline__ float wsd_thres(const WsdMaskArgs& a) { return 10.0f * log10f(wsd_decode_max(a.max_energy) + a.eps) - a.db_interval; }
 
 template <int V>
 __global__ void __launch_bounds__(256) wsd_mask_sums_kernel(const WsdMaskArgs a) {
@@ -537,7 +404,7 @@ __global__ void __launch_bounds__(256) wsd_mask_sums_kernel(const WsdMaskArgs a)
     const int per = (valid + a.chunks - 1) / a.chunks;
     const int f_lo = chunk * per, f_hi = min(valid, f_lo + per);
     const long long row0 = (long long)u * a.n_frames;
-    const float thres = wsd_thres(a);
+    const float thres = wsd_threshold(*a.max_energy, a.eps, a.db_interval);
     float acc[2] = {0.f, 0.f};
     const int items = max(f_hi - f_lo, 0) * KV;
 #pragma unroll 4
@@ -548,7 +415,7 @@ __global__ void __launch_bounds__(256) wsd_mask_sums_kernel(const WsdMaskArgs a)
         ldv<V>(a.inp + r * a.ld_inp + c, x);
         ldv<V>(a.tar + r * a.ld_tar + c, t);
         ldv<V>(a.offset + r * a.ld_off + c, o);
-        const bool voiced = 10.0f * log10f(a.energy[r] + a.eps) > thres;
+        const bool voiced = wsd_voiced(a.energy[r], a.eps, thres);
 #pragma unroll
         for (int e = 0; e < V; ++e)
             if (c + e < a.K) {
@@ -561,7 +428,7 @@ __global__ void __launch_bounds__(256) wsd_mask_sums_kernel(const WsdMaskArgs a)
     block_accumulate_to<2, float>(acc, a.sums3 + (long long)u * 2);
 }
 
-// one block: loss_per_utt[u] = alpha sd_u + (1 - alpha) rn_u and the batch mean (the arithmetic of wsd_finish_kernel)
+// one block: loss_per_utt[u] = alpha sd_u + (1 - alpha) rn_u and the batch mean
 __global__ void __launch_bounds__(256) wsd_finish_mean_kernel(const double* __restrict__ sums2, int n_utt, float alpha,
                                                               float* __restrict__ loss, float* __restrict__ loss_mean) {
     __shared__ double part[2][8];
@@ -591,14 +458,14 @@ __global__ void __launch_bounds__(256) wsd_eval_finish_kernel(const float2* __re
                                                               float* wsd_state, float* __restrict__ loss, double* __restrict__ metric_acc) {
     __shared__ double part[8];
     const int u = blockIdx.x;
-    const float thres = 10.0f * log10f(__ldcg(wsd_state) + eps) - db_interval;     // after any all-reduce of wsd_state[0]
+    const float thres = wsd_threshold(__ldcg(wsd_state), eps, db_interval);          // after any all-reduce of wsd_state[0]
     const float2* row = terms + (long long)u * n_frames;
     const int per = (n_frames + blockDim.x - 1) / blockDim.x;
     const int lo = threadIdx.x * per, hi = min(n_frames, lo + per);
     double sd = 0.0;
     for (int f = lo; f < hi; ++f) {
         const float2 t = row[f];
-        if (10.0f * log10f(t.x + eps) > thres) sd += (double)t.y;
+        if (wsd_voiced(t.x, eps, thres)) sd += (double)t.y;
     }
     sd = secommon::warp_sum(sd);
     if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = sd;
@@ -619,7 +486,8 @@ __global__ void __launch_bounds__(256) wsd_eval_finish_kernel(const float2* __re
     }
 }
 
-// d loss_mean / d offset (upstream gradient grad_uniform = 1 / B), whole rows of grad_offset: 0 on padded frames and pad columns
+// d L / d offset for L = grad_out[0] * loss_mean (grad_out null: L = loss_mean), whole rows of grad_offset: 0 on padded frames and
+// pad columns
 template <int V>
 __global__ void __launch_bounds__(256) wsd_mask_bwd_kernel(const WsdMaskArgs a) {
     const int u = blockIdx.x / a.chunks, chunk = blockIdx.x - u * a.chunks;
@@ -627,8 +495,8 @@ __global__ void __launch_bounds__(256) wsd_mask_bwd_kernel(const WsdMaskArgs a) 
     const int KV = (int)(a.ld_g / V) < (a.K + V - 1) / V ? (a.K + V - 1) / V : (int)(a.ld_g / V);
     const int per = (a.n_frames + a.chunks - 1) / a.chunks;
     const int f_lo = chunk * per, f_hi = min(a.n_frames, f_lo + per);
-    const float thres = wsd_thres(a);
-    const float scale = a.grad_uniform;
+    const float thres = wsd_threshold(*a.max_energy, a.eps, a.db_interval);
+    const float scale = a.grad_out ? a.grad_out[0] / (float)a.n_utt : a.grad_uniform;
     const long long row0 = (long long)u * a.n_frames;
     const int items = max(f_hi - f_lo, 0) * KV;
 #pragma unroll 4
@@ -644,13 +512,10 @@ __global__ void __launch_bounds__(256) wsd_mask_bwd_kernel(const WsdMaskArgs a) 
             ldv<V>(a.inp + r * a.ld_inp + c, x);
             ldv<V>(a.tar + r * a.ld_tar + c, t);
             ldv<V>(a.offset + r * a.ld_off + c, o);
-            const bool voiced = 10.0f * log10f(a.energy[r] + a.eps) > thres;
+            const bool voiced = wsd_voiced(a.energy[r], a.eps, thres);
 #pragma unroll
             for (int e = 0; e < V; ++e)
-                if (c + e < a.K) {
-                    const float S = t[e], G = o[e], n = fmaxf(x[e] - S, 0.0f);
-                    g[e] = scale * ((voiced ? a.alpha * 2.0f * (S - G * S) * (-S) : 0.0f) + (1.0f - a.alpha) * 2.0f * G * n * n);
-                }
+                if (c + e < a.K) g[e] = wsd_grad(o[e], x[e], t[e], voiced, a.alpha, scale);
         }
         if (c + V <= a.ld_g) stv<V>(a.grad_offset + r * a.ld_g + c, g);
     }
@@ -1039,6 +904,22 @@ int pick_chunks(long long n_utt, long long work_per_utt, long long min_per_chunk
     return (int)want;
 }
 
+bool vec4_ok(const float* p, long long ld, long long K) {
+    return p == nullptr || ((reinterpret_cast<uintptr_t>(p) & 15) == 0 && ld % 4 == 0 && ld >= (K + 3) / 4 * 4);
+}
+
+// The fields every launch of the strided objective kernels shares (the dense entry points pass ld = K, len_hop = 0), chunks of at
+// least min_per_chunk elements.  Returns whether the float4 variant applies: the rows of every operand given, grad_offset
+// included, are 16-byte aligned, a multiple of 4 floats apart and cover K rounded up to 4.
+bool set_mask_args(SisdrMaskArgs& a, const float* offset, long long ld_off, const float* inp, long long ld_inp, const float* tar,
+                   long long ld_tar, const int64_t* lengths, long long len_hop, long long n_utt, long long n_frames, long long K,
+                   long long min_per_chunk, double* sums, float eps, float* grad_offset, long long ld_g) {
+    a.offset = offset; a.inp = inp; a.tar = tar; a.ld_off = ld_off; a.ld_inp = ld_inp; a.ld_tar = ld_tar;
+    a.stft_len = (const long long*)lengths; a.len_hop = (int)len_hop; a.n_utt = (int)n_utt; a.n_frames = (int)n_frames; a.K = (int)K;
+    a.chunks = pick_chunks(n_utt, n_frames * K, min_per_chunk); a.sums3 = sums; a.eps = eps; a.grad_offset = grad_offset; a.ld_g = ld_g;
+    return vec4_ok(offset, ld_off, K) && vec4_ok(inp, ld_inp, K) && vec4_ok(tar, ld_tar, K) && vec4_ok(grad_offset, ld_g, K);
+}
+
 }  // namespace
 
 extern "C" {
@@ -1081,26 +962,29 @@ int se_sisdr_spec_fwd(const float* predicted, const float* linear_tar, const int
     SE_REQUIRE(predicted && linear_tar && sums3 && n_utt > 0 && n_frames > 0 && K > 0, "bad argument");
     cudaStream_t st = (cudaStream_t)stream;
     SE_CUDA_CHECK(cudaMemsetAsync(sums3, 0, sizeof(double) * 3 * n_utt, st));
-    const int chunks = pick_chunks(n_utt, n_frames * K, 8192);
-    sisdr_spec_sums_kernel<<<(unsigned)(n_utt * chunks), kThreads, 0, st>>>(predicted, linear_tar, (const long long*)stft_len,
-                                                                            (int)n_frames, (int)K, sums3, chunks);
-    int rc = secommon::check_launch("sisdr_spec_sums_kernel");
+    SisdrMaskArgs a{};
+    const bool v4 = set_mask_args(a, nullptr, K, predicted, K, linear_tar, K, stft_len, 0, n_utt, n_frames, K, 8192, sums3, eps, nullptr, 0);
+    if (v4) sisdr_mask_sums_kernel<4><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
+    else sisdr_mask_sums_kernel<1><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
+    int rc = secommon::check_launch("sisdr_mask_sums_kernel");
     if (rc != SE_OK || !loss_per_utt) return rc;
-    sisdr_spec_finish_kernel<<<(unsigned)((n_utt + 127) / 128), 128, 0, st>>>(sums3, (int)n_utt, eps, loss_per_utt);
-    return secommon::check_launch("sisdr_spec_finish_kernel");
+    sisdr_finish_mean_kernel<<<1, 256, 0, st>>>(sums3, (int)n_utt, eps, loss_per_utt, nullptr);
+    return secommon::check_launch("sisdr_finish_mean_kernel");
 }
 
 int se_sisdr_spec_bwd(const float* predicted, const float* linear_tar, const int64_t* stft_len, int64_t n_utt,
                       int64_t n_frames, int64_t K, float eps, const double* sums3, const float* grad_out,
                       float* grad_predicted, void* stream) {
     SE_REQUIRE(predicted && linear_tar && sums3 && grad_out && grad_predicted && n_utt > 0, "bad argument");
-    const int chunks = pick_chunks(n_utt, n_frames * K, 8192);
-    sisdr_spec_bwd_kernel<<<(unsigned)(n_utt * chunks), kThreads, 0, (cudaStream_t)stream>>>(
-        predicted, linear_tar, (const long long*)stft_len, (int)n_utt, (int)n_frames, (int)K, eps, sums3, grad_out, grad_predicted, chunks);
-    return secommon::check_launch("sisdr_spec_bwd_kernel");
+    SisdrMaskArgs a{};
+    const bool v4 = set_mask_args(a, nullptr, K, predicted, K, linear_tar, K, stft_len, 0, n_utt, n_frames, K, 8192,
+                                  const_cast<double*>(sums3), eps, grad_predicted, K);
+    a.grad_out = grad_out;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (v4) sisdr_mask_bwd_kernel<4><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
+    else sisdr_mask_bwd_kernel<1><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
+    return secommon::check_launch("sisdr_mask_bwd_kernel");
 }
-
-static bool vec4_ok(const float* p, long long ld) { return p == nullptr || (((reinterpret_cast<uintptr_t>(p) & 15) == 0) && (ld % 4 == 0)); }
 
 int se_sisdr_mask_fwd(const float* offset, int64_t ld_off, const float* linear_inp, int64_t ld_inp, const float* linear_tar,
                       int64_t ld_tar, const int64_t* stft_len, int64_t n_utt, int64_t n_frames, int64_t K, float eps,
@@ -1110,18 +994,14 @@ int se_sisdr_mask_fwd(const float* offset, int64_t ld_off, const float* linear_i
     cudaStream_t st = (cudaStream_t)stream;
     SE_CUDA_CHECK(cudaMemsetAsync(sums3, 0, sizeof(double) * 3 * n_utt, st));
     SisdrMaskArgs a{};
-    a.offset = offset; a.inp = linear_inp; a.tar = linear_tar; a.ld_off = ld_off; a.ld_inp = ld_inp; a.ld_tar = ld_tar;
-    a.stft_len = (const long long*)stft_len; a.n_utt = (int)n_utt; a.n_frames = (int)n_frames; a.K = (int)K;
-    a.chunks = pick_chunks(n_utt, n_frames * K, 2048); a.sums3 = sums3; a.eps = eps;
-    const long long need = (K + 3) / 4 * 4;
-    const bool v4 = vec4_ok(offset, ld_off) && vec4_ok(linear_inp, ld_inp) && vec4_ok(linear_tar, ld_tar) && ld_inp >= need &&
-                    ld_tar >= need && (!offset || ld_off >= need);
+    const bool v4 = set_mask_args(a, offset, ld_off, linear_inp, ld_inp, linear_tar, ld_tar, stft_len, 0, n_utt, n_frames, K, 2048, sums3,
+                                  eps, nullptr, 0);
     if (v4) sisdr_mask_sums_kernel<4><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
     else sisdr_mask_sums_kernel<1><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
     int rc = secommon::check_launch("sisdr_mask_sums_kernel");
     if (rc != SE_OK || !loss_per_utt) return rc;
-    sisdr_spec_finish_kernel<<<(unsigned)((n_utt + 127) / 128), 128, 0, st>>>(sums3, (int)n_utt, eps, loss_per_utt);
-    return secommon::check_launch("sisdr_spec_finish_kernel");
+    sisdr_finish_mean_kernel<<<1, 256, 0, st>>>(sums3, (int)n_utt, eps, loss_per_utt, nullptr);
+    return secommon::check_launch("sisdr_finish_mean_kernel");
 }
 
 int se_sisdr_mask_bwd(const float* offset, int64_t ld_off, const float* linear_inp, int64_t ld_inp, const float* linear_tar,
@@ -1130,13 +1010,9 @@ int se_sisdr_mask_bwd(const float* offset, int64_t ld_off, const float* linear_i
     SE_REQUIRE(linear_inp && linear_tar && sums3 && grad_out && grad_offset && n_utt > 0 && n_frames > 0 && K > 0, "bad argument");
     SE_REQUIRE(ld_inp >= K && ld_tar >= K && ld_g >= K && (!offset || ld_off >= K), "row stride smaller than K");
     SisdrMaskArgs a{};
-    a.offset = offset; a.inp = linear_inp; a.tar = linear_tar; a.ld_off = ld_off; a.ld_inp = ld_inp; a.ld_tar = ld_tar;
-    a.stft_len = (const long long*)stft_len; a.n_utt = (int)n_utt; a.n_frames = (int)n_frames; a.K = (int)K;
-    a.chunks = pick_chunks(n_utt, n_frames * K, 2048); a.sums3 = const_cast<double*>(sums3); a.eps = eps;
-    a.grad_out = grad_out; a.grad_offset = grad_offset; a.ld_g = ld_g;
-    const long long need = (K + 3) / 4 * 4;
-    const bool v4 = vec4_ok(offset, ld_off) && vec4_ok(linear_inp, ld_inp) && vec4_ok(linear_tar, ld_tar) && vec4_ok(grad_offset, ld_g) &&
-                    ld_inp >= need && ld_tar >= need && ld_g >= need && (!offset || ld_off >= need);
+    const bool v4 = set_mask_args(a, offset, ld_off, linear_inp, ld_inp, linear_tar, ld_tar, stft_len, 0, n_utt, n_frames, K, 2048,
+                                  const_cast<double*>(sums3), eps, grad_offset, ld_g);
+    a.grad_out = grad_out;
     cudaStream_t st = (cudaStream_t)stream;
     if (v4) sisdr_mask_bwd_kernel<4><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
     else sisdr_mask_bwd_kernel<1><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
@@ -1153,13 +1029,9 @@ int se_sisdr_mask_step(const float* offset, int64_t ld_off, const float* linear_
     cudaStream_t st = (cudaStream_t)stream;
     if (!sums_zeroed) SE_CUDA_CHECK(cudaMemsetAsync(sums3, 0, sizeof(double) * 3 * n_utt, st));
     SisdrMaskArgs a{};
-    a.offset = offset; a.inp = linear_inp; a.tar = linear_tar; a.ld_off = ld_off; a.ld_inp = ld_inp; a.ld_tar = ld_tar;
-    a.stft_len = (const long long*)lengths; a.len_hop = (int)len_hop; a.n_utt = (int)n_utt; a.n_frames = (int)n_frames; a.K = (int)K;
-    a.chunks = pick_chunks(n_utt, n_frames * K, 2048); a.sums3 = sums3; a.eps = eps;
-    a.grad_out = nullptr; a.grad_uniform = 1.0f / (float)n_utt; a.grad_offset = grad_offset; a.ld_g = ld_g;
-    const long long need = (K + 3) / 4 * 4;
-    const bool v4 = vec4_ok(offset, ld_off) && vec4_ok(linear_inp, ld_inp) && vec4_ok(linear_tar, ld_tar) && ld_inp >= need && ld_tar >= need &&
-                    (!offset || ld_off >= need) && (!grad_offset || (vec4_ok(grad_offset, ld_g) && ld_g >= need));
+    const bool v4 = set_mask_args(a, offset, ld_off, linear_inp, ld_inp, linear_tar, ld_tar, lengths, len_hop, n_utt, n_frames, K, 2048,
+                                  sums3, eps, grad_offset, ld_g);
+    a.grad_uniform = 1.0f / (float)n_utt;
     if (v4) sisdr_mask_sums_kernel<4><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
     else sisdr_mask_sums_kernel<1><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
     int rc = secommon::check_launch("sisdr_mask_sums_kernel");
@@ -1260,25 +1132,29 @@ int se_wsd_fwd(const float* linear_inp, const float* offset, const float* linear
     SE_CUDA_CHECK(cudaMemsetAsync(ws_sums2, 0, sizeof(double) * 2 * n_utt, st));
     int rc = launch_wsd_energy(linear_tar, K, n_utt * n_frames, (int)K, ws_energy, ws_max, st);
     if (rc != SE_OK) return rc;
-    const int chunks = pick_chunks(n_utt, n_frames * K, 8192);
-    wsd_sums_kernel<<<(unsigned)(n_utt * chunks), kThreads, 0, st>>>(linear_inp, offset, linear_tar, (const long long*)stft_len,
-                                                                     (int)n_frames, (int)K, db_interval, eps, ws_energy, ws_max,
-                                                                     ws_sums2, chunks);
-    if ((rc = secommon::check_launch("wsd_sums_kernel")) != SE_OK) return rc;
-    wsd_finish_kernel<<<1, 32, 0, st>>>(ws_sums2, (int)n_utt, alpha, loss);
-    return secommon::check_launch("wsd_finish_kernel");
+    WsdMaskArgs a{};
+    const bool v4 = set_mask_args(a, offset, K, linear_inp, K, linear_tar, K, stft_len, 0, n_utt, n_frames, K, 8192, ws_sums2, eps,
+                                  nullptr, 0);
+    a.alpha = alpha; a.db_interval = db_interval; a.energy = ws_energy; a.max_energy = ws_max;
+    if (v4) wsd_mask_sums_kernel<4><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
+    else wsd_mask_sums_kernel<1><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
+    if ((rc = secommon::check_launch("wsd_mask_sums_kernel")) != SE_OK) return rc;
+    wsd_finish_mean_kernel<<<1, 256, 0, st>>>(ws_sums2, (int)n_utt, alpha, nullptr, loss);
+    return secommon::check_launch("wsd_finish_mean_kernel");
 }
 
 int se_wsd_bwd(const float* linear_inp, const float* offset, const float* linear_tar, const int64_t* stft_len, int64_t n_utt,
                int64_t n_frames, int64_t K, float alpha, float db_interval, float eps, const float* ws_energy,
                const float* ws_max, const float* grad_loss, float* grad_offset, void* stream) {
     SE_REQUIRE(linear_inp && offset && linear_tar && ws_energy && ws_max && grad_loss && grad_offset && n_utt > 0, "bad argument");
-    const long long total = n_utt * n_frames * K;
-    const long long want = (total + 1023) / 1024;
-    wsd_bwd_kernel<<<(unsigned)(want < 148 * 16 ? want : 148 * 16), 256, 0, (cudaStream_t)stream>>>(
-        linear_inp, offset, linear_tar, (const long long*)stft_len, (int)n_utt, (int)n_frames, (int)K, alpha, db_interval, eps,
-        ws_energy, ws_max, grad_loss, grad_offset, total);
-    return secommon::check_launch("wsd_bwd_kernel");
+    WsdMaskArgs a{};
+    const bool v4 = set_mask_args(a, offset, K, linear_inp, K, linear_tar, K, stft_len, 0, n_utt, n_frames, K, 8192, nullptr, eps,
+                                  grad_offset, K);
+    a.grad_out = grad_loss; a.alpha = alpha; a.db_interval = db_interval; a.energy = ws_energy; a.max_energy = ws_max;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (v4) wsd_mask_bwd_kernel<4><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
+    else wsd_mask_bwd_kernel<1><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
+    return secommon::check_launch("wsd_mask_bwd_kernel");
 }
 
 int se_wsd_energy(const float* linear_tar, int64_t ld_tar, int64_t n_utt, int64_t n_frames, int64_t K, float* energy, float* max_energy,
@@ -1299,14 +1175,9 @@ int se_wsd_mask_step(const float* offset, int64_t ld_off, const float* linear_in
     cudaStream_t st = (cudaStream_t)stream;
     if (!sums_zeroed) SE_CUDA_CHECK(cudaMemsetAsync(sums2, 0, sizeof(double) * 2 * n_utt, st));
     WsdMaskArgs a{};
-    a.offset = offset; a.inp = linear_inp; a.tar = linear_tar; a.ld_off = ld_off; a.ld_inp = ld_inp; a.ld_tar = ld_tar;
-    a.stft_len = (const long long*)lengths; a.len_hop = (int)len_hop; a.n_utt = (int)n_utt; a.n_frames = (int)n_frames; a.K = (int)K;
-    a.chunks = pick_chunks(n_utt, n_frames * K, 2048); a.sums3 = sums2; a.eps = eps;
-    a.grad_uniform = 1.0f / (float)n_utt; a.grad_offset = grad_offset; a.ld_g = ld_g;
-    a.alpha = alpha; a.db_interval = db_interval; a.energy = energy; a.max_energy = max_energy;
-    const long long need = (K + 3) / 4 * 4;
-    const bool v4 = vec4_ok(offset, ld_off) && vec4_ok(linear_inp, ld_inp) && vec4_ok(linear_tar, ld_tar) && ld_inp >= need && ld_tar >= need &&
-                    ld_off >= need && (!grad_offset || (vec4_ok(grad_offset, ld_g) && ld_g >= need));
+    const bool v4 = set_mask_args(a, offset, ld_off, linear_inp, ld_inp, linear_tar, ld_tar, lengths, len_hop, n_utt, n_frames, K, 2048,
+                                  sums2, eps, grad_offset, ld_g);
+    a.grad_uniform = 1.0f / (float)n_utt; a.alpha = alpha; a.db_interval = db_interval; a.energy = energy; a.max_energy = max_energy;
     if (v4) wsd_mask_sums_kernel<4><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
     else wsd_mask_sums_kernel<1><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
     int rc = secommon::check_launch("wsd_mask_sums_kernel");

@@ -1037,6 +1037,18 @@ def test_wsd_matches_oracle_and_autograd(se, B, F, K, alpha, db):
     # frame counts instead of masks (what the fused step passes)
     loss2, _ = se.WSD(alpha=alpha, db_interval=db)(inp.cuda(), off.cuda(), tar.cuda(), stft_lengths=lens.cuda())
     assert loss2.item() == pytest.approx(loss.item(), rel=1e-6)
+    # the one-call form se_wsd_fwd through the C ABI: the oracle's loss, and the energies / batch maximum of se_wsd_energy
+    from speech_enhancement_by_s3prl_b200 import _lib, ops
+    inp_d, off_d, tar_d, lens_d = inp.cuda(), off.cuda(), tar.cuda(), lens.cuda()
+    energy, emax = ops.wsd_energy(tar_d, K)
+    ws_energy, ws_max, loss3 = torch.empty(B * F, device="cuda"), torch.empty(1, device="cuda"), torch.empty(1, device="cuda")
+    ws_sums2 = torch.empty(B, 2, device="cuda", dtype=torch.float64)
+    rc = _lib.load().se_wsd_fwd(inp_d.data_ptr(), off_d.data_ptr(), tar_d.data_ptr(), lens_d.data_ptr(), B, F, K, alpha, db, 1e-10,
+                                ws_energy.data_ptr(), ws_max.data_ptr(), ws_sums2.data_ptr(), loss3.data_ptr(),
+                                torch.cuda.current_stream().cuda_stream)
+    assert rc == 0, _lib.last_error()
+    assert loss3.item() == pytest.approx(ref.item(), rel=2e-5)
+    assert torch.equal(ws_max, emax) and torch.equal(ws_energy, energy.flatten())
 
 
 # ------------------------------------------------------------------------------ on-device batch synthesis (SURVEY 8f, rank 3)
@@ -1316,7 +1328,8 @@ def test_fused_training_step_matches_autograd_path(se, B, T, ragged):
 
 
 def test_sisdr_mask_kernels_match_unfused_objective(se):
-    """se_sisdr_mask_fwd / _bwd (strided, float4 and scalar variants) against sisdr_spec on predicted = offset * linear_inp."""
+    """se_sisdr_mask_fwd / _bwd (strided, float4 and scalar variants) and the dense sisdr_spec against the float64 oracle of
+    objective.SISDR on predicted = offset * linear_inp."""
     from speech_enhancement_by_s3prl_b200 import ops
     B, F, K = 5, 77, 257
     g = torch.Generator().manual_seed(2)
@@ -1325,14 +1338,19 @@ def test_sisdr_mask_kernels_match_unfused_objective(se):
     tar = (torch.randn(B, F, K, generator=g) ** 2).cuda()
     inp[0, 3, 5] = 0.0                                                         # predicted == 0: zero gradient, no NaN
     frames = torch.LongTensor([77, 60, 1, 77, 33]).cuda()
-    pred = (off * inp).requires_grad_(True)
-    loss_ref = ops.sisdr_spec(pred, tar, frames, 1e-10)
-    loss_ref.mean().backward()
-    g_ref = pred.grad * inp
+    off64 = off.double().cpu().requires_grad_(True)
+    _, ref_u = sp.sisdr_spectral(off64 * inp.double().cpu(), tar.double().cpu(), sp.length_masks(frames.cpu()))
+    ref_u.mean().backward()
+    loss_ref, g_ref = ref_u.detach(), off64.grad.cuda()
+    pred = (off * inp).requires_grad_(True)                                    # the dense entry points (autograd route)
+    loss_dense = ops.sisdr_spec(pred, tar, frames, 1e-10)
+    loss_dense.mean().backward()
+    np.testing.assert_allclose(loss_dense.detach().cpu().numpy(), loss_ref.cpu().numpy(), rtol=1e-5, atol=1e-5)
+    assert (pred.grad * inp - g_ref).abs().max().item() < 1e-5 * g_ref.abs().max().item()
     for LD in (K, 260):                                                        # scalar and float4 variants
         pad = lambda x: torch.nn.functional.pad(x, (0, LD - K), value=float("nan")).contiguous()
         loss, sums3 = ops.sisdr_mask_fwd(pad(off), pad(inp), pad(tar), frames, K)
-        np.testing.assert_allclose(loss.cpu().numpy(), loss_ref.detach().cpu().numpy(), rtol=1e-5, atol=1e-5)
+        np.testing.assert_allclose(loss.cpu().numpy(), loss_ref.cpu().numpy(), rtol=1e-5, atol=1e-5)
         go = torch.full((B,), 1.0 / B, device="cuda")
         gr = ops.sisdr_mask_bwd(pad(off), pad(inp), pad(tar), frames, K, sums3, go)
         assert gr.shape == (B, F, LD) and torch.isfinite(gr).all() and (gr[..., K:] == 0).all()
@@ -1340,7 +1358,7 @@ def test_sisdr_mask_kernels_match_unfused_objective(se):
         assert (gr[..., :K] - g_ref).abs().max().item() < 1e-5 * scale
         assert (gr[1, 60:] == 0).all() and (gr[2, 1:] == 0).all()
         loss_p, _ = ops.sisdr_mask_fwd(None, pad(off * inp), pad(tar), frames, K)   # offset = None: predicted given
-        np.testing.assert_allclose(loss_p.cpu().numpy(), loss_ref.detach().cpu().numpy(), rtol=1e-5, atol=1e-5)
+        np.testing.assert_allclose(loss_p.cpu().numpy(), loss_ref.cpu().numpy(), rtol=1e-5, atol=1e-5)
         # the training step's three-launch form: frames = lengths // hop + 1 in the kernels, batch-mean loss, uniform 1 / B gradient
         hop = 160
         lens = (frames - 1) * hop + torch.LongTensor([0, 159, 7, 80, 1]).cuda()
