@@ -117,6 +117,11 @@ int se_mask_istft_strided(const float* noisy, const float* clean, int64_t utt_st
                                       caller filling it every step: se_stft_features zeroes the `sums` part (consumed by the
                                       previous step's se_finalize_metrics), se_mask_istft_ex zeroes the stat_sums part (consumed
                                       by this step's head) -- a captured step then has no fill node at its start */
+#define SE_FLAG_MASK_IS_LOG_POWER 16 /* se_mask_istft_ex: `mask` holds the LOG of a target power spectrum (model.LSTM's
+                                      log_predicted, model.py:37-60): wav_out = iSTFT(exp(lp / 2) X / |X|), exp(lp / 2) where
+                                      X = 0 -- _decode_wav(exp(lp), phase_inp) without the phase or an exp pass; with
+                                      SE_FLAG_WANT_SPEC the spectral SI-SDR sums take s = exp(lp / 2) as the estimate's
+                                      magnitude.  Mutually exclusive with SE_FLAG_MASK_IS_POWER */
 int se_mask_istft_ex(const float* noisy, const float* clean, int64_t utt_stride, const float* mask, int64_t mask_stride,
                      const int64_t* lengths, int64_t n_utt, int64_t T, int n_fft, int hop, const float* window,
                      float* wav_out, int64_t out_stride, int64_t pad_to, double* sums, int flags, void* stream);
@@ -228,6 +233,34 @@ int se_mask_istft_wsd(const float* noisy, const float* clean, int64_t utt_stride
                       int flags, void* stream);
 int se_wsd_eval_finish(const float* frame_terms, const double* sums, int64_t n_utt, int64_t n_frames, float alpha, float db_interval,
                        float eps, float* wsd_state, float* loss_per_utt, double* metric_acc, void* stream);
+
+/* ---- the evaluation step with objective.L1 (objective.py:109-117) and model.LSTM (log_predicted) ------------------------
+ * se_mask_istft_l1: se_mask_istft_ex with SE_FLAG_MASK_IS_LOG_POWER (same waveform output and SE_SUM_YC / SE_SUM_CC / SE_SUM_YY
+ *   sums; clean and sums required) whose clean-frame pass computes, for lp = `mask` and C = STFT(clean), over the valid frames
+ *   f < lengths[u] // hop + 1 and the K bins:
+ *     sums[u * SE_NSUMS + SE_SUM_SPEC_ST] += sum |lp - log(|C|^2 + eps)|   (SE_SUM_SPEC_TT / _SS stay 0);
+ *     l1_acc[0] += the same sums over the batch, l1_acc[1] += sum_u valid_frames_u * K
+ *   (2 caller-owned doubles that rest at 0: the numerator and the element count of the global mean, which is what a data-parallel
+ *   evaluation all-reduces before se_l1_eval_finish; one double atomic per run).
+ *   flags: SE_FLAG_SUMS_ZEROED and SE_FLAG_WS_SELF_CLEAN as in se_mask_istft_ex.  Register-resident geometries only
+ *   (se_mask_istft_l1_supported, and T / hop + 1 >= 6 frames); otherwise SE_ERR_UNSUPPORTED: use se_mask_istft_ex with
+ *   SE_FLAG_MASK_IS_LOG_POWER and se_l1_eval_sums on the clean power spectrum.
+ * se_l1_eval_sums: the same sums from materialised row-strided tensors (n_utt, T / hop + 1, ld): log_predicted and the clean
+ *   power linear_tar; sums[u, SE_SUM_SPEC_ST] (zeroed by the caller) += the utterance's sum, l1_acc[0] += the batch's, l1_acc[1] +=
+ *   sum_u valid_frames_u * K.
+ * se_l1_eval_finish: after any all-reduce of l1_acc: loss_per_utt[u] = sums[u, SE_SUM_SPEC_ST] / (valid_frames_u * K) (the
+ *   utterance's own L1, a batch of one), loss[0] = l1_acc[0] / l1_acc[1] (objective.L1 of the global batch), metric_acc (or NULL)
+ *   [0] += n_utt * loss[0] (so that the pass mean of dp.means_from_acc stays the mean of the batch losses, weighted by their
+ *   utterances), then l1_acc = {0, 0} for the next step.  Lengths are clamped to [0, T] as the mask-iSTFT kernels clamp them. */
+int se_mask_istft_l1_supported(int n_fft, int hop);
+int se_mask_istft_l1(const float* noisy, const float* clean, int64_t utt_stride, const float* mask, int64_t mask_stride,
+                     const int64_t* lengths, int64_t n_utt, int64_t T, int n_fft, int hop, const float* window,
+                     float* wav_out, int64_t out_stride, int64_t pad_to, double* sums, double* l1_acc, float eps, int flags,
+                     void* stream);
+int se_l1_eval_sums(const float* log_predicted, int64_t ld_lp, const float* linear_tar, int64_t ld_tar, const int64_t* lengths,
+                    int64_t n_utt, int64_t T, int hop, int64_t K, float eps, double* sums, double* l1_acc, void* stream);
+int se_l1_eval_finish(const double* sums, const int64_t* lengths, int64_t n_utt, int64_t T, int hop, int64_t K, double* l1_acc,
+                      float* loss_per_utt, float* loss, double* metric_acc, void* stream);
 
 /* ---- K4c: batched waveform SI-SDR (evaluation.py:5-10 over runner.py:587-602) -----
  * sisdr[u] = sisdr_eval(src[u, :len[u]], tar[u, :len[u]]).  ws_sums3: caller workspace of

@@ -71,6 +71,10 @@ _SIGNATURES = {
     "se_mask_istft_wsd_supported": [c_int, c_int],
     "se_mask_istft_wsd": [c_f, c_f, i64, c_f, i64, c_f, i64, i64, c_int, c_int, c_f, c_f, i64, i64, c_f, c_f, c_f, c_int, c_f],
     "se_wsd_eval_finish": [c_f, c_f, i64, i64, c_float, c_float, c_float, c_f, c_f, c_f, c_f],
+    "se_mask_istft_l1_supported": [c_int, c_int],
+    "se_mask_istft_l1": [c_f, c_f, i64, c_f, i64, c_f, i64, i64, c_int, c_int, c_f, c_f, i64, i64, c_f, c_f, c_float, c_int, c_f],
+    "se_l1_eval_sums": [c_f, i64, c_f, i64, c_f, i64, i64, c_int, i64, c_float, c_f, c_f, c_f],
+    "se_l1_eval_finish": [c_f, c_f, i64, i64, c_int, i64, c_f, c_f, c_f, c_f, c_f],
     "se_linear_head_bwd_wsd_supported": [i64, i64, i64, i64, i64, i64, i64, i64],
     "se_linear_head_bwd_wsd": [c_f, i64, c_f, i64, c_float, c_f, i64, c_f, i64, c_f, i64, c_f, i64, c_f, c_f, c_float, c_float, c_float, i64,
                                i64, i64, i64, c_int, c_f, i64, c_f, c_f, c_f],

@@ -63,20 +63,25 @@ __device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wa
 __device__ __forceinline__ void griddep_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
 // One masked pair of bins: spectral-loss terms (own) and the merged, conjugated inverse-FFT input
-// PM ("power mode"): ga / gb are the target POWER of the bins, the output keeps the phase of X: Y = sqrt(g) X / |X|, and
-// Y = sqrt(g) where X = 0 (atan2(0, 0) = 0) -- OnlinePreprocessor.istft(linears, phase_inp) without the phase (runner.py:266-281)
-template <bool PM> __device__ __forceinline__ float2 apply_gain(float2 x, float g) {
+// PM ("power mode"): 0 = ga / gb multiply |X|^2; 1 = ga / gb are the target POWER of the bins, the output keeps the phase of X:
+// Y = sqrt(g) X / |X|, and Y = sqrt(g) where X = 0 (atan2(0, 0) = 0) -- OnlinePreprocessor.istft(linears, phase_inp) without the
+// phase (runner.py:266-281); 2 (SE_FLAG_MASK_IS_LOG_POWER) = ga / gb are the LOG of the target power (model.LSTM's
+// log_predicted): as 1 with g = exp(g)
+template <int PM> __device__ __forceinline__ float target_power(float g) { return PM == 2 ? __expf(g) : g; }
+template <int PM> __device__ __forceinline__ float2 apply_gain(float2 x, float g) {
     if (!PM) return cscale(x, fast_sqrt(g));
     const float p = x.x * x.x + x.y * x.y;
-    return p > 0.0f ? cscale(x, fast_sqrt(g) * rsqrtf(p)) : make_float2(fast_sqrt(g), 0.0f);
+    if (PM == 1) return p > 0.0f ? cscale(x, fast_sqrt(g) * rsqrtf(p)) : make_float2(fast_sqrt(g), 0.0f);
+    const float s = __expf(0.5f * g);                                         // exp(lp / 2) = sqrt(exp(lp))
+    return p > 0.0f ? cscale(x, s * rsqrtf(p)) : make_float2(s, 0.0f);
 }
 // RELU = false (the WSD variant of K3): ra / rb keep the signed mask * |X|^2
-template <bool PM, bool RELU = true>
+template <int PM, bool RELU = true>
 __device__ __forceinline__ void mask_merge(float2 xa, float2 xb, float ga, float gb, float2 w, bool own, float& ra, float& rb,
                                            float2& ca, float2& cb) {
     if (own) {
-        ra = PM ? ga : ga * (xa.x * xa.x + xa.y * xa.y);
-        rb = PM ? gb : gb * (xb.x * xb.x + xb.y * xb.y);
+        ra = PM ? target_power<PM>(ga) : ga * (xa.x * xa.x + xa.y * xa.y);
+        rb = PM ? target_power<PM>(gb) : gb * (xb.x * xb.x + xb.y * xb.y);
         if (RELU) { ra = fmaxf(ra, 0.0f); rb = fmaxf(rb, 0.0f); }
     }
     merge_pair_conj(apply_gain<PM>(xa, ga), apply_gain<PM>(xb, gb), w, ca, cb);

@@ -563,9 +563,14 @@ template <class Geo> __device__ __forceinline__ float2 group_sum(float2 v, int l
 // utterance's valid length included: the reference does not mask the energies) and writes per frame {E_f = sum_k S,
 // D_f = sum_k (S - G S)^2 (0 past the valid length)} to a.wsd_terms; sum_k (G max(X - S, 0))^2 over valid frames goes to the
 // SE_SUM_SPEC_ST slot of the sums, and the run's largest E_f to *a.wsd_max (float bits, atomicMax: energies are >= 0).
-template <class Geo, bool PM, bool TRACE, bool WSD = false>
+// L1: the variant for objective.L1 (objective.py:109-117), with PM = 2 (the mask is model.LSTM's log_predicted).  Pass 2 runs
+// for the valid frames and sums |lp - log(|C|^2 + eps)| over their K bins into the SE_SUM_SPEC_ST slot of the sums and into
+// a.l1_acc[0] (one double atomic per run each); the run that starts the utterance adds its valid_frames * K to a.l1_acc[1].
+// PM: 0 = mask of |X|^2, 1 = target power, 2 = log target power (fast_common.cuh).
+template <class Geo, int PM, bool TRACE, bool WSD = false, bool L1 = false>
 __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS) mask_istft_run_kernel(MaskIstftArgs a, GeoRunPlan plan) {
-    using Z = K3Sz<Geo, WSD ? 2 : 1>;
+    constexpr bool MB2 = WSD || L1;                                                 // pass 2 re-reads the frame's mask row
+    using Z = K3Sz<Geo, MB2 ? 2 : 1>;
     extern __shared__ __align__(128) unsigned char smem[];
     if (TRACE) trace_begin(smem + Z::SMEM);
     using S = Sz<Geo>;
@@ -581,7 +586,7 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
     const int dgrp = grp < Geo::GPW ? grp : Geo::GPW - 1;
     float* nring = reinterpret_cast<float*>(smem + S::TAB_BYTES + (size_t)warp * Z::WARP_BYTES + (size_t)dgrp * Z::GSTRIDE + Geo::XBUF);
     float* cring = nring + RB * Bs;
-    float* mb = cring + RB * Bs;                                                    // WSD: two rows, frame f_first + it in row (it & 1)
+    float* mb = cring + RB * Bs;                                                    // MB2: two rows, frame f_first + it in row (it & 1)
     const bool lane_active = grp < Geo::GPW;
     const long long unit = (long long)blockIdx.x * GROUPS + warp * Geo::GPW + grp;
     const bool active = lane_active && unit < plan.total_runs;
@@ -660,9 +665,10 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
         const bool real = live && f <= F - 1;
         const bool emit = live && f >= e0;
         // WSD: own = every real frame of the run (energies), wval = the valid ones among them (loss terms)
-        const bool own = WSD ? need_clean && real && (f >= e0 || ri == 0) : spec && real && f < valid_frames && (f >= e0 || ri == 0);
+        const bool own = WSD ? need_clean && real && (f >= e0 || ri == 0)
+                             : (L1 ? need_clean : spec) && real && f < valid_frames && (f >= e0 || ri == 0);
         const bool wval = WSD && own && f < valid_frames;
-        const int moff = WSD ? (it & 1) * S::MROW : 0;
+        const int moff = MB2 ? (it & 1) * S::MROW : 0;
         const bool next_real = it + 1 < my_iters && f + 1 <= F - 1;
         if (next_real) {                                                            // the hop of frame f + 1 -> the free ring slots
 #pragma unroll
@@ -706,18 +712,18 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
                     // (Geo1024: q >= 1 keeps k and M - k inside one 128-bin skew block per lane: constant offsets from mlo / mhi)
                     const float ga = (Geo::G == 32 && q > 0) ? mlo[moff + 16 * q] : mb[moff + mpos<Geo>(k)];
                     const float gb = (Geo::G == 32 && q > 0) ? mhi[moff - 16 * q] : mb[moff + mpos<Geo>(M - k)];
-                    mask_merge<PM, !WSD>(xa, xb, ga, gb, core.twn[q], WSD ? wval : own, ra[q], rb[q], ca[q], cbv[q]);
+                    mask_merge<PM, !WSD>(xa, xb, ga, gb, core.twn[q], WSD ? wval : own && !L1, ra[q], rb[q], ca[q], cbv[q]);
                 }
                 const float gmid = mb[moff + mpos<Geo>(M / 2)];
                 const float2 xmid = make_float2(2.0f * v[V / 2].x, -2.0f * v[V / 2].y);   // bin M/2 pairs with itself: X = 2 conj(Z[M/2])
                 if (WSD) { if (wval) rmid = gmid * (xmid.x * xmid.x + xmid.y * xmid.y); }
-                else if (own) rmid = fmaxf(PM ? gmid : gmid * (xmid.x * xmid.x + xmid.y * xmid.y), 0.0f);
+                else if (own && !L1) rmid = fmaxf(PM ? target_power<PM>(gmid) : gmid * (xmid.x * xmid.x + xmid.y * xmid.y), 0.0f);
                 __syncwarp();
-                if (next_real) stage_mask_row<Geo>(mb + (S::MROW - moff) * WSD, mrow0 + (long long)(f + 1) * a.mask_stride, mask_padded, jg);
+                if (next_real) stage_mask_row<Geo>(mb + (S::MROW - moff) * MB2, mrow0 + (long long)(f + 1) * a.mask_stride, mask_padded, jg);
                 cp_async_commit();                                                  // group M(f + 1)
                 mask_group_open = false;
                 float2 ymid;                                                        // 2 Y[M/2]: conj(Zinv[M/2]), same factor 2 as merge_pair_conj
-                if (PM) { ymid = apply_gain<true>(xmid, gmid); ymid.x *= 2.0f; ymid.y *= 2.0f; }
+                if (PM) { ymid = apply_gain<PM>(xmid, gmid); ymid.x *= 2.0f; ymid.y *= 2.0f; }
                 else { const float sm = 2.0f * fast_sqrt(gmid); ymid = make_float2(sm * xmid.x, sm * xmid.y); }
                 core.scatter_mirror(ca, cbv, ymid, v);
                 core.pre_inverse(v);
@@ -817,6 +823,26 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
                     reinterpret_cast<float2*>(a.wsd_terms)[(long long)u * F + f] = ed;
                     wmax = fmaxf(wmax, ed.x);
                 }
+            } else if (L1) {
+                // |lp - log(|C|^2 + eps)| with lp re-read from the frame's mask row (st2: this lane's part of the run's sum)
+                float2 zm[NP];
+                core.fetch_mirror(v, zm, lane);
+                if (own) {
+#pragma unroll
+                    for (int q = 0; q < NP; ++q) {
+                        const int k = core.pair_bin(q);
+                        float2 xa, xb;
+                        split_pair(v[q], zm[q], core.twn[q], xa, xb);
+                        const float ga = (Geo::G == 32 && q > 0) ? mlo[moff + 16 * q] : mb[moff + mpos<Geo>(k)];
+                        const float gb = (Geo::G == 32 && q > 0) ? mhi[moff - 16 * q] : mb[moff + mpos<Geo>(M - k)];
+                        st2.x += fabsf(ga - fast_log(xa.x * xa.x + xa.y * xa.y + a.l1_eps));
+                        st2.y += fabsf(gb - fast_log(xb.x * xb.x + xb.y * xb.y + a.l1_eps));
+                    }
+                    if (core.leader) {
+                        const float ptm = 4.0f * (v[V / 2].x * v[V / 2].x + v[V / 2].y * v[V / 2].y);
+                        acc[sekern::SUM_SPEC_ST] += fabsf(mb[moff + mpos<Geo>(M / 2)] - fast_log(ptm + a.l1_eps));
+                    }
+                }
             } else {
                 float2 zm[NP];
                 core.fetch_mirror(v, zm, lane);
@@ -868,7 +894,10 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
                 float s = acc[i];
 #pragma unroll
                 for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(kFull, s, o);
-                if (lane == 0 && active && s != 0.0f) atomicAdd(a.sums + (long long)u * sekern::NSUMS + i, (double)s);
+                if (lane == 0 && active && s != 0.0f) {
+                    atomicAdd(a.sums + (long long)u * sekern::NSUMS + i, (double)s);
+                    if (L1 && i == sekern::SUM_SPEC_ST) atomicAdd(a.l1_acc, (double)s);
+                }
             }
         } else {
             // groups of G lanes: through the group's (now idle) transpose buffer
@@ -880,12 +909,16 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
             if (active && jg < sekern::NSUMS) {
                 float s = 0.0f;
                 for (int l = 0; l < G; ++l) s += red[jg * G + l];
-                if (s != 0.0f) atomicAdd(a.sums + (long long)u * sekern::NSUMS + jg, (double)s);
+                if (s != 0.0f) {
+                    atomicAdd(a.sums + (long long)u * sekern::NSUMS + jg, (double)s);
+                    if (L1 && jg == sekern::SUM_SPEC_ST) atomicAdd(a.l1_acc, (double)s);
+                }
             }
         }
     }
     // one atomic per run; the buffer rests at 0.0f, and non-negative floats order as their bit patterns
     if (WSD && active && core.leader && wmax > 0.0f) atomicMax(reinterpret_cast<int*>(a.wsd_max), __float_as_int(wmax));
+    if (L1 && active && core.leader && ri == 0) atomicAdd(a.l1_acc + 1, (double)valid_frames * (M + 1));   // the element count
     if (TRACE) trace_end(a.trace, 3, smem + Z::SMEM);
 }
 
@@ -898,9 +931,11 @@ template <class Geo, bool TRACE> int prepare_geo() {
     SE_OPT((stft_run_kernel<Geo, false, false, TRACE>), K1Sz<Geo>::SMEM);
     SE_OPT((stft_run_kernel<Geo, true, false, TRACE>), K1Sz<Geo>::SMEM);
     SE_OPT((stft_run_kernel<Geo, false, true, TRACE>), K1Sz<Geo>::SMEM);
-    SE_OPT((mask_istft_run_kernel<Geo, false, TRACE>), K3Sz<Geo>::SMEM);
-    SE_OPT((mask_istft_run_kernel<Geo, true, TRACE>), K3Sz<Geo>::SMEM);
-    SE_OPT((mask_istft_run_kernel<Geo, false, TRACE, true>), (K3Sz<Geo, 2>::SMEM));
+    SE_OPT((mask_istft_run_kernel<Geo, 0, TRACE>), K3Sz<Geo>::SMEM);
+    SE_OPT((mask_istft_run_kernel<Geo, 1, TRACE>), K3Sz<Geo>::SMEM);
+    SE_OPT((mask_istft_run_kernel<Geo, 2, TRACE>), K3Sz<Geo>::SMEM);
+    SE_OPT((mask_istft_run_kernel<Geo, 0, TRACE, true>), (K3Sz<Geo, 2>::SMEM));
+    SE_OPT((mask_istft_run_kernel<Geo, 2, TRACE, false, true>), (K3Sz<Geo, 2>::SMEM));
 #undef SE_OPT
     return TRACE ? SE_OK : prepare_geo<Geo, true>();
 }
@@ -963,7 +998,7 @@ template <class Geo> int launch_mask_istft_geo(const MaskIstftArgs& a, cudaStrea
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3((unsigned)grid);
     cfg.blockDim = dim3(WARPS * 32);
-    cfg.dynamicSmemBytes = a.wsd_terms ? K3Sz<Geo, 2>::SMEM : K3Sz<Geo>::SMEM;
+    cfg.dynamicSmemBytes = (a.wsd_terms || a.l1_acc) ? K3Sz<Geo, 2>::SMEM : K3Sz<Geo>::SMEM;
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;       // prologue overlaps the upstream kernel's tail
@@ -971,9 +1006,11 @@ template <class Geo> int launch_mask_istft_geo(const MaskIstftArgs& a, cudaStrea
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     void (*kernel)(MaskIstftArgs, GeoRunPlan) =
-        a.wsd_terms ? (a.trace ? mask_istft_run_kernel<Geo, false, true, true> : mask_istft_run_kernel<Geo, false, false, true>)
-        : a.mask_is_power ? (a.trace ? mask_istft_run_kernel<Geo, true, true> : mask_istft_run_kernel<Geo, true, false>)
-                          : (a.trace ? mask_istft_run_kernel<Geo, false, true> : mask_istft_run_kernel<Geo, false, false>);
+        a.wsd_terms ? (a.trace ? mask_istft_run_kernel<Geo, 0, true, true> : mask_istft_run_kernel<Geo, 0, false, true>)
+        : a.l1_acc ? (a.trace ? mask_istft_run_kernel<Geo, 2, true, false, true> : mask_istft_run_kernel<Geo, 2, false, false, true>)
+        : a.mask_is_power == 2 ? (a.trace ? mask_istft_run_kernel<Geo, 2, true> : mask_istft_run_kernel<Geo, 2, false>)
+        : a.mask_is_power ? (a.trace ? mask_istft_run_kernel<Geo, 1, true> : mask_istft_run_kernel<Geo, 1, false>)
+                          : (a.trace ? mask_istft_run_kernel<Geo, 0, true> : mask_istft_run_kernel<Geo, 0, false>);
     SE_CUDA_CHECK(cudaLaunchKernelEx(&cfg, kernel, a, plan));
     return secommon::check_launch("mask_istft_run_kernel");
 }

@@ -453,6 +453,54 @@ __global__ void __launch_bounds__(256) wsd_finish_mean_kernel(const double* __re
 // the evaluation step's WSD terms (se_mask_istft_wsd) -> loss_per_utt; one CTA per utterance.  Every thread sums its own run of
 // consecutive frames, then a fixed reduction order: the result does not change from run to run.  The last CTA to finish puts the
 // maximum and the CTA counter back to 0 for the next step (a captured step then needs no fill node).
+// the slow route of the evaluation step's L1: sum |lp - log(tar + eps)| over each utterance's valid frames of row-strided
+// (n_utt, n_frames, ld) tensors -> sums[u, SE_SUM_SPEC_ST] and l1_acc[0]; the first chunk of each utterance adds its element count
+// to l1_acc[1] (the same contract as se_mask_istft_l1's sums)
+__global__ void __launch_bounds__(256) l1_eval_sums_kernel(const float* __restrict__ logp, long long ld_lp, const float* __restrict__ tar,
+                                                           long long ld_tar, const long long* __restrict__ lengths, long long T, int hop,
+                                                           int K, float eps, double* sums, double* l1_acc, int chunks) {
+    const int u = blockIdx.x / chunks, chunk = blockIdx.x - u * chunks;
+    const long long F = T / hop + 1;
+    const long long len = lengths ? min(T, max(0LL, lengths[u])) : T;
+    const long long valid = min(F, len / hop + 1) * K;
+    const long long per = (valid + chunks - 1) / chunks;
+    const long long lo = chunk * per, hi = min(valid, lo + per);
+    const float* p = logp + (long long)u * F * ld_lp;
+    const float* t = tar + (long long)u * F * ld_tar;
+    float acc[1] = {0.f};
+    for (long long i = lo + threadIdx.x; i < hi; i += blockDim.x) {
+        const long long f = i / K, k = i - f * K;
+        acc[0] += fabsf(p[f * ld_lp + k] - logf(t[f * ld_tar + k] + eps));
+    }
+    block_accumulate_to<1, float>(acc, sums + (long long)u * SE_NSUMS + SE_SUM_SPEC_ST);
+    block_accumulate_to<1, float>(acc, l1_acc);
+    if (chunk == 0 && threadIdx.x == 0) atomicAdd(l1_acc + 1, (double)valid);
+}
+
+// the evaluation step's L1 (se_mask_istft_l1, or the slow route's se_l1_eval_sums) -> per-utterance and batch losses; one
+// CTA.  Thread 0 reads the (all-reduced) [sum, count] pair before the barrier and clears it after: a captured step needs no fill.
+__global__ void __launch_bounds__(256) l1_eval_finish_kernel(const double* __restrict__ sums, const long long* __restrict__ lengths,
+                                                             int n_utt, long long T, int hop, long long K, double* l1_acc,
+                                                             float* __restrict__ loss_per_utt, float* __restrict__ loss,
+                                                             double* __restrict__ metric_acc) {
+    __shared__ double s_acc[2];
+    if (threadIdx.x == 0) { s_acc[0] = __ldcg(l1_acc); s_acc[1] = __ldcg(l1_acc + 1); }
+    const long long F = T / hop + 1;
+    for (int u = threadIdx.x; u < n_utt; u += blockDim.x) {
+        const long long len = lengths ? min(T, max(0LL, lengths[u])) : T;
+        const long long frames = min(F, len / hop + 1);
+        loss_per_utt[u] = (float)(sums[(long long)u * SE_NSUMS + SE_SUM_SPEC_ST] / (double)(frames * K));
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const float l = (float)(s_acc[0] / s_acc[1]);
+        loss[0] = l;
+        if (metric_acc) metric_acc[0] += (double)n_utt * (double)l;
+        l1_acc[0] = 0.0;
+        l1_acc[1] = 0.0;
+    }
+}
+
 __global__ void __launch_bounds__(256) wsd_eval_finish_kernel(const float2* __restrict__ terms, const double* __restrict__ sums,
                                                               int n_frames, float alpha, float db_interval, float eps,
                                                               float* wsd_state, float* __restrict__ loss, double* __restrict__ metric_acc) {
@@ -1197,6 +1245,27 @@ int se_wsd_eval_finish(const float* frame_terms, const double* sums, int64_t n_u
                                                                               (int)n_frames, alpha, db_interval, eps, wsd_state,
                                                                               loss_per_utt, metric_acc);
     return secommon::check_launch("wsd_eval_finish_kernel");
+}
+
+int se_l1_eval_sums(const float* log_predicted, int64_t ld_lp, const float* linear_tar, int64_t ld_tar, const int64_t* lengths,
+                    int64_t n_utt, int64_t T, int hop, int64_t K, float eps, double* sums, double* l1_acc, void* stream) {
+    SE_REQUIRE(log_predicted && linear_tar && sums && l1_acc && n_utt > 0 && T > 0 && hop > 0 && K > 0, "bad argument");
+    SE_REQUIRE(ld_lp >= K && ld_tar >= K && K <= 0x7fffffffLL, "ld_lp / ld_tar smaller than K");
+    const int chunks = pick_chunks(n_utt, (T / hop + 1) * K, 8192);
+    SE_REQUIRE(n_utt * chunks <= 0x7fffffffLL, "too many utterances");
+    l1_eval_sums_kernel<<<(unsigned)(n_utt * chunks), 256, 0, (cudaStream_t)stream>>>(
+        log_predicted, (long long)ld_lp, linear_tar, (long long)ld_tar, reinterpret_cast<const long long*>(lengths), (long long)T, hop,
+        (int)K, eps, sums, l1_acc, chunks);
+    return secommon::check_launch("l1_eval_sums_kernel");
+}
+
+int se_l1_eval_finish(const double* sums, const int64_t* lengths, int64_t n_utt, int64_t T, int hop, int64_t K, double* l1_acc,
+                      float* loss_per_utt, float* loss, double* metric_acc, void* stream) {
+    SE_REQUIRE(sums && l1_acc && loss_per_utt && loss && n_utt > 0 && T > 0 && hop > 0 && K > 0, "bad argument");
+    SE_REQUIRE(n_utt <= 0x7fffffffLL, "too many utterances");
+    l1_eval_finish_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(sums, reinterpret_cast<const long long*>(lengths), (int)n_utt,
+                                                              (long long)T, hop, (long long)K, l1_acc, loss_per_utt, loss, metric_acc);
+    return secommon::check_launch("l1_eval_finish_kernel");
 }
 
 int se_l1_logspec_fwd(const float* log_predicted, const float* linear_tar, const int64_t* stft_len, int64_t n_utt,

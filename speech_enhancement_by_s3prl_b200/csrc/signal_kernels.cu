@@ -330,6 +330,8 @@ int se_mask_istft_ex(const float* noisy, const float* clean, int64_t utt_stride,
     const int want_spec = (flags & SE_FLAG_WANT_SPEC) ? 1 : 0;
     SE_REQUIRE(noisy && mask && window && wav_out, "null pointer");
     SE_REQUIRE(mask_stride >= n_fft / 2 + 1, "mask_stride=%lld smaller than K", (long long)mask_stride);
+    SE_REQUIRE(!((flags & SE_FLAG_MASK_IS_POWER) && (flags & SE_FLAG_MASK_IS_LOG_POWER)),
+               "SE_FLAG_MASK_IS_POWER and SE_FLAG_MASK_IS_LOG_POWER are mutually exclusive");
     int rc = check_geometry(n_utt, T, n_fft, hop);
     if (rc != SE_OK) return rc;
     DeviceTables t;
@@ -341,7 +343,7 @@ int se_mask_istft_ex(const float* noisy, const float* clean, int64_t utt_stride,
     a.tab.window = window; a.tab.twM = t.twM; a.tab.twN = t.twN;
     a.wav_out = wav_out; a.out_stride = out_stride; a.out_len = hop * (a.n_frames - 1); a.pad_to = (int)pad_to;
     a.sums = sums; a.want_spec = (want_spec && clean && sums) ? 1 : 0; a.mask_stride = mask_stride;
-    a.mask_is_power = (flags & SE_FLAG_MASK_IS_POWER) ? 1 : 0;
+    a.mask_is_power = (flags & SE_FLAG_MASK_IS_LOG_POWER) ? 2 : (flags & SE_FLAG_MASK_IS_POWER) ? 1 : 0;
     a.trace = secommon::trace_ptr();
     SE_REQUIRE(out_stride >= a.out_len && out_stride >= pad_to, "out_stride=%lld too small", (long long)out_stride);
     cudaStream_t st = (cudaStream_t)stream;
@@ -381,6 +383,43 @@ int se_mask_istft_wsd(const float* noisy, const float* clean, int64_t utt_stride
     a.wav_out = wav_out; a.out_stride = out_stride; a.out_len = hop * (a.n_frames - 1); a.pad_to = (int)pad_to;
     a.sums = sums; a.want_spec = 0; a.mask_stride = mask_stride;
     a.wsd_terms = frame_terms; a.wsd_max = wsd_state;
+    a.trace = secommon::trace_ptr();
+    SE_REQUIRE(out_stride >= a.out_len && out_stride >= pad_to, "out_stride=%lld too small", (long long)out_stride);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!(flags & SE_FLAG_SUMS_ZEROED)) SE_CUDA_CHECK(cudaMemsetAsync(sums, 0, sizeof(double) * SE_NSUMS * n_utt, st));
+    if (flags & SE_FLAG_WS_SELF_CLEAN) {
+        a.zero_ptr = sums - 2LL * ((n_fft / 2 + 1 + 3) / 4 * 4) * n_utt;
+        a.zero_count = 2LL * ((n_fft / 2 + 1 + 3) / 4 * 4) * n_utt;
+    }
+    return sefast::launch_mask_istft_run(a, n_fft, st);
+}
+
+int se_mask_istft_l1_supported(int n_fft, int hop) { return (sefast::geo_supported(n_fft, hop) && !g_force_generic) ? 1 : 0; }
+
+int se_mask_istft_l1(const float* noisy, const float* clean, int64_t utt_stride, const float* mask, int64_t mask_stride,
+                     const int64_t* lengths, int64_t n_utt, int64_t T, int n_fft, int hop, const float* window,
+                     float* wav_out, int64_t out_stride, int64_t pad_to, double* sums, double* l1_acc, float eps, int flags,
+                     void* stream) {
+    SE_REQUIRE(noisy && clean && mask && window && wav_out && sums && l1_acc, "null pointer");
+    SE_REQUIRE(mask_stride >= n_fft / 2 + 1, "mask_stride=%lld smaller than K", (long long)mask_stride);
+    SE_REQUIRE(eps > 0.0f, "eps=%g must be positive", (double)eps);
+    SE_REQUIRE(!(flags & (SE_FLAG_WANT_SPEC | SE_FLAG_MASK_IS_POWER)), "se_mask_istft_l1: flags may hold SE_FLAG_SUMS_ZEROED, "
+               "SE_FLAG_WS_SELF_CLEAN and SE_FLAG_MASK_IS_LOG_POWER only");
+    int rc = check_geometry(n_utt, T, n_fft, hop);
+    if (rc != SE_OK) return rc;
+    if (!se_mask_istft_l1_supported(n_fft, hop) || T / hop + 1 < 6)        // the frame count se_mask_istft_ex's fast path needs
+        return fail(SE_ERR_UNSUPPORTED, "se_mask_istft_l1: n_fft=%d hop=%d T=%lld has no register-resident kernel (use se_mask_istft_ex "
+                    "with SE_FLAG_MASK_IS_LOG_POWER and se_l1_logspec_fwd on the clean power spectrum)", n_fft, hop, (long long)T);
+    DeviceTables t;
+    if ((rc = get_tables(n_fft, &t)) != SE_OK) return rc;
+    MaskIstftArgs a{};
+    a.noisy = noisy; a.clean = clean; a.utt_stride = utt_stride; a.mask = mask;
+    a.lengths = reinterpret_cast<const long long*>(lengths);
+    a.n_utt = (int)n_utt; a.T = (int)T; a.hop = hop; a.n_frames = (int)(T / hop) + 1;
+    a.tab.window = window; a.tab.twM = t.twM; a.tab.twN = t.twN;
+    a.wav_out = wav_out; a.out_stride = out_stride; a.out_len = hop * (a.n_frames - 1); a.pad_to = (int)pad_to;
+    a.sums = sums; a.want_spec = 0; a.mask_stride = mask_stride;
+    a.mask_is_power = 2; a.l1_acc = l1_acc; a.l1_eps = eps;
     a.trace = secommon::trace_ptr();
     SE_REQUIRE(out_stride >= a.out_len && out_stride >= pad_to, "out_stride=%lld too small", (long long)out_stride);
     cudaStream_t st = (cudaStream_t)stream;

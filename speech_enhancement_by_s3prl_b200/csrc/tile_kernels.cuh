@@ -84,9 +84,12 @@ struct MaskIstftArgs {
     unsigned long long* trace; // CTA timeline buffer (se_set_trace) or null
     double* zero_ptr;          // SE_FLAG_WS_SELF_CLEAN: doubles zeroed after the upstream kernel has completed (or null)
     long long zero_count;
-    int mask_is_power;         // `mask` holds the TARGET power spectrum: output = iSTFT(sqrt(mask) e^{i phase(noisy)}) (runner.py:266-281)
+    int mask_is_power;         // 1: `mask` holds the TARGET power spectrum: output = iSTFT(sqrt(mask) e^{i phase(noisy)}) (runner.py:266-281);
+                               // 2: its log (SE_FLAG_MASK_IS_LOG_POWER, model.LSTM's log_predicted): the target power is exp(mask)
     float* wsd_terms;          // se_mask_istft_wsd (fastgeo.cu only): (n_utt, n_frames) float2 {E_f, D_f}, or null
     float* wsd_max;            // idem: the batch's largest E_f (1 float, at rest 0.0f)
+    double* l1_acc;            // se_mask_istft_l1 (fastgeo.cu only): [sum |lp - log(|C|^2 + eps)|, element count] += this batch's, or null
+    float l1_eps;
 };
 
 SE_HD int imin(int a, int b) { return a < b ? a : b; }
@@ -366,7 +369,8 @@ SE_HD void mask_istft_tile(Exec& ex, const MaskIstftArgs& a, int utt, int tile, 
             float2 xa = rfft_split(za, zb, s.twN[k]);
             float2 xb = rfft_split(zb, za, s.twN[k2]);
             if (k == 0) { xa.y = 0.0f; xb.y = 0.0f; }
-            const float ga = mk[k], gb = mk[k2];
+            float ga = mk[k], gb = mk[k2];
+            if (a.mask_is_power == 2) { ga = expf(ga); gb = expf(gb); }     // log target power -> power
             float2 ya, yb;
             if (a.mask_is_power) {            // polar(sqrt(power), phase(X)); phase(0) = 0
                 const float qa = xa.x * xa.x + xa.y * xa.y, qb = xb.x * xb.x + xb.y * xb.y;

@@ -25,22 +25,43 @@ def _c64(lengths):
     return lengths if lengths.dtype == torch.int64 and lengths.is_contiguous() else lengths.to(torch.int64).contiguous()
 
 
-def _eval_wsd(criterion):
-    """The evaluation step's loss: False for None / objective.SISDR (spectral SI-SDR), True for objective.WSD."""
-    from . import objective as obj
+def _eval_loss(criterion, head=None):
+    """The evaluation step's loss: "sisdr" for None / objective.SISDR (spectral SI-SDR), "wsd" for objective.WSD, "l1" for
+    objective.L1.  The pairs follow the reference's ``criterion(**locals(), **model_results)`` call (runner.py:575): WSD reads
+    ``offset`` (LinearResidual, Residual), L1 reads ``log_predicted`` (LSTM); any other pair raises, as the reference raises
+    TypeError."""
+    from . import model, objective as obj
+    kind = type(head).__name__ if head is not None else None
     if criterion is None or type(criterion) is obj.SISDR:
-        return False
-    if type(criterion) is obj.WSD:
-        return True
-    raise RuntimeError(f"EnhancementEngine: no evaluation route for the criterion {type(criterion).__name__} (supported: None, "
-                       "objective.SISDR, objective.WSD)")
+        return "sisdr"
+    if type(criterion) is obj.WSD and (head is None or type(head) in (model.LinearResidual, model.Residual)):
+        return "wsd"
+    if type(criterion) is obj.L1 and (head is None or type(head) is model.LSTM):
+        return "l1"
+    raise RuntimeError(f"EnhancementEngine: no evaluation route for the criterion {type(criterion).__name__}"
+                       f"{' with a ' + kind + ' head' if kind else ''} (supported: None, objective.SISDR, objective.WSD with "
+                       "LinearResidual / Residual, objective.L1 with LSTM)")
+
+
+def _eval_wsd(criterion):
+    """True for objective.WSD (see _eval_loss)."""
+    return _eval_loss(criterion) == "wsd"
 
 
 def _criterion_key(criterion):
     """What a captured evaluation step bakes in of its criterion."""
-    if not _eval_wsd(criterion):
-        return None
-    return ("WSD", float(criterion.alpha), float(criterion.db_interval), float(criterion.eps))
+    loss = _eval_loss(criterion)
+    if loss == "wsd":
+        return ("WSD", float(criterion.alpha), float(criterion.db_interval), float(criterion.eps))
+    if loss == "l1":
+        return ("L1", float(criterion.eps))
+    return None
+
+
+def _recurrent(head):
+    """True for the heads with a cuDNN LSTM body (model.LSTM, model.Residual)."""
+    from . import model
+    return type(head) in (model.LSTM, model.Residual)
 
 
 class EnhancementEngine:
@@ -67,10 +88,11 @@ class EnhancementEngine:
     # ------------------------------------------------------------------ device-resident step
     def step_workspace(self, B, device, criterion=None):
         """Persistent, zeroed workspace of one captured evaluation step: [CMVN sums (B, round4(K), 2) | K3 sums (B, 6)] doubles,
-        + one double (the WSD maximum and the finish kernel's CTA counter) with an objective.WSD criterion.
+        + one double (the WSD maximum and the finish kernel's CTA counter) with an objective.WSD criterion, or two (the L1 sum
+        and element count) with objective.L1.
         The step's kernels leave it zeroed for the next replay (SE_FLAG_WS_SELF_CLEAN), so the graph has no fill node."""
         LD = ops.round4(self.n_fft // 2 + 1)
-        extra = 1 if _eval_wsd(criterion) else 0
+        extra = {"sisdr": 0, "wsd": 1, "l1": 2}[_eval_loss(criterion)]
         return torch.zeros(B * (2 * LD + ops.NSUMS) + extra, device=device, dtype=torch.float64)
 
     def eval_step(self, lengths, wavs, want_spec_loss=True, metric_acc=None, ws=None, want_stoi=False, stoi_acc=None,
@@ -83,6 +105,11 @@ class EnhancementEngine:
         global batch, so under data parallelism every rank must run the step for every batch).  On the register-resident
         geometries (n_fft / hop 512 / 256, 1024 / 256, 400 / 160) the WSD terms come out of K3 itself; on any other geometry
         from both channels' power spectra through ops.wsd_energy / ops.wsd_mask_step -- a slower route that materialises them.
+        objective.L1 (model.LSTM heads only): loss_per_utt[u] is utterance u's own L1 and out["loss"] (1,) the batch's -- the
+        element mean over every rank's valid frames (its [sum, count] pair is all-reduced), which is what the criterion returns;
+        metric_acc[0] += B * loss.  Other geometries and steps under 6 frames take a slower route through the clean power spectrum.
+        head: LinearResidual (fused K1 / K2), or a recurrent LSTM / Residual: the cuDNN body runs through torch between K1 and the
+        library's projection; LSTM's output is log_predicted and K3 decodes exp(log_predicted) with the noisy phase.
         metric_acc: float64 (3,) device tensor += [sum loss, sum SI-SDR, utterances] (the running sums of an evaluation
         pass, runner.py:587-602; ``dp.means_from_acc`` turns them into the global means with one all-reduce).  Without
         want_spec_loss the loss sum is left as it is; SI-SDR and the count are still added.
@@ -90,15 +117,17 @@ class EnhancementEngine:
         fresh one per call.
         want_stoi: also return "stoi" and "estoi" (B,) of wav_predicted against the target channel, at the preprocessor's
         sample rate (``ops.stoi``); stoi_acc: float64 (3,) device tensor += [sum STOI, sum ESTOI, utterances]."""
-        wsd = _eval_wsd(criterion) and want_spec_loss
-        want_spec_loss = want_spec_loss and not wsd             # the spectral SI-SDR sums of K3
+        head = self.head
+        crit = _eval_loss(criterion, head) if want_spec_loss else (_eval_loss(criterion, head) and "sisdr")
+        wsd, l1 = crit == "wsd", crit == "l1"
+        want_spec_loss = want_spec_loss and crit == "sisdr"     # the spectral SI-SDR sums of K3
+        log_power = type(head).__name__ == "LSTM"               # K3 decodes exp(log_predicted)
         B, C, T = wavs.shape
         dev = wavs.device
         window = self.pre._frame_window
         if window.device != dev:
             self.pre.to(dev)
             window = self.pre._frame_window
-        head = self.head
         K = self.n_fft // 2 + 1
         with torch.no_grad():
             # internal tensors use rows padded to 16 bytes (K = 257 -> 260 floats): TMA / 128-bit loads for the
@@ -108,7 +137,10 @@ class EnhancementEngine:
             wpad = self._padded_weight()
             Dout = wpad.shape[0]
             D = self._mel_feature_dim() if self.feat_cfg is not None else K
-            if self.feat_cfg is not None:
+            if _recurrent(head):
+                mask = self._recurrent_front(wavs, D, wpad)
+                k3 = {}
+            elif self.feat_cfg is not None:
                 # head input = a mel feature config (e.g. pseudo_noise.yaml:10-15) built by the fused K1b kernel from the
                 # power spectrum; the mask still applies to the K bins of the noisy spectrum
                 if D is None or D % 4 or Dout != K or not ops.linear_head_tma_supported(B, F, D, K, D, wpad.shape[1], LD):
@@ -145,11 +177,39 @@ class EnhancementEngine:
                 mask = ops.linear_head_padded(feats, K, wpad, head.linear.bias, head.activation, mean, std,
                                               head.eps, precision=self.precision)
                 k3 = {}
-            if wsd and ops.mask_istft_wsd_supported(self.n_fft, self.hop) and F >= 6:
+            extra = None                                         # the criterion's persistent state at the workspace's end
+            if ws is not None and ws.numel() > B * (2 * LD + ops.NSUMS):
+                extra = ws[B * (2 * LD + ops.NSUMS):]
+            batch_loss = None
+            if l1:
+                # K3 (log-power target) with the L1 sums, or the slow route -> all-reduce of [sum, count] on the side stream under
+                # K3' -> the finish kernel
+                l1_acc = extra if extra is not None and extra.numel() == 2 else torch.zeros(2, device=dev, dtype=torch.float64)
+                self.launches_per_step += 1                         # the finish kernel (K3-L1 replaces K3)
+                if ops.mask_istft_l1_supported(self.n_fft, self.hop) and F >= 6:
+                    wav, sums = ops.mask_istft_l1(wavs, self.ch_inp, self.ch_tar, mask, lengths, self.n_fft, self.hop, window,
+                                                  pad_to=T, l1_acc=l1_acc, eps=criterion.eps, **k3)
+                else:
+                    wav, sums = ops.mask_istft(wavs, self.ch_inp, self.ch_tar, mask, lengths, self.n_fft, self.hop, window,
+                                               pad_to=T, want_sums=True, want_spec=False, mask_padded=True, mask_is_log_power=True,
+                                               **k3)
+                    self._l1_terms_from_spectra(wavs, mask, lengths, criterion, sums, l1_acc)
+                main = torch.cuda.current_stream(dev)
+                side = self._side_stream(dev) if dp.world()[1] > 1 else None
+                if side is not None:
+                    side.wait_stream(main)
+                    with torch.cuda.stream(side):
+                        dp.reduce_sums(l1_acc)
+                gain, sisdr, _ = ops.finalize_metrics(sums, lengths, T, wav=wav, target_db=None, want_loss=False,
+                                                      metric_acc=metric_acc)
+                if side is not None:
+                    main.wait_stream(side)
+                loss, batch_loss = ops.l1_eval_finish(sums, lengths, T, self.hop, K, l1_acc, metric_acc)
+            elif wsd and ops.mask_istft_wsd_supported(self.n_fft, self.hop) and F >= 6:
                 # K3 with the WSD terms -> all-reduce(max) of its 4-byte maximum on the side stream under K3' -> the finish kernel
                 self.launches_per_step += 1
-                if ws is not None and ws.numel() == B * (2 * LD + ops.NSUMS) + 1:
-                    state = ws[B * (2 * LD + ops.NSUMS):].view(torch.float32)    # the step leaves it zeroed
+                if extra is not None and extra.numel() == 1:
+                    state = extra.view(torch.float32)                  # the step leaves it zeroed
                 else:
                     state = torch.zeros(2, device=dev, dtype=torch.float32)
                 wav, sums, terms = ops.mask_istft_wsd(wavs, self.ch_inp, self.ch_tar, mask, lengths, self.n_fft, self.hop, window,
@@ -167,17 +227,72 @@ class EnhancementEngine:
                 loss = ops.wsd_eval_finish(terms, sums, state, criterion.alpha, criterion.db_interval, criterion.eps, metric_acc)
             else:
                 wav, sums = ops.mask_istft(wavs, self.ch_inp, self.ch_tar, mask, lengths, self.n_fft, self.hop, window,
-                                           pad_to=T, want_sums=True, want_spec=want_spec_loss, mask_padded=True, **k3)
+                                           pad_to=T, want_sums=True, want_spec=want_spec_loss, mask_padded=True,
+                                           mask_is_log_power=log_power, **k3)
                 gain, sisdr, loss = ops.finalize_metrics(sums, lengths, T, wav=wav, target_db=None, want_loss=want_spec_loss,
                                                          metric_acc=metric_acc)
                 if wsd:
                     self.launches_per_step += 8     # 2 STFTs, energies (+ fill), sums (+ fill), finish, the accumulator's sum + add
                     loss = self._wsd_terms_from_spectra(wavs, mask, lengths, criterion, metric_acc)
             out = {"loss_per_utt": loss, "sisdr": sisdr, "wav_predicted": wav, "gain": gain, "mask": mask[..., :K]}
+            if batch_loss is not None:
+                out["loss"] = batch_loss
             if want_stoi:
                 # after K3' (both metrics are invariant to the gain of the estimate); the clean channel is read in place
                 out["stoi"], out["estoi"] = ops.stoi(wav, wavs[:, self.ch_tar], lengths, fs=self.pre._sample_rate, acc=stoi_acc)
         return out
+
+    def _recurrent_front(self, wavs, D, wpad):
+        """K1 -> cuDNN LSTM body (torch, no_grad) -> [Residual's CMVN over the hidden states, torch] -> the library's projection
+        (TMA head when the hidden width is a multiple of 4 and precision=1, else the padded head) -> mask (B, F, round4(K)):
+        model.LSTM's log_predicted or model.Residual's offset.  launches_per_step counts everything but the body."""
+        head, dev = self.head, wavs.device
+        window = self.pre._frame_window
+        K = self.n_fft // 2 + 1
+        if self.feat_cfg is not None:
+            if D is None:
+                raise RuntimeError("EnhancementEngine.eval_step: feat_cfg must be a mel config (log / delta <= 2, no CMVN of its own)")
+            cfg = self.feat_cfg
+            power = ops.stft_padded(wavs, self.ch_inp, self.n_fft, self.hop, window, logpower=False)
+            feats = ops.mel_features(power, self.pre._tables(dev)[1], bool(cfg.get("log", False)), self.pre.eps,
+                                     order=int(cfg.get("delta", 0)), K=K)
+            self.launches_per_step = 2
+        else:
+            feats = ops.stft_padded(wavs, self.ch_inp, self.n_fft, self.hop, window, logpower=self.log_features, log_eps=self.pre.eps)
+            self.launches_per_step = 1
+        if head.lstm.input_size != D:
+            raise RuntimeError(f"EnhancementEngine.eval_step: the {type(head).__name__} head takes {head.lstm.input_size} features, "
+                               f"the engine's feature has {D}")
+        x = feats[..., :D]
+        if not x.is_contiguous():
+            x = x.contiguous()                                           # out of the 16-byte padded rows
+            self.launches_per_step += 1
+        hidden, _ = head.lstm(x)                                         # the cuDNN body (DESIGN section 7)
+        if type(head).__name__ == "Residual" and head.cmvn:              # model.py:88, over every frame of the padded batch
+            hidden = (hidden - hidden.mean(dim=1, keepdim=True)) / (hidden.std(dim=1, keepdim=True) + head.eps)
+            self.launches_per_step += 5
+        B, F, H = hidden.shape
+        hidden = hidden.contiguous()
+        if self.precision == 1 and H % 4 == 0 and ops.linear_head_tma_supported(B, F, H, K, H, wpad.shape[1], ops.round4(K)):
+            mask = ops.linear_head_tma(hidden, H, wpad, self._proj().bias, head.activation, None, 0.0)
+        else:
+            mask = ops.linear_head_padded(hidden, H, wpad, self._proj().bias, head.activation, None, None, 0.0,
+                                          precision=self.precision)
+        self.launches_per_step += 1 + 3                                  # projection, K3's sums fill, K3, K3'
+        return mask
+
+    def _l1_terms_from_spectra(self, wavs, mask, lengths, criterion, sums, l1_acc):
+        """objective.L1's sums where K3 has no L1 variant (other geometries, or fewer than 6 frames): the clean power spectrum is
+        materialised (one more STFT) and one reduction (se_l1_eval_sums) adds each utterance's sum to its SE_SUM_SPEC_ST column of
+        `sums` and the batch's [sum, count] to l1_acc -- what K3-L1 adds on the fused route."""
+        T = wavs.shape[2]
+        tar = ops.stft_padded(wavs, self.ch_tar, self.n_fft, self.hop, self.pre._frame_window, logpower=False)
+        ops.l1_eval_sums(mask, tar, lengths, T, self.hop, self.n_fft // 2 + 1, sums, l1_acc, criterion.eps)
+        self.launches_per_step += 2
+
+    def _proj(self):
+        """The head's output layer: LinearResidual.linear, or LSTM / Residual.scaling_layer[0]."""
+        return self.head.scaling_layer[0] if _recurrent(self.head) else self.head.linear
 
     def _wsd_terms_from_spectra(self, wavs, mask, lengths, criterion, metric_acc):
         """objective.WSD's per-utterance terms where K3 has no WSD variant (other geometries, or fewer than 6 frames): both
@@ -201,7 +316,7 @@ class EnhancementEngine:
         ONE persistent buffer per (shape, device): captured graphs bake its address in, so it is refreshed IN PLACE --
         eagerly here when the parameter's version changed (optimizer.step / load_state_dict), and by kernels inside the
         captured training step after every update (``force``; graph replays never bump ``_version``)."""
-        w = self.head.linear.weight
+        w = self._proj().weight
         Dout, Din = w.shape
         buf = getattr(self, "_wpad", None)
         if buf is None or buf.device != w.device or buf.shape != (Dout, ops.round4(Din)):
@@ -238,8 +353,15 @@ class EnhancementEngine:
         torch.cuda.current_stream(device).wait_stream(side)
         torch.cuda.synchronize(device)
         graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(graph):
-            out = self.eval_step(lengths, wavs, metric_acc=metric_acc, ws=ws, want_stoi=want_stoi, stoi_acc=stoi_acc, criterion=criterion)
+        try:
+            with torch.cuda.graph(graph):
+                out = self.eval_step(lengths, wavs, metric_acc=metric_acc, ws=ws, want_stoi=want_stoi, stoi_acc=stoi_acc,
+                                     criterion=criterion)
+        except RuntimeError as exc:
+            if not _recurrent(self.head):
+                raise
+            raise RuntimeError(f"EnhancementEngine.capture_bound: the evaluation step of the {type(self.head).__name__} head could "
+                               f"not be captured into a CUDA graph (eager eval_step still runs it): {exc}") from exc
         static = {"lengths": lengths, "wavs": wavs, "graph": graph, "ws": ws}
         static.update(out)
         return static
@@ -266,17 +388,26 @@ class EnhancementEngine:
     # ------------------------------------------------------------------ host-facing step (e2e)
     def eval_step_host(self, lengths_cpu, wavs_cpu, criterion=None):
         """The call a user makes with collate_fn's output (CPU tensors): H2D of the batch, the fused
-        step, D2H of the per-utterance loss terms and SI-SDR.  Returns (mean_loss, mean_sisdr, wav_predicted on device)."""
+        step, D2H of the per-utterance loss terms and SI-SDR.  Returns (mean_loss, mean_sisdr, wav_predicted on device).
+        mean_loss is the criterion's value of the batch: the mean of the per-utterance terms, and for objective.L1 (an element
+        mean) their mean weighted by each utterance's valid frames."""
         pipe = self.host_pipeline(*wavs_cpu.shape, depth=1, criterion=criterion)
         pipe.submit(lengths_cpu, wavs_cpu)
         loss, sisdr = pipe.drain()[0]
-        return float(loss.mean()), float(sisdr.mean()), pipe.slots[0]["wav_predicted"]
+        if _eval_loss(criterion) == "l1":
+            T = wavs_cpu.shape[2]
+            frames = (lengths_cpu.to(torch.int64).clamp(0, T) // self.hop + 1).clamp(max=T // self.hop + 1).double()
+            mean_loss = float((loss.double() * frames).sum() / frames.sum())
+        else:
+            mean_loss = float(loss.mean())
+        return mean_loss, float(sisdr.mean()), pipe.slots[0]["wav_predicted"]
 
     def host_pipeline(self, B, C, T, depth=2, device=None, pcm16=False, want_wav=False, copy_wav=True, criterion=None):
         """Host-facing evaluation loop for (B, C, T) batches; see HostPipeline.  pcm16: the host batches are int16 PCM
         (half the PCIe bytes; widened on the device); want_wav: the enhanced waveforms come back to pinned host memory
         (copy_wav=False: as views of the slot's pinned buffer, valid until that slot is submitted to again);
-        criterion: the loss the per-utterance terms are in (see eval_step)."""
+        criterion: the loss the per-utterance terms are in (see eval_step); with objective.L1 they are each utterance's own L1,
+        whose batch value is their mean weighted by valid frames, not their plain mean (eval_step_host returns the weighted one)."""
         key = ("pipe", B, C, T, depth, bool(pcm16), bool(want_wav), bool(copy_wav), _criterion_key(criterion))
         if key not in self._graphs:
             device = device or torch.device("cuda", torch.cuda.current_device())
@@ -530,7 +661,7 @@ class HostPipeline:
         self.pending = []
         self.h2d_bytes = B * self.N_CH * T * (2 if pcm16 else 4) + B * 8
         self.d2h_bytes = 2 * B * 4 + (B * T * 4 if want_wav else 0)
-        self.launches_per_step = 5 + (1 if pcm16 else 0) + (1 if _eval_wsd(criterion) else 0)   # (+ the WSD finish kernel)
+        self.launches_per_step = 5 + (1 if pcm16 else 0) + (0 if _eval_loss(criterion) == "sisdr" else 1)   # (+ a finish kernel)
         with torch.cuda.stream(self.compute_stream):
             for _ in range(depth):
                 lengths = torch.full((B,), T, dtype=torch.int64, device=device)
@@ -546,6 +677,8 @@ class HostPipeline:
                 st["busy"] = False
                 self.slots.append(st)
         torch.cuda.synchronize(device)
+        if _recurrent(engine.head):              # (the library's launches around the cuDNN body, see eval_step)
+            self.launches_per_step = engine.launches_per_step + (1 if pcm16 else 0)
         self._next = 0
 
     def submit(self, lengths_cpu, wavs_cpu):

@@ -102,7 +102,7 @@ def stft_padded(wavs, channel, n_fft, hop, window, logpower=True, log_eps=1e-10)
     return out
 
 
-FLAG_WANT_SPEC, FLAG_SUMS_ZEROED, FLAG_MASK_IS_POWER, FLAG_WS_SELF_CLEAN = 1, 2, 4, 8
+FLAG_WANT_SPEC, FLAG_SUMS_ZEROED, FLAG_MASK_IS_POWER, FLAG_WS_SELF_CLEAN, FLAG_MASK_IS_LOG_POWER = 1, 2, 4, 8, 16
 
 
 def stft_features(wavs, channel, n_fft, hop, window, logpower=True, log_eps=1e-10, stat_sums=None, self_clean=False):
@@ -437,10 +437,14 @@ def istft(power, phase, n_fft, hop, window, pad_to=0):
 
 
 def mask_istft(wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, want_sums=True, want_spec=True,
-               out=None, sums=None, mask_padded=False, sums_zeroed=False, mask_is_power=False, self_clean=False):
+               out=None, sums=None, mask_padded=False, sums_zeroed=False, mask_is_power=False, self_clean=False,
+               mask_is_log_power=False):
     """Fused ``istft(linear_inp * mask, phase_inp)`` straight from the noisy waveform.
 
-    wavs (B, C, T); mask (B, F, K); lengths (B,) int64 or None.  Returns (wav (B, width), sums (B, 6) float64|None)."""
+    wavs (B, C, T); mask (B, F, K); lengths (B,) int64 or None.  Returns (wav (B, width), sums (B, 6) float64|None).
+    mask_is_power: ``mask`` is the target power (``istft(mask, phase_inp)``); mask_is_log_power: it is the log of the target
+    power, e.g. model.LSTM's log_predicted (``istft(exp(mask), phase_inp)`` without the exp pass)."""
+    assert not (mask_is_power and mask_is_log_power), "mask_is_power and mask_is_log_power are mutually exclusive"
     wavs, mask, window = _chk(wavs, "wavs"), _c(mask, "mask"), _c(window, "window")
     assert wavs.dim() == 3 and wavs.is_contiguous()
     B, C, T = wavs.shape
@@ -458,6 +462,7 @@ def mask_istft(wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, 
         clean = None if ch_tar is None else wavs.data_ptr() + 4 * int(ch_tar) * T
         flags = (FLAG_WANT_SPEC if want_spec else 0) | (FLAG_SUMS_ZEROED if sums_zeroed else 0)
         flags |= FLAG_MASK_IS_POWER if mask_is_power else 0     # `mask` = target power; output keeps the noisy phase
+        flags |= FLAG_MASK_IS_LOG_POWER if mask_is_log_power else 0
         flags |= FLAG_WS_SELF_CLEAN if self_clean else 0        # `sums` is the tail of a persistent step workspace (see stft_features)
         rc = _lib.load().se_mask_istft_ex(wavs.data_ptr() + 4 * int(ch_inp) * T, clean, C * T, mask.data_ptr(), mask_stride,
                                           _p(lengths), B, T, n_fft, hop, window.data_ptr(), out.data_ptr(), out.stride(0),
@@ -512,6 +517,76 @@ def wsd_eval_finish(frame_terms, sums, wsd_state, alpha=0.5, db_interval=30.0, e
                                             wsd_state.data_ptr(), loss.data_ptr(), _p(metric_acc), _stream())
         _lib.check(rc, "se_wsd_eval_finish")
     return loss
+
+
+def mask_istft_l1_supported(n_fft, hop):
+    """True if ``mask_istft_l1`` has a kernel for this geometry (it also needs T // hop + 1 >= 6 frames)."""
+    return bool(_lib.load().se_mask_istft_l1_supported(int(n_fft), int(hop)))
+
+
+def mask_istft_l1(wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, l1_acc, eps=1e-10, sums=None, sums_zeroed=False,
+                  self_clean=False):
+    """``mask_istft(mask_is_log_power=True)`` whose clean-frame pass sums objective.L1's terms (se_mask_istft_l1).
+
+    mask (B, F, LD) row-padded log target power; l1_acc: float64 (2,) device buffer, zero at rest (``l1_eval_finish`` resets it),
+    += [sum |lp - log(|C|^2 + eps)|, element count] of the batch's valid frames (all-reduce it with ``dp.reduce_sums`` before the
+    finish).  Returns (wav (B, width), sums (B, 6) float64 with each utterance's L1 sum in column 3, SE_SUM_SPEC_ST)."""
+    wavs, mask, window = _chk(wavs, "wavs"), _chk(mask, "mask"), _c(window, "window")
+    l1_acc = _chk(l1_acc, "l1_acc", torch.float64)
+    assert wavs.dim() == 3 and wavs.is_contiguous()
+    assert l1_acc.numel() == 2 and l1_acc.is_contiguous()
+    B, C, T = wavs.shape
+    F, K = T // hop + 1, n_fft // 2 + 1
+    assert mask.dim() == 3 and mask.shape[:2] == (B, F) and mask.shape[2] >= K and mask.stride(2) == 1 and mask.stride(1) == mask.shape[2]
+    assert mask.stride(0) == F * mask.shape[2], "mask must be contiguous along the batch (the kernel reads row u at u * F * LD)"
+    lengths = _c(lengths, "lengths", torch.int64)
+    width = max(hop * (F - 1), int(pad_to))
+    with torch.cuda.device(wavs.device):
+        out = torch.empty(B, width, device=wavs.device, dtype=torch.float32)
+        if sums is None:
+            sums = torch.empty(B, NSUMS, device=wavs.device, dtype=torch.float64)
+        flags = (FLAG_SUMS_ZEROED if sums_zeroed else 0) | (FLAG_WS_SELF_CLEAN if self_clean else 0)
+        rc = _lib.load().se_mask_istft_l1(wavs.data_ptr() + 4 * int(ch_inp) * T, wavs.data_ptr() + 4 * int(ch_tar) * T, C * T,
+                                          mask.data_ptr(), mask.shape[2], _p(lengths), B, T, n_fft, hop, window.data_ptr(),
+                                          out.data_ptr(), out.stride(0), int(pad_to), sums.data_ptr(), l1_acc.data_ptr(), float(eps),
+                                          flags, _stream())
+        _lib.check(rc, "se_mask_istft_l1")
+    return out, sums
+
+
+def l1_eval_sums(log_predicted, linear_tar, lengths, T, hop, K, sums, l1_acc, eps=1e-10):
+    """The sums of ``mask_istft_l1`` from materialised spectra (the slow route): log_predicted and linear_tar (B, F, LD) row-padded,
+    F = T // hop + 1.  sums[:, 3] (zero) += each utterance's sum |lp - log(tar + eps)| over its valid frames; l1_acc += [batch sum,
+    element count]."""
+    B, F, LDp = log_predicted.shape
+    assert linear_tar.shape[:2] == (B, F) and F == T // hop + 1 and min(LDp, linear_tar.shape[2]) >= K
+    for t in (log_predicted, linear_tar):
+        assert t.dtype == torch.float32 and t.stride(2) == 1 and t.stride(1) == t.shape[2] and t.stride(0) == F * t.shape[2]
+    assert sums.dtype == torch.float64 and sums.shape == (B, NSUMS) and sums.is_contiguous()
+    assert l1_acc.dtype == torch.float64 and l1_acc.numel() == 2 and l1_acc.is_contiguous()
+    lengths = _c(lengths, "lengths", torch.int64)
+    with torch.cuda.device(log_predicted.device):
+        rc = _lib.load().se_l1_eval_sums(log_predicted.data_ptr(), LDp, linear_tar.data_ptr(), linear_tar.shape[2], _p(lengths), B, int(T),
+                                         int(hop), int(K), float(eps), sums.data_ptr(), l1_acc.data_ptr(), _stream())
+        _lib.check(rc, "se_l1_eval_sums")
+
+
+def l1_eval_finish(sums, lengths, T, hop, K, l1_acc, metric_acc=None):
+    """objective.L1 from ``mask_istft_l1``'s outputs (after any all-reduce of l1_acc) -> (loss_per_utt (B,), loss (1,)):
+    each utterance's own L1 and the batch's (global) L1; metric_acc (float64 (3,) or None) [0] += B * loss.  Leaves l1_acc
+    zeroed for the next step."""
+    B = sums.shape[0]
+    lengths = _c(lengths, "lengths", torch.int64)
+    assert l1_acc.dtype == torch.float64 and l1_acc.numel() == 2 and l1_acc.is_contiguous()
+    if metric_acc is not None:
+        assert metric_acc.dtype == torch.float64 and metric_acc.numel() >= 3 and metric_acc.is_contiguous()
+    with torch.cuda.device(sums.device):
+        loss_per_utt = torch.empty(B, device=sums.device)
+        loss = torch.empty(1, device=sums.device)
+        rc = _lib.load().se_l1_eval_finish(sums.data_ptr(), _p(lengths), B, int(T), int(hop), int(K), l1_acc.data_ptr(),
+                                           loss_per_utt.data_ptr(), loss.data_ptr(), _p(metric_acc), _stream())
+        _lib.check(rc, "se_l1_eval_finish")
+    return loss_per_utt, loss
 
 
 def finalize_metrics(sums, lengths, T, wav=None, target_db=None, want_gain=True, want_sisdr=True, want_loss=True,
