@@ -116,7 +116,9 @@ int se_mask_istft_strided(const float* noisy, const float* clean, int64_t utt_st
                                       SE_FLAG_SUMS_ZEROED) the step's kernels leave it zeroed for the next replay instead of the
                                       caller filling it every step: se_stft_features zeroes the `sums` part (consumed by the
                                       previous step's se_finalize_metrics), se_mask_istft_ex zeroes the stat_sums part (consumed
-                                      by this step's head) -- a captured step then has no fill node at its start */
+                                      by this step's head) -- a captured step then has no fill node at its start.  The STFT
+                                      entry points require ld_stats == round4(K) with it (SE_ERR_BAD_ARG otherwise): both ends
+                                      find the boundary from that layout */
 #define SE_FLAG_MASK_IS_LOG_POWER 16 /* se_mask_istft_ex: `mask` holds the LOG of a target power spectrum (model.LSTM's
                                       log_predicted, model.py:37-60): wav_out = iSTFT(exp(lp / 2) X / |X|), exp(lp / 2) where
                                       X = 0 -- _decode_wav(exp(lp), phase_inp) without the phase or an exp pass; with

@@ -147,9 +147,91 @@ int check_geometry(int64_t n_utt, int64_t T, int n_fft, int hop) {
     return SE_OK;
 }
 
-}  // namespace
+int g_force_generic = 0;
+constexpr int64_t kMinK3Frames = 6;     // the register-resident mask-iSTFT needs this many frames; the STFT has no minimum
 
-static int g_force_generic = 0;
+// The register-resident kernels of fastgeo.cu run this geometry (and, for K3, this many frames).
+bool register_resident(int n_fft, int hop, int64_t n_frames = kMinK3Frames) {
+    return sefast::geo_supported(n_fft, hop) && n_frames >= kMinK3Frames && !g_force_generic;
+}
+
+// SE_FLAG_WS_SELF_CLEAN's workspace opens with the CMVN statistics (n_utt, round4(K), 2), right before the K3 sums.
+int64_t ws_ld_stats(int n_fft) { return (n_fft / 2 + 1 + 3) / 4 * 4; }
+int64_t ws_stat_doubles(int n_fft, int64_t n_utt) { return 2 * ws_ld_stats(n_fft) * n_utt; }
+
+int launch_stft_generic(const StftArgs& a, int n_fft, cudaStream_t st) { SE_DISPATCH_NFFT(n_fft, launch_stft, a, st) }
+
+// K1 of every STFT entry point: validates, zeroes stat_sums unless SE_FLAG_SUMS_ZEROED, fills StftArgs and runs the
+// register-resident kernel, or the generic one (then se_feature_sums over the feature for the statistics).
+// stat_sums: the CMVN sums of logpower (else of power), or null for a plain STFT.  pair: rows n_utt .. 2 n_utt - 1 are the
+// power of a second channel chan_step floats further in every utterance (register-resident kernels only).
+int stft_entry(const float* wav, int64_t n_utt, int64_t utt_stride, bool pair, int64_t chan_step, int64_t T, int n_fft, int hop,
+               const float* window, float log_eps, float* power, float* phase, float* logpower, int64_t spec_stride,
+               double* stat_sums, int64_t ld_stats, int flags, void* stream) {
+    SE_REQUIRE(wav && window, "wav and window must not be null");
+    SE_REQUIRE(spec_stride >= n_fft / 2 + 1 && (!stat_sums || ld_stats >= n_fft / 2 + 1), "spec_stride / ld_stats smaller than K");
+    const bool self_clean = stat_sums && (flags & SE_FLAG_WS_SELF_CLEAN);
+    SE_REQUIRE(!self_clean || ld_stats == ws_ld_stats(n_fft), "SE_FLAG_WS_SELF_CLEAN: ld_stats=%lld must be round4(K)=%lld, the "
+               "step workspace's layout", (long long)ld_stats, (long long)ws_ld_stats(n_fft));
+    int rc = check_geometry(pair ? 2 * n_utt : n_utt, T, n_fft, hop);
+    if (rc != SE_OK) return rc;
+    const bool fast = register_resident(n_fft, hop);
+    if (pair && !fast)
+        return fail(SE_ERR_UNSUPPORTED, "se_stft_features_pair: n_fft=%d hop=%d has no register-resident kernel (use two "
+                    "se_stft_features2 calls)", n_fft, hop);
+    DeviceTables t;
+    if ((rc = get_tables(n_fft, &t)) != SE_OK) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (stat_sums && !(flags & SE_FLAG_SUMS_ZEROED)) SE_CUDA_CHECK(cudaMemsetAsync(stat_sums, 0, sizeof(double) * 2 * ld_stats * n_utt, st));
+    StftArgs a{};
+    a.wav = wav; a.utt_stride = utt_stride; a.n_utt = (int)(pair ? 2 * n_utt : n_utt); a.T = (int)T; a.hop = hop;
+    a.n_frames = (int)(T / hop) + 1;
+    a.tab.window = window; a.tab.twM = t.twM; a.tab.twN = t.twN;
+    a.power = power; a.phase = phase; a.logp = logpower; a.log_eps = log_eps; a.spec_stride = spec_stride;
+    a.stat_sums = stat_sums; a.ld_stats = ld_stats;
+    a.trace = stat_sums ? secommon::trace_ptr() : nullptr;
+    if (pair) { a.n_real = (int)n_utt; a.chan_step = chan_step; }
+    if (self_clean) { a.zero_ptr = stat_sums + ws_stat_doubles(n_fft, n_utt); a.zero_count = (long long)SE_NSUMS * n_utt; }
+    if (fast) return sefast::launch_stft_run(a, n_fft, st);
+    if (a.zero_ptr) SE_CUDA_CHECK(cudaMemsetAsync(a.zero_ptr, 0, sizeof(double) * a.zero_count, st));   // generic path: by a memset
+    if ((rc = launch_stft_generic(a, n_fft, st)) != SE_OK || !stat_sums) return rc;
+    return se_feature_sums(logpower ? logpower : power, spec_stride, n_utt, a.n_frames, n_fft / 2 + 1, stat_sums, ld_stats, stream);
+}
+
+// K3 of every mask-iSTFT entry point: the shared checks, the tables, MaskIstftArgs, the sums' memset unless SE_FLAG_SUMS_ZEROED,
+// the self-clean region (the statistics right before `sums`) and the register-resident kernel or the generic one.  `a` arrives
+// with the entry point's own fields set; no_generic: the entry point has no generic kernel, SE_ERR_UNSUPPORTED points there.
+int mask_istft_entry(MaskIstftArgs a, const char* who, const char* no_generic, const float* noisy, const float* clean,
+                     int64_t utt_stride, const float* mask, int64_t mask_stride, const int64_t* lengths, int64_t n_utt, int64_t T,
+                     int n_fft, int hop, const float* window, float* wav_out, int64_t out_stride, int64_t pad_to, double* sums,
+                     int flags, void* stream) {
+    SE_REQUIRE(noisy && mask && window && wav_out, "null pointer");
+    SE_REQUIRE(mask_stride >= n_fft / 2 + 1, "mask_stride=%lld smaller than K", (long long)mask_stride);
+    int rc = check_geometry(n_utt, T, n_fft, hop);
+    if (rc != SE_OK) return rc;
+    const bool fast = register_resident(n_fft, hop, T / hop + 1);
+    if (no_generic && !fast)
+        return fail(SE_ERR_UNSUPPORTED, "%s: n_fft=%d hop=%d T=%lld has no register-resident kernel (%s)", who, n_fft, hop,
+                    (long long)T, no_generic);
+    DeviceTables t;
+    if ((rc = get_tables(n_fft, &t)) != SE_OK) return rc;
+    a.noisy = noisy; a.clean = clean; a.utt_stride = utt_stride; a.mask = mask;
+    a.lengths = reinterpret_cast<const long long*>(lengths);
+    a.n_utt = (int)n_utt; a.T = (int)T; a.hop = hop; a.n_frames = (int)(T / hop) + 1;
+    a.tab.window = window; a.tab.twM = t.twM; a.tab.twN = t.twN;
+    a.wav_out = wav_out; a.out_stride = out_stride; a.out_len = hop * (a.n_frames - 1); a.pad_to = (int)pad_to;
+    a.sums = sums; a.mask_stride = mask_stride;
+    a.trace = secommon::trace_ptr();
+    SE_REQUIRE(out_stride >= a.out_len && out_stride >= pad_to, "out_stride=%lld too small", (long long)out_stride);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (sums && !(flags & SE_FLAG_SUMS_ZEROED)) SE_CUDA_CHECK(cudaMemsetAsync(sums, 0, sizeof(double) * SE_NSUMS * n_utt, st));
+    if (sums && (flags & SE_FLAG_WS_SELF_CLEAN)) { a.zero_count = ws_stat_doubles(n_fft, n_utt); a.zero_ptr = sums - a.zero_count; }
+    if (fast) return sefast::launch_mask_istft_run(a, n_fft, st);
+    if (a.zero_ptr) SE_CUDA_CHECK(cudaMemsetAsync(a.zero_ptr, 0, sizeof(double) * a.zero_count, st));   // generic path: by a memset
+    SE_DISPATCH_NFFT(n_fft, launch_mask_istft, a, st)
+}
+
+}  // namespace
 
 extern "C" {
 
@@ -184,113 +266,33 @@ int se_stft(const float* wav, int64_t n_utt, int64_t utt_stride, int64_t T, int 
 
 int se_stft_strided(const float* wav, int64_t n_utt, int64_t utt_stride, int64_t T, int n_fft, int hop, const float* window,
                     float log_eps, float* power, float* phase, float* logpower, int64_t spec_stride, void* stream) {
-    SE_REQUIRE(wav && window, "wav and window must not be null");
-    SE_REQUIRE(spec_stride >= n_fft / 2 + 1, "spec_stride=%lld smaller than K", (long long)spec_stride);
-    int rc = check_geometry(n_utt, T, n_fft, hop);
-    if (rc != SE_OK) return rc;
-    DeviceTables t;
-    if ((rc = get_tables(n_fft, &t)) != SE_OK) return rc;
-    StftArgs a{};
-    a.wav = wav; a.utt_stride = utt_stride; a.n_utt = (int)n_utt; a.T = (int)T; a.hop = hop;
-    a.n_frames = (int)(T / hop) + 1;
-    a.tab.window = window; a.tab.twM = t.twM; a.tab.twN = t.twN;
-    a.power = power; a.phase = phase; a.logp = logpower; a.log_eps = log_eps; a.spec_stride = spec_stride;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (sefast::geo_supported(n_fft, hop) && !g_force_generic) return sefast::launch_stft_run(a, n_fft, st);
-    SE_DISPATCH_NFFT(n_fft, launch_stft, a, st)
+    return stft_entry(wav, n_utt, utt_stride, false, 0, T, n_fft, hop, window, log_eps, power, phase, logpower, spec_stride, nullptr,
+                      0, 0, stream);
 }
-
-static int stft_features_impl(const float* wav, int64_t n_utt, int64_t utt_stride, int64_t T, int n_fft, int hop, const float* window,
-                              float log_eps, int take_log, float* feat, int64_t feat_stride, double* stat_sums, int64_t ld_stats,
-                              int flags, void* stream);
 
 int se_stft_features(const float* wav, int64_t n_utt, int64_t utt_stride, int64_t T, int n_fft, int hop, const float* window,
                      float log_eps, int take_log, float* feat, int64_t feat_stride, double* stat_sums, int64_t ld_stats,
                      int flags, void* stream) {
-    return stft_features_impl(wav, n_utt, utt_stride, T, n_fft, hop, window, log_eps, take_log, feat, feat_stride, stat_sums,
-                              ld_stats, flags, stream);
-}
-
-static int stft_features_impl(const float* wav, int64_t n_utt, int64_t utt_stride, int64_t T, int n_fft, int hop, const float* window,
-                              float log_eps, int take_log, float* feat, int64_t feat_stride, double* stat_sums, int64_t ld_stats,
-                              int flags, void* stream) {
-    SE_REQUIRE(wav && window && feat && stat_sums, "null pointer");
-    SE_REQUIRE(feat_stride >= n_fft / 2 + 1 && ld_stats >= n_fft / 2 + 1, "feat_stride / ld_stats smaller than K");
-    int rc = check_geometry(n_utt, T, n_fft, hop);
-    if (rc != SE_OK) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (!(flags & SE_FLAG_SUMS_ZEROED)) SE_CUDA_CHECK(cudaMemsetAsync(stat_sums, 0, sizeof(double) * 2 * ld_stats * n_utt, st));
-    if (sefast::geo_supported(n_fft, hop) && !g_force_generic) {
-        DeviceTables t;
-        if ((rc = get_tables(n_fft, &t)) != SE_OK) return rc;
-        StftArgs a{};
-        a.wav = wav; a.utt_stride = utt_stride; a.n_utt = (int)n_utt; a.T = (int)T; a.hop = hop;
-        a.n_frames = (int)(T / hop) + 1;
-        a.tab.window = window; a.tab.twM = t.twM; a.tab.twN = t.twN;
-        a.power = take_log ? nullptr : feat; a.logp = take_log ? feat : nullptr; a.log_eps = log_eps; a.spec_stride = feat_stride;
-        a.stat_sums = stat_sums; a.ld_stats = ld_stats;
-        a.trace = secommon::trace_ptr();
-        if (flags & SE_FLAG_WS_SELF_CLEAN) { a.zero_ptr = stat_sums + 2 * ld_stats * n_utt; a.zero_count = (long long)SE_NSUMS * n_utt; }
-        return sefast::launch_stft_run(a, n_fft, st);
-    }
-    if (flags & SE_FLAG_WS_SELF_CLEAN)                      // no fast path for this geometry: the same contract by a memset
-        SE_CUDA_CHECK(cudaMemsetAsync(stat_sums + 2 * ld_stats * n_utt, 0, sizeof(double) * SE_NSUMS * n_utt, st));
-    // other n_fft: generic STFT, then one pass over the features for the sums
-    rc = se_stft_strided(wav, n_utt, utt_stride, T, n_fft, hop, window, log_eps, take_log ? nullptr : feat, nullptr,
-                         take_log ? feat : nullptr, feat_stride, stream);
-    if (rc != SE_OK) return rc;
-    return se_feature_sums(feat, feat_stride, n_utt, T / hop + 1, n_fft / 2 + 1, stat_sums, ld_stats, stream);
+    return se_stft_features2(wav, n_utt, utt_stride, T, n_fft, hop, window, log_eps, take_log ? nullptr : feat,
+                             take_log ? feat : nullptr, feat_stride, stat_sums, ld_stats, flags, stream);
 }
 
 int se_stft_features2(const float* wav, int64_t n_utt, int64_t utt_stride, int64_t T, int n_fft, int hop, const float* window,
                       float log_eps, float* power, float* logpower, int64_t spec_stride, double* stat_sums, int64_t ld_stats,
                       int flags, void* stream) {
-    SE_REQUIRE(wav && window && (power || logpower) && stat_sums, "null pointer");
-    SE_REQUIRE(spec_stride >= n_fft / 2 + 1 && ld_stats >= n_fft / 2 + 1, "spec_stride / ld_stats smaller than K");
-    int rc = check_geometry(n_utt, T, n_fft, hop);
-    if (rc != SE_OK) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (!(flags & SE_FLAG_SUMS_ZEROED)) SE_CUDA_CHECK(cudaMemsetAsync(stat_sums, 0, sizeof(double) * 2 * ld_stats * n_utt, st));
-    if (sefast::geo_supported(n_fft, hop) && !g_force_generic) {
-        DeviceTables t;
-        if ((rc = get_tables(n_fft, &t)) != SE_OK) return rc;
-        StftArgs a{};
-        a.wav = wav; a.utt_stride = utt_stride; a.n_utt = (int)n_utt; a.T = (int)T; a.hop = hop;
-        a.n_frames = (int)(T / hop) + 1;
-        a.tab.window = window; a.tab.twM = t.twM; a.tab.twN = t.twN;
-        a.power = power; a.logp = logpower; a.log_eps = log_eps; a.spec_stride = spec_stride;
-        a.stat_sums = stat_sums; a.ld_stats = ld_stats;
-        a.trace = secommon::trace_ptr();
-        return sefast::launch_stft_run(a, n_fft, st);
-    }
-    rc = se_stft_strided(wav, n_utt, utt_stride, T, n_fft, hop, window, log_eps, power, nullptr, logpower, spec_stride, stream);
-    if (rc != SE_OK) return rc;
-    return se_feature_sums(logpower ? logpower : power, spec_stride, n_utt, T / hop + 1, n_fft / 2 + 1, stat_sums, ld_stats, stream);
+    SE_REQUIRE((power || logpower) && stat_sums, "null pointer");
+    return stft_entry(wav, n_utt, utt_stride, false, 0, T, n_fft, hop, window, log_eps, power, nullptr, logpower, spec_stride,
+                      stat_sums, ld_stats, flags, stream);
 }
 
-int se_stft_features_pair_supported(int n_fft, int hop) { return (sefast::geo_supported(n_fft, hop) && !g_force_generic) ? 1 : 0; }
+int se_stft_features_pair_supported(int n_fft, int hop) { return register_resident(n_fft, hop) ? 1 : 0; }
 
 int se_stft_features_pair(const float* wav, int64_t n_utt, int64_t utt_stride, int64_t chan_step, int64_t T, int n_fft, int hop,
                           const float* window, float log_eps, float* power2, float* logpower, int64_t spec_stride, double* stat_sums,
                           int64_t ld_stats, int flags, void* stream) {
-    SE_REQUIRE(wav && window && power2 && stat_sums, "null pointer");
-    SE_REQUIRE(spec_stride >= n_fft / 2 + 1 && ld_stats >= n_fft / 2 + 1, "spec_stride / ld_stats smaller than K");
-    int rc = check_geometry(2 * n_utt, T, n_fft, hop);
-    if (rc != SE_OK) return rc;
-    if (!se_stft_features_pair_supported(n_fft, hop))
-        return fail(SE_ERR_UNSUPPORTED, "se_stft_features_pair: n_fft=%d hop=%d has no register-resident kernel (use two se_stft_features2 calls)", n_fft, hop);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (!(flags & SE_FLAG_SUMS_ZEROED)) SE_CUDA_CHECK(cudaMemsetAsync(stat_sums, 0, sizeof(double) * 2 * ld_stats * n_utt, st));
-    DeviceTables t;
-    if ((rc = get_tables(n_fft, &t)) != SE_OK) return rc;
-    StftArgs a{};
-    a.wav = wav; a.utt_stride = utt_stride; a.n_utt = (int)(2 * n_utt); a.n_real = (int)n_utt; a.chan_step = chan_step;
-    a.T = (int)T; a.hop = hop; a.n_frames = (int)(T / hop) + 1;
-    a.tab.window = window; a.tab.twM = t.twM; a.tab.twN = t.twN;
-    a.power = power2; a.logp = logpower; a.log_eps = log_eps; a.spec_stride = spec_stride;
-    a.stat_sums = stat_sums; a.ld_stats = ld_stats;
-    a.trace = secommon::trace_ptr();
-    return sefast::launch_stft_run(a, n_fft, st);
+    SE_REQUIRE(power2 && stat_sums, "null pointer");
+    return stft_entry(wav, n_utt, utt_stride, true, chan_step, T, n_fft, hop, window, log_eps, power2, nullptr, logpower, spec_stride,
+                      stat_sums, ld_stats, flags, stream);
 }
 
 int se_istft(const float* power, const float* phase, int64_t n_utt, int64_t n_frames, int n_fft, int hop,
@@ -327,108 +329,47 @@ int se_mask_istft_strided(const float* noisy, const float* clean, int64_t utt_st
 int se_mask_istft_ex(const float* noisy, const float* clean, int64_t utt_stride, const float* mask, int64_t mask_stride,
                      const int64_t* lengths, int64_t n_utt, int64_t T, int n_fft, int hop, const float* window,
                      float* wav_out, int64_t out_stride, int64_t pad_to, double* sums, int flags, void* stream) {
-    const int want_spec = (flags & SE_FLAG_WANT_SPEC) ? 1 : 0;
-    SE_REQUIRE(noisy && mask && window && wav_out, "null pointer");
-    SE_REQUIRE(mask_stride >= n_fft / 2 + 1, "mask_stride=%lld smaller than K", (long long)mask_stride);
     SE_REQUIRE(!((flags & SE_FLAG_MASK_IS_POWER) && (flags & SE_FLAG_MASK_IS_LOG_POWER)),
                "SE_FLAG_MASK_IS_POWER and SE_FLAG_MASK_IS_LOG_POWER are mutually exclusive");
-    int rc = check_geometry(n_utt, T, n_fft, hop);
-    if (rc != SE_OK) return rc;
-    DeviceTables t;
-    if ((rc = get_tables(n_fft, &t)) != SE_OK) return rc;
     MaskIstftArgs a{};
-    a.noisy = noisy; a.clean = clean; a.utt_stride = utt_stride; a.mask = mask;
-    a.lengths = reinterpret_cast<const long long*>(lengths);
-    a.n_utt = (int)n_utt; a.T = (int)T; a.hop = hop; a.n_frames = (int)(T / hop) + 1;
-    a.tab.window = window; a.tab.twM = t.twM; a.tab.twN = t.twN;
-    a.wav_out = wav_out; a.out_stride = out_stride; a.out_len = hop * (a.n_frames - 1); a.pad_to = (int)pad_to;
-    a.sums = sums; a.want_spec = (want_spec && clean && sums) ? 1 : 0; a.mask_stride = mask_stride;
+    a.want_spec = ((flags & SE_FLAG_WANT_SPEC) && clean && sums) ? 1 : 0;
     a.mask_is_power = (flags & SE_FLAG_MASK_IS_LOG_POWER) ? 2 : (flags & SE_FLAG_MASK_IS_POWER) ? 1 : 0;
-    a.trace = secommon::trace_ptr();
-    SE_REQUIRE(out_stride >= a.out_len && out_stride >= pad_to, "out_stride=%lld too small", (long long)out_stride);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (sums && !(flags & SE_FLAG_SUMS_ZEROED)) SE_CUDA_CHECK(cudaMemsetAsync(sums, 0, sizeof(double) * SE_NSUMS * n_utt, st));
-    const long long stat_doubles = 2LL * ((n_fft / 2 + 1 + 3) / 4 * 4) * n_utt;         // (n_utt, round4(K), 2) right before `sums`
-    const bool self_clean = (flags & SE_FLAG_WS_SELF_CLEAN) && sums;
-    if (self_clean) { a.zero_ptr = sums - stat_doubles; a.zero_count = stat_doubles; }
-    if (sefast::geo_supported(n_fft, hop) && a.n_frames >= 6 && !g_force_generic) return sefast::launch_mask_istft_run(a, n_fft, st);
-    if (self_clean) SE_CUDA_CHECK(cudaMemsetAsync(sums - stat_doubles, 0, sizeof(double) * stat_doubles, st));   // generic path: by a memset
-    SE_DISPATCH_NFFT(n_fft, launch_mask_istft, a, st)
+    return mask_istft_entry(a, "se_mask_istft_ex", nullptr, noisy, clean, utt_stride, mask, mask_stride, lengths, n_utt, T, n_fft, hop,
+                            window, wav_out, out_stride, pad_to, sums, flags, stream);
 }
 
-int se_mask_istft_wsd_supported(int n_fft, int hop) { return (sefast::geo_supported(n_fft, hop) && !g_force_generic) ? 1 : 0; }
+int se_mask_istft_wsd_supported(int n_fft, int hop) { return register_resident(n_fft, hop) ? 1 : 0; }
 
 int se_mask_istft_wsd(const float* noisy, const float* clean, int64_t utt_stride, const float* mask, int64_t mask_stride,
                       const int64_t* lengths, int64_t n_utt, int64_t T, int n_fft, int hop, const float* window,
                       float* wav_out, int64_t out_stride, int64_t pad_to, double* sums, float* frame_terms, float* wsd_state,
                       int flags, void* stream) {
-    SE_REQUIRE(noisy && clean && mask && window && wav_out && sums && frame_terms && wsd_state, "null pointer");
-    SE_REQUIRE(mask_stride >= n_fft / 2 + 1, "mask_stride=%lld smaller than K", (long long)mask_stride);
+    SE_REQUIRE(clean && sums && frame_terms && wsd_state, "null pointer");
     SE_REQUIRE((reinterpret_cast<uintptr_t>(frame_terms) & 7) == 0 && (reinterpret_cast<uintptr_t>(wsd_state) & 7) == 0,
                "frame_terms / wsd_state must be 8-byte aligned");
     SE_REQUIRE(!(flags & (SE_FLAG_WANT_SPEC | SE_FLAG_MASK_IS_POWER)), "se_mask_istft_wsd: flags may hold SE_FLAG_SUMS_ZEROED and "
                "SE_FLAG_WS_SELF_CLEAN only");
-    int rc = check_geometry(n_utt, T, n_fft, hop);
-    if (rc != SE_OK) return rc;
-    if (!se_mask_istft_wsd_supported(n_fft, hop) || T / hop + 1 < 6)       // the frame count se_mask_istft_ex's fast path needs
-        return fail(SE_ERR_UNSUPPORTED, "se_mask_istft_wsd: n_fft=%d hop=%d T=%lld has no register-resident kernel (use se_wsd_energy "
-                    "and se_wsd_mask_step on the spectra)", n_fft, hop, (long long)T);
-    DeviceTables t;
-    if ((rc = get_tables(n_fft, &t)) != SE_OK) return rc;
     MaskIstftArgs a{};
-    a.noisy = noisy; a.clean = clean; a.utt_stride = utt_stride; a.mask = mask;
-    a.lengths = reinterpret_cast<const long long*>(lengths);
-    a.n_utt = (int)n_utt; a.T = (int)T; a.hop = hop; a.n_frames = (int)(T / hop) + 1;
-    a.tab.window = window; a.tab.twM = t.twM; a.tab.twN = t.twN;
-    a.wav_out = wav_out; a.out_stride = out_stride; a.out_len = hop * (a.n_frames - 1); a.pad_to = (int)pad_to;
-    a.sums = sums; a.want_spec = 0; a.mask_stride = mask_stride;
     a.wsd_terms = frame_terms; a.wsd_max = wsd_state;
-    a.trace = secommon::trace_ptr();
-    SE_REQUIRE(out_stride >= a.out_len && out_stride >= pad_to, "out_stride=%lld too small", (long long)out_stride);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (!(flags & SE_FLAG_SUMS_ZEROED)) SE_CUDA_CHECK(cudaMemsetAsync(sums, 0, sizeof(double) * SE_NSUMS * n_utt, st));
-    if (flags & SE_FLAG_WS_SELF_CLEAN) {
-        a.zero_ptr = sums - 2LL * ((n_fft / 2 + 1 + 3) / 4 * 4) * n_utt;
-        a.zero_count = 2LL * ((n_fft / 2 + 1 + 3) / 4 * 4) * n_utt;
-    }
-    return sefast::launch_mask_istft_run(a, n_fft, st);
+    return mask_istft_entry(a, "se_mask_istft_wsd", "use se_wsd_energy and se_wsd_mask_step on the spectra", noisy, clean, utt_stride,
+                            mask, mask_stride, lengths, n_utt, T, n_fft, hop, window, wav_out, out_stride, pad_to, sums, flags, stream);
 }
 
-int se_mask_istft_l1_supported(int n_fft, int hop) { return (sefast::geo_supported(n_fft, hop) && !g_force_generic) ? 1 : 0; }
+int se_mask_istft_l1_supported(int n_fft, int hop) { return register_resident(n_fft, hop) ? 1 : 0; }
 
 int se_mask_istft_l1(const float* noisy, const float* clean, int64_t utt_stride, const float* mask, int64_t mask_stride,
                      const int64_t* lengths, int64_t n_utt, int64_t T, int n_fft, int hop, const float* window,
                      float* wav_out, int64_t out_stride, int64_t pad_to, double* sums, double* l1_acc, float eps, int flags,
                      void* stream) {
-    SE_REQUIRE(noisy && clean && mask && window && wav_out && sums && l1_acc, "null pointer");
-    SE_REQUIRE(mask_stride >= n_fft / 2 + 1, "mask_stride=%lld smaller than K", (long long)mask_stride);
+    SE_REQUIRE(clean && sums && l1_acc, "null pointer");
     SE_REQUIRE(eps > 0.0f, "eps=%g must be positive", (double)eps);
     SE_REQUIRE(!(flags & (SE_FLAG_WANT_SPEC | SE_FLAG_MASK_IS_POWER)), "se_mask_istft_l1: flags may hold SE_FLAG_SUMS_ZEROED, "
                "SE_FLAG_WS_SELF_CLEAN and SE_FLAG_MASK_IS_LOG_POWER only");
-    int rc = check_geometry(n_utt, T, n_fft, hop);
-    if (rc != SE_OK) return rc;
-    if (!se_mask_istft_l1_supported(n_fft, hop) || T / hop + 1 < 6)        // the frame count se_mask_istft_ex's fast path needs
-        return fail(SE_ERR_UNSUPPORTED, "se_mask_istft_l1: n_fft=%d hop=%d T=%lld has no register-resident kernel (use se_mask_istft_ex "
-                    "with SE_FLAG_MASK_IS_LOG_POWER and se_l1_logspec_fwd on the clean power spectrum)", n_fft, hop, (long long)T);
-    DeviceTables t;
-    if ((rc = get_tables(n_fft, &t)) != SE_OK) return rc;
     MaskIstftArgs a{};
-    a.noisy = noisy; a.clean = clean; a.utt_stride = utt_stride; a.mask = mask;
-    a.lengths = reinterpret_cast<const long long*>(lengths);
-    a.n_utt = (int)n_utt; a.T = (int)T; a.hop = hop; a.n_frames = (int)(T / hop) + 1;
-    a.tab.window = window; a.tab.twM = t.twM; a.tab.twN = t.twN;
-    a.wav_out = wav_out; a.out_stride = out_stride; a.out_len = hop * (a.n_frames - 1); a.pad_to = (int)pad_to;
-    a.sums = sums; a.want_spec = 0; a.mask_stride = mask_stride;
     a.mask_is_power = 2; a.l1_acc = l1_acc; a.l1_eps = eps;
-    a.trace = secommon::trace_ptr();
-    SE_REQUIRE(out_stride >= a.out_len && out_stride >= pad_to, "out_stride=%lld too small", (long long)out_stride);
-    cudaStream_t st = (cudaStream_t)stream;
-    if (!(flags & SE_FLAG_SUMS_ZEROED)) SE_CUDA_CHECK(cudaMemsetAsync(sums, 0, sizeof(double) * SE_NSUMS * n_utt, st));
-    if (flags & SE_FLAG_WS_SELF_CLEAN) {
-        a.zero_ptr = sums - 2LL * ((n_fft / 2 + 1 + 3) / 4 * 4) * n_utt;
-        a.zero_count = 2LL * ((n_fft / 2 + 1 + 3) / 4 * 4) * n_utt;
-    }
-    return sefast::launch_mask_istft_run(a, n_fft, st);
+    return mask_istft_entry(a, "se_mask_istft_l1", "use se_mask_istft_ex with SE_FLAG_MASK_IS_LOG_POWER and se_l1_eval_sums on the "
+                            "clean power spectrum", noisy, clean, utt_stride, mask, mask_stride, lengths, n_utt, T, n_fft, hop, window,
+                            wav_out, out_stride, pad_to, sums, flags, stream);
 }
 
 __global__ void __launch_bounds__(256) pcm16_to_float_kernel(const short4* __restrict__ src, float4* __restrict__ dst, long long n4,

@@ -43,11 +43,6 @@ def _eval_loss(criterion, head=None):
                        "LinearResidual / Residual, objective.L1 with LSTM)")
 
 
-def _eval_wsd(criterion):
-    """True for objective.WSD (see _eval_loss)."""
-    return _eval_loss(criterion) == "wsd"
-
-
 def _criterion_key(criterion):
     """What a captured evaluation step bakes in of its criterion."""
     loss = _eval_loss(criterion)
@@ -91,9 +86,7 @@ class EnhancementEngine:
         + one double (the WSD maximum and the finish kernel's CTA counter) with an objective.WSD criterion, or two (the L1 sum
         and element count) with objective.L1.
         The step's kernels leave it zeroed for the next replay (SE_FLAG_WS_SELF_CLEAN), so the graph has no fill node."""
-        LD = ops.round4(self.n_fft // 2 + 1)
-        extra = {"sisdr": 0, "wsd": 1, "l1": 2}[_eval_loss(criterion)]
-        return torch.zeros(B * (2 * LD + ops.NSUMS) + extra, device=device, dtype=torch.float64)
+        return torch.zeros(ops.step_workspace_doubles(B, self.n_fft, _eval_loss(criterion)), device=device, dtype=torch.float64)
 
     def eval_step(self, lengths, wavs, want_spec_loss=True, metric_acc=None, ws=None, want_stoi=False, stoi_acc=None,
                   criterion=None):
@@ -137,6 +130,9 @@ class EnhancementEngine:
             wpad = self._padded_weight()
             Dout = wpad.shape[0]
             D = self._mel_feature_dim() if self.feat_cfg is not None else K
+            state = None                                         # the criterion's persistent state at the workspace's end
+            if ws is not None:
+                state = ops.step_workspace_views(ws, B, self.n_fft)[2]
             if _recurrent(head):
                 mask = self._recurrent_front(wavs, D, wpad)
                 k3 = {}
@@ -158,16 +154,15 @@ class EnhancementEngine:
                 # K1 (+ CMVN sums) -> K2 (TMA + tcgen05 head) -> K3 -> K3': one zeroed workspace, no other memset, so
                 # the four kernels are chained by programmatic dependent launches
                 self.launches_per_step = 4      # K1, K2, K3, K3' (+ torch's fill of the workspace unless `ws` is given)
-                self_clean = ws is not None
-                if ws is None:
-                    ws = torch.zeros(B * (2 * LD + ops.NSUMS), device=dev, dtype=torch.float64)
-                stat_sums = ws[:B * 2 * LD].view(B, LD, 2)
-                sums = ws[B * 2 * LD:B * (2 * LD + ops.NSUMS)].view(B, ops.NSUMS)
-                feats, _ = ops.stft_features(wavs, self.ch_inp, self.n_fft, self.hop, window, logpower=self.log_features,
-                                             log_eps=self.pre.eps, stat_sums=stat_sums, self_clean=self_clean)
+                if ws is None:                  # a fresh zeroed one, used once: the kernels need not clean it
+                    stat_sums, sums, state = ops.step_workspace_views(self.step_workspace(B, dev, criterion), B, self.n_fft)
+                    k1, k3 = dict(stat_sums=stat_sums), dict(sums=sums, sums_zeroed=True)
+                else:
+                    k1 = k3 = dict(ws=ws)
+                feats, stat_sums = ops.stft_features(wavs, self.ch_inp, self.n_fft, self.hop, window, logpower=self.log_features,
+                                                     log_eps=self.pre.eps, **k1)
                 mask = ops.linear_head_tma(feats, K, wpad, head.linear.bias, head.activation,
                                              stat_sums if head.cmvn else None, head.eps)
-                k3 = dict(sums=sums, sums_zeroed=True, self_clean=self_clean)
             else:
                 self.launches_per_step = 5      # K1, K2 (+ CMVN statistics), the sums' fill, K3, K3'
                 feats = ops.stft_padded(wavs, self.ch_inp, self.n_fft, self.hop, window, logpower=self.log_features, log_eps=self.pre.eps)
@@ -177,16 +172,15 @@ class EnhancementEngine:
                 mask = ops.linear_head_padded(feats, K, wpad, head.linear.bias, head.activation, mean, std,
                                               head.eps, precision=self.precision)
                 k3 = {}
-            extra = None                                         # the criterion's persistent state at the workspace's end
-            if ws is not None and ws.numel() > B * (2 * LD + ops.NSUMS):
-                extra = ws[B * (2 * LD + ops.NSUMS):]
             batch_loss = None
+            # K3' without the loss terms, for the L1 / WSD routes (their finish kernels compute those after the all-reduce)
+            finalize = lambda: ops.finalize_metrics(sums, lengths, T, wav=wav, target_db=None, want_loss=False, metric_acc=metric_acc)
             if l1:
                 # K3 (log-power target) with the L1 sums, or the slow route -> all-reduce of [sum, count] on the side stream under
                 # K3' -> the finish kernel
-                l1_acc = extra if extra is not None and extra.numel() == 2 else torch.zeros(2, device=dev, dtype=torch.float64)
+                l1_acc = state if state is not None and state.numel() == 2 else torch.zeros(2, device=dev, dtype=torch.float64)
                 self.launches_per_step += 1                         # the finish kernel (K3-L1 replaces K3)
-                if ops.mask_istft_l1_supported(self.n_fft, self.hop) and F >= 6:
+                if ops.mask_istft_register_resident(self.n_fft, self.hop, T):
                     wav, sums = ops.mask_istft_l1(wavs, self.ch_inp, self.ch_tar, mask, lengths, self.n_fft, self.hop, window,
                                                   pad_to=T, l1_acc=l1_acc, eps=criterion.eps, **k3)
                 else:
@@ -194,36 +188,18 @@ class EnhancementEngine:
                                                pad_to=T, want_sums=True, want_spec=False, mask_padded=True, mask_is_log_power=True,
                                                **k3)
                     self._l1_terms_from_spectra(wavs, mask, lengths, criterion, sums, l1_acc)
-                main = torch.cuda.current_stream(dev)
-                side = self._side_stream(dev) if dp.world()[1] > 1 else None
-                if side is not None:
-                    side.wait_stream(main)
-                    with torch.cuda.stream(side):
-                        dp.reduce_sums(l1_acc)
-                gain, sisdr, _ = ops.finalize_metrics(sums, lengths, T, wav=wav, target_db=None, want_loss=False,
-                                                      metric_acc=metric_acc)
-                if side is not None:
-                    main.wait_stream(side)
+                gain, sisdr, _ = self._all_reduce_beside(dp.reduce_sums, l1_acc, finalize)
                 loss, batch_loss = ops.l1_eval_finish(sums, lengths, T, self.hop, K, l1_acc, metric_acc)
-            elif wsd and ops.mask_istft_wsd_supported(self.n_fft, self.hop) and F >= 6:
+            elif wsd and ops.mask_istft_register_resident(self.n_fft, self.hop, T):
                 # K3 with the WSD terms -> all-reduce(max) of its 4-byte maximum on the side stream under K3' -> the finish kernel
                 self.launches_per_step += 1
-                if extra is not None and extra.numel() == 1:
-                    state = extra.view(torch.float32)                  # the step leaves it zeroed
+                if state is not None and state.numel() == 1:
+                    state = state.view(torch.float32)                  # the step leaves it zeroed
                 else:
                     state = torch.zeros(2, device=dev, dtype=torch.float32)
                 wav, sums, terms = ops.mask_istft_wsd(wavs, self.ch_inp, self.ch_tar, mask, lengths, self.n_fft, self.hop, window,
                                                       pad_to=T, wsd_state=state, **k3)
-                main = torch.cuda.current_stream(dev)
-                side = self._side_stream(dev) if dp.world()[1] > 1 else None
-                if side is not None:
-                    side.wait_stream(main)
-                    with torch.cuda.stream(side):
-                        dp.global_max(state[:1])
-                gain, sisdr, _ = ops.finalize_metrics(sums, lengths, T, wav=wav, target_db=None, want_loss=False,
-                                                      metric_acc=metric_acc)
-                if side is not None:
-                    main.wait_stream(side)
+                gain, sisdr, _ = self._all_reduce_beside(dp.global_max, state[:1], finalize)
                 loss = ops.wsd_eval_finish(terms, sums, state, criterion.alpha, criterion.db_interval, criterion.eps, metric_acc)
             else:
                 wav, sums = ops.mask_istft(wavs, self.ch_inp, self.ch_tar, mask, lengths, self.n_fft, self.hop, window,
@@ -487,24 +463,19 @@ class EnhancementEngine:
                 linear_tar = ops.stft_padded(wavs, self.ch_tar, self.n_fft, self.hop, window, logpower=False)
             wpad = self._padded_weight()            # current: refreshed in place after every update (_clip_and_step)
             stats = stat_sums if head.cmvn else None
+            head_fwd = lambda: ops.linear_head_tma(feats, D, wpad, head.linear.bias, head.activation, stats, head.eps)
             if wsd:
                 # the voicing threshold needs the loudest frame of the GLOBAL batch: its 4-byte all-reduce runs on a side stream
-                # under the head's forward (nothing to fork at world size 1)
+                # under the head's forward
                 energy, emax = ops.wsd_energy(linear_tar, K)
-                main = torch.cuda.current_stream(dev)
-                side = self._side_stream(dev) if dp.world()[1] > 1 else None
-                if side is not None:
-                    side.wait_stream(main)
-                    with torch.cuda.stream(side):
-                        dp.global_max(emax)
-            offset = ops.linear_head_tma(feats, D, wpad, head.linear.bias, head.activation, stats, head.eps)
+                offset = self._all_reduce_beside(dp.global_max, emax, head_fwd)
+            else:
+                offset = head_fwd()
             # frames = lengths // hop + 1, the batch-mean loss and d loss / d offset inside three launches
             lens = _c64(lengths)
             fold = (ops.linear_head_bwd_wsd_supported if wsd else ops.linear_head_bwd_sisdr_supported)(
                 B, feats.shape[1], D, K, feats.shape[2], offset.shape[2], linear_inp.shape[2], linear_tar.shape[2])
             if wsd:
-                if side is not None:
-                    main.wait_stream(side)
                 sums2 = sums3.view(-1)[:2 * B].view(B, 2)          # the zeroed workspace's sums part, as (B, 2)
                 loss, _, grad_offset, _ = ops.wsd_mask_step(offset, linear_inp, linear_tar, lens, self.hop, K, energy, emax,
                                                             objective.alpha, objective.db_interval, objective.eps, sums2=sums2,
@@ -527,12 +498,22 @@ class EnhancementEngine:
                     p.grad.add_(g)
         return loss
 
-    def _side_stream(self, device):
-        """One side stream per device for the WSD maximum's all-reduce (kept: a captured step records it as a fork / join)."""
-        key = str(device)
+    def _all_reduce_beside(self, all_reduce, buf, work):
+        """all_reduce(buf) (dp.global_max / dp.reduce_sums) on the device's side stream while the current stream runs work();
+        returns work()'s result with the current stream joined to the side stream.  At world size 1 there is nothing to reduce:
+        only work() runs.  The side stream is one per device and kept, so that a captured step records it as a fork / join."""
+        if dp.world()[1] == 1:
+            return work()
+        key = str(buf.device)
         if key not in self._side_streams:
-            self._side_streams[key] = torch.cuda.Stream(device=device)
-        return self._side_streams[key]
+            self._side_streams[key] = torch.cuda.Stream(device=buf.device)
+        main, side = torch.cuda.current_stream(buf.device), self._side_streams[key]
+        side.wait_stream(main)
+        with torch.cuda.stream(side):
+            all_reduce(buf)
+        result = work()
+        main.wait_stream(side)
+        return result
 
     def _clip_and_step(self, optimizer, grad_clip):
         """runner.py:463-470; two launches with se_b200.ClipAdam (NaN / inf norms skipped on the device), torch's kernels
@@ -559,25 +540,20 @@ class EnhancementEngine:
     def train_step(self, lengths, wavs, objective, optimizer=None, grad_clip=None):
         """runner.py:431-471 on the kernels: preprocessor tensors -> head -> criterion -> backward
         (+ gradient all-reduce under DP) -> optimizer step.  Returns the loss tensor."""
-        if optimizer is not None and self.fused_training_supported(objective, wavs.shape[0], wavs.shape[2]):
-            optimizer.zero_grad(set_to_none=True)
-            loss = self._fused_forward_backward(lengths, wavs, objective)
-            dp.allreduce_gradients(self.head.parameters())
-            self._clip_and_step(optimizer, grad_clip)
-            return loss
+        if optimizer is None:
+            return self._autograd_loss(lengths, wavs, objective)
+        optimizer.zero_grad(set_to_none=True)
+        return self._train_body(lengths, wavs, objective, optimizer, grad_clip)
+
+    def _autograd_loss(self, lengths, wavs, objective):
+        """The reference's forward through the custom ops (preprocessor -> head -> objective), recorded for autograd."""
         c = self.pre.get_feat_config
         feat_cfg = self.feat_cfg or c("linear", self.ch_inp, log=self.log_features)
         feats, linear_inp, linear_tar = self.pre(wavs, [feat_cfg, c("linear", self.ch_inp), c("linear", self.ch_tar)])
         predicted, extra = self.head(features=feats, linears=linear_inp)
         frames = lengths // self.hop + 1
         loss, _ = objective(predicted=predicted, linear_tar=linear_tar, linear_inp=linear_inp, stft_lengths=frames, **extra)
-        if optimizer is not None:
-            optimizer.zero_grad(set_to_none=True)
-            loss.backward()
-            dp.allreduce_gradients(self.head.parameters())
-            self._clip_and_step(optimizer, grad_clip)
         return loss
-
 
     def capture_train(self, lengths, wavs, objective, optimizer, grad_clip=None):
         """Capture the training step of one batch shape -- forward, backward, gradient all-reduce (NCCL under DP), clipping
@@ -619,16 +595,9 @@ class EnhancementEngine:
         """forward + backward + update without ``zero_grad`` (inside a graph the gradients live in the graph's pool)."""
         if self.fused_training_supported(objective, wavs.shape[0], wavs.shape[2]):
             loss = self._fused_forward_backward(lengths, wavs, objective)
-            dp.allreduce_gradients(self.head.parameters())
-            self._clip_and_step(optimizer, grad_clip)
-            return loss
-        c = self.pre.get_feat_config
-        feat_cfg = self.feat_cfg or c("linear", self.ch_inp, log=self.log_features)
-        feats, linear_inp, linear_tar = self.pre(wavs, [feat_cfg, c("linear", self.ch_inp), c("linear", self.ch_tar)])
-        predicted, extra = self.head(features=feats, linears=linear_inp)
-        frames = lengths // self.hop + 1
-        loss, _ = objective(predicted=predicted, linear_tar=linear_tar, linear_inp=linear_inp, stft_lengths=frames, **extra)
-        loss.backward()
+        else:
+            loss = self._autograd_loss(lengths, wavs, objective)
+            loss.backward()
         dp.allreduce_gradients(self.head.parameters())
         self._clip_and_step(optimizer, grad_clip)
         return loss

@@ -103,14 +103,33 @@ def stft_padded(wavs, channel, n_fft, hop, window, logpower=True, log_eps=1e-10)
 
 
 FLAG_WANT_SPEC, FLAG_SUMS_ZEROED, FLAG_MASK_IS_POWER, FLAG_WS_SELF_CLEAN, FLAG_MASK_IS_LOG_POWER = 1, 2, 4, 8, 16
+STATE_DOUBLES = {"sisdr": 0, "wsd": 1, "l1": 2}     # the criterion's state at the end of a step workspace
 
 
-def stft_features(wavs, channel, n_fft, hop, window, logpower=True, log_eps=1e-10, stat_sums=None, self_clean=False):
+def step_workspace_doubles(B, n_fft, criterion="sisdr"):
+    """Length of a fused evaluation step's workspace (see ``step_workspace_views``) for the criterion "sisdr", "wsd" or "l1"."""
+    return B * (2 * round4(n_fft // 2 + 1) + NSUMS) + STATE_DOUBLES[criterion]
+
+
+def step_workspace_views(ws, B, n_fft):
+    """The fused evaluation step's workspace: ONE float64 vector [stat_sums (B, round4(K), 2) | sums (B, NSUMS) | state], zeroed
+    once, that the step's kernels keep ready for the next replay (SE_FLAG_WS_SELF_CLEAN): K1 zeroes `sums`, which the previous
+    step's K3' has read, and K3 zeroes `stat_sums` after the head has read them; the finish kernels reset `state`.  state: 0
+    doubles for the spectral SI-SDR, 1 for objective.WSD (its maximum and the finish kernel's CTA counter), 2 for objective.L1
+    (its sum and element count).  Returns the views (stat_sums, sums, state)."""
+    LD = round4(n_fft // 2 + 1)
+    n_stat, n_sums = B * 2 * LD, B * NSUMS
+    assert ws.dtype == torch.float64 and ws.dim() == 1 and ws.is_contiguous(), "a step workspace is one contiguous float64 vector"
+    assert ws.numel() - n_stat - n_sums in STATE_DOUBLES.values(), f"{ws.numel()} doubles is no step workspace of B={B}, n_fft={n_fft}"
+    return ws[:n_stat].view(B, LD, 2), ws[n_stat:n_stat + n_sums].view(B, NSUMS), ws[n_stat + n_sums:]
+
+
+def stft_features(wavs, channel, n_fft, hop, window, logpower=True, log_eps=1e-10, stat_sums=None, ws=None):
     """Fused-step K1: ONE feature tensor (B, F, round4(K)) -- log-power or power -- plus the CMVN sums
     (B, round4(K), 2) float64 = [sum_f x, sum_f x^2].  If ``stat_sums`` is given it must already be zero
     (the caller zeroed its workspace once for the whole step); otherwise it is allocated and zeroed here.
-    self_clean: ``stat_sums`` is the head of a persistent step workspace ``[stat_sums | K3 sums]`` (SE_FLAG_WS_SELF_CLEAN):
-    this kernel zeroes the K3 sums that follow it, ``mask_istft(self_clean=True)`` zeroes ``stat_sums`` after the head."""
+    ws: a whole step workspace (``step_workspace_views``) instead: the sums go to its stat_sums, and this kernel zeroes its
+    K3 sums for ``mask_istft(ws=)`` (and _wsd / _l1), which zeroes the stat_sums after the head."""
     wavs = _chk(wavs, "wavs")
     B, C, T = wavs.shape
     F, K = T // hop + 1, n_fft // 2 + 1
@@ -118,9 +137,12 @@ def stft_features(wavs, channel, n_fft, hop, window, logpower=True, log_eps=1e-1
     window = _c(window, "window")
     with torch.cuda.device(wavs.device):
         out = torch.empty(B, F, LD, device=wavs.device, dtype=torch.float32)
-        flags = FLAG_SUMS_ZEROED | (FLAG_WS_SELF_CLEAN if self_clean else 0)
-        if stat_sums is None:
-            assert not self_clean
+        flags = FLAG_SUMS_ZEROED
+        if ws is not None:
+            assert stat_sums is None, "stat_sums comes from the workspace"
+            stat_sums = step_workspace_views(ws, B, n_fft)[0]
+            flags |= FLAG_WS_SELF_CLEAN
+        elif stat_sums is None:
             stat_sums = torch.empty(B, LD, 2, device=wavs.device, dtype=torch.float64)
             flags = 0
         assert stat_sums.shape == (B, LD, 2) and stat_sums.dtype == torch.float64 and stat_sums.is_contiguous()
@@ -436,39 +458,55 @@ def istft(power, phase, n_fft, hop, window, pad_to=0):
     return wav
 
 
-def mask_istft(wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, want_sums=True, want_spec=True,
-               out=None, sums=None, mask_padded=False, sums_zeroed=False, mask_is_power=False, self_clean=False,
-               mask_is_log_power=False):
-    """Fused ``istft(linear_inp * mask, phase_inp)`` straight from the noisy waveform.
-
-    wavs (B, C, T); mask (B, F, K); lengths (B,) int64 or None.  Returns (wav (B, width), sums (B, 6) float64|None).
-    mask_is_power: ``mask`` is the target power (``istft(mask, phase_inp)``); mask_is_log_power: it is the log of the target
-    power, e.g. model.LSTM's log_predicted (``istft(exp(mask), phase_inp)`` without the exp pass)."""
-    assert not (mask_is_power and mask_is_log_power), "mask_is_power and mask_is_log_power are mutually exclusive"
-    wavs, mask, window = _chk(wavs, "wavs"), _c(mask, "mask"), _c(window, "window")
+def _mask_istft_call(entry, wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, out, want_sums, sums, sums_zeroed,
+                     ws, flags, *own):
+    """What the mask-iSTFT wrappers share: the checks, the output and sums buffers, the sums' flags and the call of the library
+    entry point ``entry`` with its own arguments ``own`` (those between the sums and the flags).  mask: (B, F, LD >= K), rows LD
+    floats apart.  sums None: allocated here; ws: a step workspace (``step_workspace_views``) whose sums this K3 fills and whose
+    stat_sums it zeroes.  Returns (wav (B, width), sums | None)."""
+    wavs, mask, window = _chk(wavs, "wavs"), _chk(mask, "mask"), _c(window, "window")
     assert wavs.dim() == 3 and wavs.is_contiguous()
     B, C, T = wavs.shape
     F, K = T // hop + 1, n_fft // 2 + 1
-    mask_stride = mask.shape[2] if mask_padded else K
-    assert mask.shape == (B, F, mask_stride) and mask_stride >= K, f"mask {tuple(mask.shape)} != {(B, F, mask_stride)}"
+    assert mask.dim() == 3 and mask.shape[:2] == (B, F) and mask.shape[2] >= K and mask.stride(2) == 1 and \
+        mask.stride(1) == mask.shape[2], f"mask {tuple(mask.shape)} is not ({B}, {F}, LD >= {K}) with rows LD floats apart"
     lengths = _c(lengths, "lengths", torch.int64)
-    out_len = hop * (F - 1)
-    width = max(out_len, int(pad_to))
+    width = max(hop * (F - 1), int(pad_to))
     with torch.cuda.device(wavs.device):
         if out is None:
             out = torch.empty(B, width, device=wavs.device, dtype=torch.float32)
-        if want_sums and sums is None:
+        flags |= FLAG_SUMS_ZEROED if sums_zeroed else 0
+        if ws is not None:
+            assert want_sums and sums is None, "the sums come from the workspace"
+            sums = step_workspace_views(ws, B, n_fft)[1]
+            flags |= FLAG_SUMS_ZEROED | FLAG_WS_SELF_CLEAN
+        elif want_sums and sums is None:
             sums = torch.empty(B, NSUMS, device=wavs.device, dtype=torch.float64)
+        sums = sums if want_sums else None
         clean = None if ch_tar is None else wavs.data_ptr() + 4 * int(ch_tar) * T
-        flags = (FLAG_WANT_SPEC if want_spec else 0) | (FLAG_SUMS_ZEROED if sums_zeroed else 0)
-        flags |= FLAG_MASK_IS_POWER if mask_is_power else 0     # `mask` = target power; output keeps the noisy phase
-        flags |= FLAG_MASK_IS_LOG_POWER if mask_is_log_power else 0
-        flags |= FLAG_WS_SELF_CLEAN if self_clean else 0        # `sums` is the tail of a persistent step workspace (see stft_features)
-        rc = _lib.load().se_mask_istft_ex(wavs.data_ptr() + 4 * int(ch_inp) * T, clean, C * T, mask.data_ptr(), mask_stride,
-                                          _p(lengths), B, T, n_fft, hop, window.data_ptr(), out.data_ptr(), out.stride(0),
-                                          int(pad_to), _p(sums) if want_sums else None, flags, _stream())
-        _lib.check(rc, "se_mask_istft_ex")
-    return out, (sums if want_sums else None)
+        rc = getattr(_lib.load(), entry)(wavs.data_ptr() + 4 * int(ch_inp) * T, clean, C * T, mask.data_ptr(), mask.shape[2],
+                                         _p(lengths), B, T, n_fft, hop, window.data_ptr(), out.data_ptr(), out.stride(0),
+                                         int(pad_to), _p(sums), *own, flags, _stream())
+        _lib.check(rc, entry)
+    return out, sums
+
+
+def mask_istft(wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, want_sums=True, want_spec=True,
+               out=None, sums=None, mask_padded=False, sums_zeroed=False, mask_is_power=False, ws=None,
+               mask_is_log_power=False):
+    """Fused ``istft(linear_inp * mask, phase_inp)`` straight from the noisy waveform.
+
+    wavs (B, C, T); mask (B, F, K), or (B, F, LD >= K) with mask_padded; lengths (B,) int64 or None.  Returns
+    (wav (B, width), sums (B, 6) float64|None).  ws: a step workspace (see ``stft_features``) instead of ``sums``.
+    mask_is_power: ``mask`` is the target power (``istft(mask, phase_inp)``); mask_is_log_power: it is the log of the target
+    power, e.g. model.LSTM's log_predicted (``istft(exp(mask), phase_inp)`` without the exp pass)."""
+    assert not (mask_is_power and mask_is_log_power), "mask_is_power and mask_is_log_power are mutually exclusive"
+    mask = _c(mask, "mask")
+    assert mask_padded or mask.shape[2] == n_fft // 2 + 1, f"mask {tuple(mask.shape)}: rows wider than K need mask_padded"
+    flags = (FLAG_WANT_SPEC if want_spec else 0) | (FLAG_MASK_IS_POWER if mask_is_power else 0)
+    flags |= FLAG_MASK_IS_LOG_POWER if mask_is_log_power else 0
+    return _mask_istft_call("se_mask_istft_ex", wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, out, want_sums,
+                            sums, sums_zeroed, ws, flags)
 
 
 def mask_istft_wsd_supported(n_fft, hop):
@@ -476,32 +514,24 @@ def mask_istft_wsd_supported(n_fft, hop):
     return bool(_lib.load().se_mask_istft_wsd_supported(int(n_fft), int(hop)))
 
 
+def mask_istft_register_resident(n_fft, hop, T):
+    """True if K3's register-resident kernel runs a step of T samples: a geometry of fastgeo.cu and T // hop + 1 >= 6 frames.
+    ``mask_istft_wsd`` and ``mask_istft_l1`` run exactly these steps (their ``_supported`` answer for the geometry)."""
+    return mask_istft_wsd_supported(n_fft, hop) and T // hop + 1 >= 6
+
+
 def mask_istft_wsd(wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, wsd_state, sums=None, sums_zeroed=False,
-                   self_clean=False):
+                   ws=None):
     """``mask_istft`` whose sums carry objective.WSD's terms instead of the spectral SI-SDR ones (se_mask_istft_wsd).
 
     mask (B, F, LD) row-padded; wsd_state: float32 (2,) device buffer, zero at rest (``se_wsd_eval_finish`` resets it); its
     element 0 receives the rank-local largest frame energy (all-reduce it with ``dp.global_max`` before the finish).
     Returns (wav (B, width), sums (B, 6) float64, frame_terms (B, F, 2) float32 = {frame energy, speech-distortion sum})."""
-    wavs, mask, window = _chk(wavs, "wavs"), _chk(mask, "mask"), _c(window, "window")
     wsd_state = _chk(wsd_state, "wsd_state")
-    assert wavs.dim() == 3 and wavs.is_contiguous() and wsd_state.numel() == 2 and wsd_state.is_contiguous()
-    B, C, T = wavs.shape
-    F, K = T // hop + 1, n_fft // 2 + 1
-    assert mask.dim() == 3 and mask.shape[:2] == (B, F) and mask.shape[2] >= K and mask.stride(2) == 1 and mask.stride(1) == mask.shape[2]
-    lengths = _c(lengths, "lengths", torch.int64)
-    width = max(hop * (F - 1), int(pad_to))
-    with torch.cuda.device(wavs.device):
-        out = torch.empty(B, width, device=wavs.device, dtype=torch.float32)
-        if sums is None:
-            sums = torch.empty(B, NSUMS, device=wavs.device, dtype=torch.float64)
-        terms = torch.empty(B, F, 2, device=wavs.device, dtype=torch.float32)
-        flags = (FLAG_SUMS_ZEROED if sums_zeroed else 0) | (FLAG_WS_SELF_CLEAN if self_clean else 0)
-        rc = _lib.load().se_mask_istft_wsd(wavs.data_ptr() + 4 * int(ch_inp) * T, wavs.data_ptr() + 4 * int(ch_tar) * T, C * T,
-                                           mask.data_ptr(), mask.shape[2], _p(lengths), B, T, n_fft, hop, window.data_ptr(),
-                                           out.data_ptr(), out.stride(0), int(pad_to), sums.data_ptr(), terms.data_ptr(),
-                                           wsd_state.data_ptr(), flags, _stream())
-        _lib.check(rc, "se_mask_istft_wsd")
+    assert wsd_state.numel() == 2 and wsd_state.is_contiguous()
+    terms = torch.empty(*mask.shape[:2], 2, device=mask.device, dtype=torch.float32)
+    out, sums = _mask_istft_call("se_mask_istft_wsd", wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, None, True,
+                                 sums, sums_zeroed, ws, 0, terms.data_ptr(), wsd_state.data_ptr())
     return out, sums, terms
 
 
@@ -525,33 +555,18 @@ def mask_istft_l1_supported(n_fft, hop):
 
 
 def mask_istft_l1(wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, l1_acc, eps=1e-10, sums=None, sums_zeroed=False,
-                  self_clean=False):
+                  ws=None):
     """``mask_istft(mask_is_log_power=True)`` whose clean-frame pass sums objective.L1's terms (se_mask_istft_l1).
 
     mask (B, F, LD) row-padded log target power; l1_acc: float64 (2,) device buffer, zero at rest (``l1_eval_finish`` resets it),
     += [sum |lp - log(|C|^2 + eps)|, element count] of the batch's valid frames (all-reduce it with ``dp.reduce_sums`` before the
     finish).  Returns (wav (B, width), sums (B, 6) float64 with each utterance's L1 sum in column 3, SE_SUM_SPEC_ST)."""
-    wavs, mask, window = _chk(wavs, "wavs"), _chk(mask, "mask"), _c(window, "window")
     l1_acc = _chk(l1_acc, "l1_acc", torch.float64)
-    assert wavs.dim() == 3 and wavs.is_contiguous()
     assert l1_acc.numel() == 2 and l1_acc.is_contiguous()
-    B, C, T = wavs.shape
-    F, K = T // hop + 1, n_fft // 2 + 1
-    assert mask.dim() == 3 and mask.shape[:2] == (B, F) and mask.shape[2] >= K and mask.stride(2) == 1 and mask.stride(1) == mask.shape[2]
-    assert mask.stride(0) == F * mask.shape[2], "mask must be contiguous along the batch (the kernel reads row u at u * F * LD)"
-    lengths = _c(lengths, "lengths", torch.int64)
-    width = max(hop * (F - 1), int(pad_to))
-    with torch.cuda.device(wavs.device):
-        out = torch.empty(B, width, device=wavs.device, dtype=torch.float32)
-        if sums is None:
-            sums = torch.empty(B, NSUMS, device=wavs.device, dtype=torch.float64)
-        flags = (FLAG_SUMS_ZEROED if sums_zeroed else 0) | (FLAG_WS_SELF_CLEAN if self_clean else 0)
-        rc = _lib.load().se_mask_istft_l1(wavs.data_ptr() + 4 * int(ch_inp) * T, wavs.data_ptr() + 4 * int(ch_tar) * T, C * T,
-                                          mask.data_ptr(), mask.shape[2], _p(lengths), B, T, n_fft, hop, window.data_ptr(),
-                                          out.data_ptr(), out.stride(0), int(pad_to), sums.data_ptr(), l1_acc.data_ptr(), float(eps),
-                                          flags, _stream())
-        _lib.check(rc, "se_mask_istft_l1")
-    return out, sums
+    assert mask.dim() == 3 and mask.stride(0) == mask.shape[1] * mask.shape[2], \
+        "mask must be contiguous along the batch (the kernel reads row u at u * F * LD)"
+    return _mask_istft_call("se_mask_istft_l1", wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, None, True, sums,
+                            sums_zeroed, ws, 0, l1_acc.data_ptr(), float(eps))
 
 
 def l1_eval_sums(log_predicted, linear_tar, lengths, T, hop, K, sums, l1_acc, eps=1e-10):
