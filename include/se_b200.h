@@ -173,6 +173,29 @@ int se_l1_logspec_bwd(const float* log_predicted, const float* linear_tar, const
                       int64_t n_frames, int64_t K, float eps, double count, const float* grad_out,
                       float* grad_log_predicted, void* stream);
 
+/* se_l1_mask_step: objective.L1's part of one training step (the counterpart of se_sisdr_mask_step) on row-strided tensors:
+ * log_predicted (n_utt, n_frames, ld_lp) and the clean power linear_tar (n_utt, n_frames, ld_tar), rows ld_* floats apart (float4
+ * loads when every ld is a multiple of 4 and the pointers are 16-byte aligned), columns >= K never read.  lengths / len_hop as in
+ * se_sisdr_mask_step.  Over the valid frames f < frames_u and the K bins, d = log_predicted - log(linear_tar + eps):
+ *   loss_mean (1 float) = sum |d| / count with count = K sum_u frames_u -- the element mean of the batch this rank holds, which is
+ *     what objective.L1 returns on each rank under data parallelism;
+ *   loss_per_utt[u] (may be NULL) = the utterance's own sum |d| / (K frames_u);
+ *   grad (may be NULL; ld_g floats between rows) = d loss_mean / d log_predicted = sign(d) / count, with se_l1_logspec_bwd's sign
+ *     (0 for d == 0 and for NaN), 0 on padded frames and on the pad columns [K, ld_g).
+ * Two launches and no atomics: every CTA writes the double sum of its frame chunk to its own slot of ws_partials
+ * (se_l1_mask_step_workspace doubles, caller-owned, no zeroing needed) and a one-CTA finish adds the slots in a fixed order, so the
+ * loss is bitwise repeatable.  No host synchronisation: capturable. */
+int64_t se_l1_mask_step_workspace(int64_t n_utt, int64_t n_frames, int64_t K);
+int se_l1_mask_step(const float* log_predicted, int64_t ld_lp, const float* linear_tar, int64_t ld_tar, const int64_t* lengths,
+                    int64_t len_hop, int64_t n_utt, int64_t n_frames, int64_t K, float eps, double* ws_partials, int64_t ws_doubles,
+                    float* loss_per_utt, float* loss_mean, float* grad, int64_t ld_g, void* stream);
+
+/* se_act_grad_inplace: grad <- grad * act'(out) on n_rows rows (grad rows ld_g floats apart, out rows ld_out apart), where out is
+ * the head's output AFTER its activation: Sigmoid out (1 - out), ReLU (out > 0); columns [K, ld_g) of grad are set to 0.  It turns
+ * an objective's d loss / d output into d loss / d pre-activation (the operand of both weight- and input-gradient GEMMs).
+ * act = SE_ACT_IDENTITY returns at once without a launch. */
+int se_act_grad_inplace(float* grad, int64_t ld_g, const float* out, int64_t ld_out, int64_t n_rows, int64_t K, int act, void* stream);
+
 /* ---- K4d: weighted speech distortion objective (objective.py:120-153) ------------------
  * loss = alpha * mean_u sum_{f<len,k} ((S - G S) voiced)^2 + (1 - alpha) * mean_u sum (G max(X - S, 0))^2 with
  * S = linear_tar, X = linear_inp, G = offset; voiced[u,f] = 10 log10(sum_k S + eps) > 10 log10(max_{u,f} sum_k S + eps)
@@ -406,7 +429,9 @@ int se_head_grad_embeddings_sisdr(const float* x, int64_t ldx, const double* sta
                                   void* stream);
 
 /* ---- gradient clipping + Adam on the head's parameters (runner.py:463-466: clip_grad_norm_ then optimizer.step) -------
- * params / grads / exp_avg / exp_avg_sq: HOST arrays of n_tensors (<= 8) device pointers, numels their sizes.  Semantics of
+ * params / grads / exp_avg / exp_avg_sq: HOST arrays of n_tensors device pointers (se_adam_clip_step: <= 8, its original limit;
+ * se_adam_clip_step_mirror: <= 32, e.g. a bidirectional 3-layer LSTM body and its projection, 26 tensors), numels their sizes.
+ * Semantics of
  * torch.nn.utils.clip_grad_norm_(max_norm) (skipped if max_norm <= 0; the scaled gradient is written back) followed by
  * torch.optim.Adam.step (L2 weight_decay, no amsgrad).  A NaN / inf gradient norm skips the update (runner.py:467-470):
  * parameters, moments and the step count keep their values and the skipped-step counter advances.  ws_acc: 1 double,

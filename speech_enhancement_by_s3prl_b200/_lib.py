@@ -62,6 +62,9 @@ _SIGNATURES = {
     "se_sisdr_spec_bwd": [c_f, c_f, c_f, i64, i64, i64, c_float, c_f, c_f, c_f, c_f],
     "se_l1_logspec_fwd": [c_f, c_f, c_f, i64, i64, i64, c_float, c_f, c_f],
     "se_l1_logspec_bwd": [c_f, c_f, c_f, i64, i64, i64, c_float, c_double, c_f, c_f, c_f],
+    "se_l1_mask_step_workspace": [i64, i64, i64],
+    "se_l1_mask_step": [c_f, i64, c_f, i64, c_f, i64, i64, i64, i64, c_float, c_f, i64, c_f, c_f, c_f, i64, c_f],
+    "se_act_grad_inplace": [c_f, i64, c_f, i64, i64, i64, c_int, c_f],
     "se_mix_batch": [c_f, i64, c_f, c_f, i64, c_f, c_f, i64, i64, c_float, c_float, c_f, c_f, c_f],
     "se_wsd_fwd": [c_f, c_f, c_f, c_f, i64, i64, i64, c_float, c_float, c_float, c_f, c_f, c_f, c_f, c_f],
     "se_wsd_bwd": [c_f, c_f, c_f, c_f, i64, i64, i64, c_float, c_float, c_float, c_f, c_f, c_f, c_f, c_f],

@@ -207,8 +207,9 @@ __global__ void __launch_bounds__(256) sisdr_mask_bwd_kernel(const SisdrMaskArgs
 // ------------------------------------------------------------------ gradient clipping + Adam for the head's parameters
 // runner.py:463-466 (clip_grad_norm_ -> optimizer.step) on a handful of small tensors: torch runs ~15 launches for it,
 // here it is two -- the squared gradient norm, then clip + update.  All state (moments, step count, norm accumulator) lives
-// on the device, so the pair replays from a CUDA graph.
-constexpr int kAdamMaxTensors = 8;
+// on the device, so the pair replays from a CUDA graph.  32 tensors cover a bidirectional 3-layer LSTM body and its projection (26);
+// AdamArgs (1976 bytes) travels by value, far inside the kernel-parameter limit.
+constexpr int kAdamMaxTensors = 32;
 struct AdamArgs {
     float* p[kAdamMaxTensors]; float* g[kAdamMaxTensors]; float* m[kAdamMaxTensors]; float* v[kAdamMaxTensors];
     long long n[kAdamMaxTensors];
@@ -566,6 +567,136 @@ __global__ void __launch_bounds__(256) wsd_mask_bwd_kernel(const WsdMaskArgs a) 
                 if (c + e < a.K) g[e] = wsd_grad(o[e], x[e], t[e], voiced, a.alpha, scale);
         }
         if (c + V <= a.ld_g) stv<V>(a.grad_offset + r * a.ld_g + c, g);
+    }
+}
+
+// ------------------------------------------------------------------ log-spectral L1 objective on row-padded tensors (training step)
+// objective.L1 of log_predicted against log(linear_tar + eps) over the valid frames: one CTA per (utterance, frame chunk) writes the
+// double sum of its chunk to its own slot of `partials` (no atomics), the finish kernel adds the slots in a fixed order -- the loss
+// is bitwise repeatable.  The same pass writes d loss / d log_predicted = sign(d) / count (the sign of se_l1_logspec_bwd: 0 for
+// d == 0 and for NaN), 0 on padded frames and on the pad columns of a row.
+struct L1MaskArgs {
+    const float* lp; const float* tar;
+    long long ld_lp, ld_tar;
+    const long long* lengths;
+    int len_hop;             // > 0: lengths holds SAMPLE lengths, frames = len / len_hop + 1 (runner.py:455)
+    int n_utt, n_frames, K, chunks;
+    float eps;
+    double* partials;        // (n_utt, chunks)
+    float* grad; long long ld_g;   // grad may be null
+};
+
+__device__ __forceinline__ int l1_valid_frames(const L1MaskArgs& a, int u) {
+    long long v = a.n_frames;
+    if (a.lengths) v = a.len_hop > 0 ? a.lengths[u] / a.len_hop + 1 : a.lengths[u];
+    return (int)max(0LL, min((long long)a.n_frames, v));
+}
+
+template <int V>
+__global__ void __launch_bounds__(256) l1_mask_step_kernel(const L1MaskArgs a) {
+    __shared__ double part[8];
+    __shared__ long long count[8];
+    const int u = blockIdx.x / a.chunks, chunk = blockIdx.x - u * a.chunks;
+    const int warp = threadIdx.x >> 5, nwarps = (int)(blockDim.x >> 5);
+    const int valid = l1_valid_frames(a, u);
+    float scale = 0.0f;
+    if (a.grad) {            // 1 / (K * sum_u valid_u): every CTA counts the batch's frames itself (n_utt loads)
+        long long c = 0;
+        for (int v = threadIdx.x; v < a.n_utt; v += blockDim.x) c += l1_valid_frames(a, v);
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
+        if ((threadIdx.x & 31) == 0) count[warp] = c;
+        __syncthreads();
+        c = 0;
+        for (int w = 0; w < nwarps; ++w) c += count[w];
+        scale = c > 0 ? (float)(1.0 / (double)(c * a.K)) : 0.0f;
+    }
+    const int KV = a.grad ? max((int)(a.ld_g / V), (a.K + V - 1) / V) : (a.K + V - 1) / V;   // whole rows of grad
+    const int per = (a.n_frames + a.chunks - 1) / a.chunks;
+    const int f_lo = chunk * per, f_hi = min(a.grad ? a.n_frames : valid, f_lo + per);
+    const long long row0 = (long long)u * a.n_frames;
+    const int items = max(f_hi - f_lo, 0) * KV;
+    float acc = 0.0f;
+#pragma unroll 4
+    for (int i = threadIdx.x; i < items; i += blockDim.x) {
+        const int fr = i / KV, c = (i - fr * KV) * V;
+        const int f = f_lo + fr;
+        const long long r = row0 + f;
+        float g[V];
+#pragma unroll
+        for (int e = 0; e < V; ++e) g[e] = 0.0f;
+        if (f < valid && c < a.K) {
+            float p[V], t[V];
+            ldv<V>(a.lp + r * a.ld_lp + c, p);
+            ldv<V>(a.tar + r * a.ld_tar + c, t);
+#pragma unroll
+            for (int e = 0; e < V; ++e)
+                if (c + e < a.K) {
+                    const float d = p[e] - logf(t[e] + a.eps);
+                    acc += fabsf(d);
+                    g[e] = d > 0.0f ? scale : (d < 0.0f ? -scale : 0.0f);
+                }
+        }
+        if (a.grad && c + V <= a.ld_g) stv<V>(a.grad + r * a.ld_g + c, g);
+    }
+    const double s = secommon::warp_sum((double)acc);
+    if ((threadIdx.x & 31) == 0) part[warp] = s;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double t = 0.0;
+        for (int w = 0; w < nwarps; ++w) t += part[w];
+        a.partials[blockIdx.x] = t;
+    }
+}
+
+// one CTA: loss_per_utt[u] = (sum of u's slots) / (valid_u K) (may be null) and loss_mean = the batch's sum / (K sum_u valid_u)
+__global__ void __launch_bounds__(256) l1_mask_finish_kernel(const L1MaskArgs a, float* __restrict__ loss_per_utt,
+                                                             float* __restrict__ loss_mean) {
+    __shared__ double part[8];
+    __shared__ long long count[8];
+    double s = 0.0;
+    long long n = 0;
+    for (int u = threadIdx.x; u < a.n_utt; u += blockDim.x) {
+        double su = 0.0;
+        for (int c = 0; c < a.chunks; ++c) su += a.partials[(long long)u * a.chunks + c];
+        const int v = l1_valid_frames(a, u);
+        if (loss_per_utt) loss_per_utt[u] = (float)(su / ((double)v * a.K));
+        s += su;
+        n += v;
+    }
+    s = secommon::warp_sum(s);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
+    if ((threadIdx.x & 31) == 0) { part[threadIdx.x >> 5] = s; count[threadIdx.x >> 5] = n; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        s = 0.0;
+        n = 0;
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) { s += part[w]; n += count[w]; }
+        *loss_mean = (float)(s / ((double)n * a.K));
+    }
+}
+
+// g <- g * act'(out) on row-strided tensors, out = the head's output AFTER the activation (Sigmoid: out (1 - out), ReLU: out > 0):
+// d loss / d output becomes d loss / d pre-activation.  Columns [K, ld_g) of g are set to 0 (the pad columns of `out` are unspecified).
+template <int V>
+__global__ void __launch_bounds__(256) act_grad_kernel(float* __restrict__ g, long long ld_g, const float* __restrict__ out, long long ld_out,
+                                                       long long n_rows, int K, int act) {
+    const long long per_row = ld_g / V, n = n_rows * per_row;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        const long long r = i / per_row;
+        const int c = (int)(i - r * per_row) * V;
+        float gv[V], o[V];
+#pragma unroll
+        for (int e = 0; e < V; ++e) o[e] = 0.0f;
+        ldv<V>(g + r * ld_g + c, gv);
+        if (c < K) ldv<V>(out + r * ld_out + c, o);
+#pragma unroll
+        for (int e = 0; e < V; ++e) {
+            const float y = o[e];
+            gv[e] = c + e >= K ? 0.0f : (act == SE_ACT_SIGMOID ? gv[e] * y * (1.0f - y) : gv[e] * (y > 0.0f ? 1.0f : 0.0f));
+        }
+        stv<V>(g + r * ld_g + c, gv);
     }
 }
 
@@ -1094,6 +1225,9 @@ int se_sisdr_mask_step(const float* offset, int64_t ld_off, const float* linear_
 int se_adam_clip_step(float* const* params, float* const* grads, float* const* exp_avg, float* const* exp_avg_sq,
                       const int64_t* numels, int n_tensors, float lr, float beta1, float beta2, float eps, float weight_decay,
                       float max_norm, double* ws_acc, int* ws_state, void* stream) {
+    // this entry keeps its original limit of 8 tensors (callers may size their arrays by it); the mirror form takes 32
+    SE_REQUIRE(n_tensors > 0 && n_tensors <= 8, "n_tensors=%d must be in [1, 8] (se_adam_clip_step_mirror takes up to %d)", n_tensors,
+               kAdamMaxTensors);
     return se_adam_clip_step_mirror(params, grads, exp_avg, exp_avg_sq, numels, n_tensors, lr, beta1, beta2, eps, weight_decay, max_norm,
                                     nullptr, nullptr, nullptr, 0, ws_acc, ws_state, stream);
 }
@@ -1266,6 +1400,49 @@ int se_l1_eval_finish(const double* sums, const int64_t* lengths, int64_t n_utt,
     l1_eval_finish_kernel<<<1, 256, 0, (cudaStream_t)stream>>>(sums, reinterpret_cast<const long long*>(lengths), (int)n_utt,
                                                               (long long)T, hop, (long long)K, l1_acc, loss_per_utt, loss, metric_acc);
     return secommon::check_launch("l1_eval_finish_kernel");
+}
+
+int64_t se_l1_mask_step_workspace(int64_t n_utt, int64_t n_frames, int64_t K) {
+    if (n_utt <= 0 || n_frames <= 0 || K <= 0) return 0;
+    return n_utt * pick_chunks(n_utt, n_frames * K, 2048);
+}
+
+int se_l1_mask_step(const float* log_predicted, int64_t ld_lp, const float* linear_tar, int64_t ld_tar, const int64_t* lengths,
+                    int64_t len_hop, int64_t n_utt, int64_t n_frames, int64_t K, float eps, double* ws_partials, int64_t ws_doubles,
+                    float* loss_per_utt, float* loss_mean, float* grad, int64_t ld_g, void* stream) {
+    SE_REQUIRE(log_predicted && linear_tar && ws_partials && loss_mean && n_utt > 0 && n_frames > 0 && K > 0, "bad argument");
+    SE_REQUIRE(ld_lp >= K && ld_tar >= K && (!grad || ld_g >= K), "row stride smaller than K");
+    SE_REQUIRE(len_hop >= 0 && len_hop < (1LL << 30), "len_hop=%lld out of range", (long long)len_hop);
+    SE_REQUIRE(n_utt <= 0x7fffffffLL && n_frames <= 0x7fffffffLL && K <= 0x7fffffffLL, "shape too large");
+    SE_REQUIRE(ws_doubles >= se_l1_mask_step_workspace(n_utt, n_frames, K), "ws_partials holds %lld doubles, %lld needed",
+               (long long)ws_doubles, (long long)se_l1_mask_step_workspace(n_utt, n_frames, K));
+    L1MaskArgs a{};
+    a.lp = log_predicted; a.tar = linear_tar; a.ld_lp = ld_lp; a.ld_tar = ld_tar;
+    a.lengths = reinterpret_cast<const long long*>(lengths); a.len_hop = (int)len_hop;
+    a.n_utt = (int)n_utt; a.n_frames = (int)n_frames; a.K = (int)K; a.chunks = pick_chunks(n_utt, n_frames * K, 2048);
+    a.eps = eps; a.partials = ws_partials; a.grad = grad; a.ld_g = ld_g;
+    cudaStream_t st = (cudaStream_t)stream;
+    const bool v4 = vec4_ok(log_predicted, ld_lp, K) && vec4_ok(linear_tar, ld_tar, K) && vec4_ok(grad, ld_g, K);
+    if (v4) l1_mask_step_kernel<4><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
+    else l1_mask_step_kernel<1><<<(unsigned)(n_utt * a.chunks), 256, 0, st>>>(a);
+    int rc = secommon::check_launch("l1_mask_step_kernel");
+    if (rc != SE_OK) return rc;
+    l1_mask_finish_kernel<<<1, 256, 0, st>>>(a, loss_per_utt, loss_mean);
+    return secommon::check_launch("l1_mask_finish_kernel");
+}
+
+int se_act_grad_inplace(float* grad, int64_t ld_g, const float* out, int64_t ld_out, int64_t n_rows, int64_t K, int act, void* stream) {
+    SE_REQUIRE(act >= SE_ACT_IDENTITY && act <= SE_ACT_SIGMOID, "unknown activation %d", act);
+    if (act == SE_ACT_IDENTITY) return SE_OK;                           // act' = 1: nothing to do
+    SE_REQUIRE(grad && out && n_rows > 0 && K > 0 && K <= 0x7fffffffLL, "bad argument");
+    SE_REQUIRE(ld_g >= K && ld_out >= K, "row stride smaller than K");
+    const bool v4 = vec4_ok(grad, ld_g, K) && vec4_ok(out, ld_out, K);
+    const long long n = n_rows * (v4 ? ld_g / 4 : ld_g);
+    const long long blocks = std::min((n + 255) / 256, 148LL * 8);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (v4) act_grad_kernel<4><<<(unsigned)blocks, 256, 0, st>>>(grad, ld_g, out, ld_out, n_rows, (int)K, act);
+    else act_grad_kernel<1><<<(unsigned)blocks, 256, 0, st>>>(grad, ld_g, out, ld_out, n_rows, (int)K, act);
+    return secommon::check_launch("act_grad_kernel");
 }
 
 int se_l1_logspec_fwd(const float* log_predicted, const float* linear_tar, const int64_t* stft_len, int64_t n_utt,

@@ -222,40 +222,71 @@ class EnhancementEngine:
         """K1 -> cuDNN LSTM body (torch, no_grad) -> [Residual's CMVN over the hidden states, torch] -> the library's projection
         (TMA head when the hidden width is a multiple of 4 and precision=1, else the padded head) -> mask (B, F, round4(K)):
         model.LSTM's log_predicted or model.Residual's offset.  launches_per_step counts everything but the body."""
-        head, dev = self.head, wavs.device
-        window = self.pre._frame_window
-        K = self.n_fft // 2 + 1
-        if self.feat_cfg is not None:
-            if D is None:
-                raise RuntimeError("EnhancementEngine.eval_step: feat_cfg must be a mel config (log / delta <= 2, no CMVN of its own)")
-            cfg = self.feat_cfg
-            power = ops.stft_padded(wavs, self.ch_inp, self.n_fft, self.hop, window, logpower=False)
-            feats = ops.mel_features(power, self.pre._tables(dev)[1], bool(cfg.get("log", False)), self.pre.eps,
-                                     order=int(cfg.get("delta", 0)), K=K)
-            self.launches_per_step = 2
-        else:
-            feats = ops.stft_padded(wavs, self.ch_inp, self.n_fft, self.hop, window, logpower=self.log_features, log_eps=self.pre.eps)
-            self.launches_per_step = 1
-        if head.lstm.input_size != D:
-            raise RuntimeError(f"EnhancementEngine.eval_step: the {type(head).__name__} head takes {head.lstm.input_size} features, "
-                               f"the engine's feature has {D}")
-        x = feats[..., :D]
-        if not x.is_contiguous():
-            x = x.contiguous()                                           # out of the 16-byte padded rows
-            self.launches_per_step += 1
-        hidden, _ = head.lstm(x)                                         # the cuDNN body (DESIGN section 7)
-        if type(head).__name__ == "Residual" and head.cmvn:              # model.py:88, over every frame of the padded batch
-            hidden = (hidden - hidden.mean(dim=1, keepdim=True)) / (hidden.std(dim=1, keepdim=True) + head.eps)
-            self.launches_per_step += 5
-        B, F, H = hidden.shape
-        hidden = hidden.contiguous()
-        if self.precision == 1 and H % 4 == 0 and ops.linear_head_tma_supported(B, F, H, K, H, wpad.shape[1], ops.round4(K)):
-            mask = ops.linear_head_tma(hidden, H, wpad, self._proj().bias, head.activation, None, 0.0)
-        else:
-            mask = ops.linear_head_padded(hidden, H, wpad, self._proj().bias, head.activation, None, None, 0.0,
-                                          precision=self.precision)
+        feats = self._recurrent_k1(wavs, D)[0]
+        hidden = self._recurrent_body(self._recurrent_input(feats, D, "eval_step"))
+        mask = self._recurrent_project(hidden, wpad)
+        self.launches_per_step = (2 if self.feat_cfg is not None else 1) + int(D != feats.shape[2])   # K1 (+ K1b), the copy
+        self.launches_per_step += 5 if self._recurrent_cmvn() else 0
         self.launches_per_step += 1 + 3                                  # projection, K3's sums fill, K3, K3'
         return mask
+
+    def _recurrent_k1(self, wavs, D, spectra=False):
+        """K1 of the recurrent routes: the head's input (B, F, LD) -- the (log-)power spectrum of the input channel, or the mel feature
+        of ``feat_cfg`` -- and with ``spectra`` also both channels' power spectra linear_inp and linear_tar (B, F, round4(K)) that the
+        training step's objectives read (one launch for all three where the register-resident pair kernel exists).  Returns
+        (feats, linear_inp | None, linear_tar | None)."""
+        dev, window = wavs.device, self.pre._frame_window
+        K = self.n_fft // 2 + 1
+        linear_inp = linear_tar = None
+        if self.feat_cfg is not None:
+            if D is None:
+                raise RuntimeError(f"EnhancementEngine.{'train_step' if spectra else 'eval_step'}: feat_cfg must be a mel config "
+                                   "(log / delta <= 2, no CMVN of its own)")
+            cfg = self.feat_cfg
+            linear_inp = ops.stft_padded(wavs, self.ch_inp, self.n_fft, self.hop, window, logpower=False)
+            feats = ops.mel_features(linear_inp, self.pre._tables(dev)[1], bool(cfg.get("log", False)), self.pre.eps,
+                                     order=int(cfg.get("delta", 0)), K=K)
+        elif not spectra:
+            feats = ops.stft_padded(wavs, self.ch_inp, self.n_fft, self.hop, window, logpower=self.log_features, log_eps=self.pre.eps)
+        elif self.log_features:
+            linear_inp, feats, linear_tar, _ = ops.stft_features_pair(wavs, self.ch_inp, self.ch_tar, self.n_fft, self.hop, window,
+                                                                      log_eps=self.pre.eps)
+        else:
+            feats = linear_inp = ops.stft_padded(wavs, self.ch_inp, self.n_fft, self.hop, window, logpower=False)
+        if spectra and linear_tar is None:
+            linear_tar = ops.stft_padded(wavs, self.ch_tar, self.n_fft, self.hop, window, logpower=False)
+        return feats, linear_inp, linear_tar
+
+    def _recurrent_input(self, feats, D, caller):
+        """The recurrent head's input (B, F, D), copied out of K1's 16-byte padded rows where they are wider than D."""
+        head = self.head
+        if head.lstm.input_size != D:
+            raise RuntimeError(f"EnhancementEngine.{caller}: the {type(head).__name__} head takes {head.lstm.input_size} features, "
+                               f"the engine's feature has {D}")
+        x = feats[..., :D]
+        return x if x.is_contiguous() else x.contiguous()
+
+    def _recurrent_cmvn(self):
+        return type(self.head).__name__ == "Residual" and self.head.cmvn
+
+    def _recurrent_body(self, x):
+        """The cuDNN LSTM body (DESIGN section 7) [+ Residual's CMVN over every frame of the padded batch, model.py:88] in torch:
+        recorded for autograd when grad mode is on.  Returns the projection's input (B, F, hidden * directions), contiguous."""
+        head = self.head
+        hidden, _ = head.lstm(x)
+        if self._recurrent_cmvn():
+            hidden = (hidden - hidden.mean(dim=1, keepdim=True)) / (hidden.std(dim=1, keepdim=True) + head.eps)
+        return hidden.contiguous()
+
+    def _recurrent_project(self, hidden, wpad):
+        """The library's projection of the hidden states -> (B, F, round4(K)): the TMA head when the hidden width is a multiple of 4
+        at precision 1, else the padded head."""
+        B, F, H = hidden.shape
+        K = self.n_fft // 2 + 1
+        if self.precision == 1 and H % 4 == 0 and ops.linear_head_tma_supported(B, F, H, K, H, wpad.shape[1], ops.round4(K)):
+            return ops.linear_head_tma(hidden, H, wpad, self._proj().bias, self.head.activation, None, 0.0)
+        return ops.linear_head_padded(hidden, H, wpad, self._proj().bias, self.head.activation, None, None, 0.0,
+                                      precision=self.precision)
 
     def _l1_terms_from_spectra(self, wavs, mask, lengths, criterion, sums, l1_acc):
         """objective.L1's sums where K3 has no L1 variant (other geometries, or fewer than 6 frames): the clean power spectrum is
@@ -307,7 +338,34 @@ class EnhancementEngine:
                     bits = buf.view(torch.int32)
                     bits.add_(0x1000).bitwise_and_(~0x1FFF)
             self._wpad_key = key
+            self._refresh_weight_t()
         return buf
+
+    def _padded_weight_t(self):
+        """The transposed copy of ``_padded_weight``, (Din, round4(Dout)) with zero pad columns: the weight operand of the recurrent
+        training step's input gradient dH = dZ W (the TMA head run on W^T).  A second persistent buffer under the same version key,
+        refreshed in place whenever the first one is (also by the captured step after every update), so graphs always read the
+        trained weights.  TF32 values copied from the rounded buffer stay TF32."""
+        buf = self._padded_weight()
+        Din = self._proj().weight.shape[1]
+        if self._weight_t() is None:
+            self._wtpad = torch.zeros(Din, ops.round4(buf.shape[0]), device=buf.device, dtype=torch.float32)
+            self._refresh_weight_t()
+        return self._wtpad
+
+    def _weight_t(self):
+        """The W^T buffer if it exists and matches the current padded weight, else None (and the stale one is dropped)."""
+        wt, buf = getattr(self, "_wtpad", None), getattr(self, "_wpad", None)
+        if wt is not None and (buf is None or wt.device != buf.device or
+                               wt.shape != (self._proj().weight.shape[1], ops.round4(buf.shape[0]))):
+            wt = self._wtpad = None
+        return wt
+
+    def _refresh_weight_t(self):
+        wt = self._weight_t()
+        if wt is not None:
+            with torch.no_grad():
+                wt[:, :self._wpad.shape[0]].copy_(self._wpad[:, :wt.shape[0]].t())
 
     # ------------------------------------------------------------------ CUDA-graph replay of the step
     def capture_bound(self, lengths, wavs, metric_acc=None, want_stoi=False, stoi_acc=None, criterion=None):
@@ -405,11 +463,16 @@ class EnhancementEngine:
     def fused_training_supported(self, objective, B, T):
         """True if train_step can take the fused route: LinearResidual with the SISDR or the WSD objective and the tensor-core
         head, on the (log-)power spectrum or on a mel feature config (pseudo_noise.yaml:10-15), shapes inside the TMA head's / the
-        split-K backward's range."""
+        split-K backward's range.  Recurrent heads: model.LSTM with objective.L1 and model.Residual with objective.SISDR / WSD (with
+        or without its CMVN), a hidden width (x directions) that is a multiple of 4, and both projections -- hidden -> K forward and
+        K -> hidden for the input gradient -- on the TMA head (see _fused_recurrent_forward_backward).  Every other pair (e.g. LSTM
+        with SISDR, or Linear) takes the autograd route."""
         from . import model, objective as obj
-        if not self.fused_training or self.precision != 1 or type(objective) not in (obj.SISDR, obj.WSD):
+        if not self.fused_training or self.precision != 1:
             return False
-        if type(self.head) is not model.LinearResidual:
+        if _recurrent(self.head):
+            return self._fused_recurrent_supported(objective, B, T)
+        if type(objective) not in (obj.SISDR, obj.WSD) or type(self.head) is not model.LinearResidual:
             return False
         F, K = T // self.hop + 1, self.n_fft // 2 + 1
         LD = ops.round4(K)
@@ -419,6 +482,72 @@ class EnhancementEngine:
         if self.head.linear.weight.shape != (K, D):
             return False
         return (ops.linear_head_tma_supported(B, F, D, K, ops.round4(D), ops.round4(D), LD) and ops.linear_head_bwd_fused_supported(B, F, D, K))
+
+    def _fused_recurrent_supported(self, objective, B, T):
+        from . import model, objective as obj
+        head = self.head
+        if not ((type(head) is model.LSTM and type(objective) is obj.L1) or
+                (type(head) is model.Residual and type(objective) in (obj.SISDR, obj.WSD))):
+            return False
+        F, K = T // self.hop + 1, self.n_fft // 2 + 1
+        LD = ops.round4(K)
+        D = K if self.feat_cfg is None else self._mel_feature_dim()
+        H = head.lstm.hidden_size * (2 if head.lstm.bidirectional else 1)
+        if D is None or head.lstm.input_size != D or getattr(head.lstm, "proj_size", 0) or H % 4 or self._proj().weight.shape != (K, H):
+            return False
+        return (ops.linear_head_tma_supported(B, F, H, K, H, H, LD) and ops.linear_head_tma_supported(B, F, K, H, LD, LD, H) and
+                ops.linear_head_bwd_fused_supported(B, F, H, K))
+
+    def _fused_recurrent_forward_backward(self, lengths, wavs, objective):
+        """runner.py:431-460 for model.LSTM + objective.L1 and model.Residual + objective.SISDR / WSD: the cuDNN body and Residual's
+        CMVN stay in torch autograd (DESIGN section 7); everything around them runs on the library's padded kernels.
+          K1 (both channels) -> copy out of the padded rows -> body (+ CMVN), recorded for autograd
+          -> projection forward on the TMA head (detached hidden states) -> the objective's step: loss and d loss / d output
+             (objective.WSD: its batch maximum all-reduced on the side stream under the projection)
+          -> act'(output) in place: dZ, read by both GEMMs -> weight / bias gradient (split-K TMA kernel)
+          -> dH = dZ W (TMA head on the persistent TF32 W^T copy) -> torch.autograd.backward(hidden, dH): cuDNN BPTT [+ CMVN's].
+        Leaves the gradients in ``.grad`` and returns the loss (objective.L1: the element mean of this rank's batch)."""
+        from . import objective as obj
+        head, dev = self.head, wavs.device
+        if self.pre._frame_window.device != dev:
+            self.pre.to(dev)
+        K = self.n_fft // 2 + 1
+        D = K if self.feat_cfg is None else self._mel_feature_dim()
+        kind = type(objective)
+        with torch.no_grad():
+            feats, linear_inp, linear_tar = self._recurrent_k1(wavs, D, spectra=True)
+            x = self._recurrent_input(feats, D, "train_step")
+        with torch.enable_grad():
+            hidden = self._recurrent_body(x)
+        proj = self._proj()
+        with torch.no_grad():
+            wpad, wt = self._padded_weight(), self._padded_weight_t()
+            h = hidden.detach()
+            H = h.shape[2]
+            head_fwd = lambda: ops.linear_head_tma(h, H, wpad, proj.bias, head.activation, None, 0.0)
+            lens = _c64(lengths)
+            if kind is obj.WSD:
+                energy, emax = ops.wsd_energy(linear_tar, K)
+                out = self._all_reduce_beside(dp.global_max, emax, head_fwd)
+                loss, _, dz, _ = ops.wsd_mask_step(out, linear_inp, linear_tar, lens, self.hop, K, energy, emax, objective.alpha,
+                                                   objective.db_interval, objective.eps)
+            elif kind is obj.SISDR:
+                out = head_fwd()
+                loss, _, dz, _ = ops.sisdr_mask_step(out, linear_inp, linear_tar, lens, self.hop, K, objective.eps)
+            else:
+                out = head_fwd()
+                loss, _, dz = ops.l1_mask_step(out, linear_tar, lens, self.hop, K, objective.eps)
+            ops.act_grad_(dz, out, K, head.activation)                  # dZ = d loss / d pre-activation; pad columns 0
+            gw, gb = ops.linear_head_bwd_fused(h, H, None, 0.0, out, dz, K, "Identity")
+            dh = ops.linear_head_tma(dz, K, wt, None, "Identity", None, 0.0)
+            for p, g in ((proj.weight, gw), (proj.bias, gb)):
+                if p.grad is None:
+                    p.grad = g
+                else:
+                    p.grad.add_(g)
+        if hidden.requires_grad:                                         # (a frozen body: nothing below the projection trains)
+            torch.autograd.backward(hidden, dh)
+        return loss
 
     def _fused_forward_backward(self, lengths, wavs, objective):
         """runner.py:431-460 in seven kernels, no autograd graph: K1 (noisy: power + log-power + CMVN sums), K1 (clean:
@@ -520,11 +649,13 @@ class EnhancementEngine:
         with any other optimizer (the guard is then the runner's host-side check, which cannot run under graph capture)."""
         from .optim import ClipAdam
         if isinstance(optimizer, ClipAdam):
-            # the update kernel also writes the padded / TF32 copy the head kernels read (one persistent buffer, see _padded_weight)
-            w = self.head.linear.weight
+            # the update kernel also writes the padded / TF32 copy the head kernels read (one persistent buffer, see _padded_weight);
+            # the recurrent step's transposed copy follows it
+            w = self._proj().weight
             buf = self._padded_weight()
             optimizer.clip_and_step(grad_clip, mirrors={w: buf}, mirror_tf32=self.precision == 1)
             self._wpad_key = (w.data_ptr(), w._version)
+            self._refresh_weight_t()
             return
         else:
             params = list(self.head.parameters())
@@ -575,8 +706,14 @@ class EnhancementEngine:
             torch.cuda.synchronize(dev)
             optimizer.zero_grad(set_to_none=True)
             graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(graph):
-                st["loss"] = self._train_body(st["lengths"], st["wavs"], objective, optimizer, grad_clip)
+            try:
+                with torch.cuda.graph(graph):
+                    st["loss"] = self._train_body(st["lengths"], st["wavs"], objective, optimizer, grad_clip)
+            except RuntimeError as exc:
+                if not _recurrent(self.head):
+                    raise
+                raise RuntimeError(f"EnhancementEngine.capture_train: the training step of the {type(self.head).__name__} head could "
+                                   f"not be captured into a CUDA graph (eager train_step still runs it): {exc}") from exc
             st["graph"] = graph
             self._graphs[key] = st
         return st
@@ -594,7 +731,8 @@ class EnhancementEngine:
     def _train_body(self, lengths, wavs, objective, optimizer, grad_clip):
         """forward + backward + update without ``zero_grad`` (inside a graph the gradients live in the graph's pool)."""
         if self.fused_training_supported(objective, wavs.shape[0], wavs.shape[2]):
-            loss = self._fused_forward_backward(lengths, wavs, objective)
+            fused = self._fused_recurrent_forward_backward if _recurrent(self.head) else self._fused_forward_backward
+            loss = fused(lengths, wavs, objective)
         else:
             loss = self._autograd_loss(lengths, wavs, objective)
             loss.backward()

@@ -342,6 +342,46 @@ def sisdr_mask_step(offset, linear_inp, linear_tar, lengths, hop, K, eps=1e-10, 
     return out[B], out[:B], grad, sums3
 
 
+def l1_mask_step(log_predicted, linear_tar, lengths, hop, K, eps=1e-10, want_grad=True):
+    """objective.L1's part of a training step on (B, F, LD) row-padded tensors (the counterpart of ``sisdr_mask_step``): the element
+    mean of |log_predicted - log(linear_tar + eps)| over the valid frames of this batch (what objective.L1 returns on each rank) and
+    d loss / d log_predicted = sign / count, in two launches with a fixed summation order (bitwise repeatable).  ``lengths``: SAMPLE
+    lengths with ``hop`` (frames = lengths // hop + 1) or frame counts with hop = 0.
+    Returns (loss (0-dim), loss_per_utt (B,), grad (B, F, LD of log_predicted; 0 on padded frames and pad columns) or None)."""
+    log_predicted, linear_tar = _chk(log_predicted, "log_predicted"), _chk(linear_tar, "linear_tar")
+    B, F, LDp = log_predicted.shape
+    assert linear_tar.shape[:2] == (B, F) and min(LDp, linear_tar.shape[2]) >= K
+    for t in (log_predicted, linear_tar):
+        assert t.stride(2) == 1 and t.stride(1) == t.shape[2] and t.stride(0) == F * t.shape[2], "rows must be packed (B, F, LD)"
+    lengths = _c(lengths, "lengths", torch.int64)
+    dev = log_predicted.device
+    lib = _lib.load()
+    with torch.cuda.device(dev):
+        n_ws = lib.se_l1_mask_step_workspace(B, F, int(K))
+        ws = torch.empty(n_ws, device=dev, dtype=torch.float64)
+        out = torch.empty(B + 1, device=dev)
+        grad = torch.empty_like(log_predicted) if want_grad else None
+        rc = lib.se_l1_mask_step(log_predicted.data_ptr(), LDp, linear_tar.data_ptr(), linear_tar.shape[2], lengths.data_ptr(), int(hop),
+                                 B, F, int(K), float(eps), ws.data_ptr(), n_ws, out.data_ptr(), out[B:].data_ptr(), _p(grad),
+                                 0 if grad is None else grad.shape[2], _stream())
+        _lib.check(rc, "se_l1_mask_step")
+    return out[B], out[:B], grad
+
+
+def act_grad_(grad, out, K, activation):
+    """grad <- grad * act'(out) in place on (B, F, LD) row-padded tensors (``out``: the head's output after the activation): d loss /
+    d output -> d loss / d pre-activation, columns >= K set to 0.  Identity: nothing to do, no launch.  Returns grad."""
+    if ACT[activation] == ACT["Identity"]:
+        return grad
+    grad, out = _chk(grad, "grad"), _chk(out, "out")
+    assert grad.shape[:2] == out.shape[:2] and grad.is_contiguous() and out.is_contiguous()
+    B, F, LDg = grad.shape
+    with torch.cuda.device(grad.device):
+        rc = _lib.load().se_act_grad_inplace(grad.data_ptr(), LDg, out.data_ptr(), out.shape[2], B * F, int(K), ACT[activation], _stream())
+        _lib.check(rc, "se_act_grad_inplace")
+    return grad
+
+
 def sisdr_mask_fwd(offset, linear_inp, linear_tar, stft_lengths, K, eps=1e-10, sums3=None):
     """objective.SISDR of predicted = offset * linear_inp on (B, F, LD) row-padded tensors (offset None: predicted =
     linear_inp).  Returns (loss_per_utt (B,), sums3 (B, 3) float64 for the backward)."""

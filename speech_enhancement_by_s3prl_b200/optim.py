@@ -13,7 +13,7 @@ import torch
 
 from . import _lib
 
-_MAX_TENSORS = 8
+_MAX_TENSORS = 32          # per parameter group (se_adam_clip_step_mirror): e.g. a bidirectional 3-layer LSTM head + projection, 26
 
 
 class ClipAdam(torch.optim.Optimizer):
