@@ -248,8 +248,19 @@ template <class Geo> struct Sz {
     static constexpr int E_MIN = EDGE / H + 1;                      // first emit window that reaches t >= 0
     static constexpr int NV = (EDGE + H - 1) / H;                   // virtual frames past the last one
     static constexpr int MROW = (K + 16 * (K >> 7) + 3) / 4 * 4;    // skewed mask row (bins 128 apart land 16 banks apart)
-    static constexpr int TAB_BYTES = (2 * M * 8 + 127) / 128 * 128; // s_win2 | s_bw2
+    static constexpr int WROW = V + 2;                              // float2 per lane row of a window table (below)
+    static constexpr int TAB_BYTES = (2 * G * WROW * 8 + 127) / 128 * 128;   // s_win2 | s_bw2
 };
+// Window tables (s_win2, s_bw2): value m = t + G r -- the one lane t of a group multiplies into its slot r -- sits in slot r of
+// row t, and a row is V float2 + 16 B.  A lane reads slots (r, r + 1) with one LDS.128 (V / 2 per table and frame instead of V
+// LDS.64); rows 4 (V + 2) words apart put the 16-byte chunks of 8 consecutive lanes on 8 disjoint 4-bank groups (V = 16: 4 t,
+// V = 20: 12 t mod 32), so the reads take the minimum number of wavefronts, as the LDS.64 did.
+template <class Geo> __device__ __forceinline__ int win_slot(int m) { return (m % Geo::G) * Sz<Geo>::WROW + m / Geo::G; }
+__device__ __forceinline__ float4 win_pair(const float2* __restrict__ row, int r) {          // slots r, r + 1 (r even)
+    return reinterpret_cast<const float4*>(row)[r >> 1];
+}
+__device__ __forceinline__ float2 lo2(float4 q) { return make_float2(q.x, q.y); }
+__device__ __forceinline__ float2 hi2(float4 q) { return make_float2(q.z, q.w); }
 // position of bin k in the staged mask row.  Geo1024: the two halves of a warp read bins 128 apart in the same instruction, so
 // every 128 bins are skewed by 16 floats (16 banks); Geo400: plain; Geo512: plain, each group reads 16 consecutive bins of its
 // own row, and the two rows of a warp sit 16 banks apart (K3Sz::GSTRIDE).
@@ -289,18 +300,24 @@ __device__ __forceinline__ void stage_mask_row(float* __restrict__ dst, const fl
         for (int k = jg; k < K; k += G) cp_async4(dst + mpos<Geo>(k), src + k);
     }
 }
-// v[r] = (x[2m], x[2m+1]) * win2[m], m = tidx + G r, from the ring (block 0 of the frame in ring slot `slot0`)
+// v[r] = (x[2m], x[2m+1]) * win2[m], m = tidx + G r, from the ring (block 0 of the frame in ring slot `slot0`); wrow = the lane's
+// row of s_win2
 template <class Geo>
-__device__ __forceinline__ void frame_from_ring(const float* __restrict__ ring, int slot0, int tidx, const float2* __restrict__ win2,
+__device__ __forceinline__ void frame_from_ring(const float* __restrict__ ring, int slot0, int tidx, const float2* __restrict__ wrow,
                                                 float2 (&v)[Geo::V]) {
     constexpr int Bs = Sz<Geo>::Bs, RB = Sz<Geo>::RB, G = Geo::G, VB = Geo::VB;
+    static_assert(VB % 2 == 0, "window slots are read in pairs within a block");
 #pragma unroll
     for (int b = 0; b < Geo::NB; ++b) {
         int slot = slot0 + b;
         slot = slot >= RB ? slot - RB : slot;
         const float2* p = reinterpret_cast<const float2*>(ring + slot * Bs) + tidx;
 #pragma unroll
-        for (int i = 0; i < VB; ++i) v[b * VB + i] = pmul(p[G * i], win2[tidx + G * (b * VB + i)]);
+        for (int i = 0; i < VB; i += 2) {
+            const float4 w = win_pair(wrow, b * VB + i);
+            v[b * VB + i] = pmul(p[G * i], lo2(w));
+            v[b * VB + i + 1] = pmul(p[G * (i + 1)], hi2(w));
+        }
     }
 }
 
@@ -408,7 +425,8 @@ __global__ void __launch_bounds__(K1Cfg<Geo>::WARPS * 32, K1Cfg<Geo>::MIN_BLOCKS
     }
     const bool second = a.n_real > 0 && u >= a.n_real;                              // pair mode, second channel: power only
     for (int i = threadIdx.x; i < M; i += THREADS)
-        s_win2[i] = make_float2(0.5f * a.tab.window[2 * i], 0.5f * a.tab.window[2 * i + 1]);
+        s_win2[win_slot<Geo>(i)] = make_float2(0.5f * a.tab.window[2 * i], 0.5f * a.tab.window[2 * i + 1]);
+    const float2* wrow = s_win2 + core.tidx * S::WROW;
     if (STATS && core.active && jg == 0) s_utt[gslot] = (active && len > 0 && !second) ? u : -1;
     float2 sacc[2 * NP + 1];
 #pragma unroll
@@ -424,7 +442,11 @@ __global__ void __launch_bounds__(K1Cfg<Geo>::WARPS * 32, K1Cfg<Geo>::MIN_BLOCKS
         const int f = fa + it;
         float2 v[V];
 #pragma unroll
-        for (int r = 0; r < V; ++r) v[r] = pmul(x[r], s_win2[core.tidx + G * r]);
+        for (int r = 0; r < V; r += 2) {
+            const float4 w = win_pair(wrow, r);
+            v[r] = pmul(x[r], lo2(w));
+            v[r + 1] = pmul(x[r + 1], hi2(w));
+        }
         if (it + 1 < len) load_frame<Geo>(x, row, a.T, (f + 1) * H - N / 2, core.tidx);   // lands behind this frame's transform
         core.fft(v);
         core.post_forward(v);
@@ -577,7 +599,7 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
     constexpr int N = S::N, M = S::M, H = S::H, G = S::G, V = S::V, NP = S::NP, Bs = S::Bs, RB = S::RB, HS = S::HS;
     constexpr int WARPS = K3Cfg<Geo>::WARPS, THREADS = WARPS * 32, GROUPS = Z::GROUPS;
     float2* s_win2 = reinterpret_cast<float2*>(smem);
-    float2* s_bw2 = s_win2 + M;
+    float2* s_bw2 = s_win2 + G * S::WROW;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int grp = Core<Geo>::group_of(lane), jg = Core<Geo>::lane_in_group(lane);
     unsigned char* region = smem + S::TAB_BYTES + (size_t)warp * Z::WARP_BYTES + (size_t)grp * Z::GSTRIDE;
@@ -611,14 +633,16 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
     }
     for (int i = threadIdx.x; i < M; i += THREADS) {
         const float w0 = a.tab.window[2 * i], w1 = a.tab.window[2 * i + 1];
-        s_win2[i] = make_float2(0.5f * w0, 0.5f * w1);
+        s_win2[win_slot<Geo>(i)] = make_float2(0.5f * w0, 0.5f * w1);
         float en0 = 0.0f, en1 = 0.0f;                                               // interior envelope: all frames that can cover the sample
         for (int n = (2 * i) % H; n < N; n += H) en0 += a.tab.window[n] * a.tab.window[n];
         for (int n = (2 * i + 1) % H; n < N; n += H) en1 += a.tab.window[n] * a.tab.window[n];
-        s_bw2[i] = make_float2(w0 / (2.0f * M * en0), -w1 / (2.0f * M * en1));     // sign: conjugation of the forward-as-inverse FFT
+        s_bw2[win_slot<Geo>(i)] = make_float2(w0 / (2.0f * M * en0), -w1 / (2.0f * M * en1));   // sign: conjugation of the forward-as-inverse FFT
     }
     Core<Geo> core;
     core.init(lane, region, a.tab);
+    const float2* wrow = s_win2 + core.tidx * S::WROW;                              // the lane's rows of the window tables
+    const float2* brow = s_bw2 + core.tidx * S::WROW;
     __syncthreads();
     griddep_launch();
     const int n_iter = __reduce_max_sync(kFull, my_iters);
@@ -688,12 +712,13 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
         for (int q = 0; q < NP; ++q) { ra[q] = 0.0f; rb[q] = 0.0f; }
         float2 v[V];
         bool mask_group_open = true;
-#pragma unroll 1
+        // unrolled: each pass is straight-line code with its own copy of the transform and no runtime dispatch (DESIGN.md 4.1)
+#pragma unroll
         for (int pass = 0; pass < 3; ++pass) {
             // a pass runs if ANY group of the warp needs it (shuffles are warp-wide); the others compute and discard
             if (!__any_sync(kFull, pass == 0 ? real : pass == 1 ? live : own)) continue;
-            if (pass == 0) frame_from_ring<Geo>(nring, slot0, tidx, s_win2, v);
-            else if (pass == 2) frame_from_ring<Geo>(cring, slot0, tidx, s_win2, v);
+            if (pass == 0) frame_from_ring<Geo>(nring, slot0, tidx, wrow, v);
+            else if (pass == 2) frame_from_ring<Geo>(cring, slot0, tidx, wrow, v);
             else if (!real) {                                                       // virtual frame (or idle): nothing to add
 #pragma unroll
                 for (int r = 0; r < V; ++r) v[r] = make_float2(0.0f, 0.0f);
@@ -729,13 +754,19 @@ __global__ void __launch_bounds__(K3Cfg<Geo>::WARPS * 32, K3Cfg<Geo>::MIN_BLOCKS
                 core.pre_inverse(v);
             } else if (pass == 1) {
                 // v[r] = conj(z[m]) unnormalised, m = tidx + G r; signs, 1/M and the interior 1/envelope are in s_bw2
-                float2 y[HS];
+                float2 y[HS], bw[V];
 #pragma unroll
-                for (int i = 0; i < HS; ++i) y[i] = pfma(s_bw2[tidx + G * i], v[i], carry[i]);
+                for (int r = 0; r < V; r += 2) {
+                    const float4 w = win_pair(brow, r);
+                    bw[r] = lo2(w);
+                    bw[r + 1] = hi2(w);
+                }
+#pragma unroll
+                for (int i = 0; i < HS; ++i) y[i] = pfma(bw[i], v[i], carry[i]);
 #pragma unroll
                 for (int i = 0; i < V - HS; ++i) {
-                    if (i < V - 2 * HS) carry[i] = pfma(s_bw2[tidx + G * (i + HS)], v[i + HS], carry[i + HS]);
-                    else carry[i] = pmul(s_bw2[tidx + G * (i + HS)], v[i + HS]);
+                    if (i < V - 2 * HS) carry[i] = pfma(bw[i + HS], v[i + HS], carry[i + HS]);
+                    else carry[i] = pmul(bw[i + HS], v[i + HS]);
                 }
                 if (emit) {
                     const int t0 = f * H - N / 2;

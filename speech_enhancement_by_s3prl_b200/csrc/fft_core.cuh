@@ -26,10 +26,15 @@ static inline float2 make_float2(float x, float y) { float2 r; r.x = x; r.y = y;
 namespace sefft {
 
 #if defined(__CUDA_ARCH__)
-// sm_100 packed fp32 arithmetic: one FADD2 / FMUL2 / FFMA2 works on a (re, im) register pair, and ptxas folds the
-// component shuffles below (broadcast, swap, per-half negation) into the operand selectors of those instructions
-// (R.F32, R.F32x2.LO_HI, .NP ...), so a complex add is ONE instruction and a complex multiply is TWO.  The rounding is
-// that of the scalar forms with the usual mul+add contraction.
+// sm_100 packed fp32 arithmetic: one FADD2 / FMUL2 / FFMA2 works on a (re, im) register pair, and ptxas folds some
+// component shuffles into the operand selectors of those instructions (R.F32 broadcast, R.F32x2.HI_LO swap, .NP), so a
+// complex add is ONE instruction.  Which shuffles fold depends on the operand: cmul is written as
+//   a * b = (a.x, a.y) * (b.x, b.x) + (a.y, a.x) * (-b.y, b.y)
+// (broadcast of b.x, swap of a, the sign pattern on the broadcast of b.y), which compiles to one FMUL2 + one FFMA2 also
+// when b is a conjugated twiddle.  The textbook form (a.x, a.x) * (b.x, b.y) + (a.y, a.y) * (-b.y, b.x) does not fold:
+// ptxas builds (-b.y, b.x) with a scalar FADD and a MOV per use (4 instructions per multiply; tools/sass_fastgeo.py).
+// The rounding is that of the scalar forms with the usual mul+add contraction (re = fma(-a.y, b.y, a.x b.x),
+// im = fma(a.x, b.y, a.y b.x)).
 typedef unsigned long long se_u64;
 __device__ __forceinline__ se_u64 pk2(float lo, float hi) { se_u64 r; asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi)); return r; }
 __device__ __forceinline__ float2 upk2(se_u64 v) { float2 r; asm("mov.b64 {%0, %1}, %2;" : "=f"(r.x), "=f"(r.y) : "l"(v)); return r; }
@@ -40,12 +45,12 @@ __device__ __forceinline__ se_u64 fma2(se_u64 a, se_u64 b, se_u64 c) { se_u64 r;
 __device__ __forceinline__ float2 cadd(float2 a, float2 b) { return upk2(add2(pk2(a.x, a.y), pk2(b.x, b.y))); }
 __device__ __forceinline__ float2 csub(float2 a, float2 b) { return upk2(sub2(pk2(a.x, a.y), pk2(b.x, b.y))); }
 __device__ __forceinline__ float2 cmul(float2 a, float2 b) {
-    return upk2(fma2(pk2(a.y, a.y), pk2(-b.y, b.x), mul2(pk2(a.x, a.x), pk2(b.x, b.y))));
+    return upk2(fma2(pk2(a.y, a.x), pk2(-b.y, b.y), mul2(pk2(a.x, a.y), pk2(b.x, b.x))));
 }
 __device__ __forceinline__ float2 cscale(float2 a, float s) { return upk2(mul2(pk2(a.x, a.y), pk2(s, s))); }
 // a * b + c (complex), and element-wise a * b / a * b + c on (x, y) pairs
 __device__ __forceinline__ float2 cmadd(float2 a, float2 b, float2 c) {
-    return upk2(fma2(pk2(a.y, a.y), pk2(-b.y, b.x), fma2(pk2(a.x, a.x), pk2(b.x, b.y), pk2(c.x, c.y))));
+    return upk2(fma2(pk2(a.y, a.x), pk2(-b.y, b.y), fma2(pk2(a.x, a.y), pk2(b.x, b.x), pk2(c.x, c.y))));
 }
 __device__ __forceinline__ float2 pmul(float2 a, float2 b) { return upk2(mul2(pk2(a.x, a.y), pk2(b.x, b.y))); }
 __device__ __forceinline__ float2 pfma(float2 a, float2 b, float2 c) { return upk2(fma2(pk2(a.x, a.y), pk2(b.x, b.y), pk2(c.x, c.y))); }
