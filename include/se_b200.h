@@ -88,6 +88,29 @@ int se_stft_strided(const float* wav, int64_t n_utt, int64_t utt_stride, int64_t
 int se_istft(const float* power, const float* phase, int64_t n_utt, int64_t n_frames, int n_fft, int hop,
              const float* window, float* wav_out, int64_t out_stride, int64_t pad_to, void* stream);
 
+/* ---- adjoint of the iSTFT (training through the waveform) -----------------------
+ * For y = iSTFT(Y) as se_istft computes it and a gradient waveform g = dL/dy (zero outside [0, hop*(n_frames-1))), the
+ * gradient of every frame's spectrum G = dL/dRe Y + i dL/dIm Y is, with w the centred window and env[p] = sum_f w[p - f hop]^2,
+ *   r_f[n] = w[n] g[f hop + n - n_fft/2] / env[f hop + n],
+ *   G_f[k] = (c_k / n_fft) sum_n r_f[n] e^{-2 pi i k n / n_fft},  c_0 = c_{n_fft/2} = 1, else 2;  Im G_f[0] = Im G_f[n_fft/2] = 0
+ * (the exact transpose of irfft + window + overlap-add + envelope division; one forward real FFT per frame).
+ * se_istft_bwd: the backward of se_istft in power and phase, Y = sqrt(P) e^{i phase}: grad_wav row u at grad_wav + u*grad_stride
+ *   (only its first hop*(n_frames-1) samples are read: the pad_to zero fill carries no gradient); power / phase / grad_power /
+ *   grad_phase dense (n_utt, n_frames, K):
+ *     grad_power = Re(G e^{-i phase}) / (2 sqrt(P)), 0 where P = 0;   grad_phase = sqrt(P) Im(G e^{-i phase}).
+ * se_mask_istft_bwd: the backward of se_mask_istft_ex in its mask, for a loss whose gradient in K3's output y (wav_out, rows
+ *   y_stride apart) is g[t] = coef[u].x y[t] + coef[u].y clean[t] for t < min(lengths[u], hop*(T/hop)) (0 elsewhere; coef (n_utt)
+ *   float pairs, e.g. from se_wave_sisdr_finish): the noisy spectrum X is recomputed from `noisy` with K3's framing, and
+ *     flags 0 (Y = sqrt(m) X):                             grad_mask = Re(G conj X) / (2 sqrt(m)), 0 where m <= 0;
+ *     SE_FLAG_MASK_IS_LOG_POWER (Y = e^{m/2} X / |X|):     grad_mask = Re(G conj Y) / 2.
+ *   mask and grad_mask are (n_utt, T/hop + 1, ld >= K) with rows ld floats apart; grad_mask's columns [K, ld) are written 0.
+ *   Every n_fft and hop of se_mask_istft_ex, on the generic tile kernel. */
+int se_istft_bwd(const float* grad_wav, int64_t grad_stride, const float* power, const float* phase, int64_t n_utt,
+                 int64_t n_frames, int n_fft, int hop, const float* window, float* grad_power, float* grad_phase, void* stream);
+int se_mask_istft_bwd(const float* noisy, const float* clean, int64_t utt_stride, const float* y, int64_t y_stride, const float* coef,
+                      const int64_t* lengths, const float* mask, int64_t ld, int64_t n_utt, int64_t T, int n_fft, int hop,
+                      const float* window, float* grad_mask, int flags, void* stream);
+
 /* ---- K3: fused mask multiply + iSTFT + overlap-add (+ metric sums) ---------------
  * wav_out = istft(linear_inp * mask, phase_inp) computed as iSTFT(sqrt(mask) * STFT(noisy))
  * without materialising the spectrum, `predicted` or the phase
@@ -292,6 +315,19 @@ int se_l1_eval_finish(const double* sums, const int64_t* lengths, int64_t n_utt,
  * n_utt x 3 doubles (overwritten: <s,t>, <t,t>, <s,s>). */
 int se_sisdr_wave(const float* src, int64_t src_stride, const float* tar, int64_t tar_stride, const int64_t* lengths,
                   int64_t n_utt, int64_t T, float eps, double* ws_sums3, float* sisdr, void* stream);
+/* ---- objective.WaveSISDR: the waveform SI-SDR as a training loss ------------------------------------------------
+ * se_wave_sisdr_finish: from s = sums + u * ld_sums = [<y,c>, <c,c>, <y,y>] (K3's SE_SUM_YC / CC / YY with ld_sums = SE_NSUMS,
+ *   or se_sisdr_wave's workspace with ld_sums = 3), in double with sisdr_eval's arithmetic (a = s0 / (s1 + eps)):
+ *     loss_per_utt[u] = -10 log10(a^2 s1 / (a^2 s1 - 2 a s0 + s2 + eps) + eps),  loss[0] = their mean over the n_utt utterances;
+ *     coef[u] = (alpha_u, beta_u), float pairs, such that d loss[0] / d y[t] = alpha_u y[t] + beta_u c[t] (the 1/n_utt included);
+ *     metric_acc[0..2] += [sum loss_per_utt, sum SI-SDR, n_utt].
+ *   Every output is optional.  A silent reference (s1 = 0) or a zero estimate gives finite values (coefficients 0).
+ * se_wave_sisdr_bwd: grad[u, t] = scale * grad_out[u] * (coef[u].x src[u, t] + coef[u].y tar[u, t]) for t < lengths[u] (clamped
+ *   to [0, T]; NULL = T), 0 for the rest of [0, T). */
+int se_wave_sisdr_finish(const double* sums, int64_t ld_sums, int64_t n_utt, float eps, float* loss_per_utt, float* loss, float* coef,
+                         double* metric_acc, void* stream);
+int se_wave_sisdr_bwd(const float* src, int64_t src_stride, const float* tar, int64_t tar_stride, const int64_t* lengths, int64_t n_utt,
+                      int64_t T, const float* coef, const float* grad_out, float scale, float* grad, int64_t grad_stride, void* stream);
 
 /* ---- STOI / ESTOI (pystoi 0.3.x: stoi(clean, processed, fs), extended=False / True) -----------------------
  * stoi[u], estoi[u] of ref[u, :len[u]] (the clean reference, pystoi's x) and est[u, :len[u]] (the processed

@@ -7,7 +7,7 @@ ABI of ``include/se_b200.h`` (``libse_b200.so``), plus the fused evaluation / tr
 """
 from .preprocessor import OnlinePreprocessor                      # noqa: F401
 from .model import Linear, LinearResidual, LSTM, Residual          # noqa: F401
-from .objective import SISDR, L1, WSD                              # noqa: F401
+from .objective import SISDR, L1, WSD, WaveSISDR                   # noqa: F401
 from .evaluation import sisdr_eval, sisdr_eval_batch, stoi_eval, estoi_eval, stoi_eval_batch  # noqa: F401
 from .utils import masked_mean, masked_normalize_decibel           # noqa: F401
 from .runner_ops import get_length_masks, decode_wav, pseudo_wav, stft_lengths  # noqa: F401

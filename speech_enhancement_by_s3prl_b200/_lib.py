@@ -28,6 +28,8 @@ _SIGNATURES = {
     "se_stft": [c_f, i64, i64, i64, c_int, c_int, c_f, c_float, c_f, c_f, c_f, c_f],
     "se_stft_strided": [c_f, i64, i64, i64, c_int, c_int, c_f, c_float, c_f, c_f, c_f, i64, c_f],
     "se_istft": [c_f, c_f, i64, i64, c_int, c_int, c_f, c_f, i64, i64, c_f],
+    "se_istft_bwd": [c_f, i64, c_f, c_f, i64, i64, c_int, c_int, c_f, c_f, c_f, c_f],
+    "se_mask_istft_bwd": [c_f, c_f, i64, c_f, i64, c_f, c_f, c_f, i64, i64, i64, c_int, c_int, c_f, c_f, c_int, c_f],
     "se_mask_istft": [c_f, c_f, i64, c_f, c_f, i64, i64, c_int, c_int, c_f, c_f, i64, i64, c_f, c_int, c_f],
     "se_mask_istft_strided": [c_f, c_f, i64, c_f, i64, c_f, i64, i64, c_int, c_int, c_f, c_f, i64, i64, c_f, c_int, c_f],
     "se_mask_istft_ex": [c_f, c_f, i64, c_f, i64, c_f, i64, i64, c_int, c_int, c_f, c_f, i64, i64, c_f, c_int, c_f],
@@ -82,6 +84,8 @@ _SIGNATURES = {
     "se_linear_head_bwd_wsd": [c_f, i64, c_f, i64, c_float, c_f, i64, c_f, i64, c_f, i64, c_f, i64, c_f, c_f, c_float, c_float, c_float, i64,
                                i64, i64, i64, c_int, c_f, i64, c_f, c_f, c_f],
     "se_sisdr_wave": [c_f, i64, c_f, i64, c_f, i64, i64, c_float, c_f, c_f, c_f],
+    "se_wave_sisdr_finish": [c_f, i64, i64, c_float, c_f, c_f, c_f, c_f, c_f],
+    "se_wave_sisdr_bwd": [c_f, i64, c_f, i64, c_f, i64, i64, c_f, c_f, c_float, c_f, i64, c_f],
     "se_stoi_workspace": [i64, i64, c_int],
     "se_stoi": [c_f, i64, c_f, i64, c_f, i64, i64, c_int, c_f, i64, c_f, c_f, c_f, c_f, c_f],
     "se_masked_normalize_db": [c_f, i64, c_f, i64, i64, c_f, c_f, i64, c_float, c_f, c_f, i64, c_f],

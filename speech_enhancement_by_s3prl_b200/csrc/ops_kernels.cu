@@ -779,6 +779,57 @@ __global__ void sisdr_wave_finish_kernel(const double* __restrict__ sums3, int n
     if (u < n_utt) out[u] = (float)sisdr_from_sums(sums3[3 * u], sums3[3 * u + 1], sums3[3 * u + 2], (double)eps);
 }
 
+// objective.WaveSISDR from [<y,c>, <c,c>, <y,y>] at sums + u * ld_sums (K3's SE_SUM_YC / CC / YY, or se_sisdr_wave's workspace):
+// loss_per_utt[u] = -sisdr_eval, loss[0] = their batch mean, coef[u] = (alpha, beta) with d loss[0] / d y = alpha y + beta c,
+// metric_acc += [sum loss, sum SI-SDR, n_utt].  One block: the mean is summed in a fixed order.
+__global__ void __launch_bounds__(256) wave_sisdr_finish_kernel(const double* __restrict__ sums, int ld_sums, int n_utt, float eps,
+                                                                float* __restrict__ loss_per_utt, float* __restrict__ loss,
+                                                                float2* __restrict__ coef, double* __restrict__ metric_acc) {
+    __shared__ double part[8];
+    double acc = 0.0;
+    for (int u = threadIdx.x; u < n_utt; u += blockDim.x) {
+        const double* s = sums + (long long)u * ld_sums;
+        const float l = (float)(-sisdr_from_sums(s[0], s[1], s[2], (double)eps));
+        if (loss_per_utt) loss_per_utt[u] = l;
+        if (coef) {
+            const float2 c = sisdr_coef(s, (double)eps, 1.0 / (double)n_utt);      // (coefficient of c, coefficient of y)
+            coef[u] = make_float2(c.y, c.x);
+        }
+        acc += (double)l;
+    }
+    acc = secommon::warp_sum(acc);
+    if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = acc;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double t = 0.0;
+        for (int w = 0; w < (int)(blockDim.x >> 5); ++w) t += part[w];
+        if (loss) *loss = (float)(t / (double)n_utt);
+        if (metric_acc) {
+            atomicAdd(metric_acc, t);
+            atomicAdd(metric_acc + 1, -t);
+            atomicAdd(metric_acc + 2, (double)n_utt);
+        }
+    }
+}
+
+// grad[u, t] = scale * grad_out[u] * (coef[u].x src[u, t] + coef[u].y tar[u, t]) for t < len[u], 0 for len[u] <= t < T
+__global__ void wave_sisdr_bwd_kernel(const float* __restrict__ src, long long src_stride, const float* __restrict__ tar,
+                                      long long tar_stride, const long long* __restrict__ lengths, int T, const float2* __restrict__ coef,
+                                      const float* __restrict__ grad_out, float scale, float* __restrict__ grad, long long grad_stride,
+                                      int chunks) {
+    const int u = blockIdx.x / chunks, chunk = blockIdx.x - u * chunks;
+    const int len = lengths ? (int)min((long long)T, max(0LL, lengths[u])) : T;
+    const int per = (T + chunks - 1) / chunks;
+    const int lo = chunk * per, hi = min(T, lo + per);
+    const float w = scale * grad_out[u];
+    const float2 c = coef[u];
+    const float a = w * c.x, b = w * c.y;
+    const float* s = src + (long long)u * src_stride;
+    const float* t = tar + (long long)u * tar_stride;
+    float* g = grad + (long long)u * grad_stride;
+    for (int i = lo + threadIdx.x; i < hi; i += blockDim.x) g[i] = i < len ? a * s[i] + b * t[i] : 0.0f;
+}
+
 // out = audio * sqrt(10^(target/10) / (mean(audio^2) + eps)); sums3[u] = (<a,r>, <r,r>, <a,a>) with r = ref.
 // The masked means divide by len + 1e-8 whatever eps is (utils.py:26 masked_mean's own default); eps enters only the
 // gain's denominator (utils.py:42).
@@ -1480,6 +1531,26 @@ int se_sisdr_wave(const float* src, int64_t src_stride, const float* tar, int64_
     if (rc != SE_OK) return rc;
     sisdr_wave_finish_kernel<<<(unsigned)((n_utt + 127) / 128), 128, 0, st>>>(ws_sums3, (int)n_utt, eps, sisdr);
     return secommon::check_launch("sisdr_wave_finish_kernel");
+}
+
+int se_wave_sisdr_finish(const double* sums, int64_t ld_sums, int64_t n_utt, float eps, float* loss_per_utt, float* loss, float* coef,
+                         double* metric_acc, void* stream) {
+    SE_REQUIRE(sums && n_utt > 0 && ld_sums >= 3, "bad argument");
+    SE_REQUIRE(!coef || (reinterpret_cast<uintptr_t>(coef) & 7) == 0, "coef must be 8-byte aligned");
+    wave_sisdr_finish_kernel<<<1, kThreads, 0, (cudaStream_t)stream>>>(sums, (int)ld_sums, (int)n_utt, eps, loss_per_utt, loss,
+                                                                      reinterpret_cast<float2*>(coef), metric_acc);
+    return secommon::check_launch("wave_sisdr_finish_kernel");
+}
+
+int se_wave_sisdr_bwd(const float* src, int64_t src_stride, const float* tar, int64_t tar_stride, const int64_t* lengths, int64_t n_utt,
+                      int64_t T, const float* coef, const float* grad_out, float scale, float* grad, int64_t grad_stride, void* stream) {
+    SE_REQUIRE(src && tar && coef && grad_out && grad && n_utt > 0 && T > 0 && T < (1LL << 31), "bad argument");
+    SE_REQUIRE((reinterpret_cast<uintptr_t>(coef) & 7) == 0, "coef must be 8-byte aligned");
+    const int chunks = pick_chunks(n_utt, T, 8192);
+    wave_sisdr_bwd_kernel<<<(unsigned)(n_utt * chunks), kThreads, 0, (cudaStream_t)stream>>>(
+        src, src_stride, tar, tar_stride, (const long long*)lengths, (int)T, reinterpret_cast<const float2*>(coef), grad_out, scale, grad,
+        grad_stride, chunks);
+    return secommon::check_launch("wave_sisdr_bwd_kernel");
 }
 
 int se_masked_normalize_db(const float* audio, int64_t stride, const int64_t* lengths, int64_t n_utt, int64_t width,

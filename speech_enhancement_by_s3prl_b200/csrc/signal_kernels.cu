@@ -50,6 +50,18 @@ template <int N> __global__ void __launch_bounds__(Cfg<N>::THREADS) mask_istft_k
     const int utt = blockIdx.x / tiles, tile = blockIdx.x - utt * tiles;
     mask_istft_tile<N>(ex, a, utt, tile, smem);
 }
+template <int N> __global__ void __launch_bounds__(Cfg<N>::THREADS) istft_bwd_kernel(IstftBwdArgs a, int tiles) {
+    extern __shared__ __align__(16) unsigned char smem[];
+    BlockExec ex;
+    const int utt = blockIdx.x / tiles, tile = blockIdx.x - utt * tiles;
+    istft_bwd_tile<N, false>(ex, a, utt, tile, smem);
+}
+template <int N> __global__ void __launch_bounds__(Cfg<N>::THREADS) mask_istft_bwd_kernel(IstftBwdArgs a, int tiles) {
+    extern __shared__ __align__(16) unsigned char smem[];
+    BlockExec ex;
+    const int utt = blockIdx.x / tiles, tile = blockIdx.x - utt * tiles;
+    istft_bwd_tile<N, true>(ex, a, utt, tile, smem);
+}
 
 // ------------------------------------------------------------------ per-device tables
 struct DeviceTables { float2* twM = nullptr; float2* twN = nullptr; };
@@ -61,6 +73,8 @@ template <int N> int opt_in_smem() {
     SE_CUDA_CHECK(cudaFuncSetAttribute(stft_kernel<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
     SE_CUDA_CHECK(cudaFuncSetAttribute(istft_kernel<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
     SE_CUDA_CHECK(cudaFuncSetAttribute(mask_istft_kernel<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+    SE_CUDA_CHECK(cudaFuncSetAttribute(istft_bwd_kernel<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
+    SE_CUDA_CHECK(cudaFuncSetAttribute(mask_istft_bwd_kernel<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxSmem));
     return SE_OK;
 }
 
@@ -127,6 +141,23 @@ template <int N> int launch_mask_istft(MaskIstftArgs a, cudaStream_t st) {
     if (blocks > 0x7fffffffLL) return fail(SE_ERR_BAD_ARG, "grid too large");
     mask_istft_kernel<N><<<(unsigned)blocks, Cfg<N>::THREADS, smem, st>>>(a, tiles);
     return secommon::check_launch("mask_istft_kernel");
+}
+
+// the adjoint of the iSTFT: istft_bwd_kernel (se_istft_bwd) or, with a.mask, mask_istft_bwd_kernel (se_mask_istft_bwd)
+template <int N> int launch_istft_bwd(IstftBwdArgs a, cudaStream_t st) {
+    const bool mask = a.mask != nullptr;
+    const int frames = istft_bwd_frames<N>(mask);
+    const int tiles = (a.n_frames + frames - 1) / frames;
+    const size_t smem = Smem<N>::bytes(istft_bwd_seg<N>(a.hop, mask), 0);
+    if (smem > kMaxSmem) return fail(SE_ERR_UNSUPPORTED, "hop=%d needs %zu B of shared memory", a.hop, smem);
+    const long long blocks = (long long)a.n_utt * tiles;
+    if (blocks > 0x7fffffffLL) return fail(SE_ERR_BAD_ARG, "grid too large");
+    if (mask) {
+        mask_istft_bwd_kernel<N><<<(unsigned)blocks, Cfg<N>::THREADS, smem, st>>>(a, tiles);
+        return secommon::check_launch("mask_istft_bwd_kernel");
+    }
+    istft_bwd_kernel<N><<<(unsigned)blocks, Cfg<N>::THREADS, smem, st>>>(a, tiles);
+    return secommon::check_launch("istft_bwd_kernel");
 }
 
 #define SE_DISPATCH_NFFT(n_fft, FN, ...)                 \
@@ -310,6 +341,46 @@ int se_istft(const float* power, const float* phase, int64_t n_utt, int64_t n_fr
     SE_REQUIRE(out_stride >= a.out_len && out_stride >= pad_to, "out_stride=%lld too small", (long long)out_stride);
     cudaStream_t st = (cudaStream_t)stream;
     SE_DISPATCH_NFFT(n_fft, launch_istft, a, st)
+}
+
+int se_istft_bwd(const float* grad_wav, int64_t grad_stride, const float* power, const float* phase, int64_t n_utt,
+                 int64_t n_frames, int n_fft, int hop, const float* window, float* grad_power, float* grad_phase, void* stream) {
+    SE_REQUIRE(grad_wav && power && phase && window && grad_power && grad_phase, "null pointer");
+    SE_REQUIRE(n_utt > 0 && n_frames > 1, "n_utt=%lld, n_frames=%lld", (long long)n_utt, (long long)n_frames);
+    SE_REQUIRE(hop > 0 && hop <= n_fft, "hop=%d must be in [1, n_fft=%d]", hop, n_fft);
+    SE_REQUIRE(n_frames < (1LL << 30) / hop, "n_frames=%lld too long", (long long)n_frames);
+    SE_REQUIRE(grad_stride >= hop * (n_frames - 1), "grad_stride=%lld smaller than hop * (n_frames - 1)", (long long)grad_stride);
+    DeviceTables t;
+    int rc = get_tables(n_fft, &t);
+    if (rc != SE_OK) return rc;
+    IstftBwdArgs a{};
+    a.n_utt = (int)n_utt; a.T = hop * ((int)n_frames - 1); a.hop = hop; a.n_frames = (int)n_frames; a.out_len = a.T;
+    a.tab.window = window; a.tab.twM = t.twM; a.tab.twN = t.twN;
+    a.grad_wav = grad_wav; a.grad_stride = grad_stride;
+    a.power = power; a.phase = phase; a.grad_power = grad_power; a.grad_phase = grad_phase;
+    SE_DISPATCH_NFFT(n_fft, launch_istft_bwd, a, (cudaStream_t)stream)
+}
+
+int se_mask_istft_bwd(const float* noisy, const float* clean, int64_t utt_stride, const float* y, int64_t y_stride, const float* coef,
+                      const int64_t* lengths, const float* mask, int64_t ld, int64_t n_utt, int64_t T, int n_fft, int hop,
+                      const float* window, float* grad_mask, int flags, void* stream) {
+    SE_REQUIRE(noisy && clean && y && coef && mask && window && grad_mask, "null pointer");
+    SE_REQUIRE(ld >= n_fft / 2 + 1, "ld=%lld smaller than K", (long long)ld);
+    SE_REQUIRE((flags & ~SE_FLAG_MASK_IS_LOG_POWER) == 0, "se_mask_istft_bwd: flags may hold SE_FLAG_MASK_IS_LOG_POWER only");
+    SE_REQUIRE((reinterpret_cast<uintptr_t>(coef) & 7) == 0, "coef must be 8-byte aligned");
+    int rc = check_geometry(n_utt, T, n_fft, hop);
+    if (rc != SE_OK) return rc;
+    const int n_frames = (int)(T / hop) + 1;
+    SE_REQUIRE(y_stride >= hop * (n_frames - 1), "y_stride=%lld smaller than hop * (T / hop)", (long long)y_stride);
+    DeviceTables t;
+    if ((rc = get_tables(n_fft, &t)) != SE_OK) return rc;
+    IstftBwdArgs a{};
+    a.n_utt = (int)n_utt; a.T = (int)T; a.hop = hop; a.n_frames = n_frames; a.out_len = hop * (n_frames - 1);
+    a.tab.window = window; a.tab.twM = t.twM; a.tab.twN = t.twN;
+    a.y = y; a.y_stride = y_stride; a.noisy = noisy; a.clean = clean; a.utt_stride = utt_stride;
+    a.coef = reinterpret_cast<const float2*>(coef); a.lengths = reinterpret_cast<const long long*>(lengths);
+    a.mask = mask; a.grad_mask = grad_mask; a.ld = ld; a.mask_is_power = (flags & SE_FLAG_MASK_IS_LOG_POWER) ? 2 : 0;
+    SE_DISPATCH_NFFT(n_fft, launch_istft_bwd, a, (cudaStream_t)stream)
 }
 
 int se_mask_istft(const float* noisy, const float* clean, int64_t utt_stride, const float* mask, const int64_t* lengths,

@@ -423,4 +423,128 @@ SE_HD void mask_istft_tile(Exec& ex, const MaskIstftArgs& a, int utt, int tile, 
     if (a.sums) ex.template block_accumulate<NSUMS>(acc, a.sums + (long long)utt * NSUMS);
 }
 
+// ------------------------------------------------------------------ adjoint of the iSTFT
+// Given dL/dy for y = iSTFT(Y) (trimmed by N/2, out_len = hop (F-1) samples), the gradient of frame f's spectrum is
+//   r_f[n] = w[n] g[f hop + n - N/2] / env[f hop + n],   env[p] = sum_f w[p - f hop]^2
+//   G_f[k] = (c_k / N) sum_n r_f[n] e^{-2 pi i k n / N},  c_0 = c_{N/2} = 1, else 2;  Im G_f[0] = Im G_f[N/2] = 0
+// with G = dL/dRe Y + i dL/dIm Y: the transpose of irfft (which drops Im of DC and Nyquist) + window + overlap-add + / env.
+// One forward real FFT per frame, as in stft_tile.
+struct IstftBwdArgs {
+    int n_utt, T, hop, n_frames, out_len;
+    Tables tab;
+    // the gradient waveform g[t], t < glen_u = min(len_u, out_len) (zero elsewhere):
+    const float* grad_wav;     // se_istft_bwd: g = grad_wav row u (grad_stride floats apart)
+    long long grad_stride;
+    const float* y;            // se_mask_istft_bwd: g = coef[u].x y[t] + coef[u].y clean[t], y = K3's output (y_stride apart)
+    long long y_stride;
+    const float* noisy;        // idem: the noisy and clean channels, rows utt_stride apart
+    const float* clean;
+    long long utt_stride;
+    const float2* coef;        // (n_utt)
+    const long long* lengths;  // (n_utt) or null (= T), clamped to [0, T]
+    // se_istft_bwd: Y = sqrt(P) e^{i phase}: dense (n_utt, n_frames, K)
+    const float* power;
+    const float* phase;
+    float* grad_power;
+    float* grad_phase;
+    // se_mask_istft_bwd: Y = sqrt(m) X (mask_is_power 0) or exp(m / 2) X / |X| (2, log target power); rows ld floats apart
+    const float* mask;
+    float* grad_mask;          // same layout as mask; columns [K, ld) are written 0
+    long long ld;
+    int mask_is_power;
+};
+
+// Frames per tile: G for se_istft_bwd; G / 2 for se_mask_istft_bwd, whose tile transforms 2 nf sequences (noisy frames, then r_f).
+template <int N> SE_HD int istft_bwd_frames(bool mask) { return mask ? Cfg<N>::G / 2 : Cfg<N>::G; }
+template <int N> SE_HD int istft_bwd_seg(int hop, bool mask) {
+    const int seg = (istft_bwd_frames<N>(mask) - 1) * hop + N;
+    return mask ? 2 * seg : seg;
+}
+
+// MASK: the se_mask_istft_bwd body (a.mask, a.y, ...), else se_istft_bwd's (a.grad_wav, a.power, ...)
+template <int N, bool MASK, class Exec>
+SE_HD void istft_bwd_tile(Exec& ex, const IstftBwdArgs& a, int utt, int tile, unsigned char* smem_raw) {
+    constexpr int M = N / 2, K = M + 1;
+    constexpr int PAD = Padded<M>::SIZE;
+    using P = Plan<M>;
+    constexpr bool mask = MASK;
+    const int GT = istft_bwd_frames<N>(mask);
+    const int hop = a.hop;
+    const int seg_len_max = (GT - 1) * hop + N;
+    Smem<N> s(smem_raw, istft_bwd_seg<N>(hop, mask));
+    const int f0 = tile * GT;
+    const int nf = imin(GT, a.n_frames - f0);
+    if (nf <= 0) return;
+    load_tables<N>(ex, a.tab, s);
+    const long long len_raw = a.lengths ? a.lengths[utt] : (long long)a.T;
+    const int len = (int)(len_raw < 0 ? 0 : (len_raw > a.T ? a.T : len_raw));
+    const int glen = imin(len, a.out_len);
+    const int t0 = f0 * hop - N / 2, n_seg = (nf - 1) * hop + N;
+    float* rseg = mask ? s.seg + seg_len_max : s.seg;
+    if (mask) load_segment(ex, a.noisy + (long long)utt * a.utt_stride, a.T, t0, n_seg, s.seg);
+    ex.sync();                                                       // the window is read below
+    {
+        const float* grow = mask ? nullptr : a.grad_wav + (long long)utt * a.grad_stride;
+        const float* yrow = mask ? a.y + (long long)utt * a.y_stride : nullptr;
+        const float* crow = mask ? a.clean + (long long)utt * a.utt_stride : nullptr;
+        const float2 cf = mask ? a.coef[utt] : make_float2(0.0f, 0.0f);
+        const float* win = s.win;
+        ex.foreach(n_seg, [&](int i) {
+            const int t = t0 + i;
+            float r = 0.0f;
+            if (t >= 0 && t < glen) {
+                const float g = mask ? cf.x * yrow[t] + cf.y * crow[t] : grow[t];
+                const int p = t + N / 2;                                // padded coordinate
+                const int fa = imax(0, floordiv(p - N, hop) + 1), fb = imin(a.n_frames - 1, floordiv(p, hop));
+                float env = 0.0f;
+                for (int f = fa; f <= fb; ++f) { const float w = win[p - f * hop]; env += w * w; }
+                r = g / env;
+            }
+            rseg[i] = r;
+        });
+    }
+    ex.sync();
+    const float* seg = s.seg;
+    const float* win = s.win;
+    auto load0 = [=](int g, int i) {
+        const float* fr = (g < nf) ? (mask ? seg : rseg) + g * hop : rseg + (g - nf) * hop;
+        return make_float2(fr[2 * i] * win[2 * i], fr[2 * i + 1] * win[2 * i + 1]);
+    };
+    const float2* Z = fft_run<P, -1>(ex, mask ? 2 * nf : nf, load0, s.bx, s.by, s.twM);
+    const int ncols = mask ? (int)a.ld : K;
+    ex.foreach(nf * ncols, [&](int w0) {
+        const int g = w0 / ncols;
+        const int k = w0 - g * ncols;
+        const long long o = ((long long)utt * a.n_frames + f0 + g) * ncols + k;
+        if (k >= K) { a.grad_mask[o] = 0.0f; return; }
+        const float2* zr = Z + (mask ? g + nf : g) * PAD;
+        float2 G = rfft_split(zr[phys(k == M ? 0 : k)], zr[phys(k == 0 ? 0 : M - k)], s.twN[k]);
+        const float ck = (k == 0 || k == M) ? 1.0f / N : 2.0f / N;
+        G = make_float2(G.x * ck, (k == 0 || k == M) ? 0.0f : G.y * ck);
+        if (!mask) {                                                    // Y = sqrt(P) e^{i phase}
+            const float pw = a.power[o];
+            float sn, cs;
+            sincosf(a.phase[o], &sn, &cs);
+            const float re = G.x * cs + G.y * sn, im = G.y * cs - G.x * sn;     // G e^{-i phase}
+            const float mag = sqrtf(pw);
+            a.grad_power[o] = pw > 0.0f ? re / (2.0f * mag) : 0.0f;
+            a.grad_phase[o] = mag * im;
+            return;
+        }
+        const float2* zx = Z + g * PAD;
+        float2 X = rfft_split(zx[phys(k == M ? 0 : k)], zx[phys(k == 0 ? 0 : M - k)], s.twN[k]);
+        if (k == 0 || k == M) X.y = 0.0f;
+        const float m = a.mask[o];
+        float gm;
+        if (a.mask_is_power == 2) {                                     // Y = e^{m/2} X / |X|, (e^{m/2}, 0) at X = 0
+            const float q = X.x * X.x + X.y * X.y;
+            const float2 Y = q > 0.0f ? cscale(X, sqrtf(expf(m)) / sqrtf(q)) : make_float2(sqrtf(expf(m)), 0.0f);
+            gm = 0.5f * (G.x * Y.x + G.y * Y.y);
+        } else {                                                        // Y = sqrt(m) X
+            gm = m > 0.0f ? (G.x * X.x + G.y * X.y) / (2.0f * sqrtf(m)) : 0.0f;
+        }
+        a.grad_mask[o] = gm;
+    });
+}
+
 }  // namespace sekern

@@ -27,7 +27,7 @@ def _c64(lengths):
 
 def _eval_loss(criterion, head=None):
     """The evaluation step's loss: "sisdr" for None / objective.SISDR (spectral SI-SDR), "wsd" for objective.WSD, "l1" for
-    objective.L1.  The pairs follow the reference's ``criterion(**locals(), **model_results)`` call (runner.py:575): WSD reads
+    objective.L1, "wave" for objective.WaveSISDR (any head: it reads the waveform).  The pairs follow the reference's ``criterion(**locals(), **model_results)`` call (runner.py:575): WSD reads
     ``offset`` (LinearResidual, Residual), L1 reads ``log_predicted`` (LSTM); any other pair raises, as the reference raises
     TypeError."""
     from . import model, objective as obj
@@ -38,9 +38,11 @@ def _eval_loss(criterion, head=None):
         return "wsd"
     if type(criterion) is obj.L1 and (head is None or type(head) is model.LSTM):
         return "l1"
+    if type(criterion) is obj.WaveSISDR:
+        return "wave"
     raise RuntimeError(f"EnhancementEngine: no evaluation route for the criterion {type(criterion).__name__}"
                        f"{' with a ' + kind + ' head' if kind else ''} (supported: None, objective.SISDR, objective.WSD with "
-                       "LinearResidual / Residual, objective.L1 with LSTM)")
+                       "LinearResidual / Residual, objective.L1 with LSTM, objective.WaveSISDR)")
 
 
 def _criterion_key(criterion):
@@ -50,6 +52,8 @@ def _criterion_key(criterion):
         return ("WSD", float(criterion.alpha), float(criterion.db_interval), float(criterion.eps))
     if loss == "l1":
         return ("L1", float(criterion.eps))
+    if loss == "wave":
+        return ("WaveSISDR",)
     return None
 
 
@@ -101,6 +105,8 @@ class EnhancementEngine:
         objective.L1 (model.LSTM heads only): loss_per_utt[u] is utterance u's own L1 and out["loss"] (1,) the batch's -- the
         element mean over every rank's valid frames (its [sum, count] pair is all-reduced), which is what the criterion returns;
         metric_acc[0] += B * loss.  Other geometries and steps under 6 frames take a slower route through the clean power spectrum.
+        objective.WaveSISDR (any head): loss_per_utt = -sisdr, the step's own waveform SI-SDR (sisdr_eval's eps, 1e-10), from the
+        same K3 sums; metric_acc[0] += their sum on the device.
         head: LinearResidual (fused K1 / K2), or a recurrent LSTM / Residual: the cuDNN body runs through torch between K1 and the
         library's projection; LSTM's output is log_predicted and K3 decodes exp(log_predicted) with the noisy phase.
         metric_acc: float64 (3,) device tensor += [sum loss, sum SI-SDR, utterances] (the running sums of an evaluation
@@ -112,7 +118,7 @@ class EnhancementEngine:
         sample rate (``ops.stoi``); stoi_acc: float64 (3,) device tensor += [sum STOI, sum ESTOI, utterances]."""
         head = self.head
         crit = _eval_loss(criterion, head) if want_spec_loss else (_eval_loss(criterion, head) and "sisdr")
-        wsd, l1 = crit == "wsd", crit == "l1"
+        wsd, l1, wave = crit == "wsd", crit == "l1", crit == "wave"
         want_spec_loss = want_spec_loss and crit == "sisdr"     # the spectral SI-SDR sums of K3
         log_power = type(head).__name__ == "LSTM"               # K3 decodes exp(log_predicted)
         B, C, T = wavs.shape
@@ -210,6 +216,12 @@ class EnhancementEngine:
                 if wsd:
                     self.launches_per_step += 8     # 2 STFTs, energies (+ fill), sums (+ fill), finish, the accumulator's sum + add
                     loss = self._wsd_terms_from_spectra(wavs, mask, lengths, criterion, metric_acc)
+                elif wave:
+                    loss = sisdr.neg()              # objective.WaveSISDR's terms are the step's own metric, bit for bit
+                    self.launches_per_step += 1
+                    if metric_acc is not None:
+                        metric_acc[:1].sub_(sisdr.sum(dtype=torch.float64))
+                        self.launches_per_step += 2
             out = {"loss_per_utt": loss, "sisdr": sisdr, "wav_predicted": wav, "gain": gain, "mask": mask[..., :K]}
             if batch_loss is not None:
                 out["loss"] = batch_loss
@@ -461,9 +473,10 @@ class EnhancementEngine:
         return (int(cfg.get("delta", 0)) + 1) * self.pre._n_mels
 
     def fused_training_supported(self, objective, B, T):
-        """True if train_step can take the fused route: LinearResidual with the SISDR or the WSD objective and the tensor-core
+        """True if train_step can take the fused route: LinearResidual with the SISDR, WSD or WaveSISDR objective and the tensor-core
         head, on the (log-)power spectrum or on a mel feature config (pseudo_noise.yaml:10-15), shapes inside the TMA head's / the
-        split-K backward's range.  Recurrent heads: model.LSTM with objective.L1 and model.Residual with objective.SISDR / WSD (with
+        split-K backward's range.  Recurrent heads: model.LSTM with objective.L1 / WaveSISDR and model.Residual with objective.SISDR / WSD /
+        WaveSISDR (with
         or without its CMVN), a hidden width (x directions) that is a multiple of 4, and both projections -- hidden -> K forward and
         K -> hidden for the input gradient -- on the TMA head (see _fused_recurrent_forward_backward).  Every other pair (e.g. LSTM
         with SISDR, or Linear) takes the autograd route."""
@@ -472,7 +485,7 @@ class EnhancementEngine:
             return False
         if _recurrent(self.head):
             return self._fused_recurrent_supported(objective, B, T)
-        if type(objective) not in (obj.SISDR, obj.WSD) or type(self.head) is not model.LinearResidual:
+        if type(objective) not in (obj.SISDR, obj.WSD, obj.WaveSISDR) or type(self.head) is not model.LinearResidual:
             return False
         F, K = T // self.hop + 1, self.n_fft // 2 + 1
         LD = ops.round4(K)
@@ -486,8 +499,8 @@ class EnhancementEngine:
     def _fused_recurrent_supported(self, objective, B, T):
         from . import model, objective as obj
         head = self.head
-        if not ((type(head) is model.LSTM and type(objective) is obj.L1) or
-                (type(head) is model.Residual and type(objective) in (obj.SISDR, obj.WSD))):
+        if not ((type(head) is model.LSTM and type(objective) in (obj.L1, obj.WaveSISDR)) or
+                (type(head) is model.Residual and type(objective) in (obj.SISDR, obj.WSD, obj.WaveSISDR))):
             return False
         F, K = T // self.hop + 1, self.n_fft // 2 + 1
         LD = ops.round4(K)
@@ -503,7 +516,8 @@ class EnhancementEngine:
         CMVN stay in torch autograd (DESIGN section 7); everything around them runs on the library's padded kernels.
           K1 (both channels) -> copy out of the padded rows -> body (+ CMVN), recorded for autograd
           -> projection forward on the TMA head (detached hidden states) -> the objective's step: loss and d loss / d output
-             (objective.WSD: its batch maximum all-reduced on the side stream under the projection)
+             (objective.WSD: its batch maximum all-reduced on the side stream under the projection; objective.WaveSISDR: K3 ->
+             se_wave_sisdr_finish -> se_mask_istft_bwd, LSTM's output decoded as a log target power)
           -> act'(output) in place: dZ, read by both GEMMs -> weight / bias gradient (split-K TMA kernel)
           -> dH = dZ W (TMA head on the persistent TF32 W^T copy) -> torch.autograd.backward(hidden, dH): cuDNN BPTT [+ CMVN's].
         Leaves the gradients in ``.grad`` and returns the loss (objective.L1: the element mean of this rank's batch)."""
@@ -514,8 +528,9 @@ class EnhancementEngine:
         K = self.n_fft // 2 + 1
         D = K if self.feat_cfg is None else self._mel_feature_dim()
         kind = type(objective)
+        wave = kind is obj.WaveSISDR
         with torch.no_grad():
-            feats, linear_inp, linear_tar = self._recurrent_k1(wavs, D, spectra=True)
+            feats, linear_inp, linear_tar = self._recurrent_k1(wavs, D, spectra=not wave)
             x = self._recurrent_input(feats, D, "train_step")
         with torch.enable_grad():
             hidden = self._recurrent_body(x)
@@ -534,6 +549,9 @@ class EnhancementEngine:
             elif kind is obj.SISDR:
                 out = head_fwd()
                 loss, _, dz, _ = ops.sisdr_mask_step(out, linear_inp, linear_tar, lens, self.hop, K, objective.eps)
+            elif wave:
+                out = head_fwd()
+                loss, dz = self._wave_sisdr_step(wavs, lens, out, objective, log_power=type(head).__name__ == "LSTM")
             else:
                 out = head_fwd()
                 loss, _, dz = ops.l1_mask_step(out, linear_tar, lens, self.hop, K, objective.eps)
@@ -558,6 +576,7 @@ class EnhancementEngine:
         its backward in the weight-gradient kernel.  Leaves the gradients in ``.grad`` and returns the loss."""
         from . import objective as obj
         wsd = type(objective) is obj.WSD
+        wave = type(objective) is obj.WaveSISDR
         B, C, T = wavs.shape
         dev = wavs.device
         head = self.head
@@ -573,7 +592,11 @@ class EnhancementEngine:
                 stat_sums = ws[:B * 2 * LD].view(B, LD, 2)
                 sums3 = ws[B * 2 * LD:].view(B, 3)
                 linear_tar = None
-                if self.log_features:        # one K1 launch for both channels where the register-resident kernel exists
+                if wave:                     # the loss reads the clean waveform: K1 on the noisy channel only
+                    linear_inp, logp, _ = ops.stft_features2(wavs, self.ch_inp, self.n_fft, self.hop, window,
+                                                             want_power=not self.log_features, want_logpower=self.log_features,
+                                                             log_eps=self.pre.eps, stat_sums=stat_sums)
+                elif self.log_features:      # one K1 launch for both channels where the register-resident kernel exists
                     linear_inp, logp, linear_tar, _ = ops.stft_features_pair(wavs, self.ch_inp, self.ch_tar, self.n_fft, self.hop, window,
                                                                              log_eps=self.pre.eps, stat_sums=stat_sums)
                 else:
@@ -588,7 +611,7 @@ class EnhancementEngine:
                                          order=int(cfg.get("delta", 0)), K=K)
                 D = feats.shape[2]
                 stat_sums = ops.feature_sums(feats, D) if head.cmvn else None
-            if self.feat_cfg is not None or linear_tar is None:
+            if not wave and (self.feat_cfg is not None or linear_tar is None):
                 linear_tar = ops.stft_padded(wavs, self.ch_tar, self.n_fft, self.hop, window, logpower=False)
             wpad = self._padded_weight()            # current: refreshed in place after every update (_clip_and_step)
             stats = stat_sums if head.cmvn else None
@@ -600,8 +623,14 @@ class EnhancementEngine:
                 offset = self._all_reduce_beside(dp.global_max, emax, head_fwd)
             else:
                 offset = head_fwd()
-            # frames = lengths // hop + 1, the batch-mean loss and d loss / d offset inside three launches
             lens = _c64(lengths)
+            if wave:
+                loss, grad_offset = self._wave_sisdr_step(wavs, lens, offset, objective)
+                gw, gb = ops.linear_head_bwd_fused(feats, D, stats, head.eps, offset, grad_offset, K, head.activation)
+                for p, g in ((head.linear.weight, gw), (head.linear.bias, gb)):
+                    p.grad = g if p.grad is None else p.grad.add_(g)
+                return loss
+            # frames = lengths // hop + 1, the batch-mean loss and d loss / d offset inside three launches
             fold = (ops.linear_head_bwd_wsd_supported if wsd else ops.linear_head_bwd_sisdr_supported)(
                 B, feats.shape[1], D, K, feats.shape[2], offset.shape[2], linear_inp.shape[2], linear_tar.shape[2])
             if wsd:
@@ -626,6 +655,18 @@ class EnhancementEngine:
                 else:
                     p.grad.add_(g)
         return loss
+
+    def _wave_sisdr_step(self, wavs, lengths, mask, objective, log_power=False):
+        """objective.WaveSISDR's step on a mask (B, F, round4(K)) of the head: K3 (the enhanced waveform y and its sums, no gain
+        pass) -> se_wave_sisdr_finish (the batch-mean loss and d loss / d y = alpha y + beta clean) -> se_mask_istft_bwd.
+        Returns (loss (1,), d loss / d mask (B, F, round4(K)), pad columns 0)."""
+        window, T = self.pre._frame_window, wavs.shape[2]
+        y, sums = ops.mask_istft(wavs, self.ch_inp, self.ch_tar, mask, lengths, self.n_fft, self.hop, window, pad_to=T,
+                                 want_sums=True, want_spec=False, mask_padded=True, mask_is_log_power=log_power)
+        _, loss, coef = ops.wave_sisdr_finish(sums, objective.eps)
+        grad = ops.mask_istft_bwd(wavs, self.ch_inp, self.ch_tar, y, coef, lengths, mask, self.n_fft, self.hop, window,
+                                  mask_is_log_power=log_power)
+        return loss, grad
 
     def _all_reduce_beside(self, all_reduce, buf, work):
         """all_reduce(buf) (dp.global_max / dp.reduce_sums) on the device's side stream while the current stream runs work();
@@ -678,8 +719,17 @@ class EnhancementEngine:
 
     def _autograd_loss(self, lengths, wavs, objective):
         """The reference's forward through the custom ops (preprocessor -> head -> objective), recorded for autograd."""
+        from . import objective as obj
         c = self.pre.get_feat_config
         feat_cfg = self.feat_cfg or c("linear", self.ch_inp, log=self.log_features)
+        if type(objective) is obj.WaveSISDR:
+            # wav_predicted = istft(predicted, phase_inp) zero-padded to T (runner.py:266-268, before the level normalisation,
+            # which the scale-invariant loss does not need), through the differentiable ops.istft
+            feats, linear_inp, phase_inp = self.pre(wavs, [feat_cfg, c("linear", self.ch_inp), c("phase", self.ch_inp)])
+            predicted, _ = self.head(features=feats, linears=linear_inp)
+            wav_predicted = ops.istft(predicted, phase_inp, self.n_fft, self.hop, self.pre._frame_window, pad_to=wavs.shape[2])
+            loss, _ = objective(wav_predicted=wav_predicted, wav_tar=wavs[:, self.ch_tar], lengths=lengths)
+            return loss
         feats, linear_inp, linear_tar = self.pre(wavs, [feat_cfg, c("linear", self.ch_inp), c("linear", self.ch_tar)])
         predicted, extra = self.head(features=feats, linears=linear_inp)
         frames = lengths // self.hop + 1

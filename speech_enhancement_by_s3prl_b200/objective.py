@@ -58,3 +58,18 @@ class WSD(nn.Module):
         loss = ops.wsd(linear_inp, offset, linear_tar, _frames(stft_length_masks, stft_lengths), self.alpha, self.db_interval,
                        self.eps)
         return loss, {}
+
+
+class WaveSISDR(nn.Module):
+    """Waveform SI-SDR as a training loss: the batch mean of -evaluation.sisdr_eval(wav_predicted[u, :len_u], wav_tar[u, :len_u])
+    (evaluation.py:5-10, eps = 1e-10 by default), the number the evaluation reports.  Differentiable in ``wav_predicted``;
+    with the differentiable ``ops.istft`` the gradient reaches the spectrum.  This is not the reference's lowercase asteroid
+    ``sisdr`` (objective.py:16-78): no zero-mean step and no asteroid eps; only sisdr_eval's arithmetic is implemented."""
+
+    def __init__(self, eps=1e-10, **kwargs):
+        super().__init__()
+        self.eps = eps
+
+    def forward(self, wav_predicted, wav_tar, lengths, **kwargs):
+        per_utt = ops.sisdr_wave(wav_predicted, wav_tar, lengths.to(wav_predicted.device, torch.int64), self.eps)
+        return -per_utt.mean(), {}

@@ -103,7 +103,7 @@ def stft_padded(wavs, channel, n_fft, hop, window, logpower=True, log_eps=1e-10)
 
 
 FLAG_WANT_SPEC, FLAG_SUMS_ZEROED, FLAG_MASK_IS_POWER, FLAG_WS_SELF_CLEAN, FLAG_MASK_IS_LOG_POWER = 1, 2, 4, 8, 16
-STATE_DOUBLES = {"sisdr": 0, "wsd": 1, "l1": 2}     # the criterion's state at the end of a step workspace
+STATE_DOUBLES = {"sisdr": 0, "wsd": 1, "l1": 2, "wave": 0}     # the criterion's state at the end of a step workspace
 
 
 def step_workspace_doubles(B, n_fft, criterion="sisdr"):
@@ -483,8 +483,8 @@ def linear_head_padded(x, D_in, weight_padded, bias, activation, mean, std, cmvn
     return out
 
 
-def istft(power, phase, n_fft, hop, window, pad_to=0):
-    """(B, F, K) power + phase -> (B, max(hop*(F-1), pad_to)); reference OnlinePreprocessor.istft."""
+@torch.library.custom_op("se_b200::istft", mutates_args=())
+def _istft(power: torch.Tensor, phase: torch.Tensor, n_fft: int, hop: int, window: torch.Tensor, pad_to: int) -> torch.Tensor:
     power, phase, window = _c(power, "linears"), _c(phase, "phases"), _c(window, "window")
     B, F, K = power.shape
     assert K == n_fft // 2 + 1 and phase.shape == power.shape
@@ -496,6 +496,54 @@ def istft(power, phase, n_fft, hop, window, pad_to=0):
                                   wav.data_ptr(), width, int(pad_to), _stream())
         _lib.check(rc, "se_istft")
     return wav
+
+
+@_istft.register_fake
+def _(power, phase, n_fft, hop, window, pad_to):
+    B, F, _ = power.shape
+    return power.new_empty(B, max(hop * (F - 1), int(pad_to)))
+
+
+@torch.library.custom_op("se_b200::istft_bwd", mutates_args=())
+def _istft_bwd(grad_wav: torch.Tensor, power: torch.Tensor, phase: torch.Tensor, n_fft: int, hop: int,
+               window: torch.Tensor) -> tuple[torch.Tensor, torch.Tensor]:
+    power, phase, window = _c(power, "linears"), _c(phase, "phases"), _c(window, "window")
+    grad_wav = _chk(grad_wav, "grad_wav")
+    if grad_wav.stride(1) != 1:
+        grad_wav = grad_wav.contiguous()
+    B, F, K = power.shape
+    with torch.cuda.device(power.device):
+        grad_power, grad_phase = torch.empty_like(power), torch.empty_like(phase)
+        rc = _lib.load().se_istft_bwd(grad_wav.data_ptr(), grad_wav.stride(0), power.data_ptr(), phase.data_ptr(), B, F, n_fft, hop,
+                                      window.data_ptr(), grad_power.data_ptr(), grad_phase.data_ptr(), _stream())
+        _lib.check(rc, "se_istft_bwd")
+    return grad_power, grad_phase
+
+
+@_istft_bwd.register_fake
+def _(grad_wav, power, phase, n_fft, hop, window):
+    return torch.empty_like(power, memory_format=torch.contiguous_format), torch.empty_like(phase, memory_format=torch.contiguous_format)
+
+
+def _istft_setup(ctx, inputs, output):
+    power, phase, n_fft, hop, window, pad_to = inputs
+    ctx.save_for_backward(power, phase, window)
+    ctx.cfg = (n_fft, hop)
+
+
+def _istft_backward(ctx, grad_wav):
+    power, phase, window = ctx.saved_tensors
+    grad_power, grad_phase = torch.ops.se_b200.istft_bwd(grad_wav, power, phase, *ctx.cfg, window)
+    return grad_power, grad_phase, None, None, None, None
+
+
+_istft.register_autograd(_istft_backward, setup_context=_istft_setup)
+
+
+def istft(power, phase, n_fft, hop, window, pad_to=0):
+    """(B, F, K) power + phase -> (B, max(hop*(F-1), pad_to)); reference OnlinePreprocessor.istft.  Differentiable in power and
+    phase (se_istft_bwd: the adjoint of the iSTFT); the zero fill up to pad_to carries no gradient."""
+    return torch.ops.se_b200.istft(power, phase, int(n_fft), int(hop), window, int(pad_to))
 
 
 def _mask_istft_call(entry, wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, out, want_sums, sums, sums_zeroed,
@@ -547,6 +595,49 @@ def mask_istft(wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, 
     flags |= FLAG_MASK_IS_LOG_POWER if mask_is_log_power else 0
     return _mask_istft_call("se_mask_istft_ex", wavs, ch_inp, ch_tar, mask, lengths, n_fft, hop, window, pad_to, out, want_sums,
                             sums, sums_zeroed, ws, flags)
+
+
+def mask_istft_bwd(wavs, ch_inp, ch_tar, y, coef, lengths, mask, n_fft, hop, window, mask_is_log_power=False):
+    """The backward of ``mask_istft`` in its mask for a loss whose gradient in K3's output y (B, >= hop * (T // hop)) is
+    coef[u, 0] y + coef[u, 1] clean on the first min(lengths[u], hop * (T // hop)) samples (se_mask_istft_bwd; coef (B, 2) float32,
+    e.g. from ``wave_sisdr_finish``).  mask (B, F, LD >= K) row-padded as the head writes it.  Returns grad_mask (B, F, LD),
+    columns [K, LD) zero: d L / d m for Y = sqrt(m) X, or with mask_is_log_power d L / d lp for Y = exp(lp / 2) X / |X|."""
+    wavs, y, mask, window = _chk(wavs, "wavs"), _chk(y, "y"), _chk(mask, "mask"), _c(window, "window")
+    coef, lengths = _c(coef, "coef"), _c(lengths, "lengths", torch.int64)
+    assert wavs.dim() == 3 and wavs.is_contiguous() and y.dim() == 2 and y.stride(1) == 1
+    B, C, T = wavs.shape
+    F, K = T // hop + 1, n_fft // 2 + 1
+    assert mask.dim() == 3 and mask.shape[:2] == (B, F) and mask.shape[2] >= K and mask.is_contiguous(), \
+        f"mask {tuple(mask.shape)} is not a contiguous ({B}, {F}, LD >= {K})"
+    assert coef.shape == (B, 2)
+    with torch.cuda.device(wavs.device):
+        grad = torch.empty_like(mask)
+        rc = _lib.load().se_mask_istft_bwd(wavs.data_ptr() + 4 * int(ch_inp) * T, wavs.data_ptr() + 4 * int(ch_tar) * T, C * T,
+                                           y.data_ptr(), y.stride(0), coef.data_ptr(), _p(lengths), mask.data_ptr(), mask.shape[2], B, T,
+                                           n_fft, hop, window.data_ptr(), grad.data_ptr(),
+                                           FLAG_MASK_IS_LOG_POWER if mask_is_log_power else 0, _stream())
+        _lib.check(rc, "se_mask_istft_bwd")
+    return grad
+
+
+def wave_sisdr_finish(sums, eps=1e-10, want_coef=True, metric_acc=None):
+    """objective.WaveSISDR from the sums [<y,c>, <c,c>, <y,y>] in the first three columns of ``sums`` (B, >= 3) float64 -- K3's
+    (B, 6) or se_sisdr_wave's (B, 3) -- in one launch (se_wave_sisdr_finish).  Returns (loss_per_utt (B,) = -sisdr_eval,
+    loss (1,) = their mean, coef (B, 2) | None): d loss / d y = coef[:, 0] y + coef[:, 1] c.  metric_acc (float64 (3,) or None)
+    += [sum loss, sum SI-SDR, B]."""
+    assert sums.dtype == torch.float64 and sums.dim() == 2 and sums.shape[1] >= 3 and sums.stride(1) == 1
+    if metric_acc is not None:
+        assert metric_acc.dtype == torch.float64 and metric_acc.numel() >= 3 and metric_acc.is_contiguous()
+    B = sums.shape[0]
+    dev = sums.device
+    with torch.cuda.device(dev):
+        loss_per_utt = torch.empty(B, device=dev)
+        loss = torch.empty(1, device=dev)
+        coef = torch.empty(B, 2, device=dev) if want_coef else None
+        rc = _lib.load().se_wave_sisdr_finish(sums.data_ptr(), sums.stride(0), B, float(eps), loss_per_utt.data_ptr(), loss.data_ptr(),
+                                              _p(coef), _p(metric_acc), _stream())
+        _lib.check(rc, "se_wave_sisdr_finish")
+    return loss_per_utt, loss, coef
 
 
 def mask_istft_wsd_supported(n_fft, hop):
@@ -689,8 +780,8 @@ def mix_batch(speech, speech_len, noise, noise_len, snr_db, target_level=-25.0, 
 
 
 # --------------------------------------------------------------------------- waveform-level helpers
-def sisdr_wave(src, tar, lengths=None, eps=1e-10):
-    """Batched evaluation.sisdr_eval: src, tar (B, T) -> (B,) dB."""
+@torch.library.custom_op("se_b200::sisdr_wave", mutates_args=())
+def _sisdr_wave(src: torch.Tensor, tar: torch.Tensor, lengths: torch.Tensor | None, eps: float) -> tuple[torch.Tensor, torch.Tensor]:
     src, tar = _chk(src, "src"), _chk(tar, "tar")
     assert src.dim() == 2 and src.shape == tar.shape and src.stride(1) == 1 and tar.stride(1) == 1
     B, T = src.shape
@@ -701,7 +792,53 @@ def sisdr_wave(src, tar, lengths=None, eps=1e-10):
         rc = _lib.load().se_sisdr_wave(src.data_ptr(), src.stride(0), tar.data_ptr(), tar.stride(0), _p(lengths), B, T,
                                        float(eps), ws.data_ptr(), out.data_ptr(), _stream())
         _lib.check(rc, "se_sisdr_wave")
-    return out
+    return out, ws
+
+
+@_sisdr_wave.register_fake
+def _(src, tar, lengths, eps):
+    B = src.shape[0]
+    return src.new_empty(B), src.new_empty(B, 3, dtype=torch.float64)
+
+
+@torch.library.custom_op("se_b200::sisdr_wave_bwd", mutates_args=())
+def _sisdr_wave_bwd(src: torch.Tensor, tar: torch.Tensor, lengths: torch.Tensor | None, eps: float, sums: torch.Tensor,
+                    grad_out: torch.Tensor) -> torch.Tensor:
+    B, T = src.shape
+    lengths = _c(lengths, "lengths", torch.int64)
+    _, _, coef = wave_sisdr_finish(sums, eps)                    # d mean_u(-sisdr_u) / d src = coef . (src, tar)
+    g = grad_out.reshape(B).to(torch.float32).contiguous()
+    with torch.cuda.device(src.device):
+        grad = torch.empty(B, T, device=src.device)
+        rc = _lib.load().se_wave_sisdr_bwd(src.data_ptr(), src.stride(0), tar.data_ptr(), tar.stride(0), _p(lengths), B, T,
+                                           coef.data_ptr(), g.data_ptr(), -float(B), grad.data_ptr(), T, _stream())
+        _lib.check(rc, "se_wave_sisdr_bwd")
+    return grad
+
+
+@_sisdr_wave_bwd.register_fake
+def _(src, tar, lengths, eps, sums, grad_out):
+    return src.new_empty(src.shape)
+
+
+def _sisdr_wave_setup(ctx, inputs, output):
+    src, tar, lengths, eps = inputs
+    ctx.save_for_backward(src, tar, lengths, output[1])
+    ctx.eps = eps
+
+
+def _sisdr_wave_backward(ctx, grad_out, grad_sums):
+    src, tar, lengths, sums = ctx.saved_tensors
+    return torch.ops.se_b200.sisdr_wave_bwd(src, tar, lengths, ctx.eps, sums, grad_out), None, None, None
+
+
+_sisdr_wave.register_autograd(_sisdr_wave_backward, setup_context=_sisdr_wave_setup)
+
+
+def sisdr_wave(src, tar, lengths=None, eps=1e-10):
+    """Batched evaluation.sisdr_eval: src, tar (B, T) -> (B,) dB.  Differentiable in src: the backward is se_wave_sisdr_finish's
+    coefficients and one se_wave_sisdr_bwd launch (samples from lengths[u] on get 0)."""
+    return torch.ops.se_b200.sisdr_wave(src, tar, lengths, float(eps))[0]
 
 
 def stoi(est, ref, lengths=None, fs=16000, want_stoi=True, want_estoi=True, acc=None, n_kept=None):
